@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """SAVSR forward hot-path benchmark (contract: see task brief / DESIGN.md section "Measurement").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload vid4_x4] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload vid4_x4] [--batch B] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 A "step" = super-resolving one synthetic Vid4-shaped clip (34 frames, 144x180 LR -> 576x720 HR at x4; every output frame is
@@ -84,6 +84,27 @@ def workload_config(name, world):
             "weights": "random init (seed 0)", "parallelism": f"frame-sharded x{world}, no data-path collective",
             # timing rule "flush L2 or use inputs larger than L2": the latter (GPU arm; the CPU arm carries the same text so the objects stay equal)
             "l2": "no explicit flush: the per-step working set (16-bit activation arenas, several GB per clip) exceeds the 126 MB L2"}
+
+
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def write_outputs(dirname, arrays):
+    """--dump-outputs: write each tensor as float32 `dirname/<name>.npy`, at most DUMP_BYTES in all, so that two builds run with the
+    same arguments can be compared output for output.  A tensor larger than its share of the budget is cut to a fixed sample of its
+    rows along dim 0 (torch.randperm with seed 0, kept in ascending order)."""
+    os.makedirs(dirname, exist_ok=True)
+    import numpy as np
+    share = DUMP_BYTES // len(arrays) - 4096                       # room for the .npy header
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if t.numel() * 4 > share:
+            keep = share // (t[0].numel() * 4)
+            if keep == 0:
+                raise ValueError(f"--dump-outputs: one row of {name} {tuple(t.shape)} is larger than its {share}-byte share")
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[rows.to(t.device)]
+        np.save(os.path.join(dirname, f"{name}.npy"), t.cpu().numpy())
 
 
 class ClockSampler(threading.Thread):
@@ -183,7 +204,7 @@ def load_reference(state_dict=None, device="cpu"):
 
 def cpu_reference_time(sd_cpu, frames, h, w, scale, threads=None):
     """Time the reference's CPU path on `frames` windows: the real reference when baseline/_ref is importable (kind
-    "reference"), else the oracle port.  Returns (HR Mpix/s, seconds, threads, kind)."""
+    "reference"), else the oracle port.  Returns (HR Mpix/s, seconds, threads, kind, output of the last window)."""
     threads = threads or os.cpu_count() or 1
     torch.set_num_threads(threads)
     H, W = hw_out(h, w, scale)
@@ -200,9 +221,9 @@ def cpu_reference_time(sd_cpu, frames, h, w, scale, threads=None):
         run(x[:, :, :, : min(h, 32), : min(w, 32)].contiguous())    # warm-up (thread pool, oneDNN primitives)
         t0 = time.perf_counter()
         for _ in range(frames):
-            run(x)
+            y = run(x)
         dt = time.perf_counter() - t0
-    return frames * H * W / dt / 1e6, dt, threads, kind
+    return frames * H * W / dt / 1e6, dt, threads, kind, y
 
 
 def run_reference(args, rank, world):
@@ -219,8 +240,10 @@ def run_reference(args, rank, world):
         cpu_reference_time(sd, 1, h, w, scale)
     t_total, n, kind, threads = 0.0, 0, "port", 1
     for _ in range(args.steps):
-        _, dt, threads, kind = cpu_reference_time(sd, per_step, h, w, scale)
+        _, dt, threads, kind, y = cpu_reference_time(sd, per_step, h, w, scale)
         t_total += dt; n += per_step
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"hr": y})
     val = n * H * W / t_total / 1e6
     what = ("the unmodified reference (baseline/_ref, lbasicsr/archs/savsr_arch.py) on CPU" if kind == "reference"
             else "oracle port of lbasicsr/archs/savsr_arch.py (pinned to the reference by tests/golden)")
@@ -450,6 +473,8 @@ def run_train(args, rank, world, local_rank):
     sampler = ClockSampler(local_rank); sampler.start()
     ms, loss = timed_steps(step, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, {"loss": torch.tensor([loss]), "params": torch.cat([p.detach().flatten() for p in net.parameters()])})
     # the same step as the reference's loop sees it (sr_model.py:101-128 + the logger reading l_pix): batches from pinned host memory
     # (already the case above) and the loss value read back by the host EVERY step, which serialises host and device
     ms_e2e, _ = timed_steps(lambda i: float(step(i)), args.steps)
@@ -519,7 +544,8 @@ def run_train(args, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of the headline, e2e, streamed, pipeline, other_scales and train_cfg5 "
+                    "measurements; cfg4_strong (2 steps), latency_b1 and gpu_reference (their own repetition counts) state theirs in the output")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="vid4_x4", choices=sorted(WORKLOADS) + ["train_cfg5"])
@@ -535,7 +561,15 @@ def main():
     ap.add_argument("--train-engine", default="native", choices=["native", "autograd"],
                     help="train_cfg5: native = savsr_b200.trainplan (static launch list, stage B); autograd = savsr_b200.train.Trainer (stage A)")
     ap.add_argument("--no-train-graph", action="store_true", help="train_cfg5: issue the step eagerly instead of replaying one CUDA graph per scale")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the timed path computed in its last step as "
+                    "DIR/<name>.npy (float32, at most 64 MB in all; rank 0's arrays): hr = the HR frames (a fixed sample of them when the clip "
+                    "is larger), or for train_cfg5 loss and params (a fixed sample of the updated parameters; its weight gradients are summed "
+                    "with fp32 atomics, so two runs agree to rounding amplified by Adam, about lr per step, not bit for bit).  For comparing two builds of "
+                    "one arm: --impl reference writes the output of its single timed window (input seed 1234), not frames of our arm's clip "
+                    "(seed 1234 + rank)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -660,6 +694,8 @@ def main():
     sampler = ClockSampler(local_rank); sampler.start()
     ms_total = timed(step_resident, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, {"hr": out_dev})
     for _ in range(2):
         step_e2e()
     ms_e2e = timed(step_e2e, args.steps)
@@ -852,7 +888,7 @@ def main():
     if rank == 0 and not args.no_cpu_baseline and world == 1:
         sd = {k: v.detach().cpu() for k, v in net.state_dict().items()}
         n_cpu = 3
-        val, dt, threads, kind = cpu_reference_time(sd, n_cpu, h, w, scale)
+        val, dt, threads, kind, _ = cpu_reference_time(sd, n_cpu, h, w, scale)
         line["cpu_baseline"] = {"value": round(val, 5), "unit": "HR Mpix/s", "cores": threads, "kind": kind,
                                 "sample": f"{n_cpu} output frames of the same clip shape ({h}x{w} -> {H}x{W}), fp32, {dt:.1f} s; "
                                           + ("the unmodified reference (baseline/_ref)" if kind == "reference" else "oracle port")}

@@ -88,31 +88,85 @@ def test_context_creation_fails_loudly_without_gpu():
     assert lib.savsr_ctx_sm_count(None) == 0
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/lbasicsr"), reason="reference tree only exists in the build container")
-def test_overlay_serves_the_new_arch_to_the_reference_registry():
+# A pristine checkout of the reference, reduced to what the overlay has to get past: lbasicsr/__init__.py imports the generated
+# version.py (absent before setup.py runs) and the archs; lbasicsr/archs/__init__.py imports every *_arch.py beside it by module name;
+# the registry asserts that a name is registered once.  The reference's own savsr_arch.py must never be the one that loads.
+REFERENCE_STAND_IN = {
+    "lbasicsr/__init__.py": "from .archs import *  # noqa: F401,F403\nfrom .version import __gitsha__, __version__  # noqa: F401\n",
+    "lbasicsr/utils/__init__.py": "",
+    "lbasicsr/utils/registry.py": (
+        "class Registry:\n"
+        "    def __init__(self, name):\n"
+        "        self._name, self._obj_map = name, {}\n"
+        "    def _do_register(self, name, obj):\n"
+        "        assert name not in self._obj_map, f\"An object named '{name}' was already registered in '{self._name}' registry!\"\n"
+        "        self._obj_map[name] = obj\n"
+        "    def register(self, obj=None):\n"
+        "        if obj is None:\n"
+        "            def deco(func_or_class):\n"
+        "                self._do_register(func_or_class.__name__, func_or_class)\n"
+        "                return func_or_class\n"
+        "            return deco\n"
+        "        self._do_register(obj.__name__, obj)\n"
+        "    def get(self, name):\n"
+        "        ret = self._obj_map.get(name)\n"
+        "        if ret is None:\n"
+        "            raise KeyError(f\"No object named '{name}' found in '{self._name}' registry!\")\n"
+        "        return ret\n"
+        "ARCH_REGISTRY = Registry('arch')\n"),
+    "lbasicsr/archs/__init__.py": (
+        "import importlib\n"
+        "from copy import deepcopy\n"
+        "from os import listdir, path as osp\n"
+        "from lbasicsr.utils.registry import ARCH_REGISTRY\n"
+        "__all__ = ['build_network']\n"
+        "arch_folder = osp.dirname(osp.abspath(__file__))\n"
+        "arch_filenames = sorted(osp.splitext(v)[0] for v in listdir(arch_folder) if v.endswith('_arch.py'))\n"
+        "_arch_modules = [importlib.import_module(f'lbasicsr.archs.{file_name}') for file_name in arch_filenames]\n"
+        "def build_network(opt):\n"
+        "    opt = deepcopy(opt)\n"
+        "    return ARCH_REGISTRY.get(opt.pop('type'))(**opt)\n"),
+    "lbasicsr/archs/savsr_arch.py": "raise ImportError('the reference savsr_arch.py was imported instead of the overlay')\n",
+    "lbasicsr/archs/edvr_arch.py": (
+        "from lbasicsr.utils.registry import ARCH_REGISTRY\n"
+        "@ARCH_REGISTRY.register()\n"
+        "class EDVR:\n"
+        "    pass\n"),
+}
+
+
+def test_overlay_serves_the_new_arch_to_the_reference_registry(tmp_path):
     import subprocess
     import sys
+    ref = tmp_path / "reference"
+    for rel, text in REFERENCE_STAND_IN.items():
+        (ref / rel).parent.mkdir(parents=True, exist_ok=True)
+        (ref / rel).write_text(text)
     code = ("import sys; sys.path.insert(0, %r)\n"
-            "from savsr_b200 import overlay; overlay.install('/root/reference')\n"
+            "from savsr_b200 import overlay; overlay.install(%r)\n"
             "import lbasicsr\n"
             "from lbasicsr.archs import build_network\n"
+            "from lbasicsr.utils.registry import ARCH_REGISTRY\n"
             "net = build_network(dict(type='SAVSR', num_in_ch=3, num_feat=64, num_frame=7, slid_win=3, fusion_win=5, interval=0,"
             " w1_num_block=4, w2_num_block=2, n_resgroups=4, n_resblocks=8, center_frame_idx=None))\n"
             "import savsr_b200.engine\n"
             "assert type(net).__module__ == 'lbasicsr.archs.savsr_arch' and hasattr(net, 'plan_for'), type(net)\n"
-            "print('OVERLAY_OK', len(net.state_dict()))\n") % ROOT
+            "assert ARCH_REGISTRY.get('EDVR').__module__ == 'lbasicsr.archs.edvr_arch'\n"
+            "print('OVERLAY_OK', len(net.state_dict()))\n") % (ROOT, str(ref))
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
     assert "OVERLAY_OK 791" in out.stdout, out.stdout[-2000:] + out.stderr[-2000:]
 
 
-def test_bench_reference_arm_contract():
-    """`bench.py --impl reference` (the CPU arm the driver runs beside ours) prints one JSON line with the contract's keys."""
+def test_bench_reference_arm_contract(tmp_path):
+    """`bench.py --impl reference` (the CPU arm the driver runs beside ours) prints one JSON line with the contract's keys, and
+    --dump-outputs writes the output of its last timed window."""
     import json
     import subprocess
     import sys
+    import numpy as np
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--workload", "cfg1_x2", "--steps", "1",
-                          "--warmup", "0"], capture_output=True, text=True, timeout=300, cwd=root)
+                          "--warmup", "0", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=300, cwd=root)
     assert out.returncode == 0, out.stderr[-2000:]
     line = json.loads(out.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["metric"] == "hr_mpix_per_s" and line["unit"] == "HR Mpix/s"
@@ -122,6 +176,30 @@ def test_bench_reference_arm_contract():
     assert line["config"]["workload"] == "cfg1_x2"
     import bench
     assert line["config"] == bench.workload_config("cfg1_x2", 1)      # both arms print the same config object
+    assert sorted(os.listdir(tmp_path)) == ["hr.npy"]
+    y = np.load(tmp_path / "hr.npy")
+    assert y.dtype == np.float32 and y.shape == (1, 3, 128, 128) and np.isfinite(y).all()
+
+
+def test_bench_dump_outputs(tmp_path):
+    """--dump-outputs: float32 .npy files within the 64 MB budget, a larger output cut to the same rows on every run, and a refusal
+    when a single row does not fit."""
+    import numpy as np
+    import bench
+    big = torch.arange(40 * 3 * 400 * 400, dtype=torch.float64).view(40, 3, 400, 400)      # 153.6 MB in float32
+    for d in ("a", "b"):
+        bench.write_outputs(str(tmp_path / d), {"hr": big, "loss": torch.tensor([0.5])})
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["hr.npy", "loss.npy"]
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) <= bench.DUMP_BYTES
+    hr = np.load(tmp_path / "a" / "hr.npy")
+    assert hr.dtype == np.float32 and hr.shape[1:] == (3, 400, 400) and 1 <= hr.shape[0] < 40
+    rows = hr[:, 0, 0, 0].astype(np.int64) // (3 * 400 * 400)
+    assert np.all(np.diff(rows) > 0) and np.array_equal(hr, big[torch.from_numpy(rows)].float().numpy())
+    assert np.array_equal(hr, np.load(tmp_path / "b" / "hr.npy"))
+    assert np.load(tmp_path / "a" / "loss.npy").tolist() == [0.5]
+    with pytest.raises(ValueError, match="larger than"):
+        bench.write_outputs(str(tmp_path / "c"), {"hr": torch.zeros(2, 3, 3000, 3000)})       # one row = 108 MB
 
 
 def test_bench_our_arm_needs_a_gpu():

@@ -159,8 +159,6 @@ def test_vid4_shape_against_oracle(G, scale, precision):
 def test_baseline_shapes_against_oracle(G, name, b, h, w, scale, precision):
     """BASELINE config 4 (UDM10 shape: 23 x 12 = 276 tiles per image, another chunking of the persistent loop) and config 1
     (64x64, x2) at full size, whole forward + stage taps vs the CPU oracle; the odd-size case exercises pad_spatial there."""
-    if b > 1 and precision == "fp16":
-        pytest.skip("one precision is enough for the ragged variant")
     torch.set_num_threads(os.cpu_count() or 1)
     info = G.check_forward(b=b, h=h, w=w, scale=scale, sd_seed=0, in_seed=1234, impl="halo", graph=True, tol=TOL[precision][0],
                            stage_tol=TOL[precision][1], precision=precision)
