@@ -278,7 +278,7 @@ int savsr_osa_prologue(savsr_ctx* ctx, const savsr_osa_params* convs, int nconvs
 /* Train-mode OSA-Conv prologue (savsr_arch.py:139-163 with ScaleAttention's BatchNorm on BATCH statistics, as nn.BatchNorm2d does
  * in train mode: biased variance normalises, running statistics move by `momentum` with the unbiased variance) and its backward.
  * convs[i] as for savsr_osa_prologue (bn_scale / bn_shift unused; scratch must be private to this convolution: it keeps the
- * forward's intermediate vectors for the backward); batch <= 8.  Besides convs[i].packed (forward operand, [n][s][9][64][64]) the
+ * forward's intermediate vectors for the backward); batch <= 32.  Besides convs[i].packed (forward operand, [n][s][9][64][64]) the
  * folded kernels are also written transposed + flipped (data-gradient operand) to extra[i].packed_t as [s][n][9][64][64]. */
 typedef struct savsr_osa_train {
   const float* bn_weight; const float* bn_bias;   /* [att]                                                        */

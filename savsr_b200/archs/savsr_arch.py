@@ -223,8 +223,8 @@ class SAVSR(nn.Module):
         if self.training:
             # optimisation path (sr_model.py:101-128 calls net_g(lq) in train mode).  Default: the native launch list of
             # savsr_b200/trainplan.py behind ONE autograd node (forward + backward of every trunk op on libsavsr_sm100; the caller's loss,
-            # optimizer, EMA and DistributedDataParallel work on the module's parameters as usual).  Fallback (odd sizes, batch > 8 per GPU,
-            # no_grad, native_training = False): savsr_b200/train.py, the ATen tape with the 3x3 convolutions on the tcgen05 kernels.
+            # optimizer, EMA and DistributedDataParallel work on the module's parameters as usual).  Fallback (odd sizes, more than
+            # trainplan.MAX_NATIVE_BATCH = 32 samples per GPU, no_grad, native_training = False): savsr_b200/train.py, the ATen tape with the 3x3 convolutions on the tcgen05 kernels.
             from savsr_b200 import trainplan as _tp
             if self.native_training and torch.is_grad_enabled() and self.precision == "bf16" and _tp.ModuleTraining.supports(x):
                 st = self.__dict__.get("_train_state")

@@ -54,7 +54,9 @@ namespace savsr {
 // Kernels that need more than 48 KB of dynamic shared memory: the attribute belongs to the device (primary context), so
 // it is tracked per savsr_ctx, not per process.
 enum AttrBit { kAttrIgemm = 0 /* + template index, 6 variants */, kAttrBigk = 8, kAttrKsta = 9, kAttrSatuHr = 10, kAttrOsaLinear = 11,
-               kAttrFused = 12, kAttrBigk128 = 13, kAttrSatuHrBf16 = 14, kAttrWgrad = 15, kAttrWgradBatched = 16 };
+               kAttrFused = 12, kAttrBigk128 = 13, kAttrSatuHrBf16 = 14, kAttrWgrad = 15, kAttrWgradBatched = 16,
+               kAttrOsaAssembleTrain = 17, kAttrOsaUnfoldBwd = 18, kAttrOsaChain = 19, kAttrOsaMatvec = 20 /* + 0, 1, 2: batch 8, 16, 32 */,
+               kAttrCaBackward = 23 };
 template <class F>
 inline int ensure_smem_attr(savsr_ctx* ctx, int bit, F func, size_t bytes) {
   if (ctx->attr_mask & (1u << bit)) return 0;

@@ -1,6 +1,6 @@
 // Train-mode attention paths of the native training step (row f1, stage B): the scale-attention prologue of OSA-Conv with
 // batch-statistics BatchNorm and its backward (savsr_arch.py:91-96, 123-128, 139-172), and the backward of the RCAB channel
-// attention (savsr_arch.py:514-524).  Small problems (a batch of B <= 8 vectors of <= 640 elements, weight banks of a few MB):
+// attention (savsr_arch.py:514-524).  Small problems (a batch of B <= 32 vectors of <= 640 elements, weight banks of a few MB):
 // latency-bound CUDA-core kernels whose job is to replace ~100 framework launches per convolution by 3-4.
 //
 // Forward:   savsr_osa_prologue's pooling and routing kernels (small_ops.cu), then osa_assemble_train_kernel: z = ReLU(BN_batch(fc v)),
@@ -15,7 +15,9 @@ namespace savsr {
 
 constexpr int kMaxOsaT = 4;
 static_assert(sizeof(savsr_osa_train) == 56 && sizeof(savsr_osa_grads) == 160, "C ABI struct layout changed: update savsr_b200/_capi.py");
-constexpr int kMaxBatchT = 8;      // samples per launch of the train-mode attention kernels
+// Samples per launch of the train-mode attention kernels.  Their per-sample arrays live in dynamic shared memory sized by the batch;
+// the chain kernel needs the most (178 KB at 32 samples and ci = 320) and would pass the 227 KB a block may use at 42.
+constexpr int kMaxBatchT = 32;
 __host__ __device__ inline int osat_scratch_stride(int ci) { return 5 * ci + 192; }
 __host__ __device__ inline int osat_off_h1(int ci) { return ci + 8; }
 __host__ __device__ inline int osat_off_v2(int ci) { return 3 * ci + 8; }
@@ -42,14 +44,15 @@ __global__ void __launch_bounds__(256) osa_assemble_train_kernel(const __grid_co
   pdl_trigger();
   const savsr_osa_params& c = L.c[blockIdx.y];
   const savsr_osa_train& tr = L.t[blockIdx.y];
-  __shared__ float zpre_s[kMaxBatchT][32];
-  __shared__ float z_s[kMaxBatchT][32];
-  __shared__ float att_s[kMaxBatchT][64 * SAVSR_MAX_SRC + 64 + 9 + 8];
+  extern __shared__ float sm[];                       // zpre [B][32] | z [B][32] | att [B][nout]
   if (blockIdx.x * blockDim.x >= c.co * c.ci) return;
   const int B = L.batch;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int stride = osat_scratch_stride(c.ci);
   const int nout = c.ci + c.co + 9 + 8;
+  float* zpre_s = sm;
+  float* z_s = sm + B * 32;
+  float* att_s = sm + 2 * B * 32;
   const bool saver = blockIdx.x == 0;
   for (int a = warp; a < c.att; a += 8) {
     float wr[10];
@@ -63,19 +66,19 @@ __global__ void __launch_bounds__(256) osa_assemble_train_kernel(const __grid_co
       for (int j = 0; j < 10; ++j) if (lane + 32 * j < c.ci) acc += wr[j] * v2[lane + 32 * j];
 #pragma unroll
       for (int off = 16; off >= 1; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
-      if (lane == 0) zpre_s[n][a] = acc;
+      if (lane == 0) zpre_s[n * 32 + a] = acc;
       s1 += acc;
     }
     const float mu = s1 / B;
     __syncwarp();
-    for (int n = 0; n < B; ++n) { const float d = zpre_s[n][a] - mu; s2 += d * d; }
+    for (int n = 0; n < B; ++n) { const float d = zpre_s[n * 32 + a] - mu; s2 += d * d; }
     const float var = s2 / B;                                  // biased variance normalises (F.batch_norm, training = True)
     const float rstd = rsqrtf(var + tr.eps);
     if (lane == 0) {
       const float gm = tr.bn_weight[a], bt = tr.bn_bias[a];
-      for (int n = 0; n < B; ++n) z_s[n][a] = fmaxf((zpre_s[n][a] - mu) * rstd * gm + bt, 0.f);
+      for (int n = 0; n < B; ++n) z_s[n * 32 + a] = fmaxf((zpre_s[n * 32 + a] - mu) * rstd * gm + bt, 0.f);
       if (saver) {
-        for (int n = 0; n < B; ++n) { tr.state[st_zpre(n) + a] = zpre_s[n][a]; tr.state[st_z(B, n) + a] = z_s[n][a]; }
+        for (int n = 0; n < B; ++n) { tr.state[st_zpre(n) + a] = zpre_s[n * 32 + a]; tr.state[st_z(B, n) + a] = z_s[n * 32 + a]; }
         tr.state[st_mu(B) + a] = mu;
         tr.state[st_rstd(B) + a] = rstd;
         if (tr.running_mean) {                                  // running statistics: momentum update with the UNBIASED variance
@@ -101,13 +104,13 @@ __global__ void __launch_bounds__(256) osa_assemble_train_kernel(const __grid_co
     for (int n = 0; n < B; ++n) {
       float acc = b;
 #pragma unroll
-      for (int a = 0; a < 32; ++a) if (a < c.att) acc += wv[a] * z_s[n][a];
-      att_s[n][j] = sig ? sigmoid_t(acc) : acc;
+      for (int a = 0; a < 32; ++a) if (a < c.att) acc += wv[a] * z_s[n * 32 + a];
+      att_s[n * nout + j] = sig ? sigmoid_t(acc) : acc;
     }
   }
   __syncthreads();
   if (threadIdx.x < B) {
-    float* ka = att_s[threadIdx.x] + c.ci + c.co + 9;
+    float* ka = att_s + threadIdx.x * nout + c.ci + c.co + 9;
     float mx = ka[0];
     for (int k = 1; k < 8; ++k) mx = fmaxf(mx, ka[k]);
     float e[8], sum = 0.f;
@@ -118,7 +121,7 @@ __global__ void __launch_bounds__(256) osa_assemble_train_kernel(const __grid_co
   if (saver) {
     for (int r = threadIdx.x; r < B * nout; r += blockDim.x) {
       const int n = r / nout, j = r - n * nout;
-      c.scratch[static_cast<long>(n) * stride + osat_off_att(c.ci) + j] = att_s[n][j];
+      c.scratch[static_cast<long>(n) * stride + osat_off_att(c.ci) + j] = att_s[r];
     }
   }
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
@@ -139,7 +142,7 @@ __global__ void __launch_bounds__(256) osa_assemble_train_kernel(const __grid_co
   const int row_t = quad_row(kk);                              // transposed operand: rows = input channels, K = output channels
   const int inner_t = row_t * 64 + ((((o >> 3) ^ (row_t & 7)) << 3) | (o & 7));
   for (int n = 0; n < B; ++n) {
-    const float* att = att_s[n];
+    const float* att = att_s + n * nout;
     const float ca = att[i], fa = att[c.ci + o];
     const float* sa = att + c.ci + c.co;
     const float* ka = sa + 9;
@@ -363,26 +366,29 @@ __global__ void __launch_bounds__(1024) osa_attn_chain_kernel(const __grid_const
 //   layer 1: dh1 = dv2 R2 ([ci][2ci]), through the ReLU of routing.0 (mask h1 > 0), written to dvec;
 //   layer 0: dvin = dh1 R0 ([2ci][ci+2]); columns 2.. are the pooled means -> dpool.
 // grid (ceil(cols/32), nconvs), 512 threads: warp w sums the rows w, w+16, ... for 32 columns (coalesced), shared-memory reduce.
+// NB: batch bucket (8, 16 or 32) >= B, the number of per-sample accumulators each thread keeps in registers.
+template <int NB>
 __global__ void __launch_bounds__(512) osa_attn_matvec_kernel(const __grid_constant__ OsaTrainLaunch L, int layer) {
   pdl_wait();
   pdl_trigger();
   const savsr_osa_params& c = L.c[blockIdx.y];
   const savsr_osa_grads& g = L.g[blockIdx.y];
-  __shared__ float red[16][kMaxBatchT][32];
-  __shared__ float in_s[kMaxBatchT * 64 * SAVSR_MAX_SRC * 2];  // [B][rows], rows <= 640
+  extern __shared__ float sm[];                       // red [16 warps][B][32] | in_s [B][rows], rows <= 640
   const int B = L.batch, ci = c.ci;
   const int nout = ci + c.co + 9 + 8;
   const int rows = layer == 1 ? ci : 2 * ci, cols = layer == 1 ? 2 * ci : ci + 2;
   if (blockIdx.x * 32 >= cols) return;
+  float* red = sm;
+  float* in_s = sm + 16 * B * 32;
   const float* W = layer == 1 ? c.r2_w : c.r0_w;
   const float* in = g.dvec + (layer == 1 ? dv_dv2(B, nout) : dv_dh1(B, nout, ci));
   for (int r = threadIdx.x; r < B * rows; r += blockDim.x) in_s[r] = in[r];
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int col = blockIdx.x * 32 + lane;
-  float acc[kMaxBatchT];
+  float acc[NB];
 #pragma unroll
-  for (int b = 0; b < kMaxBatchT; ++b) acc[b] = 0.f;
+  for (int b = 0; b < NB; ++b) acc[b] = 0.f;
   if (col < cols) {
     int r = warp;
     for (; r + 48 < rows; r += 64) {                          // four independent weight loads in flight per warp
@@ -392,23 +398,22 @@ __global__ void __launch_bounds__(512) osa_attn_matvec_kernel(const __grid_const
 #pragma unroll
       for (int q = 0; q < 4; ++q) {
 #pragma unroll
-        for (int b = 0; b < kMaxBatchT; ++b) if (b < B) acc[b] += in_s[b * rows + r + 16 * q] * w[q];
+        for (int b = 0; b < NB; ++b) if (b < B) acc[b] += in_s[b * rows + r + 16 * q] * w[q];
       }
     }
     for (; r < rows; r += 16) {
       const float w = __ldg(W + static_cast<long>(r) * cols + col);
 #pragma unroll
-      for (int b = 0; b < kMaxBatchT; ++b) if (b < B) acc[b] += in_s[b * rows + r] * w;
+      for (int b = 0; b < NB; ++b) if (b < B) acc[b] += in_s[b * rows + r] * w;
     }
   }
 #pragma unroll
-  for (int b = 0; b < kMaxBatchT; ++b) red[warp][b][lane] = acc[b];
+  for (int b = 0; b < NB; ++b) if (b < B) red[(warp * B + b) * 32 + lane] = acc[b];
   __syncthreads();
-  const int b = threadIdx.x >> 5;                              // the first warps finish: one sample each
-  if (b < B && col < cols) {
+  for (int b = threadIdx.x >> 5; b < B && col < cols; b += 16) {   // the warps finish one sample each (two at B > 16)
     float v = 0.f;
 #pragma unroll
-    for (int w = 0; w < 16; ++w) v += red[w][b][lane];
+    for (int w = 0; w < 16; ++w) v += red[(w * B + b) * 32 + lane];
     const int stride = osat_scratch_stride(ci);
     if (layer == 1) {
       g.dvec[dv_dh1(B, nout, ci) + b * 2 * ci + col] = c.scratch[static_cast<long>(b) * stride + osat_off_h1(ci) + col] > 0.f ? v : 0.f;
@@ -525,10 +530,14 @@ struct CaBwdParams {
 __global__ void __launch_bounds__(1024) ca_backward_kernel(const CaBwdParams p) {
   pdl_wait();
   pdl_trigger();
-  __shared__ float part[16][kMaxBatchT][64];
-  __shared__ float mean[kMaxBatchT][64], ds[kMaxBatchT][64], hid[kMaxBatchT][4], dhid[kMaxBatchT][4];
   const int tid = threadIdx.x;
   const int B = p.batch;
+  extern __shared__ float sm[];                       // part [16][B][64] | mean [B][64] | ds [B][64] | hid [B][4] | dhid [B][4]
+  float* part = sm;
+  float* mean = part + 16 * B * 64;
+  float* ds = mean + B * 64;
+  float* hid = ds + B * 64;
+  float* dhid = hid + B * 4;
   {
     const int c = tid & 63, q16 = tid >> 6;
     for (int n = 0; n < B; ++n) {
@@ -540,7 +549,7 @@ __global__ void __launch_bounds__(1024) ca_backward_kernel(const CaBwdParams p) 
         for (int j = 0; j < 4; ++j) a[j] += src[(q + 16 * j) * kC + c];
       }
       for (; q < p.npart; q += 16) a[0] += src[q * kC + c];
-      part[q16][n][c] = (a[0] + a[1]) + (a[2] + a[3]);
+      part[(q16 * B + n) * 64 + c] = (a[0] + a[1]) + (a[2] + a[3]);
     }
   }
   __syncthreads();
@@ -548,35 +557,35 @@ __global__ void __launch_bounds__(1024) ca_backward_kernel(const CaBwdParams p) 
     const int n = r >> 6, c = r & 63;
     float m = 0.f;
 #pragma unroll
-    for (int q = 0; q < 16; ++q) m += part[q][n][c];
-    mean[n][c] = m * p.inv_npix;
+    for (int q = 0; q < 16; ++q) m += part[(q * B + n) * 64 + c];
+    mean[r] = m * p.inv_npix;
     const float yy = p.y[r];
-    ds[n][c] = p.dy[r] * yy * (1.f - yy);
+    ds[r] = p.dy[r] * yy * (1.f - yy);
     p.dy[r] = 0.f;
   }
   __syncthreads();
   if (tid < B * 4) {
     const int n = tid >> 2, k = tid & 3;
     float a = p.b1[k], d = 0.f;
-    for (int c = 0; c < 64; ++c) { a += p.w1[k * 64 + c] * mean[n][c]; d += p.w2[c * 4 + k] * ds[n][c]; }
-    hid[n][k] = fmaxf(a, 0.f);
-    dhid[n][k] = a > 0.f ? d : 0.f;
+    for (int c = 0; c < 64; ++c) { a += p.w1[k * 64 + c] * mean[n * 64 + c]; d += p.w2[c * 4 + k] * ds[n * 64 + c]; }
+    hid[tid] = fmaxf(a, 0.f);
+    dhid[tid] = a > 0.f ? d : 0.f;
   }
   __syncthreads();
   if (tid < 256) {                                             // weight gradients: 256 threads = w2 [64][4] and w1 [4][64]
     const int c = tid >> 2, k = tid & 3;
     float a2 = 0.f, a1 = 0.f;
-    for (int n = 0; n < B; ++n) { a2 += ds[n][c] * hid[n][k]; a1 += dhid[n][k] * mean[n][c]; }
+    for (int n = 0; n < B; ++n) { a2 += ds[n * 64 + c] * hid[n * 4 + k]; a1 += dhid[n * 4 + k] * mean[n * 64 + c]; }
     p.dw2[c * 4 + k] += a2;
     p.dw1[k * 64 + c] += a1;
-    if (tid < 64) { float s = 0.f; for (int n = 0; n < B; ++n) s += ds[n][tid]; p.db2[tid] += s; }
-    if (tid < 4) { float s = 0.f; for (int n = 0; n < B; ++n) s += dhid[n][tid]; p.db1[tid] += s; }
+    if (tid < 64) { float s = 0.f; for (int n = 0; n < B; ++n) s += ds[n * 64 + tid]; p.db2[tid] += s; }
+    if (tid < 4) { float s = 0.f; for (int n = 0; n < B; ++n) s += dhid[n * 4 + tid]; p.db1[tid] += s; }
   }
   for (int r = tid; r < B * 64; r += blockDim.x) {
     const int n = r >> 6, c = r & 63;
     float a = 0.f;
 #pragma unroll
-    for (int k = 0; k < 4; ++k) a += p.w1[k * 64 + c] * dhid[n][k];
+    for (int k = 0; k < 4; ++k) a += p.w1[k * 64 + c] * dhid[n * 4 + k];
     p.dmean[r] = a;
   }
 }
@@ -588,6 +597,18 @@ using namespace savsr;
 // defined in small_ops.cu: the pooling + scale_routing launches shared with the inference prologue
 namespace savsr { int osa_prologue_front(savsr_ctx* ctx, const savsr_osa_params* convs, int nconvs, int batch, int npart, int npix, float inv_scale_h,
                                          float inv_scale_w, cudaStream_t st); }
+
+// Dynamic shared memory of each kernel (bytes) for `batch` samples and a largest input width of `ci` channels (nout = ci + 64 + 17);
+// the attribute of each kernel is raised once per context to its size at kMaxBatchT samples and ci = 64 * SAVSR_MAX_SRC.
+constexpr size_t smem_assemble(int batch, int ci) { return (2 * 32 + static_cast<size_t>(ci + 81)) * batch * sizeof(float); }
+constexpr size_t smem_unfold(int batch, int ci) { return (static_cast<size_t>(ci + 81) + 4 * 18) * batch * sizeof(float); }
+constexpr size_t smem_chain(int batch, int ci) { return (static_cast<size_t>(ci + 81) + 32 + 3 * static_cast<size_t>(ci) + 1) * batch * sizeof(float); }
+constexpr size_t smem_matvec(int batch, int ci) { return (16 * 32 + 2 * static_cast<size_t>(ci)) * batch * sizeof(float); }
+constexpr size_t smem_ca_backward(int batch) { return (16 * 64 + 2 * 64 + 2 * 4) * static_cast<size_t>(batch) * sizeof(float); }
+constexpr int kCiMaxT = 64 * SAVSR_MAX_SRC;
+static_assert(smem_assemble(kMaxBatchT, kCiMaxT) <= 227 * 1024 && smem_unfold(kMaxBatchT, kCiMaxT) <= 227 * 1024 &&
+              smem_chain(kMaxBatchT, kCiMaxT) <= 227 * 1024 && smem_matvec(kMaxBatchT, kCiMaxT) <= 227 * 1024 &&
+              smem_ca_backward(kMaxBatchT) <= 227 * 1024, "kMaxBatchT samples exceed the 227 KB of shared memory a block may use");
 
 static int fill_launch(const char* who, OsaTrainLaunch& L, savsr_ctx* ctx, const savsr_osa_params* convs, const savsr_osa_train* extra,
                        const savsr_osa_grads* grads, int nconvs, int batch) {
@@ -626,7 +647,11 @@ extern "C" int savsr_osa_prologue_train(savsr_ctx* ctx, const savsr_osa_params* 
   if (int rc = osa_prologue_front(ctx, convs, nconvs, batch, npart, npix, inv_scale_h, inv_scale_w, st)) return rc;
   int max_ci = 0;
   for (int i = 0; i < nconvs; ++i) max_ci = convs[i].ci > max_ci ? convs[i].ci : max_ci;
-  (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, osa_assemble_train_kernel, dim3((64 * max_ci + 255) / 256, nconvs), dim3(256), 0, st, L);
+  const size_t smem = smem_assemble(batch, max_ci);
+  if (smem > 48 * 1024) {
+    if (int rc = ensure_smem_attr(ctx, kAttrOsaAssembleTrain, osa_assemble_train_kernel, smem_assemble(kMaxBatchT, kCiMaxT))) return rc;
+  }
+  (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, osa_assemble_train_kernel, dim3((64 * max_ci + 255) / 256, nconvs), dim3(256), smem, st, L);
   SAVSR_CUDA(cudaGetLastError());
   return 0;
 }
@@ -643,15 +668,27 @@ extern "C" int savsr_osa_fold_backward(savsr_ctx* ctx, const savsr_osa_params* c
   cudaStream_t st = static_cast<cudaStream_t>(st_);
   int max_ci = 0;
   for (int i = 0; i < nconvs; ++i) max_ci = convs[i].ci > max_ci ? convs[i].ci : max_ci;
-  const int nout = max_ci + 64 + 17;
-  const size_t smem1 = (static_cast<size_t>(batch) * nout + 4 * static_cast<size_t>(batch) * 18) * sizeof(float);
-  SAVSR_REQUIRE(smem1 <= 48 * 1024, "savsr_osa_fold_backward: batch %d too large", batch);
+  const size_t smem1 = smem_unfold(batch, max_ci);
+  if (smem1 > 48 * 1024) {
+    if (int rc = ensure_smem_attr(ctx, kAttrOsaUnfoldBwd, osa_unfold_bwd_kernel, smem_unfold(kMaxBatchT, kCiMaxT))) return rc;
+  }
   (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, osa_unfold_bwd_kernel, dim3(max_ci / 2, nconvs), dim3(128), smem1, st, L);
-  const size_t smem2 = (static_cast<size_t>(batch) * nout + batch * 32 + 3 * static_cast<size_t>(batch) * max_ci + 16) * sizeof(float);
-  SAVSR_REQUIRE(smem2 <= 48 * 1024, "savsr_osa_fold_backward: batch %d too large for the chain kernel", batch);
+  const size_t smem2 = smem_chain(batch, max_ci);
+  if (smem2 > 48 * 1024) {
+    if (int rc = ensure_smem_attr(ctx, kAttrOsaChain, osa_attn_chain_kernel, smem_chain(kMaxBatchT, kCiMaxT))) return rc;
+  }
   (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, osa_attn_chain_kernel, dim3(nconvs), dim3(1024), smem2, st, L);
-  (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, osa_attn_matvec_kernel, dim3((2 * max_ci + 31) / 32, nconvs), dim3(512), 0, st, L, 1);
-  (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, osa_attn_matvec_kernel, dim3((max_ci + 2 + 31) / 32, nconvs), dim3(512), 0, st, L, 0);
+  // the smallest batch bucket that holds the batch: b <= 8 keeps eight accumulators per thread
+  void (*matvec)(const OsaTrainLaunch, int) = osa_attn_matvec_kernel<32>;
+  int matvec_bit = kAttrOsaMatvec + 2;
+  if (batch <= 8) { matvec = osa_attn_matvec_kernel<8>; matvec_bit = kAttrOsaMatvec; }
+  else if (batch <= 16) { matvec = osa_attn_matvec_kernel<16>; matvec_bit = kAttrOsaMatvec + 1; }
+  const size_t smem3 = smem_matvec(batch, max_ci);
+  if (smem3 > 48 * 1024) {
+    if (int rc = ensure_smem_attr(ctx, matvec_bit, matvec, smem_matvec(kMaxBatchT, kCiMaxT))) return rc;
+  }
+  (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, matvec, dim3((2 * max_ci + 31) / 32, nconvs), dim3(512), smem3, st, L, 1);
+  (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, matvec, dim3((max_ci + 2 + 31) / 32, nconvs), dim3(512), smem3, st, L, 0);
   (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, osa_attn_wgrad_kernel, dim3(2 * ctx->sm_count / nconvs + 1, nconvs), dim3(256), 0, st, L);
   SAVSR_CUDA(cudaGetLastError());
   return 0;
@@ -681,7 +718,11 @@ extern "C" int savsr_ca_backward(savsr_ctx* ctx, const float* pool, int npart, i
   CaBwdParams p;
   p.pool = pool; p.npart = npart; p.inv_npix = 1.f / static_cast<float>(npix);
   p.w1 = w1; p.b1 = b1; p.w2 = w2; p.b2 = b2; p.dy = dy; p.y = y; p.dw1 = dw1; p.db1 = db1; p.dw2 = dw2; p.db2 = db2; p.dmean = dmean; p.batch = batch;
-  (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, ca_backward_kernel, dim3(1), dim3(1024), 0, static_cast<cudaStream_t>(st), p);
+  const size_t smem = smem_ca_backward(batch);
+  if (smem > 48 * 1024) {
+    if (int rc = ensure_smem_attr(ctx, kAttrCaBackward, ca_backward_kernel, smem_ca_backward(kMaxBatchT))) return rc;
+  }
+  (void)launch_k(ctx->opt[SAVSR_OPT_PDL] != 0, ca_backward_kernel, dim3(1), dim3(1024), smem, static_cast<cudaStream_t>(st), p);
   SAVSR_CUDA(cudaGetLastError());
   return 0;
 }

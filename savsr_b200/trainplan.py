@@ -42,6 +42,7 @@ from . import train as T
 from .engine import context, get_hw, normalize_scale, pdl
 
 L_ACT = K.ACT_LRELU
+MAX_NATIVE_BATCH = 32      # samples per GPU the native attention kernels take (kMaxBatchT, csrc/train_attn.cu); above it they run as ATen islands
 CHUNK3 = 9 * 8192          # bytes of the nine [64][64] 16-bit blocks of one (64 x 64 channel) filter corner
 
 
@@ -318,7 +319,7 @@ class TrainPlan:
         device = flat.device
         self.own_loss = own_loss                            # False: the caller computes the loss from the returned output and passes its gradient back
         self.dsr: Optional[torch.Tensor] = None
-        self.native_attn = native_attn and batch <= 8      # False: the attention MLPs run as ATen islands (cross-check / larger batches)
+        self.native_attn = native_attn and batch <= MAX_NATIVE_BATCH      # False: the attention MLPs run as ATen islands (cross-check / larger batches)
         self.native_mask = native_mask                      # False: the OSAdapt mask net + combination run as an ATen island (cross-check)
         self._mask_scratch: Optional[dict] = None
         self.nbt_counts: Dict[str, int] = {}
@@ -1244,7 +1245,8 @@ class ModuleTraining:
 
     @staticmethod
     def supports(x: torch.Tensor) -> bool:
-        return x.is_cuda and x.dim() == 5 and x.shape[1] == 7 and x.shape[3] % 2 == 0 and x.shape[4] % 2 == 0 and x.shape[0] <= 8
+        return (x.is_cuda and x.dim() == 5 and x.shape[1] == 7 and x.shape[3] % 2 == 0 and x.shape[4] % 2 == 0
+                and x.shape[0] <= MAX_NATIVE_BATCH)
 
     def forward(self, x: torch.Tensor, scale) -> torch.Tensor:
         return _NativeNet.apply(x, self, self.plan_for(x, scale), *self.params)
