@@ -248,6 +248,11 @@ int savsr_conv_wgrad_batched(savsr_ctx* ctx, const void* tbase, int ntslots, int
  * 1 - beta^t).  grad_scale multiplies the gradient first (1 / world size after a summing all-reduce).  ema may be NULL. */
 int savsr_adam_ema(savsr_ctx* ctx, float* param, const float* grad, float* exp_avg, float* exp_avg_sq, float* ema, long n, float lr,
                    float beta1, float beta2, float eps, const float* step_dev, float ema_decay, float grad_scale, savsr_stream st);
+/* savsr_adam_ema with the learning rate read from device memory (lr_dev: one float, read when the kernel starts), so a captured CUDA
+ * graph follows a schedule that rewrites *lr_dev between replays.  Same arithmetic: bit-identical to savsr_adam_ema at the same lr. */
+int savsr_adam_ema_dev(savsr_ctx* ctx, float* param, const float* grad, float* exp_avg, float* exp_avg_sq, float* ema, long n,
+                       const float* lr_dev, float beta1, float beta2, float eps, const float* step_dev, float ema_decay, float grad_scale,
+                       savsr_stream st);
 
 /* ---- OSA-Conv prologue (savsr_arch.py:143-163, 91-96, 123-128) ---------------------------------- */
 typedef struct savsr_osa_params {

@@ -153,6 +153,7 @@ SIGNATURES = {
     "savsr_pack_conv_chunks": (_I, [_VP, _VP, _I, _I, _VP]),
     "savsr_conv_wgrad_batched": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _VP, _I, _I, _VP]),
     "savsr_adam_ema": (_I, [_VP, _VP, _VP, _VP, _VP, _VP, C.c_long, _F, _F, _F, _F, _VP, _F, _F, _VP]),
+    "savsr_adam_ema_dev": (_I, [_VP, _VP, _VP, _VP, _VP, _VP, C.c_long, _VP, _F, _F, _F, _VP, _F, _F, _VP]),
     "savsr_osa_train_state_floats": (_SZ, [_I]),
     "savsr_osa_train_dvec_floats": (_SZ, [_I, _I]),
     "savsr_osa_prologue_train": (_I, [_VP, C.POINTER(OsaParams), C.POINTER(OsaTrain), _I, _I, _I, _I, _F, _F, _VP]),

@@ -12,6 +12,7 @@
 //                             transposed + flipped (data gradient), in ONE launch per step
 //   savsr_conv_wgrad_batched  table-driven tcgen05 weight gradient: all (conv, source) pairs of a step in one persistent launch
 //   savsr_adam_ema            Adam + EMA over the flat parameter / gradient / moment buffers
+//   savsr_adam_ema_dev        the same with the learning rate read from device memory (a replayed graph follows a schedule)
 #include "common.cuh"
 
 namespace savsr {
@@ -438,11 +439,13 @@ typedef CUresult (*EncodeTiledFnT)(CUtensorMap*, CUtensorMapDataType, cuuint32_t
 
 // ------------------------------------------------------------------------------------------------ Adam + EMA
 __global__ void __launch_bounds__(256) adam_ema_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
-                                                       float* __restrict__ v, float* __restrict__ ema, long n, float lr, float b1,
-                                                       float b2, float eps, const float* __restrict__ step, float decay, float gscale) {
+                                                       float* __restrict__ v, float* __restrict__ ema, long n, float lr,
+                                                       const float* __restrict__ lr_dev, float b1, float b2, float eps,
+                                                       const float* __restrict__ step, float decay, float gscale) {
   const float t = *step;
+  const float lr_t = lr_dev ? *lr_dev : lr;          // device-resident lr: a replayed CUDA graph follows a schedule
   const float bc1 = 1.f - powf(b1, t), bc2s = sqrtf(1.f - powf(b2, t));
-  const float step_size = lr / bc1;
+  const float step_size = lr_t / bc1;
   for (long i = blockIdx.x * static_cast<long>(blockDim.x) + threadIdx.x; i < n; i += static_cast<long>(gridDim.x) * blockDim.x) {
     const float gi = g[i] * gscale;
     const float mi = b1 * m[i] + (1.f - b1) * gi;
@@ -585,16 +588,31 @@ extern "C" int savsr_conv_wgrad_batched(savsr_ctx* ctx, const void* tbase, int n
   return 0;
 }
 
-extern "C" int savsr_adam_ema(savsr_ctx* ctx, float* param, const float* grad, float* exp_avg, float* exp_avg_sq, float* ema, long n, float lr,
-                              float beta1, float beta2, float eps, const float* step_dev, float ema_decay, float grad_scale, savsr_stream st) {
-  SAVSR_REQUIRE(ctx && param && grad && exp_avg && exp_avg_sq && step_dev, "savsr_adam_ema: null pointer");
-  SAVSR_REQUIRE(n >= 0, "savsr_adam_ema: negative length");
+static int launch_adam_ema(const char* who, savsr_ctx* ctx, float* param, const float* grad, float* exp_avg, float* exp_avg_sq, float* ema, long n,
+                           float lr, const float* lr_dev, float beta1, float beta2, float eps, const float* step_dev, float ema_decay,
+                           float grad_scale, savsr_stream st) {
+  SAVSR_REQUIRE(ctx && param && grad && exp_avg && exp_avg_sq && step_dev, "%s: null pointer", who);
+  SAVSR_REQUIRE(n >= 0, "%s: negative length", who);
   if (n == 0) return 0;
   DeviceGuard guard(ctx->device);
   long blocks = (n + 255) / 256;
   if (blocks > 8L * ctx->sm_count) blocks = 8L * ctx->sm_count;
-  adam_ema_kernel<<<static_cast<unsigned>(blocks), 256, 0, static_cast<cudaStream_t>(st)>>>(param, grad, exp_avg, exp_avg_sq, ema, n, lr, beta1, beta2,
-                                                                                          eps, step_dev, ema_decay, grad_scale);
+  adam_ema_kernel<<<static_cast<unsigned>(blocks), 256, 0, static_cast<cudaStream_t>(st)>>>(param, grad, exp_avg, exp_avg_sq, ema, n, lr, lr_dev, beta1,
+                                                                                          beta2, eps, step_dev, ema_decay, grad_scale);
   SAVSR_CUDA(cudaGetLastError());
   return 0;
+}
+
+extern "C" int savsr_adam_ema(savsr_ctx* ctx, float* param, const float* grad, float* exp_avg, float* exp_avg_sq, float* ema, long n, float lr,
+                              float beta1, float beta2, float eps, const float* step_dev, float ema_decay, float grad_scale, savsr_stream st) {
+  return launch_adam_ema("savsr_adam_ema", ctx, param, grad, exp_avg, exp_avg_sq, ema, n, lr, nullptr, beta1, beta2, eps, step_dev, ema_decay,
+                         grad_scale, st);
+}
+
+extern "C" int savsr_adam_ema_dev(savsr_ctx* ctx, float* param, const float* grad, float* exp_avg, float* exp_avg_sq, float* ema, long n,
+                                  const float* lr_dev, float beta1, float beta2, float eps, const float* step_dev, float ema_decay, float grad_scale,
+                                  savsr_stream st) {
+  SAVSR_REQUIRE(lr_dev, "savsr_adam_ema_dev: null lr pointer");
+  return launch_adam_ema("savsr_adam_ema_dev", ctx, param, grad, exp_avg, exp_avg_sq, ema, n, 0.f, lr_dev, beta1, beta2, eps, step_dev, ema_decay,
+                         grad_scale, st);
 }

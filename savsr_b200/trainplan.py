@@ -103,6 +103,146 @@ class FlatParams:
         o, p = self.offsets[name], self.P[name]
         return self.ema[o:o + p.numel()].view(p.shape)
 
+    def view(self, buf: torch.Tensor, name: str) -> torch.Tensor:
+        """Parameter `name`'s slice of one of the flat buffers (p, g, m, v, ema), in the parameter's shape."""
+        o, p = self.offsets[name], self.P[name]
+        return buf[o:o + p.numel()].view(p.shape)
+
+
+class FlatAdam(torch.optim.Optimizer):
+    """Adam + EMA over the flat buffers of `FlatParams` (one savsr_adam_ema launch) as a torch.optim.Optimizer, so that the reference's
+    schedulers (torch.optim.lr_scheduler, BasicSR's warm-up / CosineAnnealingRestartLR) drive it and its state_dict is the one
+    torch.optim.Adam writes for the same parameters: one group, the module's trainable parameters in named_parameters() order
+    (the order of the reference's setup_optimizers), state[i] = {'step', 'exp_avg', 'exp_avg_sq'}.  The moments are views of the flat
+    buffers, so state_dict() copies nothing and load_state_dict() copies into them.
+
+    step(): eagerly, savsr_adam_ema with the group's lr; with use_graph, the captured savsr_adam_ema_dev reads the lr from a device
+    scalar that is rewritten (one small fill on the current stream) only when the group's lr changed since the last write.  No weight
+    decay, no AMSGrad, no maximize: load_state_dict refuses state that asks for them."""
+
+    def __init__(self, flat: FlatParams, ctx: K.Context, lr: float = 2e-4, betas=(0.9, 0.99), eps: float = 1e-8, ema_decay: float = 0.999,
+                 world_size: int = 1, use_graph: bool = False):
+        defaults = dict(torch.optim.Adam([torch.zeros(1)], lr=lr, betas=betas, eps=eps).defaults)      # torch's group keys, whatever its version
+        super().__init__(list(flat.P.values()), defaults)
+        self.flat, self.ctx = flat, ctx
+        self.names = list(flat.P)
+        self.ema_decay, self.world, self.use_graph = ema_decay, world_size, use_graph
+        self.lr_dev = torch.full((1,), float(lr), device=flat.device)     # what the captured launch reads
+        self._lr_written = float(lr)
+        self._graph: Optional[torch.cuda.CUDAGraph] = None
+        self._graph_key: Optional[tuple] = None                           # (betas, eps) baked into the captured launch
+
+    @property
+    def group(self) -> dict:
+        return self.param_groups[0]
+
+    def _hyper(self) -> tuple:
+        g = self.group
+        if g.get("weight_decay", 0) != 0 or g.get("amsgrad", False) or g.get("maximize", False):
+            raise ValueError("the flat Adam kernel implements neither weight decay nor AMSGrad nor maximize")
+        return float(g["betas"][0]), float(g["betas"][1]), float(g["eps"])
+
+    def _launch(self, lr_dev: bool) -> None:
+        f = self.flat
+        b1, b2, eps = self._hyper()
+        st = torch.cuda.current_stream(f.device).cuda_stream
+        ema = f.ema.data_ptr() if f.ema is not None else None
+        f.step_t.add_(1.0)
+        if lr_dev:
+            K.check(self.ctx.lib.savsr_adam_ema_dev(self.ctx.handle, f.p.data_ptr(), f.g.data_ptr(), f.m.data_ptr(), f.v.data_ptr(), ema, f.n,
+                                                    self.lr_dev.data_ptr(), b1, b2, eps, f.step_t.data_ptr(), self.ema_decay, 1.0 / self.world, st))
+        else:
+            K.check(self.ctx.lib.savsr_adam_ema(self.ctx.handle, f.p.data_ptr(), f.g.data_ptr(), f.m.data_ptr(), f.v.data_ptr(), ema, f.n,
+                                                float(self.group["lr"]), b1, b2, eps, f.step_t.data_ptr(), self.ema_decay, 1.0 / self.world, st))
+
+    @torch.no_grad()
+    def step(self, closure=None):
+        """One Adam + EMA update from the flat gradient buffer (the caller has filled it: NativeTrainer.step does)."""
+        loss = None
+        if closure is not None:
+            with torch.enable_grad():
+                loss = closure()
+        if not self.use_graph:
+            self._launch(lr_dev=False)
+            return loss
+        dev = self.flat.device
+        if self._graph is None or self._graph_key != self._hyper():
+            og = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(og, stream=torch.cuda.Stream(dev)):
+                self._launch(lr_dev=True)
+            self._graph, self._graph_key = og, self._hyper()           # (capture does not execute: nothing to roll back)
+        lr = float(self.group["lr"])
+        if lr != self._lr_written:
+            self.lr_dev.fill_(lr)
+            self._lr_written = lr
+        self._graph.replay()
+        return loss
+
+    def zero_grad(self, set_to_none: bool = True) -> None:
+        """The gradients are views of the flat gradient buffer and stay so: zero it (set_to_none is ignored)."""
+        self.flat.g.zero_()
+
+    # ---- checkpoints: the layout of torch.optim.Adam.state_dict()
+    def state_dict(self) -> dict:
+        f = self.flat
+        step = float(f.step_t.item())
+        self.state.clear()
+        if step > 0:
+            for n, p in f.P.items():
+                self.state[p] = {"step": torch.tensor(step, dtype=torch.float32), "exp_avg": f.view(f.m, n), "exp_avg_sq": f.view(f.v, n)}
+        try:
+            return super().state_dict()
+        finally:
+            self.state.clear()
+
+    def load_state_dict(self, state_dict: dict) -> None:
+        """Take over a state written by FlatAdam or torch.optim.Adam for the same parameters: moments, step, the group's lr / initial_lr /
+        betas / eps.  Raises ValueError on what the kernel cannot continue (several groups, other parameters, per-parameter step
+        counts, weight decay, AMSGrad, maximize)."""
+        groups = state_dict.get("param_groups", [])
+        if len(groups) != 1:
+            raise ValueError(f"FlatAdam holds one parameter group; the state has {len(groups)}")
+        saved = groups[0]
+        if saved.get("weight_decay", 0) != 0:
+            raise ValueError(f"weight_decay={saved['weight_decay']} is not implemented by the flat Adam kernel (it needs 0)")
+        for key in ("amsgrad", "maximize"):
+            if saved.get(key, False):
+                raise ValueError(f"{key}=True is not implemented by the flat Adam kernel")
+        f = self.flat
+        ids = list(saved["params"])
+        if len(ids) != len(self.names):
+            raise ValueError(f"the state holds {len(ids)} parameters, this optimizer {len(self.names)}")
+        st = state_dict.get("state", {})
+        steps = set()
+        for pid, n in zip(ids, self.names):
+            s = st.get(pid)
+            if s is None:
+                steps.add(0.0)
+                continue
+            steps.add(float(s["step"]))
+            for key in ("exp_avg", "exp_avg_sq"):
+                if tuple(s[key].shape) != tuple(f.P[n].shape):
+                    raise ValueError(f"parameter {pid} ({n}): {key} has shape {tuple(s[key].shape)}, the parameter {tuple(f.P[n].shape)}")
+        if len(steps) > 1:
+            raise ValueError(f"the parameters have different step counts {sorted(steps)}; the flat kernel keeps one")
+        with torch.no_grad():
+            for pid, n in zip(ids, self.names):
+                s = st.get(pid)
+                for buf, key in ((f.m, "exp_avg"), (f.v, "exp_avg_sq")):
+                    if s is None:
+                        f.view(buf, n).zero_()
+                    else:
+                        f.view(buf, n).copy_(s[key])
+            f.step_t.fill_(steps.pop() if steps else 0.0)
+        group = {k: v for k, v in saved.items() if k != "params"}      # as torch's load_state_dict: the saved group with our parameters
+        for k, v in self.defaults.items():
+            group.setdefault(k, v)
+        group["params"] = self.group["params"]
+        self.param_groups[0] = group
+        self.state.clear()
+        if self._graph is not None and self._graph_key != self._hyper():
+            self._graph = None                                          # betas / eps are baked into the captured launch
+
 
 # ====================================================================================================== packed weights
 class TrainWeights:
@@ -1119,7 +1259,9 @@ class TrainPlan:
 class NativeTrainer:
     """The optimisation step of lbasicsr/models/sr_model.py:101-128 on the native plan: pack weights -> forward -> Charbonnier ->
     backward -> (all-reduce of the flat gradient over NCCL when torch.distributed is initialised) -> Adam + EMA, one CUDA graph per
-    (scale, batch shape).  lr / betas: the train YAML's Adam (2e-4, 0.9 / 0.99); EMA 0.999 (base_model.py:75-82)."""
+    (scale, batch shape).  lr / betas: the train YAML's Adam (2e-4, 0.9 / 0.99); EMA 0.999 (base_model.py:75-82).
+    `optimizer` (FlatAdam) takes the caller's lr schedulers and checkpoints in torch.optim.Adam's layout; ema_state_dict() is the EMA
+    network's full state_dict (params_ema); training_state() / resume() are BasicSR's .state file."""
 
     def __init__(self, net: torch.nn.Module, lr: float = 2e-4, betas=(0.9, 0.99), eps: float = 1e-8, ema_decay: float = 0.999,
                  use_graph: bool = True, world_size: int = 1, native_attn: bool = True, native_mask: bool = True):
@@ -1129,16 +1271,91 @@ class NativeTrainer:
         dev = self.flat.device
         self.ctx = context(_dev_index(dev))
         self.weights = TrainWeights(self.flat, self.ctx)
-        self.lr, self.betas, self.eps, self.ema_decay = lr, betas, eps, ema_decay
-        self.use_graph = use_graph
+        self.ema_decay = ema_decay
         self.world = world_size
+        self.optimizer = FlatAdam(self.flat, self.ctx, lr=lr, betas=betas, eps=eps, ema_decay=ema_decay, world_size=world_size, use_graph=use_graph)
+        self.use_graph = use_graph
         self.plans: Dict[tuple, TrainPlan] = {}
         self._graphs: Dict[int, tuple] = {}
-        self._opt_graph: Optional[torch.cuda.CUDAGraph] = None
+        self._ema_buffers = self._snapshot_buffers(net.state_dict())
 
+    # ---- hyper-parameters: the optimizer's group, which schedulers rewrite
+    @property
+    def lr(self) -> float:
+        return self.optimizer.param_groups[0]["lr"]
+
+    @lr.setter
+    def lr(self, value: float) -> None:
+        self.optimizer.param_groups[0]["lr"] = value
+
+    @property
+    def betas(self) -> tuple:
+        return tuple(self.optimizer.param_groups[0]["betas"])
+
+    @property
+    def eps(self) -> float:
+        return self.optimizer.param_groups[0]["eps"]
+
+    @property
+    def use_graph(self) -> bool:
+        return self._use_graph
+
+    @use_graph.setter
+    def use_graph(self, value: bool) -> None:
+        self._use_graph = self.optimizer.use_graph = bool(value)
+
+    # ---- EMA in the reference's layout
     @property
     def ema(self) -> Optional[Dict[str, torch.Tensor]]:
         return {n: self.flat.ema_view(n) for n in self.flat.P} if self.flat.ema is not None else None
+
+    def _snapshot_buffers(self, sd: Dict[str, torch.Tensor]) -> Dict[str, torch.Tensor]:
+        """BasicSR's model_ema averages named_parameters() only: net_g_ema keeps the buffers (BatchNorm running statistics, call
+        counters) it was built or loaded with.  So do we: a copy of the buffers taken when the EMA is initialised."""
+        return {k: v.detach().clone() for k, v in sd.items() if k not in self.flat.P}
+
+    def ema_state_dict(self) -> Optional[Dict[str, torch.Tensor]]:
+        """The EMA network's full state_dict (every key of net.state_dict(), in its order), the `params_ema` of a BasicSR checkpoint:
+        the averaged parameters (views of the flat EMA buffer) and the buffers snapshot at construction / load_ema_state_dict.
+        None when the trainer keeps no EMA (ema_decay 0)."""
+        if self.flat.ema is None:
+            return None
+        return {k: (self.flat.ema_view(k) if k in self.flat.P else self._ema_buffers[k]) for k in self.net.state_dict()}
+
+    def load_ema_state_dict(self, sd: Dict[str, torch.Tensor]) -> None:
+        """Reverse of ema_state_dict, with strict key checking: parameters into the flat EMA buffer, buffers into the snapshot."""
+        if self.flat.ema is None:
+            raise ValueError("this trainer keeps no EMA (ema_decay 0)")
+        want = self.net.state_dict()
+        missing, unexpected = [k for k in want if k not in sd], [k for k in sd if k not in want]
+        if missing or unexpected:
+            raise ValueError(f"EMA state_dict keys differ from the network's: missing {missing[:4]} ({len(missing)}), "
+                             f"unexpected {unexpected[:4]} ({len(unexpected)})")
+        for k, v in want.items():
+            if tuple(sd[k].shape) != tuple(v.shape):
+                raise ValueError(f"EMA state_dict: {k} has shape {tuple(sd[k].shape)}, the network {tuple(v.shape)}")
+        with torch.no_grad():
+            for n in self.flat.P:
+                self.flat.ema_view(n).copy_(sd[n])
+        self._ema_buffers = {k: sd[k].detach().to(want[k].device, want[k].dtype, copy=True) for k in want if k not in self.flat.P}
+
+    # ---- BasicSR's training state (base_model.py save_training_state / resume_training)
+    def training_state(self, iter: int, epoch: int, schedulers: Sequence = ()) -> dict:
+        """{'epoch', 'iter', 'optimizers': [optimizer state], 'schedulers': [their states]}: the .state file BasicSR writes."""
+        return {"epoch": epoch, "iter": iter, "optimizers": [self.optimizer.state_dict()], "schedulers": [s.state_dict() for s in schedulers]}
+
+    def resume(self, state: dict, schedulers: Sequence = ()) -> Tuple[int, int]:
+        """Load a training_state() (or BasicSR's resume state for one Adam) into the optimizer and `schedulers`; returns (epoch, iter).
+        With several ranks every rank loads the same state."""
+        opts, scheds = state["optimizers"], state["schedulers"]
+        if len(opts) != 1:
+            raise ValueError(f"the state holds {len(opts)} optimizers; NativeTrainer has one")
+        if len(scheds) != len(schedulers):
+            raise ValueError(f"the state holds {len(scheds)} schedulers, {len(schedulers)} were given")
+        self.optimizer.load_state_dict(opts[0])
+        for s, sd in zip(schedulers, scheds):
+            s.load_state_dict(sd)
+        return state["epoch"], state["iter"]
 
     def plan_for(self, lq: torch.Tensor, scale) -> TrainPlan:
         b, t, c, h, w = lq.shape
@@ -1155,14 +1372,6 @@ class NativeTrainer:
         loss = plan.run()
         self.weights.scatter_expanded_grads()
         return loss
-
-    def _optim(self) -> None:
-        f = self.flat
-        st = torch.cuda.current_stream(f.device).cuda_stream
-        f.step_t.add_(1.0)
-        K.check(self.ctx.lib.savsr_adam_ema(self.ctx.handle, f.p.data_ptr(), f.g.data_ptr(), f.m.data_ptr(), f.v.data_ptr(),
-                                            f.ema.data_ptr() if f.ema is not None else None, f.n, self.lr, self.betas[0], self.betas[1], self.eps,
-                                            f.step_t.data_ptr(), self.ema_decay, 1.0 / self.world, st))
 
     def _allreduce(self) -> None:
         if self.world > 1:
@@ -1181,7 +1390,7 @@ class NativeTrainer:
             if not self.use_graph:
                 loss = self._fwd_bwd(plan)
                 self._allreduce()
-                self._optim()
+                self.optimizer.step()
                 return loss
             key = id(plan)
             ent = self._graphs.get(key)
@@ -1201,15 +1410,10 @@ class NativeTrainer:
                 with torch.cuda.graph(g, stream=torch.cuda.Stream(dev)):
                     loss = self._fwd_bwd(plan)
                 ent = self._graphs[key] = (g, loss)
-                if self._opt_graph is None:
-                    og = torch.cuda.CUDAGraph()
-                    with torch.cuda.graph(og, stream=torch.cuda.Stream(dev)):
-                        self._optim()
-                    self._opt_graph = og                      # (capture does not execute: nothing to roll back)
             g, loss = ent
             g.replay()
             self._allreduce()
-            self._opt_graph.replay()
+            self.optimizer.step()                             # replays the optimizer's own graph (captured at its first step)
             return loss
 
 

@@ -2,6 +2,8 @@
 (16 x 7 x 3 x 60 x 60 per GPU), one scale per step from a fixed rotation.  Three arms in one process, timed alternately:
 
   native_trainer  trainplan.NativeTrainer, one CUDA graph per scale (forward + loss + backward) plus one for Adam + EMA
+  native_trainer_cosine  the same with a cosine schedule stepped after every step (torch.optim.lr_scheduler.CosineAnnealingLR on
+                  tr.optimizer): the lr changes every step, so each step adds one one-float fill of the device lr before the optimizer graph
   module_native   the module as the reference's optimize_parameters drives it: SAVSR.train(), net(lq), the caller's Charbonnier,
                   backward(), torch.optim.Adam -- the native launch list behind one autograd node (trainplan.ModuleTraining)
   module_stage_a  the same loop with native_training = False: the ATen tape of savsr_b200/train.py (what this shape ran before
@@ -9,6 +11,7 @@
 
 Every scale of the rotation is warmed up first (graphs captured).  Each timed window is a host clock around --steps steps that ends in a
 device synchronise.  Prints one JSON line.  Usage: python scripts/bench_train_shape.py --batch 16 --lq 60 --steps 16 [--rounds 3]
+(the cost of a schedule: --batch 4 --lq 64 --arms native_trainer,native_trainer_cosine)
 """
 import argparse
 import json
@@ -78,12 +81,16 @@ def main():
         mem0 = torch.cuda.memory_allocated(dev)
         torch.cuda.reset_peak_memory_stats(dev)
         net = new_net()
-        if name == "native_trainer":
+        if name in ("native_trainer", "native_trainer_cosine"):
             tr = TP.NativeTrainer(net, use_graph=True)
+            sched = torch.optim.lr_scheduler.CosineAnnealingLR(tr.optimizer, T_max=1_000_000, eta_min=1e-7) if name.endswith("cosine") else None
 
-            def step(i, tr=tr):
+            def step(i, tr=tr, sched=sched):
                 s = SCALES[i % len(SCALES)]
-                return tr.step(lq, gts[s], s)
+                loss = tr.step(lq, gts[s], s)
+                if sched is not None:
+                    sched.step()
+                return loss
             warm = len(SCALES)                                 # the first step of each scale captures its graph
         elif name in ("module_native", "module_stage_a"):
             net.native_training = name == "module_native"
@@ -106,7 +113,7 @@ def main():
         ent = dict(step=step, ms=[], loss=None, net=net,
                    max_memory_allocated_gib=round(torch.cuda.max_memory_allocated(dev) / 2 ** 30, 2),
                    arm_memory_gib=round((torch.cuda.max_memory_allocated(dev) - mem0) / 2 ** 30, 2))
-        if name == "native_trainer":
+        if name.startswith("native_trainer"):
             plan = next(iter(tr.plans.values()))
             ent["arena_gib"] = round(plan.arena_t.numel() * 2 / 2 ** 30, 2)
             ent["t_arena_gib"] = round(plan.tarena.numel() * 2 / 2 ** 30, 2)
@@ -147,6 +154,8 @@ def main():
             if k in ent:
                 row[k] = ent[k]
         out["arms"][name] = row
+    if "native_trainer" in arms and "native_trainer_cosine" in arms:
+        out["cosine_schedule_cost_ms"] = round(statistics.median(arms["native_trainer_cosine"]["ms"]) - statistics.median(arms["native_trainer"]["ms"]), 3)
     if "module_native" in arms and "module_stage_a" in arms:
         out["module_native_speedup_vs_stage_a"] = round(statistics.median(arms["module_stage_a"]["ms"]) / statistics.median(arms["module_native"]["ms"]), 2)
     out["memory_note"] = ("max_memory_allocated_gib: the process peak after the arm's warm-up over the whole rotation (arms are built in the order "
