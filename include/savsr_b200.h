@@ -160,6 +160,13 @@ int savsr_conv(savsr_ctx* ctx, savsr_arena* arena, const savsr_conv_group* group
  */
 int savsr_pack_frames(savsr_ctx* ctx, savsr_arena* arena, const float* x, int t, int h, int w, int dst_slot,
                       savsr_stream st);
+/*
+ * The same from a decoded 8-bit window: x uint8 [batch][t][h][w][3], BGR (the layout cv2.imread and video decoders produce).
+ * Each value becomes float(u) / 255 correctly rounded (the reference's img.astype(np.float32) / 255.) with channels swapped to RGB,
+ * so the slot is bit-identical to savsr_pack_frames of that fp32 window.
+ */
+int savsr_pack_frames_u8(savsr_ctx* ctx, savsr_arena* arena, const uint8_t* x, int t, int h, int w, int dst_slot,
+                         savsr_stream st);
 
 /* ---- backward of the 3x3 convolution (next row 8f1: training step, lbasicsr/models/sr_model.py:101-128) ----------------------
  * Data gradient: a 3x3 convolution of dY with the transposed, spatially flipped filter -- call savsr_conv with those weights
@@ -427,6 +434,15 @@ int savsr_satu_hr(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int
                   const float* table, const float* base_y, const float* base_x, const void* weights,
                   const float* zbias, const float* tail_bias, const float* x_in, int t, int centre, float* out,
                   savsr_stream st);
+/*
+ * The same with 8-bit I/O: x_in is the uint8 BGR window [batch][t][h][w][3] given to savsr_pack_frames_u8 (the bilinear skip reads
+ * its centre frame through the same u / 255), and out is uint8 HWC BGR [batch][H][W][3]: every pixel quantised as tensor2img does
+ * (clamp to [0, 1], * 255, round half to even; what savsr_img_metrics writes to bgr_u8 from savsr_satu_hr's fp32 output).
+ */
+int savsr_satu_hr_u8(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
+                     const float* table, const float* base_y, const float* base_x, const void* weights,
+                     const float* zbias, const float* tail_bias, const uint8_t* x_in, int t, int centre, uint8_t* out,
+                     savsr_stream st);
 
 /* ---- the forward as one call -----------------------------------------------------------------------------------------------------
  * savsr_plan = an ordered list of recorded launches of the entry points above (argument structures copied at record time), replayed on
@@ -440,7 +456,11 @@ int savsr_plan_create(savsr_ctx* ctx, savsr_plan** out);
 void savsr_plan_destroy(savsr_plan* plan);
 int savsr_plan_size(const savsr_plan* plan);                 /* recorded launches */
 int savsr_plan_set_io(savsr_plan* plan, float* x_in, size_t x_bytes, float* out, size_t out_bytes, int format /* enum savsr_format */);
+/* 8-bit I/O: x_in uint8 BGR [batch][7][h][w][3], out uint8 BGR [batch][H][W][3] (the plan records savsr_pack_frames_u8 and
+ * savsr_satu_hr_u8 on them).  A plan has one I/O mode, set by whichever of the two set_io calls came last. */
+int savsr_plan_set_io_u8(savsr_plan* plan, uint8_t* x_in, size_t x_bytes, uint8_t* out, size_t out_bytes, int format);
 int savsr_plan_add_pack_frames(savsr_plan* plan, savsr_arena* arena, const float* x, int t, int h, int w, int dst_slot);
+int savsr_plan_add_pack_frames_u8(savsr_plan* plan, savsr_arena* arena, const uint8_t* x, int t, int h, int w, int dst_slot);
 int savsr_plan_add_conv(savsr_plan* plan, savsr_arena* arena, const savsr_conv_group* groups, int ngroups, int ksize, int n_tile,
                         int dst_mode, int impl);
 int savsr_plan_add_osa_prologue(savsr_plan* plan, const savsr_osa_params* convs, int nconvs, int batch, int npart, int npix,
@@ -454,10 +474,16 @@ int savsr_plan_add_satu_kconv_sta(savsr_plan* plan, savsr_arena* arena, int a_sl
 int savsr_plan_add_satu_hr(savsr_plan* plan, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W, const float* table,
                            const float* base_y, const float* base_x, const void* weights, const float* zbias, const float* tail_bias,
                            const float* x_in, int t, int centre, float* out);
+int savsr_plan_add_satu_hr_u8(savsr_plan* plan, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W, const float* table,
+                              const float* base_y, const float* base_x, const void* weights, const float* zbias, const float* tail_bias,
+                              const uint8_t* x_in, int t, int centre, uint8_t* out);
 int savsr_plan_add_arena_export(savsr_plan* plan, savsr_arena* arena, int slot, float* nchw);   /* debug taps */
 int savsr_plan_run(savsr_plan* plan, savsr_stream st);
 /* x -> the plan's input staging buffer (device-to-device, skipped when x IS that buffer), replay, output staging buffer -> out. */
 int savsr_forward(savsr_plan* plan, const float* x, float* out, savsr_stream st);
+/* The same for a plan with 8-bit I/O (savsr_plan_set_io_u8): x uint8 BGR [batch][7][h][w][3] -> out uint8 BGR [batch][H][W][3].
+ * Each of savsr_forward / savsr_forward_u8 returns an error, before any copy or launch, on a plan of the other I/O mode. */
+int savsr_forward_u8(savsr_plan* plan, const uint8_t* x, uint8_t* out, savsr_stream st);
 
 /* ---- post-processing / metrics on the device (next row 8f3) -------------------------------------------------------
  * tensor2img (lbasicsr/utils/img_util.py:38-94): sr fp32 NCHW [batch][3][H][W] RGB -> uint8 HWC BGR [batch][H][W][3]

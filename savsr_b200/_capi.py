@@ -168,23 +168,29 @@ SIGNATURES = {
     "savsr_plan_destroy": (None, [_VP]),
     "savsr_plan_size": (_I, [_VP]),
     "savsr_plan_set_io": (_I, [_VP, _VP, _SZ, _VP, _SZ, _I]),
+    "savsr_plan_set_io_u8": (_I, [_VP, _VP, _SZ, _VP, _SZ, _I]),
     "savsr_plan_add_pack_frames": (_I, [_VP, _VP, _VP, _I, _I, _I, _I]),
+    "savsr_plan_add_pack_frames_u8": (_I, [_VP, _VP, _VP, _I, _I, _I, _I]),
     "savsr_plan_add_conv": (_I, [_VP, _VP, C.POINTER(ConvGroup), _I, _I, _I, _I, _I]),
     "savsr_plan_add_osa_prologue": (_I, [_VP, C.POINTER(OsaParams), _I, _I, _I, _I, _F, _F]),
     "savsr_plan_add_ca_scale_residual": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _VP, _VP, _VP, _VP, _VP]),
     "savsr_plan_add_osadapt_mask": (_I, [_VP, _VP, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     "savsr_plan_add_satu_kconv_sta": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _VP, _VP, _F]),
     "savsr_plan_add_satu_hr": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP]),
+    "savsr_plan_add_satu_hr_u8": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP]),
     "savsr_plan_add_arena_export": (_I, [_VP, _VP, _I, _VP]),
     "savsr_plan_run": (_I, [_VP, _VP]),
     "savsr_forward": (_I, [_VP, _VP, _VP, _VP]),
+    "savsr_forward_u8": (_I, [_VP, _VP, _VP, _VP]),
     "savsr_pack_frames": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),
+    "savsr_pack_frames_u8": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),
     "savsr_osa_prologue": (_I, [_VP, C.POINTER(OsaParams), _I, _I, _I, _I, _F, _F, _VP]),
     "savsr_ca_scale_residual": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _VP, _VP, _VP, _VP, _VP, _VP]),
     "savsr_osadapt_mask": (_I, [_VP, _VP, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
     "savsr_satu_index": (_I, [_VP, C.POINTER(SatuWeights), _I, _I, _I, _I, _F, _F] + [_VP] * 9 + [_VP]),
     "savsr_satu_kconv_sta": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _VP, _VP, _F, _VP]),
     "savsr_satu_hr": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP, _VP]),
+    "savsr_satu_hr_u8": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP, _VP]),
     "savsr_img_metrics_blocks": (_I, [_VP, _I, _I]),
     "savsr_img_metrics": (_I, [_VP, _VP, _VP, _I, _I, _I, _VP, _VP, _VP]),
     "savsr_ssim_y_blocks": (_I, [_I, _I]),

@@ -237,7 +237,24 @@ class SAVSR(nn.Module):
         if x.dim() == 5 and x.shape[0] == 0 and x.is_cuda:        # an empty batch of windows (a rank with no frames of the clip): nothing to launch
             H, W = engine.get_hw(x.shape[3], x.shape[4], self.scale)
             return x.new_empty((0, 3, H, W))
-        plan = self.plan_for(x)
+        return self._run_plan(self.plan_for(x), x)
+
+    def forward_bgr_u8(self, x: torch.Tensor, scale=None) -> torch.Tensor:
+        """Upscale decoded 8-bit video: x uint8 [b, 7, h, w, 3] BGR windows (the layout cv2.imread and video decoders produce) ->
+        a fresh uint8 [b, H, W, 3] BGR tensor.  Bit for bit the image tensor2img makes of forward(x') (postproc.tensor2img_psnr),
+        where x' = the windows as fp32 RGB planes, u / 255 correctly rounded, as the reference's img.astype(np.float32) / 255.
+        Inference only (training takes fp32 windows through forward); same plan cache, precision, conv_impl and CUDA graphs as
+        forward, with its own plan per shape."""
+        if self.training:
+            raise RuntimeError("forward_bgr_u8 is inference only: call eval() first (training takes fp32 windows through forward)")
+        if scale is not None:
+            self.scale = scale
+        b, h, w = self._window_shape(x, "bgr_u8")
+        if b == 0:                  # an empty batch of windows (a rank with no frames of the clip): nothing to launch
+            return x.new_empty((0, *engine.get_hw(h, w, self.scale), 3))
+        return self._run_plan(self.plan_for(x, io="bgr_u8"), x)
+
+    def _run_plan(self, plan: engine.Plan, x: torch.Tensor) -> torch.Tensor:
         with torch.cuda.device(plan.device):
             out = torch.empty_like(plan.out)
             plan.forward_into(x, out, graph=self.use_graph)
@@ -291,20 +308,34 @@ class SAVSR(nn.Module):
             self._stores[key] = st
         return st
 
-    def plan_for(self, x: torch.Tensor) -> engine.Plan:
-        if x.dim() != 5 or x.shape[1] != self.num_frame or x.shape[2] != 3:
-            raise ValueError(f"expected input [b, {self.num_frame}, 3, h, w], got {tuple(x.shape)}")
+    def _window_shape(self, x: torch.Tensor, io: str) -> Tuple[int, int, int]:
+        """(b, h, w) of a batch of windows in the layout of `io`, after checking that it can run on this module's device."""
+        if io == "bgr_u8":
+            if x.dtype != torch.uint8:
+                raise TypeError(f"forward_bgr_u8 takes uint8 windows, got {x.dtype}")
+            if x.dim() != 5 or x.shape[1] != self.num_frame or x.shape[4] != 3:
+                raise ValueError(f"expected uint8 BGR windows [b, {self.num_frame}, h, w, 3], got {tuple(x.shape)}")
+            b, _, h, w, _ = x.shape
+        else:
+            if x.dim() != 5 or x.shape[1] != self.num_frame or x.shape[2] != 3:
+                raise ValueError(f"expected input [b, {self.num_frame}, 3, h, w], got {tuple(x.shape)}")
+            b, _, _, h, w = x.shape
         if not x.is_cuda:
             raise RuntimeError("savsr_b200.SAVSR runs on CUDA (sm_100a) only; there is no CPU fallback")
-        if self.training:
-            raise RuntimeError("plans are the inference path; in train mode forward() runs savsr_b200.train.forward")
         p0 = self.gamma
         if p0.device != x.device:
             raise RuntimeError(f"module parameters on {p0.device}, input on {x.device}")
-        b, _, _, h, w = x.shape
+        return b, h, w
+
+    def plan_for(self, x: torch.Tensor, io: str = "f32") -> engine.Plan:
+        """The cached plan for windows like `x`: io="f32" takes [b, 7, 3, h, w] (forward), io="bgr_u8" uint8 [b, 7, h, w, 3]
+        (forward_bgr_u8).  Plans of both modes share one WeightStore."""
+        b, h, w = self._window_shape(x, io)
+        if self.training:
+            raise RuntimeError("plans are the inference path; in train mode forward() runs savsr_b200.train.forward")
         s = engine.normalize_scale(self.scale)
         wkey = self._weights_version()
-        key = (b, h, w, float(s[0]), float(s[1]), self.conv_impl, self.precision, tuple(self.debug_taps), x.device.index) + wkey
+        key = (b, h, w, float(s[0]), float(s[1]), self.conv_impl, self.precision, tuple(self.debug_taps), x.device.index, io) + wkey
         plan = self._plans.get(key)
         if plan is not None:
             self._plans.move_to_end(key)
@@ -313,7 +344,7 @@ class SAVSR(nn.Module):
         t0 = time.perf_counter()
         params = {k: v for k, v in self.state_dict(keep_vars=True).items()}
         plan = engine.Plan(params, b, h, w, s, x.device, conv_impl=self.conv_impl, num_frame=self.num_frame,
-                           taps=self.debug_taps, precision=self.precision, store=self._store_for(x.device, wkey))
+                           taps=self.debug_taps, precision=self.precision, store=self._store_for(x.device, wkey), io=io)
         self.last_plan_build_ms = 1e3 * (time.perf_counter() - t0)
         self._plans[key] = plan
         # bound the device memory held by cached plans (arenas + graphs): evict least recently used down to the byte budget

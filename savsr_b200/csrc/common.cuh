@@ -56,7 +56,7 @@ namespace savsr {
 enum AttrBit { kAttrIgemm = 0 /* + template index, 6 variants */, kAttrBigk = 8, kAttrKsta = 9, kAttrSatuHr = 10, kAttrOsaLinear = 11,
                kAttrFused = 12, kAttrBigk128 = 13, kAttrSatuHrBf16 = 14, kAttrWgrad = 15, kAttrWgradBatched = 16,
                kAttrOsaAssembleTrain = 17, kAttrOsaUnfoldBwd = 18, kAttrOsaChain = 19, kAttrOsaMatvec = 20 /* + 0, 1, 2: batch 8, 16, 32 */,
-               kAttrCaBackward = 23 };
+               kAttrCaBackward = 23, kAttrSatuHrU8 = 24 /* + format: 8-bit I/O instantiations of satu_hr */ };
 template <class F>
 inline int ensure_smem_attr(savsr_ctx* ctx, int bit, F func, size_t bytes) {
   if (ctx->attr_mask & (1u << bit)) return 0;
@@ -124,6 +124,16 @@ __device__ __forceinline__ float h_lo(uint32_t v, int fmt) {
 __device__ __forceinline__ float h_hi(uint32_t v, int fmt) {
   return fmt ? __half2float(__ushort_as_half(static_cast<unsigned short>(v >> 16))) : __uint_as_float(v & 0xffff0000u);
 }
+// 8-bit pixel <-> [0, 1] float.  In: the reference's img.astype(np.float32) / 255., correctly rounded.  A multiply by the rounded
+// reciprocal alone is off by one ulp for 126 of the 256 values; with one fma correction of the remainder it is exact for all of them
+// (checked exhaustively, tests/test_video_u8_io.py), and unlike __fdiv_rn it has no slow-path call.
+// Out: tensor2img (lbasicsr/utils/img_util.py:38-94): clamp to [0, 1], * 255, round half to even.
+__device__ __forceinline__ float u8_to_unit(uint8_t u) {
+  const float a = static_cast<float>(u), r = 1.0f / 255.0f;
+  const float q = __fmul_rn(a, r);
+  return __fmaf_rn(__fmaf_rn(-q, 255.0f, a), r, q);
+}
+__device__ __forceinline__ int unit_to_u8(float v) { return __float2int_rn(fminf(fmaxf(v, 0.f), 1.f) * 255.0f); }
 __device__ __forceinline__ float h_to_float(uint16_t raw, int fmt) { return h_lo(raw, fmt); }
 __device__ __forceinline__ uint16_t float_to_h(float x, int fmt) { return static_cast<uint16_t>(pack_h2(x, 0.f, fmt) & 0xffffu); }
 

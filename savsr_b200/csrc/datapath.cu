@@ -92,7 +92,7 @@ __global__ void __launch_bounds__(256) lr_width_kernel(const LrParams p) {
     float v;
     if (p.frames != nullptr) {
       const uint8_t* row = p.frames + ((static_cast<long>(t) * p.H + y) * p.W) * 3 + (2 - c);
-      auto load = [&](int x) { return __fdiv_rn(static_cast<float>(row[static_cast<long>(x) * 3]), 255.0f); };
+      auto load = [&](int x) { return u8_to_unit(row[static_cast<long>(x) * 3]); };
       if (p.ow == p.wc) {
         v = load(ox);
       } else {
@@ -141,7 +141,7 @@ __global__ void __launch_bounds__(256) gt_rgb_kernel(const LrParams p) {
     const int y = r % p.hc; r /= p.hc;
     const int c = r % 3;
     const int t = r / 3;
-    p.gt[idx] = __fdiv_rn(static_cast<float>(p.frames[((static_cast<long>(t) * p.H + y) * p.W + x) * 3 + (2 - c)]), 255.0f);
+    p.gt[idx] = u8_to_unit(p.frames[((static_cast<long>(t) * p.H + y) * p.W + x) * 3 + (2 - c)]);
   }
 }
 

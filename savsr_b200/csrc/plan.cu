@@ -12,10 +12,11 @@
 struct savsr_plan {
   savsr_ctx* ctx;
   std::vector<std::function<int(savsr_stream)>> ops;
-  float* x_in = nullptr;
-  float* out = nullptr;
+  void* x_in = nullptr;
+  void* out = nullptr;
   size_t x_bytes = 0, out_bytes = 0;
   int format = SAVSR_FMT_BF16;
+  bool u8 = false;                 // I/O mode: fp32 (savsr_forward) or uint8 BGR (savsr_forward_u8)
 };
 
 using namespace savsr;
@@ -32,17 +33,32 @@ extern "C" int savsr_plan_create(savsr_ctx* ctx, savsr_plan** out) {
 extern "C" void savsr_plan_destroy(savsr_plan* plan) { delete plan; }
 extern "C" int savsr_plan_size(const savsr_plan* plan) { return plan ? static_cast<int>(plan->ops.size()) : 0; }
 
-extern "C" int savsr_plan_set_io(savsr_plan* plan, float* x_in, size_t x_bytes, float* out, size_t out_bytes, int format) {
-  SAVSR_REQUIRE(plan && x_in && out && x_bytes && out_bytes, "savsr_plan_set_io: null pointer / empty buffer");
-  SAVSR_REQUIRE(format == SAVSR_FMT_BF16 || format == SAVSR_FMT_FP16, "savsr_plan_set_io: unknown format %d", format);
-  plan->x_in = x_in; plan->x_bytes = x_bytes; plan->out = out; plan->out_bytes = out_bytes; plan->format = format;
+static int set_io(const char* name, savsr_plan* plan, void* x_in, size_t x_bytes, void* out, size_t out_bytes, int format, bool u8) {
+  SAVSR_REQUIRE(plan && x_in && out && x_bytes && out_bytes, "%s: null pointer / empty buffer", name);
+  SAVSR_REQUIRE(format == SAVSR_FMT_BF16 || format == SAVSR_FMT_FP16, "%s: unknown format %d", name, format);
+  plan->x_in = x_in; plan->x_bytes = x_bytes; plan->out = out; plan->out_bytes = out_bytes; plan->format = format; plan->u8 = u8;
   return 0;
+}
+
+extern "C" int savsr_plan_set_io(savsr_plan* plan, float* x_in, size_t x_bytes, float* out, size_t out_bytes, int format) {
+  return set_io("savsr_plan_set_io", plan, x_in, x_bytes, out, out_bytes, format, false);
+}
+
+extern "C" int savsr_plan_set_io_u8(savsr_plan* plan, uint8_t* x_in, size_t x_bytes, uint8_t* out, size_t out_bytes, int format) {
+  return set_io("savsr_plan_set_io_u8", plan, x_in, x_bytes, out, out_bytes, format, true);
 }
 
 extern "C" int savsr_plan_add_pack_frames(savsr_plan* plan, savsr_arena* arena, const float* x, int t, int h, int w, int dst_slot) {
   SAVSR_REQUIRE(plan && arena && x, "savsr_plan_add_pack_frames: null pointer");
   savsr_ctx* ctx = plan->ctx;
   plan->ops.push_back([=](savsr_stream st) { return savsr_pack_frames(ctx, arena, x, t, h, w, dst_slot, st); });
+  return 0;
+}
+
+extern "C" int savsr_plan_add_pack_frames_u8(savsr_plan* plan, savsr_arena* arena, const uint8_t* x, int t, int h, int w, int dst_slot) {
+  SAVSR_REQUIRE(plan && arena && x, "savsr_plan_add_pack_frames_u8: null pointer");
+  savsr_ctx* ctx = plan->ctx;
+  plan->ops.push_back([=](savsr_stream st) { return savsr_pack_frames_u8(ctx, arena, x, t, h, w, dst_slot, st); });
   return 0;
 }
 
@@ -100,6 +116,17 @@ extern "C" int savsr_plan_add_satu_hr(savsr_plan* plan, savsr_arena* lr, int x_s
   return 0;
 }
 
+extern "C" int savsr_plan_add_satu_hr_u8(savsr_plan* plan, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
+                                         const float* table, const float* base_y, const float* base_x, const void* weights,
+                                         const float* zbias, const float* tail_bias, const uint8_t* x_in, int t, int centre, uint8_t* out) {
+  SAVSR_REQUIRE(plan && lr, "savsr_plan_add_satu_hr_u8: null pointer");
+  savsr_ctx* ctx = plan->ctx;
+  plan->ops.push_back([=](savsr_stream st) {
+    return savsr_satu_hr_u8(ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias, x_in, t, centre, out, st);
+  });
+  return 0;
+}
+
 extern "C" int savsr_plan_add_arena_export(savsr_plan* plan, savsr_arena* arena, int slot, float* nchw) {
   SAVSR_REQUIRE(plan && arena && nchw, "savsr_plan_add_arena_export: null pointer");
   plan->ops.push_back([=](savsr_stream st) { return savsr_arena_export(arena, slot, nchw, st); });
@@ -116,13 +143,23 @@ extern "C" int savsr_plan_run(savsr_plan* plan, savsr_stream st) {
   return 0;
 }
 
-extern "C" int savsr_forward(savsr_plan* plan, const float* x, float* out, savsr_stream st) {
-  SAVSR_REQUIRE(plan && x && out, "savsr_forward: null pointer");
-  SAVSR_REQUIRE(plan->x_in && plan->out, "savsr_forward: the plan has no I/O staging buffers (savsr_plan_set_io)");
+static int forward(const char* name, savsr_plan* plan, const void* x, void* out, bool u8, savsr_stream st) {
+  SAVSR_REQUIRE(plan && x && out, "%s: null pointer", name);
+  SAVSR_REQUIRE(plan->x_in && plan->out, "%s: the plan has no I/O staging buffers (savsr_plan_set_io / savsr_plan_set_io_u8)", name);
+  SAVSR_REQUIRE(plan->u8 == u8, "%s: the plan was set up for %s I/O; call %s", name, plan->u8 ? "uint8 BGR" : "fp32",
+                plan->u8 ? "savsr_forward_u8" : "savsr_forward");
   DeviceGuard guard(plan->ctx->device);
   cudaStream_t s = static_cast<cudaStream_t>(st);
   if (x != plan->x_in) SAVSR_CUDA(cudaMemcpyAsync(plan->x_in, x, plan->x_bytes, cudaMemcpyDeviceToDevice, s));
   if (int rc = savsr_plan_run(plan, st)) return rc;
   if (out != plan->out) SAVSR_CUDA(cudaMemcpyAsync(out, plan->out, plan->out_bytes, cudaMemcpyDeviceToDevice, s));
   return 0;
+}
+
+extern "C" int savsr_forward(savsr_plan* plan, const float* x, float* out, savsr_stream st) {
+  return forward("savsr_forward", plan, x, out, false, st);
+}
+
+extern "C" int savsr_forward_u8(savsr_plan* plan, const uint8_t* x, uint8_t* out, savsr_stream st) {
+  return forward("savsr_forward_u8", plan, x, out, true, st);
 }

@@ -342,6 +342,10 @@ __device__ __forceinline__ int swz(int r, int c) { return r * 128 + ((c ^ (r & 7
 //                          8      MMA issuer (tcgen05, accumulators U and Z in TMEM, double buffered)
 //                          0..7   consumers, two groups alternating tiles: routing (U -> V tile), Z -> smem, and, once per
 //                                 block and sample, the 9-tap sum + bias + bilinear skip -> fp32 NCHW stores (128 B per warp row)
+//
+// I/O modes (template U8): fp32 (the module's forward contract) reads the skip from the fp32 window and stores fp32 NCHW; 8-bit reads it
+// from the uint8 BGR window [batch][t][h][w][3] through the same u / 255 as the first layer, so the skip is the same fp32 number, and
+// stores tensor2img's uint8 HWC BGR [batch][H][W][3] of the same fp32 value the fp32 mode would have written.
 struct HrParams {
   const __nv_bfloat16* lr;
   const float* table;        // [H*W][8]: offset x,y | st_offset x,y | r0..r3
@@ -350,8 +354,8 @@ struct HrParams {
   const uint8_t* weights;    // 4 x [32 rows][128 B] K-major swizzled: Wc (rows e*8+k) | Wcf | Wcs | Wv (K = 32), rows of Wcf/Wcs/Wv = tap*3+c
   const float* zbias;        // [32]: zb[tap*3+c], 27 used
   const float* tail_bias;    // [3]
-  const float* x_in;         // [batch][t][3][h][w] fp32 (bilinear skip of the centre frame)
-  float* out;                // [batch][3][H][W] fp32
+  const void* x_in;          // bilinear skip of the centre frame: fp32 [batch][t][3][h][w], or uint8 BGR [batch][t][h][w][3]
+  void* out;                 // fp32 [batch][3][H][W], or uint8 BGR [batch][H][W][3]
   int batch, hp, wp, h, w, H, W;
   int x_slot, sta_slot;
   int t, centre;
@@ -424,7 +428,7 @@ __device__ __forceinline__ void bilinear_src_scaled(int dst, float scale, int in
   l1 = src - static_cast<float>(i0);
 }
 
-template <int FMT>
+template <int FMT, bool U8>
 __global__ void __launch_bounds__(kHrThreads, 1) satu_hr_kernel(const __grid_constant__ HrParams p) {
   extern __shared__ uint8_t raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(raw) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -489,13 +493,20 @@ __global__ void __launch_bounds__(kHrThreads, 1) satu_hr_kernel(const __grid_con
           float ly, lx;
           bilinear_src_scaled(Y, sk_sy, p.h, y0, y1, ly);
           bilinear_src_scaled(X, sk_sx, p.w, x0, x1, lx);
-          const float* xc = p.x_in + static_cast<long>(n * p.t + p.centre) * 3 * plane;
+          const long xc = static_cast<long>(n * p.t + p.centre) * 3 * plane;   // centre frame of sample n (elements, either layout)
           const int o00 = y0 * p.w + x0, o01 = y0 * p.w + x1, o10 = y1 * p.w + x0, o11 = y1 * p.w + x1;
           float sk[3];
 #pragma unroll
           for (int ch = 0; ch < 3; ++ch) {
-            const float* pl = xc + ch * plane;
-            const float a = __ldg(pl + o00), bb = __ldg(pl + o01), cc = __ldg(pl + o10), d = __ldg(pl + o11);
+            float a, bb, cc, d;
+            if constexpr (U8) {
+              const uint8_t* pl = static_cast<const uint8_t*>(p.x_in) + xc + 2 - ch;
+              a = u8_to_unit(__ldg(pl + 3 * o00)); bb = u8_to_unit(__ldg(pl + 3 * o01));
+              cc = u8_to_unit(__ldg(pl + 3 * o10)); d = u8_to_unit(__ldg(pl + 3 * o11));
+            } else {
+              const float* pl = static_cast<const float*>(p.x_in) + xc + ch * plane;
+              a = __ldg(pl + o00); bb = __ldg(pl + o01); cc = __ldg(pl + o10); d = __ldg(pl + o11);
+            }
             sk[ch] = (1.f - ly) * ((1.f - lx) * a + lx * bb) + ly * ((1.f - lx) * cc + lx * d);
           }
           float acc0 = bt0, acc1 = bt1, acc2 = bt2;
@@ -511,8 +522,15 @@ __global__ void __launch_bounds__(kHrThreads, 1) satu_hr_kernel(const __grid_con
               acc2 += v ? __half2float(z[2 * kHrPix]) : 0.f;
             }
           }
-          float* o = p.out + static_cast<long>(n) * 3 * NPIX + static_cast<long>(Y) * p.W + X;
-          o[0] = acc0 + sk[0]; o[NPIX] = acc1 + sk[1]; o[2 * NPIX] = acc2 + sk[2];
+          if constexpr (U8) {
+            // 3 bytes per pixel: W * 3 has any alignment, so plain byte stores (a warp row is 96 contiguous bytes)
+            uint8_t* o = static_cast<uint8_t*>(p.out) + (static_cast<long>(n) * NPIX + static_cast<long>(Y) * p.W + X) * 3;
+            o[0] = static_cast<uint8_t>(unit_to_u8(acc2 + sk[2])); o[1] = static_cast<uint8_t>(unit_to_u8(acc1 + sk[1]));
+            o[2] = static_cast<uint8_t>(unit_to_u8(acc0 + sk[0]));
+          } else {
+            float* o = static_cast<float*>(p.out) + static_cast<long>(n) * 3 * NPIX + static_cast<long>(Y) * p.W + X;
+            o[0] = acc0 + sk[0]; o[NPIX] = acc1 + sk[1]; o[2 * NPIX] = acc2 + sk[2];
+          }
         }
       }
       __syncwarp();
@@ -756,20 +774,21 @@ extern "C" int savsr_satu_kconv_sta(savsr_ctx* ctx, savsr_arena* arena, int a_sl
   return 0;
 }
 
-extern "C" int savsr_satu_hr(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
-                             const float* table, const float* base_y, const float* base_x, const void* weights,
-                             const float* zbias, const float* tail_bias, const float* x_in, int t, int centre, float* out,
-                             savsr_stream st) {
-  SAVSR_REQUIRE(ctx && lr && table && base_y && base_x && weights && zbias && tail_bias && x_in && out, "savsr_satu_hr: null pointer");
+template <bool U8>
+static int satu_hr(const char* name, savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W, const float* table,
+                   const float* base_y, const float* base_x, const void* weights, const float* zbias, const float* tail_bias,
+                   const void* x_in, int t, int centre, void* out, savsr_stream st) {
+  SAVSR_REQUIRE(ctx && lr && table && base_y && base_x && weights && zbias && tail_bias && x_in && out, "%s: null pointer", name);
   DeviceGuard guard(ctx->device);
-  SAVSR_REQUIRE(x_slot >= 0 && x_slot < lr->nslots && sta_slot >= 0 && sta_slot < lr->nslots, "savsr_satu_hr: LR slot out of range");
-  SAVSR_REQUIRE(h >= 2 && w >= 2 && h <= lr->height && w <= lr->width, "savsr_satu_hr: region %dx%d exceeds LR arena", h, w);
-  SAVSR_REQUIRE(h < 65536 && w < 65536, "savsr_satu_hr: LR frames larger than 65535 pixels per side are not supported");
-  SAVSR_REQUIRE(H >= 1 && W >= 1 && t >= 1 && centre >= 0 && centre < t, "savsr_satu_hr: bad HR size %dx%d or window (%d, %d)", H, W, t, centre);
+  SAVSR_REQUIRE(x_slot >= 0 && x_slot < lr->nslots && sta_slot >= 0 && sta_slot < lr->nslots, "%s: LR slot out of range", name);
+  SAVSR_REQUIRE(h >= 2 && w >= 2 && h <= lr->height && w <= lr->width, "%s: region %dx%d exceeds LR arena", name, h, w);
+  SAVSR_REQUIRE(h < 65536 && w < 65536, "%s: LR frames larger than 65535 pixels per side are not supported", name);
+  SAVSR_REQUIRE(H >= 1 && W >= 1 && t >= 1 && centre >= 0 && centre < t, "%s: bad HR size %dx%d or window (%d, %d)", name, H, W, t, centre);
   if (lr->batch == 0) return 0;
   const bool fp16 = ctx->fmt == SAVSR_FMT_FP16;
-  if (int rc = fp16 ? ensure_smem_attr(ctx, kAttrSatuHr + 0, satu_hr_kernel<SAVSR_FMT_FP16>, kHrSmem)
-                    : ensure_smem_attr(ctx, kAttrSatuHrBf16, satu_hr_kernel<SAVSR_FMT_BF16>, kHrSmem)) return rc;
+  auto kernel = fp16 ? satu_hr_kernel<SAVSR_FMT_FP16, U8> : satu_hr_kernel<SAVSR_FMT_BF16, U8>;
+  const int bit = U8 ? kAttrSatuHrU8 + (fp16 ? 1 : 0) : (fp16 ? kAttrSatuHr : kAttrSatuHrBf16);
+  if (int rc = ensure_smem_attr(ctx, bit, kernel, kHrSmem)) return rc;
   HrParams p;
   p.lr = lr->base; p.table = table; p.base_y = base_y; p.base_x = base_x;
   p.weights = static_cast<const uint8_t*>(weights); p.zbias = zbias; p.tail_bias = tail_bias; p.x_in = x_in; p.out = out;
@@ -778,8 +797,23 @@ extern "C" int savsr_satu_hr(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int st
   p.regions_x = (W + kHrRW - 1) / kHrRW;
   p.nregions = p.regions_x * ((H + kHrRH - 1) / kHrRH);
   const int grid = p.nregions < ctx->sm_count ? p.nregions : ctx->sm_count;
-  if (fp16) satu_hr_kernel<SAVSR_FMT_FP16><<<grid, kHrThreads, kHrSmem, static_cast<cudaStream_t>(st)>>>(p);
-  else satu_hr_kernel<SAVSR_FMT_BF16><<<grid, kHrThreads, kHrSmem, static_cast<cudaStream_t>(st)>>>(p);
+  kernel<<<grid, kHrThreads, kHrSmem, static_cast<cudaStream_t>(st)>>>(p);
   SAVSR_CUDA(cudaGetLastError());
   return 0;
+}
+
+extern "C" int savsr_satu_hr(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
+                             const float* table, const float* base_y, const float* base_x, const void* weights,
+                             const float* zbias, const float* tail_bias, const float* x_in, int t, int centre, float* out,
+                             savsr_stream st) {
+  return satu_hr<false>("savsr_satu_hr", ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias, x_in, t,
+                        centre, out, st);
+}
+
+extern "C" int savsr_satu_hr_u8(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
+                                const float* table, const float* base_y, const float* base_x, const void* weights,
+                                const float* zbias, const float* tail_bias, const uint8_t* x_in, int t, int centre, uint8_t* out,
+                                savsr_stream st) {
+  return satu_hr<true>("savsr_satu_hr_u8", ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias, x_in, t,
+                       centre, out, st);
 }

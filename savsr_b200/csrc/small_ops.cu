@@ -7,10 +7,12 @@
 namespace savsr {
 
 // ------------------------------------------------------------------------------------------------ first layer: frame packing
-// fp32 NCHW window [B][t][3][h][w] -> one bf16 arena slot whose channels 0..3t-1 are the frames' RGB planes
-// (channel 3f + c), the rest zero, reflect-padded to the even arena size (savsr_arch.py:670-690).  With this slot the
-// first-layer convs (conv_c / conv_sup, savsr_arch.py:456-457) run on the tensor-core kernel with zero-expanded weights.
-__global__ void __launch_bounds__(256) pack_frames_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ dst, int batch,
+// The input window -> one bf16 arena slot whose channels 0..3t-1 are the frames' RGB planes (channel 3f + c), the rest zero,
+// reflect-padded to the even arena size (savsr_arch.py:670-690).  With this slot the first-layer convs (conv_c / conv_sup,
+// savsr_arch.py:456-457) run on the tensor-core kernel with zero-expanded weights.  T = float: fp32 NCHW window [B][t][3][h][w] RGB;
+// T = uint8_t: the decoded 8-bit window [B][t][h][w][3] BGR, converted exactly as the reference's img.astype(np.float32) / 255.
+template <class T>
+__global__ void __launch_bounds__(256) pack_frames_kernel(const T* __restrict__ x, __nv_bfloat16* __restrict__ dst, int batch,
                                                           int t, int h, int w, int hp, int wp, int fmt) {
   const long npix = static_cast<long>(hp) * wp;
   const long total = static_cast<long>(batch) * npix * 8;
@@ -25,7 +27,12 @@ __global__ void __launch_bounds__(256) pack_frames_kernel(const float* __restric
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       const int ch = chunk * 8 + e;
-      v[e] = ch < 3 * t ? __ldg(x + ((static_cast<long>(n) * t * 3 + ch) * h + ry) * w + rx) : 0.f;
+      if constexpr (sizeof(T) == 1) {
+        const int f = ch / 3, c = ch - 3 * f;
+        v[e] = ch < 3 * t ? u8_to_unit(__ldg(x + ((static_cast<long>(n) * t + f) * h + ry) * w * 3 + rx * 3 + 2 - c)) : 0.f;
+      } else {
+        v[e] = ch < 3 * t ? __ldg(x + ((static_cast<long>(n) * t * 3 + ch) * h + ry) * w + rx) : 0.f;
+      }
     }
     uint4 o;
     o.x = pack_h2(v[0], v[1], fmt); o.y = pack_h2(v[2], v[3], fmt); o.z = pack_h2(v[4], v[5], fmt); o.w = pack_h2(v[6], v[7], fmt);
@@ -442,8 +449,8 @@ __global__ void __launch_bounds__(256) img_metrics_kernel(const float* __restric
     int q[3], qg[3];
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-      q[c] = __float2int_rn(fminf(fmaxf(s[c * npix + pix], 0.f), 1.f) * 255.0f);
-      if (g) qg[c] = __float2int_rn(fminf(fmaxf(g[c * npix + pix], 0.f), 1.f) * 255.0f);
+      q[c] = unit_to_u8(s[c * npix + pix]);
+      if (g) qg[c] = unit_to_u8(g[c * npix + pix]);
     }
     if (bgr) {
       uint8_t* o = bgr + (static_cast<long>(n) * npix + pix) * 3;
@@ -500,8 +507,8 @@ __global__ void __launch_bounds__(256) ssim_y_kernel(const __grid_constant__ Ssi
       int q[3], qg[3];
 #pragma unroll
       for (int ch = 0; ch < 3; ++ch) {
-        q[ch] = __float2int_rn(fminf(fmaxf(s[ch * npix + pix], 0.f), 1.f) * 255.0f);
-        qg[ch] = __float2int_rn(fminf(fmaxf(g[ch * npix + pix], 0.f), 1.f) * 255.0f);
+        q[ch] = unit_to_u8(s[ch * npix + pix]);
+        qg[ch] = unit_to_u8(g[ch * npix + pix]);
       }
       a = static_cast<double>(y_of_u8(q[2], q[1], q[0]));
       b = static_cast<double>(y_of_u8(qg[2], qg[1], qg[0]));
@@ -537,22 +544,31 @@ __global__ void __launch_bounds__(256) ssim_y_kernel(const __grid_constant__ Ssi
   }
 }
 
-extern "C" int savsr_pack_frames(savsr_ctx* ctx, savsr_arena* arena, const float* x, int t, int h, int w, int dst_slot, savsr_stream st) {
-  SAVSR_REQUIRE(ctx && arena && x, "savsr_pack_frames: null pointer");
+template <class T>
+static int pack_frames(const char* name, savsr_ctx* ctx, savsr_arena* arena, const T* x, int t, int h, int w, int dst_slot, savsr_stream st) {
+  SAVSR_REQUIRE(ctx && arena && x, "%s: null pointer", name);
   DeviceGuard guard(ctx->device);
-  SAVSR_REQUIRE(t >= 1 && 3 * t <= kC, "savsr_pack_frames: %d frames do not fit 64 channels", t);
-  SAVSR_REQUIRE(h >= 2 && w >= 2, "savsr_pack_frames: LR frame %dx%d too small for reflect padding", h, w);
+  SAVSR_REQUIRE(t >= 1 && 3 * t <= kC, "%s: %d frames do not fit 64 channels", name, t);
+  SAVSR_REQUIRE(h >= 2 && w >= 2, "%s: LR frame %dx%d too small for reflect padding", name, h, w);
   SAVSR_REQUIRE(arena->height == h + (h & 1) && arena->width == w + (w & 1),
-                "savsr_pack_frames: arena %dx%d is not the even-padded size of %dx%d", arena->height, arena->width, h, w);
-  SAVSR_REQUIRE(dst_slot >= 0 && dst_slot < arena->nslots, "savsr_pack_frames: slot %d out of range", dst_slot);
+                "%s: arena %dx%d is not the even-padded size of %dx%d", name, arena->height, arena->width, h, w);
+  SAVSR_REQUIRE(dst_slot >= 0 && dst_slot < arena->nslots, "%s: slot %d out of range", name, dst_slot);
   if (arena->batch == 0) return 0;
   const long npix = static_cast<long>(arena->height) * arena->width;
   const long total = arena->batch * npix * 8;
   const int blocks = static_cast<int>((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096);
-  pack_frames_kernel<<<blocks, 256, 0, static_cast<cudaStream_t>(st)>>>(x, arena->base + static_cast<long>(dst_slot) * arena->batch * npix * kC,
-                                                                       arena->batch, t, h, w, arena->height, arena->width, ctx->fmt);
+  pack_frames_kernel<T><<<blocks, 256, 0, static_cast<cudaStream_t>(st)>>>(x, arena->base + static_cast<long>(dst_slot) * arena->batch * npix * kC,
+                                                                          arena->batch, t, h, w, arena->height, arena->width, ctx->fmt);
   SAVSR_CUDA(cudaGetLastError());
   return 0;
+}
+
+extern "C" int savsr_pack_frames(savsr_ctx* ctx, savsr_arena* arena, const float* x, int t, int h, int w, int dst_slot, savsr_stream st) {
+  return pack_frames("savsr_pack_frames", ctx, arena, x, t, h, w, dst_slot, st);
+}
+
+extern "C" int savsr_pack_frames_u8(savsr_ctx* ctx, savsr_arena* arena, const uint8_t* x, int t, int h, int w, int dst_slot, savsr_stream st) {
+  return pack_frames("savsr_pack_frames_u8", ctx, arena, x, t, h, w, dst_slot, st);
 }
 
 namespace savsr {

@@ -25,6 +25,7 @@ import torch
 from . import _capi as K
 
 BN_EPS = 1e-5
+IO_MODES = ("f32", "bgr_u8")
 
 
 def normalize_scale(scale) -> Tuple[float, float]:
@@ -159,15 +160,22 @@ def satu_hr_pack(parts, fmt: int, device: torch.device) -> torch.Tensor:
 
 
 class Plan:
+    """I/O modes (`io`): "f32" stages the module's forward contract, x fp32 [B,7,3,h,w] RGB in [0, 1] -> out fp32 [B,3,H,W];
+    "bgr_u8" stages decoded 8-bit video, x uint8 [B,7,h,w,3] BGR -> out uint8 [B,H,W,3] BGR, the image tensor2img makes of the
+    fp32 output of x / 255.  The two modes differ only in their first and last launch (savsr_pack_frames[_u8], savsr_satu_hr[_u8])."""
+    io = "f32"
+
     def __init__(self, params: Dict[str, torch.Tensor], batch: int, h: int, w: int, scale, device: torch.device,
                  conv_impl: str = "tap", num_frame: int = 7, taps: Optional[Sequence[str]] = None, precision: str = "bf16",
-                 store: Optional[WeightStore] = None):
+                 store: Optional[WeightStore] = None, io: str = "f32"):
         if device.type != "cuda":
             raise K.SavsrError("savsr_b200 runs on CUDA (sm_100a) only; there is no CPU fallback")
         if num_frame != 7:
             raise NotImplementedError("only the shipped 7-frame configuration is implemented")
         if h < 2 or w < 2:
             raise ValueError(f"LR frames must be at least 2x2, got {h}x{w}")
+        if io not in IO_MODES:
+            raise ValueError(f"io must be one of {IO_MODES}, got {io!r}")
         self.device = device
         self.ctx = context(device.index if device.index is not None else torch.cuda.current_device())
         self.lib = self.ctx.lib
@@ -175,6 +183,7 @@ class Plan:
         if precision not in K.FMT_NAMES:
             raise ValueError(f"precision must be one of {sorted(K.FMT_NAMES)}, got {precision!r}")
         self.fmt = K.FMT_NAMES[precision]
+        self.io = io
         self.B, self.h, self.w, self.t = batch, h, w, num_frame
         self.scale = normalize_scale(scale)
         self.hp, self.wp = h + (h & 1), w + (w & 1)
@@ -199,8 +208,9 @@ class Plan:
             self._build()
             if self.cplan is not None:
                 if self._recorded == len(self.ops):
-                    K.check(self.lib.savsr_plan_set_io(self.cplan.handle, self.x_in.data_ptr(), self.x_in.numel() * 4, self.out.data_ptr(),
-                                                       self.out.numel() * 4, self.fmt))
+                    set_io = self.lib.savsr_plan_set_io_u8 if self.io == "bgr_u8" else self.lib.savsr_plan_set_io
+                    K.check(set_io(self.cplan.handle, self.x_in.data_ptr(), self.x_in.numel() * self.x_in.element_size(), self.out.data_ptr(),
+                                   self.out.numel() * self.out.element_size(), self.fmt))
                 else:
                     self.cplan = None                       # an op without a C-side record: keep the Python loop
 
@@ -401,14 +411,22 @@ class Plan:
         self.arena_lr_t.zero_()                  # the zero slot must be zero; the rest so that activation_absmax never reads stale memory
         self.lr = K.Arena(self.ctx, self.arena_lr_t.data_ptr(), self.n_lr_slots, B, self.hp, self.wp)
         lr = self.lr
-        self.x_in = self._buf(B, t, 3, self.h, self.w)
-        self.out = self._buf(B, 3, self.H, self.W)
+        u8 = self.io == "bgr_u8"
+        if u8:
+            self.x_in = self._buf(B, t, self.h, self.w, 3, dtype=torch.uint8)
+            self.out = self._buf(B, self.H, self.W, 3, dtype=torch.uint8)
+        else:
+            self.x_in = self._buf(B, t, 3, self.h, self.w)
+            self.out = self._buf(B, 3, self.H, self.W)
         xin = self.x_in.data_ptr()
+        sfx = "_u8" if u8 else ""               # the I/O mode picks the first and the last launch; everything between is shared
+        pack_frames, add_pack_frames = getattr(lib, "savsr_pack_frames" + sfx), getattr(lib, "savsr_plan_add_pack_frames" + sfx)
+        satu_hr, add_satu_hr = getattr(lib, "savsr_satu_hr" + sfx), getattr(lib, "savsr_plan_add_satu_hr" + sfx)
 
         # ---- 1. bi-directional propagation (savsr_arch.py:703-719), both directions per launch
         lrh0, hh0, ww0 = lr.handle, self.h, self.w
-        self._emit(lambda st: lib.savsr_pack_frames(ctx, lrh0, xin, t, hh0, ww0, FR, st), kind="pack_frames",
-                   rec=lambda cp: lib.savsr_plan_add_pack_frames(cp, lrh0, xin, t, hh0, ww0, FR))
+        self._emit(lambda st: pack_frames(ctx, lrh0, xin, t, hh0, ww0, FR, st), kind="pack_frames",
+                   rec=lambda cp: add_pack_frames(cp, lrh0, xin, t, hh0, ww0, FR))
         hpast = [zero, zero]
         for idx in range(n_it):
             centre = [t - 1 - 1 - idx, idx + 1]                     # f2p walks back, p2f forward
@@ -570,9 +588,9 @@ class Plan:
         tb = self._ptr("tail.bias")
         hwp, outp, cen = hw.data_ptr(), self.out.data_ptr(), t // 2
         hr_flops = 2.0 * B * self.H * self.W * (64 * 32 + 32 * 64 + 128 * 64 + 64 * 3 * 9)      # compress, expand, fusion, tail (reference counts)
-        self._emit(lambda st: lib.savsr_satu_hr(ctx, lrh, TR, STA, hh, ww, H, W, tab, by, bx, hwp, zb, tb, xin, t, cen, outp, st),
+        self._emit(lambda st: satu_hr(ctx, lrh, TR, STA, hh, ww, H, W, tab, by, bx, hwp, zb, tb, xin, t, cen, outp, st),
                    kind="satu_hr", flops=hr_flops,
-                   rec=lambda cp: lib.savsr_plan_add_satu_hr(cp, lrh, TR, STA, hh, ww, H, W, tab, by, bx, hwp, zb, tb, xin, t, cen, outp))
+                   rec=lambda cp: add_satu_hr(cp, lrh, TR, STA, hh, ww, H, W, tab, by, bx, hwp, zb, tb, xin, t, cen, outp))
         # declared traffic beyond the compulsory SATU bytes (per sample): only the 16-bit sta intermediate (written by kconv_sta, read here)
         self.satu_extra_bytes_per_sample = 2 * 64 * self.hp * self.wp * 2
         self._stream().synchronize()
@@ -670,8 +688,8 @@ class Plan:
             self.graph.replay()
 
     def forward_into(self, x: torch.Tensor, out: torch.Tensor, graph: bool = True) -> None:
-        """x [B,7,3,h,w] fp32 -> out [B,3,H,W] fp32 through the plan's staging buffers (graph replay reads / writes fixed
-        addresses), all on the device's current stream."""
+        """x -> out through the plan's staging buffers (graph replay reads / writes fixed addresses), all on the device's current
+        stream: fp32 [B,7,3,h,w] -> [B,3,H,W], or with io="bgr_u8" uint8 [B,7,h,w,3] -> [B,H,W,3]."""
         with torch.cuda.device(self.device):
             self.x_in.copy_(x, non_blocking=True)
             if graph:
@@ -689,16 +707,19 @@ class Plan:
             return peak if peak == peak else float("inf")                                                          # NaN counts as overflow
 
     def forward_c(self, x: torch.Tensor, out: torch.Tensor) -> None:
-        """x [B,7,3,h,w] fp32 -> out [B,3,H,W] fp32 through ONE C call (savsr_forward: staging copies + the recorded launch list), eagerly on the
-        device's current stream -- what a non-Python host would call."""
+        """x -> out through ONE C call (savsr_forward, or savsr_forward_u8 for io="bgr_u8": staging copies + the recorded launch list),
+        eagerly on the device's current stream -- what a non-Python host would call.  Shapes and dtypes as in forward_into."""
         if self.cplan is None:
             raise K.SavsrError("this plan has no C-side launch list")
-        if not (x.is_cuda and out.is_cuda and x.is_contiguous() and out.is_contiguous() and x.dtype == out.dtype == torch.float32):
-            raise ValueError("savsr_forward takes contiguous fp32 CUDA tensors")
+        u8 = self.io == "bgr_u8"
+        dt = torch.uint8 if u8 else torch.float32
+        if not (x.is_cuda and out.is_cuda and x.is_contiguous() and out.is_contiguous() and x.dtype == out.dtype == dt):
+            raise ValueError(f"savsr_forward{'_u8' if u8 else ''} takes contiguous {'uint8' if u8 else 'fp32'} CUDA tensors")
         if tuple(x.shape) != tuple(self.x_in.shape) or tuple(out.shape) != tuple(self.out.shape):
             raise ValueError(f"plan built for {tuple(self.x_in.shape)} -> {tuple(self.out.shape)}, got {tuple(x.shape)} -> {tuple(out.shape)}")
+        fwd = self.lib.savsr_forward_u8 if u8 else self.lib.savsr_forward
         with torch.cuda.device(self.device):
-            K.check(self.lib.savsr_forward(self.cplan.handle, x.data_ptr(), out.data_ptr(), self._stream().cuda_stream))
+            K.check(fwd(self.cplan.handle, x.data_ptr(), out.data_ptr(), self._stream().cuda_stream))
 
     def release(self) -> None:
         """Drop the CUDA graph and every device buffer now (plan-cache eviction), instead of waiting for the collector."""

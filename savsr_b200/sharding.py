@@ -58,7 +58,8 @@ def _window_index(T: int, frames: Sequence[int], num_frames: int, device: torch.
 
 
 def gather_windows(clip: torch.Tensor, frames: Sequence[int], num_frames: int = 7) -> torch.Tensor:
-    """clip [T, 3, h, w] -> windows [len(frames), num_frames, 3, h, w] (temporal halo = duplicated input)."""
+    """clip [T, ...] -> windows [len(frames), num_frames, ...] (temporal halo = duplicated input): fp32 [T, 3, h, w] planes for
+    SAVSR.forward, or uint8 [T, h, w, 3] BGR frames for SAVSR.forward_bgr_u8."""
     idx = _window_index(clip.shape[0], frames, num_frames, clip.device)
     return clip.index_select(0, idx).reshape(len(frames), num_frames, *clip.shape[1:])
 
@@ -83,7 +84,8 @@ def infer_clip(net: Callable[[torch.Tensor], torch.Tensor], clip: torch.Tensor, 
                batch=1, num_frames: int = 7, out: Optional[torch.Tensor] = None, copy_stream: Optional["torch.cuda.Stream"] = None,
                join: bool = True) -> torch.Tensor:
     """Run `net` on the windows of `frames` (default: all), `batch` windows per forward (int or a schedule, see batch_schedule).
-    Returns [len(frames), 3, H, W].  The last, ragged batch is run at its own size.
+    Returns [len(frames), ...] of whatever `net` returns per window: [n, 3, H, W] fp32 for SAVSR (clip [T, 3, h, w] fp32), or
+    [n, H, W, 3] uint8 BGR for SAVSR.forward_bgr_u8 (clip [T, h, w, 3] uint8).  The last, ragged batch is run at its own size.
     If `out` (e.g. a pinned host tensor) is given, each batch is copied into it on a side stream while the next
     batch computes, and `out` is returned once all copies are enqueued behind the current stream.
     `copy_stream` / `join=False`: for a stream of clips -- the caller owns ONE copy stream, the compute stream does not wait for the copies
@@ -116,7 +118,7 @@ def infer_clip(net: Callable[[torch.Tensor], torch.Tensor], clip: torch.Tensor, 
 def gather_outputs(local: torch.Tensor, n_frames: int, rank: int, world_size: int, dst: Optional[int] = 0,
                    contiguous: bool = False, group=None, out: Optional[torch.Tensor] = None,
                    async_op: bool = False):
-    """Collect per-rank results [n_local, ...] (frames owned per `shard_frames(n_frames, rank, world_size, contiguous)`) into
+    """Collect per-rank results [n_local, ...] of any dtype (frames owned per `shard_frames(n_frames, rank, world_size, contiguous)`) into
     clip order [n_frames, ...].  One pre-sized collective, no pickled metadata: every rank derives every other rank's frame
     list from the same deterministic `shard_frames`, so only payload travels.
 
