@@ -167,6 +167,20 @@ int savsr_pack_frames(savsr_ctx* ctx, savsr_arena* arena, const float* x, int t,
  */
 int savsr_pack_frames_u8(savsr_ctx* ctx, savsr_arena* arena, const uint8_t* x, int t, int h, int w, int dst_slot,
                          savsr_stream st);
+/*
+ * The same from a frame table: frames is a DEVICE array const uint8_t* [batch][t] (savsr_write_frame_table), and entry n * t + f points
+ * at frame f of sample n, one contiguous uint8 [h][w][3] BGR frame.  The slot is bit-identical to savsr_pack_frames_u8 of the window
+ * those frames would form.  Frames may repeat and may lie anywhere on the context's device (a ring of decoded frames, read in place).
+ * Ownership: the table and every frame it points at must stay valid, in stream order, until the launch that reads them has run.
+ */
+int savsr_pack_frames_u8_table(savsr_ctx* ctx, savsr_arena* arena, const uint8_t* const* frames, int t, int h, int w, int dst_slot,
+                               savsr_stream st);
+/*
+ * Frame table writer: table_dev[i] = ptrs_host[i] for i < n, on stream st.  The pointers travel in the launches' by-value arguments
+ * (448 per launch, more launches above that), never through a host-to-device copy, so the call returns at once and can be enqueued
+ * in stream order in front of a graph replay that reads the table.  Refuses a null entry before any launch.
+ */
+int savsr_write_frame_table(savsr_ctx* ctx, const uint8_t** table_dev, const uint8_t* const* ptrs_host, int n, savsr_stream st);
 
 /* ---- backward of the 3x3 convolution (next row 8f1: training step, lbasicsr/models/sr_model.py:101-128) ----------------------
  * Data gradient: a 3x3 convolution of dY with the transposed, spatially flipped filter -- call savsr_conv with those weights
@@ -443,6 +457,11 @@ int savsr_satu_hr_u8(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, 
                      const float* table, const float* base_y, const float* base_x, const void* weights,
                      const float* zbias, const float* tail_bias, const uint8_t* x_in, int t, int centre, uint8_t* out,
                      savsr_stream st);
+/* The same with the skip read from the frame table given to savsr_pack_frames_u8_table (entry n * t + centre); same ownership rule. */
+int savsr_satu_hr_u8_table(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
+                           const float* table, const float* base_y, const float* base_x, const void* weights,
+                           const float* zbias, const float* tail_bias, const uint8_t* const* frames, int t, int centre, uint8_t* out,
+                           savsr_stream st);
 
 /* ---- the forward as one call -----------------------------------------------------------------------------------------------------
  * savsr_plan = an ordered list of recorded launches of the entry points above (argument structures copied at record time), replayed on
@@ -459,8 +478,12 @@ int savsr_plan_set_io(savsr_plan* plan, float* x_in, size_t x_bytes, float* out,
 /* 8-bit I/O: x_in uint8 BGR [batch][7][h][w][3], out uint8 BGR [batch][H][W][3] (the plan records savsr_pack_frames_u8 and
  * savsr_satu_hr_u8 on them).  A plan has one I/O mode, set by whichever of the two set_io calls came last. */
 int savsr_plan_set_io_u8(savsr_plan* plan, uint8_t* x_in, size_t x_bytes, uint8_t* out, size_t out_bytes, int format);
+/* 8-bit I/O from a frame table: table_dev is the device array of `entries` = batch * 7 frame pointers that the plan's
+ * savsr_pack_frames_u8_table and savsr_satu_hr_u8_table launches read, out uint8 BGR [batch][H][W][3].  A third I/O mode. */
+int savsr_plan_set_io_u8_table(savsr_plan* plan, const uint8_t** table_dev, int entries, uint8_t* out, size_t out_bytes, int format);
 int savsr_plan_add_pack_frames(savsr_plan* plan, savsr_arena* arena, const float* x, int t, int h, int w, int dst_slot);
 int savsr_plan_add_pack_frames_u8(savsr_plan* plan, savsr_arena* arena, const uint8_t* x, int t, int h, int w, int dst_slot);
+int savsr_plan_add_pack_frames_u8_table(savsr_plan* plan, savsr_arena* arena, const uint8_t* const* frames, int t, int h, int w, int dst_slot);
 int savsr_plan_add_conv(savsr_plan* plan, savsr_arena* arena, const savsr_conv_group* groups, int ngroups, int ksize, int n_tile,
                         int dst_mode, int impl);
 int savsr_plan_add_osa_prologue(savsr_plan* plan, const savsr_osa_params* convs, int nconvs, int batch, int npart, int npix,
@@ -477,6 +500,9 @@ int savsr_plan_add_satu_hr(savsr_plan* plan, savsr_arena* lr, int x_slot, int st
 int savsr_plan_add_satu_hr_u8(savsr_plan* plan, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W, const float* table,
                               const float* base_y, const float* base_x, const void* weights, const float* zbias, const float* tail_bias,
                               const uint8_t* x_in, int t, int centre, uint8_t* out);
+int savsr_plan_add_satu_hr_u8_table(savsr_plan* plan, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W, const float* table,
+                                    const float* base_y, const float* base_x, const void* weights, const float* zbias, const float* tail_bias,
+                                    const uint8_t* const* frames, int t, int centre, uint8_t* out);
 int savsr_plan_add_arena_export(savsr_plan* plan, savsr_arena* arena, int slot, float* nchw);   /* debug taps */
 int savsr_plan_run(savsr_plan* plan, savsr_stream st);
 /* x -> the plan's input staging buffer (device-to-device, skipped when x IS that buffer), replay, output staging buffer -> out. */
@@ -484,6 +510,12 @@ int savsr_forward(savsr_plan* plan, const float* x, float* out, savsr_stream st)
 /* The same for a plan with 8-bit I/O (savsr_plan_set_io_u8): x uint8 BGR [batch][7][h][w][3] -> out uint8 BGR [batch][H][W][3].
  * Each of savsr_forward / savsr_forward_u8 returns an error, before any copy or launch, on a plan of the other I/O mode. */
 int savsr_forward_u8(savsr_plan* plan, const uint8_t* x, uint8_t* out, savsr_stream st);
+/* The same for a plan with frame-table I/O (savsr_plan_set_io_u8_table): ptrs_host holds batch * 7 DEVICE frame pointers, window n =
+ * entries 7n .. 7n + 6, each one contiguous uint8 BGR [h][w][3] frame.  Writes the table (savsr_write_frame_table), replays, and copies
+ * the output staging buffer to out uint8 BGR [batch][H][W][3].  The host array may be reused when the call returns; the frames must stay
+ * valid, in stream order, until this forward has run.  Returns an error, before any launch, on a plan of another I/O mode, and
+ * savsr_forward / savsr_forward_u8 refuse a frame-table plan. */
+int savsr_forward_u8_frames(savsr_plan* plan, const uint8_t* const* ptrs_host, uint8_t* out, savsr_stream st);
 
 /* ---- post-processing / metrics on the device (next row 8f3) -------------------------------------------------------
  * tensor2img (lbasicsr/utils/img_util.py:38-94): sr fp32 NCHW [batch][3][H][W] RGB -> uint8 HWC BGR [batch][H][W][3]

@@ -18,7 +18,7 @@ from __future__ import annotations
 import math
 import os
 from collections import OrderedDict
-from typing import Dict, Tuple, Union
+from typing import Dict, Optional, Tuple, Union
 
 import torch
 import torch.nn as nn
@@ -254,10 +254,52 @@ class SAVSR(nn.Module):
             return x.new_empty((0, *engine.get_hw(h, w, self.scale), 3))
         return self._run_plan(self.plan_for(x, io="bgr_u8"), x)
 
-    def _run_plan(self, plan: engine.Plan, x: torch.Tensor) -> torch.Tensor:
+    def forward_bgr_u8_indexed(self, pool: torch.Tensor, windows, scale=None) -> torch.Tensor:
+        """forward_bgr_u8(pool[windows]), bit for bit, without gathering the windows: pool is a uint8 CUDA tensor [N, h, w, 3] whose
+        rows are BGR frames (a clip, or a ring of decoded frames), windows a host sequence or CPU integer tensor [b, 7] of row
+        indices (any order, repeats allowed).  Each forward reads its frames in place through a device table of frame addresses,
+        so every frame is read once per window instead of being copied 7 times.  Returns a fresh uint8 [b, H, W, 3] BGR tensor.
+        The pool is read on the device's current stream: it must stay valid, in stream order, until the forward has run."""
+        if scale is not None:
+            self.scale = scale
+        return self._forward_bgr_u8_indexed(pool, windows, self.scale)
+
+    def _forward_bgr_u8_indexed(self, pool: torch.Tensor, windows, scale) -> torch.Tensor:
+        """forward_bgr_u8_indexed at `scale`, leaving self.scale as it is (savsr_b200.VideoUpscaler keeps its own scale)."""
+        if self.training:
+            raise RuntimeError("forward_bgr_u8_indexed is inference only: call eval() first (training takes fp32 windows through forward)")
+        if pool.dtype != torch.uint8:
+            raise TypeError(f"forward_bgr_u8_indexed takes a uint8 frame pool, got {pool.dtype}")
+        if pool.dim() != 4 or pool.shape[3] != 3:
+            raise ValueError(f"expected a uint8 BGR frame pool [N, h, w, 3], got {tuple(pool.shape)}")
+        if not pool.is_contiguous():
+            raise ValueError("the frame pool must be contiguous (each row one [h, w, 3] frame)")
+        idx = torch.as_tensor(windows)
+        if idx.numel() == 0 and not idx.is_cuda:
+            idx = idx.reshape(0, self.num_frame).long()
+        if idx.is_cuda or idx.is_floating_point() or idx.is_complex() or idx.dtype == torch.bool:
+            raise TypeError(f"windows must be a host sequence or CPU integer tensor of row indices, got {idx.dtype} on {idx.device}")
+        if idx.dim() != 2 or idx.shape[1] != self.num_frame:
+            raise ValueError(f"expected windows [b, {self.num_frame}] of row indices, got shape {tuple(idx.shape)}")
+        n, h, w, _ = pool.shape
+        b = idx.shape[0]
+        self._check_device(pool)
+        if b == 0:
+            return pool.new_empty((0, *engine.get_hw(h, w, scale), 3))
+        idx = idx.to(torch.int64)
+        lo, hi = int(idx.min()), int(idx.max())
+        if lo < 0 or hi >= n:
+            raise IndexError(f"window row index {lo if lo < 0 else hi} out of range for a pool of {n} frames")
+        ptrs = (idx.reshape(-1) * (h * w * 3) + pool.data_ptr()).tolist()
+        return self._run_plan(self._plan(b, h, w, pool.device, "bgr_u8_frames", scale), frames=ptrs)
+
+    def _run_plan(self, plan: engine.Plan, x: Optional[torch.Tensor] = None, frames: Optional[list] = None) -> torch.Tensor:
         with torch.cuda.device(plan.device):
             out = torch.empty_like(plan.out)
-            plan.forward_into(x, out, graph=self.use_graph)
+            if frames is None:
+                plan.forward_into(x, out, graph=self.use_graph)
+            else:
+                plan.forward_frames_into(frames, out, graph=self.use_graph)
             if self.precision == "fp16" and not plan.__dict__.get("_range_checked"):
                 # fp16 operands meet the <= 1e-3 bound but saturate at 65504: look at every trunk activation of this plan's FIRST forward
                 # (one pass over the arena, once per plan) and refuse to continue silently when the headroom is below 4x
@@ -320,22 +362,28 @@ class SAVSR(nn.Module):
             if x.dim() != 5 or x.shape[1] != self.num_frame or x.shape[2] != 3:
                 raise ValueError(f"expected input [b, {self.num_frame}, 3, h, w], got {tuple(x.shape)}")
             b, _, _, h, w = x.shape
+        self._check_device(x)
+        return b, h, w
+
+    def _check_device(self, x: torch.Tensor) -> None:
         if not x.is_cuda:
             raise RuntimeError("savsr_b200.SAVSR runs on CUDA (sm_100a) only; there is no CPU fallback")
         p0 = self.gamma
         if p0.device != x.device:
             raise RuntimeError(f"module parameters on {p0.device}, input on {x.device}")
-        return b, h, w
 
     def plan_for(self, x: torch.Tensor, io: str = "f32") -> engine.Plan:
         """The cached plan for windows like `x`: io="f32" takes [b, 7, 3, h, w] (forward), io="bgr_u8" uint8 [b, 7, h, w, 3]
-        (forward_bgr_u8).  Plans of both modes share one WeightStore."""
+        (forward_bgr_u8).  Plans of every I/O mode (also "bgr_u8_frames", forward_bgr_u8_indexed) share one WeightStore."""
         b, h, w = self._window_shape(x, io)
+        return self._plan(b, h, w, x.device, io, self.scale)
+
+    def _plan(self, b: int, h: int, w: int, device: torch.device, io: str, scale) -> engine.Plan:
         if self.training:
             raise RuntimeError("plans are the inference path; in train mode forward() runs savsr_b200.train.forward")
-        s = engine.normalize_scale(self.scale)
+        s = engine.normalize_scale(scale)
         wkey = self._weights_version()
-        key = (b, h, w, float(s[0]), float(s[1]), self.conv_impl, self.precision, tuple(self.debug_taps), x.device.index, io) + wkey
+        key = (b, h, w, float(s[0]), float(s[1]), self.conv_impl, self.precision, tuple(self.debug_taps), device.index, io) + wkey
         plan = self._plans.get(key)
         if plan is not None:
             self._plans.move_to_end(key)
@@ -343,8 +391,8 @@ class SAVSR(nn.Module):
         import time
         t0 = time.perf_counter()
         params = {k: v for k, v in self.state_dict(keep_vars=True).items()}
-        plan = engine.Plan(params, b, h, w, s, x.device, conv_impl=self.conv_impl, num_frame=self.num_frame,
-                           taps=self.debug_taps, precision=self.precision, store=self._store_for(x.device, wkey), io=io)
+        plan = engine.Plan(params, b, h, w, s, device, conv_impl=self.conv_impl, num_frame=self.num_frame,
+                           taps=self.debug_taps, precision=self.precision, store=self._store_for(device, wkey), io=io)
         self.last_plan_build_ms = 1e3 * (time.perf_counter() - t0)
         self._plans[key] = plan
         # bound the device memory held by cached plans (arenas + graphs): evict least recently used down to the byte budget

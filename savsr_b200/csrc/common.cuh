@@ -56,7 +56,16 @@ namespace savsr {
 enum AttrBit { kAttrIgemm = 0 /* + template index, 6 variants */, kAttrBigk = 8, kAttrKsta = 9, kAttrSatuHr = 10, kAttrOsaLinear = 11,
                kAttrFused = 12, kAttrBigk128 = 13, kAttrSatuHrBf16 = 14, kAttrWgrad = 15, kAttrWgradBatched = 16,
                kAttrOsaAssembleTrain = 17, kAttrOsaUnfoldBwd = 18, kAttrOsaChain = 19, kAttrOsaMatvec = 20 /* + 0, 1, 2: batch 8, 16, 32 */,
-               kAttrCaBackward = 23, kAttrSatuHrU8 = 24 /* + format: 8-bit I/O instantiations of satu_hr */ };
+               kAttrCaBackward = 23, kAttrSatuHrU8 = 24 /* + format: 8-bit I/O instantiations of satu_hr */,
+               kAttrSatuHrU8Table = 26 /* + format: 8-bit frame-table instantiations of satu_hr */ };
+// Input addressing of the two launches that read a forward's input (pack_frames, satu_hr's bilinear skip):
+//   kIoF32      fp32 NCHW window [batch][t][3][h][w] RGB
+//   kIoU8       uint8 window [batch][t][h][w][3] BGR
+//   kIoU8Table  frame table: device array const uint8_t* [batch][t], entry (n, f) -> one contiguous uint8 [h][w][3] BGR frame
+enum IoMode { kIoF32 = 0, kIoU8 = 1, kIoU8Table = 2 };
+// One launch of the frame-table writer carries at most this many pointers in its by-value argument (3.6 KB, under the 4 KB
+// parameter limit of older drivers); 448 = 64 windows of 7 frames.
+constexpr int kFrameTableChunk = 448;
 template <class F>
 inline int ensure_smem_attr(savsr_ctx* ctx, int bit, F func, size_t bytes) {
   if (ctx->attr_mask & (1u << bit)) return 0;
@@ -134,6 +143,10 @@ __device__ __forceinline__ float u8_to_unit(uint8_t u) {
   return __fmaf_rn(__fmaf_rn(-q, 255.0f, a), r, q);
 }
 __device__ __forceinline__ int unit_to_u8(float v) { return __float2int_rn(fminf(fmaxf(v, 0.f), 1.f) * 255.0f); }
+// Entry i of a frame table (kIoU8Table), through the read-only cache: every thread of a launch reads the same few entries.
+__device__ __forceinline__ const uint8_t* frame_at(const uint8_t* const* table, long i) {
+  return reinterpret_cast<const uint8_t*>(__ldg(reinterpret_cast<const unsigned long long*>(table) + i));
+}
 __device__ __forceinline__ float h_to_float(uint16_t raw, int fmt) { return h_lo(raw, fmt); }
 __device__ __forceinline__ uint16_t float_to_h(float x, int fmt) { return static_cast<uint16_t>(pack_h2(x, 0.f, fmt) & 0xffffu); }
 

@@ -12,11 +12,11 @@
 struct savsr_plan {
   savsr_ctx* ctx;
   std::vector<std::function<int(savsr_stream)>> ops;
-  void* x_in = nullptr;
+  void* x_in = nullptr;            // input staging buffer, or the frame table (kIoU8Table)
   void* out = nullptr;
   size_t x_bytes = 0, out_bytes = 0;
   int format = SAVSR_FMT_BF16;
-  bool u8 = false;                 // I/O mode: fp32 (savsr_forward) or uint8 BGR (savsr_forward_u8)
+  int io = savsr::kIoF32;          // I/O mode: fp32 (savsr_forward), uint8 BGR (savsr_forward_u8), frame table (savsr_forward_u8_frames)
 };
 
 using namespace savsr;
@@ -33,19 +33,25 @@ extern "C" int savsr_plan_create(savsr_ctx* ctx, savsr_plan** out) {
 extern "C" void savsr_plan_destroy(savsr_plan* plan) { delete plan; }
 extern "C" int savsr_plan_size(const savsr_plan* plan) { return plan ? static_cast<int>(plan->ops.size()) : 0; }
 
-static int set_io(const char* name, savsr_plan* plan, void* x_in, size_t x_bytes, void* out, size_t out_bytes, int format, bool u8) {
+static int set_io(const char* name, savsr_plan* plan, void* x_in, size_t x_bytes, void* out, size_t out_bytes, int format, int io) {
   SAVSR_REQUIRE(plan && x_in && out && x_bytes && out_bytes, "%s: null pointer / empty buffer", name);
   SAVSR_REQUIRE(format == SAVSR_FMT_BF16 || format == SAVSR_FMT_FP16, "%s: unknown format %d", name, format);
-  plan->x_in = x_in; plan->x_bytes = x_bytes; plan->out = out; plan->out_bytes = out_bytes; plan->format = format; plan->u8 = u8;
+  plan->x_in = x_in; plan->x_bytes = x_bytes; plan->out = out; plan->out_bytes = out_bytes; plan->format = format; plan->io = io;
   return 0;
 }
 
 extern "C" int savsr_plan_set_io(savsr_plan* plan, float* x_in, size_t x_bytes, float* out, size_t out_bytes, int format) {
-  return set_io("savsr_plan_set_io", plan, x_in, x_bytes, out, out_bytes, format, false);
+  return set_io("savsr_plan_set_io", plan, x_in, x_bytes, out, out_bytes, format, kIoF32);
 }
 
 extern "C" int savsr_plan_set_io_u8(savsr_plan* plan, uint8_t* x_in, size_t x_bytes, uint8_t* out, size_t out_bytes, int format) {
-  return set_io("savsr_plan_set_io_u8", plan, x_in, x_bytes, out, out_bytes, format, true);
+  return set_io("savsr_plan_set_io_u8", plan, x_in, x_bytes, out, out_bytes, format, kIoU8);
+}
+
+extern "C" int savsr_plan_set_io_u8_table(savsr_plan* plan, const uint8_t** table_dev, int entries, uint8_t* out, size_t out_bytes, int format) {
+  SAVSR_REQUIRE(entries >= 0, "savsr_plan_set_io_u8_table: negative entry count %d", entries);
+  return set_io("savsr_plan_set_io_u8_table", plan, const_cast<uint8_t**>(table_dev), entries * sizeof(*table_dev), out, out_bytes, format,
+                kIoU8Table);
 }
 
 extern "C" int savsr_plan_add_pack_frames(savsr_plan* plan, savsr_arena* arena, const float* x, int t, int h, int w, int dst_slot) {
@@ -59,6 +65,14 @@ extern "C" int savsr_plan_add_pack_frames_u8(savsr_plan* plan, savsr_arena* aren
   SAVSR_REQUIRE(plan && arena && x, "savsr_plan_add_pack_frames_u8: null pointer");
   savsr_ctx* ctx = plan->ctx;
   plan->ops.push_back([=](savsr_stream st) { return savsr_pack_frames_u8(ctx, arena, x, t, h, w, dst_slot, st); });
+  return 0;
+}
+
+extern "C" int savsr_plan_add_pack_frames_u8_table(savsr_plan* plan, savsr_arena* arena, const uint8_t* const* frames, int t, int h, int w,
+                                                   int dst_slot) {
+  SAVSR_REQUIRE(plan && arena && frames, "savsr_plan_add_pack_frames_u8_table: null pointer");
+  savsr_ctx* ctx = plan->ctx;
+  plan->ops.push_back([=](savsr_stream st) { return savsr_pack_frames_u8_table(ctx, arena, frames, t, h, w, dst_slot, st); });
   return 0;
 }
 
@@ -127,6 +141,19 @@ extern "C" int savsr_plan_add_satu_hr_u8(savsr_plan* plan, savsr_arena* lr, int 
   return 0;
 }
 
+extern "C" int savsr_plan_add_satu_hr_u8_table(savsr_plan* plan, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
+                                               const float* table, const float* base_y, const float* base_x, const void* weights,
+                                               const float* zbias, const float* tail_bias, const uint8_t* const* frames, int t, int centre,
+                                               uint8_t* out) {
+  SAVSR_REQUIRE(plan && lr, "savsr_plan_add_satu_hr_u8_table: null pointer");
+  savsr_ctx* ctx = plan->ctx;
+  plan->ops.push_back([=](savsr_stream st) {
+    return savsr_satu_hr_u8_table(ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias, frames, t, centre,
+                                  out, st);
+  });
+  return 0;
+}
+
 extern "C" int savsr_plan_add_arena_export(savsr_plan* plan, savsr_arena* arena, int slot, float* nchw) {
   SAVSR_REQUIRE(plan && arena && nchw, "savsr_plan_add_arena_export: null pointer");
   plan->ops.push_back([=](savsr_stream st) { return savsr_arena_export(arena, slot, nchw, st); });
@@ -143,11 +170,19 @@ extern "C" int savsr_plan_run(savsr_plan* plan, savsr_stream st) {
   return 0;
 }
 
-static int forward(const char* name, savsr_plan* plan, const void* x, void* out, bool u8, savsr_stream st) {
+// Refuses a call of the wrong I/O mode before any copy or launch.
+static int check_io(const char* name, const savsr_plan* plan, int io) {
+  static const char* const kModeName[] = {"fp32", "uint8 BGR", "uint8 BGR frame-table"};
+  static const char* const kForward[] = {"savsr_forward", "savsr_forward_u8", "savsr_forward_u8_frames"};
+  SAVSR_REQUIRE(plan->x_in && plan->out,
+                "%s: the plan has no I/O staging buffers (savsr_plan_set_io / savsr_plan_set_io_u8 / savsr_plan_set_io_u8_table)", name);
+  SAVSR_REQUIRE(plan->io == io, "%s: the plan was set up for %s I/O; call %s", name, kModeName[plan->io], kForward[plan->io]);
+  return 0;
+}
+
+static int forward(const char* name, savsr_plan* plan, const void* x, void* out, int io, savsr_stream st) {
   SAVSR_REQUIRE(plan && x && out, "%s: null pointer", name);
-  SAVSR_REQUIRE(plan->x_in && plan->out, "%s: the plan has no I/O staging buffers (savsr_plan_set_io / savsr_plan_set_io_u8)", name);
-  SAVSR_REQUIRE(plan->u8 == u8, "%s: the plan was set up for %s I/O; call %s", name, plan->u8 ? "uint8 BGR" : "fp32",
-                plan->u8 ? "savsr_forward_u8" : "savsr_forward");
+  if (int rc = check_io(name, plan, io)) return rc;
   DeviceGuard guard(plan->ctx->device);
   cudaStream_t s = static_cast<cudaStream_t>(st);
   if (x != plan->x_in) SAVSR_CUDA(cudaMemcpyAsync(plan->x_in, x, plan->x_bytes, cudaMemcpyDeviceToDevice, s));
@@ -157,9 +192,20 @@ static int forward(const char* name, savsr_plan* plan, const void* x, void* out,
 }
 
 extern "C" int savsr_forward(savsr_plan* plan, const float* x, float* out, savsr_stream st) {
-  return forward("savsr_forward", plan, x, out, false, st);
+  return forward("savsr_forward", plan, x, out, kIoF32, st);
 }
 
 extern "C" int savsr_forward_u8(savsr_plan* plan, const uint8_t* x, uint8_t* out, savsr_stream st) {
-  return forward("savsr_forward_u8", plan, x, out, true, st);
+  return forward("savsr_forward_u8", plan, x, out, kIoU8, st);
+}
+
+extern "C" int savsr_forward_u8_frames(savsr_plan* plan, const uint8_t* const* ptrs_host, uint8_t* out, savsr_stream st) {
+  SAVSR_REQUIRE(plan && ptrs_host && out, "savsr_forward_u8_frames: null pointer");
+  if (int rc = check_io("savsr_forward_u8_frames", plan, kIoU8Table)) return rc;
+  DeviceGuard guard(plan->ctx->device);
+  const int entries = static_cast<int>(plan->x_bytes / sizeof(const uint8_t*));
+  if (int rc = savsr_write_frame_table(plan->ctx, static_cast<const uint8_t**>(plan->x_in), ptrs_host, entries, st)) return rc;
+  if (int rc = savsr_plan_run(plan, st)) return rc;
+  if (out != plan->out) SAVSR_CUDA(cudaMemcpyAsync(out, plan->out, plan->out_bytes, cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(st)));
+  return 0;
 }

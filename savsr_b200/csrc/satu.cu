@@ -343,9 +343,10 @@ __device__ __forceinline__ int swz(int r, int c) { return r * 128 + ((c ^ (r & 7
 //                          0..7   consumers, two groups alternating tiles: routing (U -> V tile), Z -> smem, and, once per
 //                                 block and sample, the 9-tap sum + bias + bilinear skip -> fp32 NCHW stores (128 B per warp row)
 //
-// I/O modes (template U8): fp32 (the module's forward contract) reads the skip from the fp32 window and stores fp32 NCHW; 8-bit reads it
-// from the uint8 BGR window [batch][t][h][w][3] through the same u / 255 as the first layer, so the skip is the same fp32 number, and
-// stores tensor2img's uint8 HWC BGR [batch][H][W][3] of the same fp32 value the fp32 mode would have written.
+// I/O modes (template IO, enum IoMode): fp32 (the module's forward contract) reads the skip from the fp32 window and stores fp32 NCHW;
+// 8-bit reads it from the uint8 BGR window [batch][t][h][w][3], or from the centre frame's entry of a frame table, through the same
+// u / 255 as the first layer, so the skip is the same fp32 number, and stores tensor2img's uint8 HWC BGR [batch][H][W][3] of the same
+// fp32 value the fp32 mode would have written.
 struct HrParams {
   const __nv_bfloat16* lr;
   const float* table;        // [H*W][8]: offset x,y | st_offset x,y | r0..r3
@@ -354,7 +355,8 @@ struct HrParams {
   const uint8_t* weights;    // 4 x [32 rows][128 B] K-major swizzled: Wc (rows e*8+k) | Wcf | Wcs | Wv (K = 32), rows of Wcf/Wcs/Wv = tap*3+c
   const float* zbias;        // [32]: zb[tap*3+c], 27 used
   const float* tail_bias;    // [3]
-  const void* x_in;          // bilinear skip of the centre frame: fp32 [batch][t][3][h][w], or uint8 BGR [batch][t][h][w][3]
+  const void* x_in;          // bilinear skip of the centre frame: fp32 [batch][t][3][h][w], uint8 BGR [batch][t][h][w][3], or the
+                             // frame table const uint8_t* [batch][t]
   void* out;                 // fp32 [batch][3][H][W], or uint8 BGR [batch][H][W][3]
   int batch, hp, wp, h, w, H, W;
   int x_slot, sta_slot;
@@ -428,7 +430,7 @@ __device__ __forceinline__ void bilinear_src_scaled(int dst, float scale, int in
   l1 = src - static_cast<float>(i0);
 }
 
-template <int FMT, bool U8>
+template <int FMT, int IO>
 __global__ void __launch_bounds__(kHrThreads, 1) satu_hr_kernel(const __grid_constant__ HrParams p) {
   extern __shared__ uint8_t raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(raw) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -493,14 +495,16 @@ __global__ void __launch_bounds__(kHrThreads, 1) satu_hr_kernel(const __grid_con
           float ly, lx;
           bilinear_src_scaled(Y, sk_sy, p.h, y0, y1, ly);
           bilinear_src_scaled(X, sk_sx, p.w, x0, x1, lx);
-          const long xc = static_cast<long>(n * p.t + p.centre) * 3 * plane;   // centre frame of sample n (elements, either layout)
+          const long xc = static_cast<long>(n * p.t + p.centre) * 3 * plane;   // centre frame of sample n (elements, either window layout)
+          const uint8_t* fc = nullptr;
+          if constexpr (IO == kIoU8Table) fc = frame_at(static_cast<const uint8_t* const*>(p.x_in), n * p.t + p.centre);
           const int o00 = y0 * p.w + x0, o01 = y0 * p.w + x1, o10 = y1 * p.w + x0, o11 = y1 * p.w + x1;
           float sk[3];
 #pragma unroll
           for (int ch = 0; ch < 3; ++ch) {
             float a, bb, cc, d;
-            if constexpr (U8) {
-              const uint8_t* pl = static_cast<const uint8_t*>(p.x_in) + xc + 2 - ch;
+            if constexpr (IO != kIoF32) {
+              const uint8_t* pl = (IO == kIoU8Table ? fc : static_cast<const uint8_t*>(p.x_in) + xc) + 2 - ch;
               a = u8_to_unit(__ldg(pl + 3 * o00)); bb = u8_to_unit(__ldg(pl + 3 * o01));
               cc = u8_to_unit(__ldg(pl + 3 * o10)); d = u8_to_unit(__ldg(pl + 3 * o11));
             } else {
@@ -522,7 +526,7 @@ __global__ void __launch_bounds__(kHrThreads, 1) satu_hr_kernel(const __grid_con
               acc2 += v ? __half2float(z[2 * kHrPix]) : 0.f;
             }
           }
-          if constexpr (U8) {
+          if constexpr (IO != kIoF32) {
             // 3 bytes per pixel: W * 3 has any alignment, so plain byte stores (a warp row is 96 contiguous bytes)
             uint8_t* o = static_cast<uint8_t*>(p.out) + (static_cast<long>(n) * NPIX + static_cast<long>(Y) * p.W + X) * 3;
             o[0] = static_cast<uint8_t>(unit_to_u8(acc2 + sk[2])); o[1] = static_cast<uint8_t>(unit_to_u8(acc1 + sk[1]));
@@ -774,7 +778,7 @@ extern "C" int savsr_satu_kconv_sta(savsr_ctx* ctx, savsr_arena* arena, int a_sl
   return 0;
 }
 
-template <bool U8>
+template <int IO>
 static int satu_hr(const char* name, savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W, const float* table,
                    const float* base_y, const float* base_x, const void* weights, const float* zbias, const float* tail_bias,
                    const void* x_in, int t, int centre, void* out, savsr_stream st) {
@@ -786,8 +790,10 @@ static int satu_hr(const char* name, savsr_ctx* ctx, savsr_arena* lr, int x_slot
   SAVSR_REQUIRE(H >= 1 && W >= 1 && t >= 1 && centre >= 0 && centre < t, "%s: bad HR size %dx%d or window (%d, %d)", name, H, W, t, centre);
   if (lr->batch == 0) return 0;
   const bool fp16 = ctx->fmt == SAVSR_FMT_FP16;
-  auto kernel = fp16 ? satu_hr_kernel<SAVSR_FMT_FP16, U8> : satu_hr_kernel<SAVSR_FMT_BF16, U8>;
-  const int bit = U8 ? kAttrSatuHrU8 + (fp16 ? 1 : 0) : (fp16 ? kAttrSatuHr : kAttrSatuHrBf16);
+  auto kernel = fp16 ? satu_hr_kernel<SAVSR_FMT_FP16, IO> : satu_hr_kernel<SAVSR_FMT_BF16, IO>;
+  const int bit = IO == kIoU8Table ? kAttrSatuHrU8Table + (fp16 ? 1 : 0)
+                : IO == kIoU8      ? kAttrSatuHrU8 + (fp16 ? 1 : 0)
+                                   : (fp16 ? kAttrSatuHr : kAttrSatuHrBf16);
   if (int rc = ensure_smem_attr(ctx, bit, kernel, kHrSmem)) return rc;
   HrParams p;
   p.lr = lr->base; p.table = table; p.base_y = base_y; p.base_x = base_x;
@@ -806,14 +812,22 @@ extern "C" int savsr_satu_hr(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int st
                              const float* table, const float* base_y, const float* base_x, const void* weights,
                              const float* zbias, const float* tail_bias, const float* x_in, int t, int centre, float* out,
                              savsr_stream st) {
-  return satu_hr<false>("savsr_satu_hr", ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias, x_in, t,
-                        centre, out, st);
+  return satu_hr<kIoF32>("savsr_satu_hr", ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias, x_in, t,
+                         centre, out, st);
 }
 
 extern "C" int savsr_satu_hr_u8(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
                                 const float* table, const float* base_y, const float* base_x, const void* weights,
                                 const float* zbias, const float* tail_bias, const uint8_t* x_in, int t, int centre, uint8_t* out,
                                 savsr_stream st) {
-  return satu_hr<true>("savsr_satu_hr_u8", ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias, x_in, t,
-                       centre, out, st);
+  return satu_hr<kIoU8>("savsr_satu_hr_u8", ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias, x_in, t,
+                        centre, out, st);
+}
+
+extern "C" int savsr_satu_hr_u8_table(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
+                                      const float* table, const float* base_y, const float* base_x, const void* weights,
+                                      const float* zbias, const float* tail_bias, const uint8_t* const* frames, int t, int centre,
+                                      uint8_t* out, savsr_stream st) {
+  return satu_hr<kIoU8Table>("savsr_satu_hr_u8_table", ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias,
+                             frames, t, centre, out, st);
 }

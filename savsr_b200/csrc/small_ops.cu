@@ -2,6 +2,8 @@
 // the OSA-Conv prologue (pool -> scale_routing MLP -> ScaleAttention -> per-sample kernel assembly),
 // RCAB channel attention, and the OSAdapt mask tail.  All HBM/L2-bound or latency-bound by nature;
 // they use coalesced 128-bit accesses and keep weights in shared memory.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace savsr {
@@ -10,7 +12,8 @@ namespace savsr {
 // The input window -> one bf16 arena slot whose channels 0..3t-1 are the frames' RGB planes (channel 3f + c), the rest zero,
 // reflect-padded to the even arena size (savsr_arch.py:670-690).  With this slot the first-layer convs (conv_c / conv_sup,
 // savsr_arch.py:456-457) run on the tensor-core kernel with zero-expanded weights.  T = float: fp32 NCHW window [B][t][3][h][w] RGB;
-// T = uint8_t: the decoded 8-bit window [B][t][h][w][3] BGR, converted exactly as the reference's img.astype(np.float32) / 255.
+// T = uint8_t: the decoded 8-bit window [B][t][h][w][3] BGR, converted exactly as the reference's img.astype(np.float32) / 255.;
+// T = const uint8_t*: a frame table (x[n * t + f] -> frame f of sample n, [h][w][3] BGR), read through the same conversion.
 template <class T>
 __global__ void __launch_bounds__(256) pack_frames_kernel(const T* __restrict__ x, __nv_bfloat16* __restrict__ dst, int batch,
                                                           int t, int h, int w, int hp, int wp, int fmt) {
@@ -27,7 +30,10 @@ __global__ void __launch_bounds__(256) pack_frames_kernel(const T* __restrict__ 
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
       const int ch = chunk * 8 + e;
-      if constexpr (sizeof(T) == 1) {
+      if constexpr (std::is_pointer<T>::value) {
+        const int f = ch / 3, c = ch - 3 * f;
+        v[e] = ch < 3 * t ? u8_to_unit(__ldg(frame_at(x, static_cast<long>(n) * t + f) + (static_cast<long>(ry) * w + rx) * 3 + 2 - c)) : 0.f;
+      } else if constexpr (sizeof(T) == 1) {
         const int f = ch / 3, c = ch - 3 * f;
         v[e] = ch < 3 * t ? u8_to_unit(__ldg(x + ((static_cast<long>(n) * t + f) * h + ry) * w * 3 + rx * 3 + 2 - c)) : 0.f;
       } else {
@@ -569,6 +575,36 @@ extern "C" int savsr_pack_frames(savsr_ctx* ctx, savsr_arena* arena, const float
 
 extern "C" int savsr_pack_frames_u8(savsr_ctx* ctx, savsr_arena* arena, const uint8_t* x, int t, int h, int w, int dst_slot, savsr_stream st) {
   return pack_frames("savsr_pack_frames_u8", ctx, arena, x, t, h, w, dst_slot, st);
+}
+
+extern "C" int savsr_pack_frames_u8_table(savsr_ctx* ctx, savsr_arena* arena, const uint8_t* const* frames, int t, int h, int w, int dst_slot,
+                                          savsr_stream st) {
+  return pack_frames("savsr_pack_frames_u8_table", ctx, arena, frames, t, h, w, dst_slot, st);
+}
+
+namespace savsr {
+// The frame table is written by kernels whose by-value argument carries the pointers, never by a host-to-device copy: a copy from
+// pageable host memory holds the host until the stream has drained, and between two forwards of a video that is an idle GPU.
+struct FrameTableChunk {
+  const uint8_t* ptrs[kFrameTableChunk];
+};
+__global__ void __launch_bounds__(kFrameTableChunk) write_frame_table_kernel(const __grid_constant__ FrameTableChunk c, const uint8_t** dst, int n) {
+  if (static_cast<int>(threadIdx.x) < n) dst[threadIdx.x] = c.ptrs[threadIdx.x];
+}
+}  // namespace savsr
+
+extern "C" int savsr_write_frame_table(savsr_ctx* ctx, const uint8_t** table_dev, const uint8_t* const* ptrs_host, int n, savsr_stream st) {
+  SAVSR_REQUIRE(ctx && table_dev && ptrs_host && n >= 0, "savsr_write_frame_table: null pointer / negative count");
+  for (int i = 0; i < n; ++i) SAVSR_REQUIRE(ptrs_host[i], "savsr_write_frame_table: frame pointer %d of %d is null", i, n);
+  DeviceGuard guard(ctx->device);
+  FrameTableChunk c = {};
+  for (int i0 = 0; i0 < n; i0 += kFrameTableChunk) {
+    const int m = n - i0 < kFrameTableChunk ? n - i0 : kFrameTableChunk;
+    memcpy(c.ptrs, ptrs_host + i0, m * sizeof(c.ptrs[0]));
+    write_frame_table_kernel<<<1, kFrameTableChunk, 0, static_cast<cudaStream_t>(st)>>>(c, table_dev + i0, m);
+    SAVSR_CUDA(cudaGetLastError());
+  }
+  return 0;
 }
 
 namespace savsr {

@@ -1,0 +1,141 @@
+"""Frame-in / frame-out upscaling of decoded 8-bit video of any length.
+
+``VideoUpscaler`` takes frames as a decoder produces them and returns HR frames in order, with the same windows, reflection and
+batch partition as ``sharding.infer_clip(net.forward_bgr_u8, clip, batch=...)`` on the whole clip, so its output is byte-identical to
+that call.  Frames are uploaded once into a device ring and read in place by ``SAVSR.forward_bgr_u8_indexed``; the ring's size depends
+on the largest batch of the schedule, not on the length of the video.
+"""
+from __future__ import annotations
+
+import contextlib
+from typing import List, Optional, Tuple
+
+import torch
+
+from . import engine, sharding
+
+
+class VideoUpscaler:
+    """Stream uint8 BGR frames through `net` (a SAVSR in eval mode)::
+
+        up = VideoUpscaler(net, lr_size=(h, w), scale=(4, 4), batch=(26, 8))
+        for frame in decoder:                  # uint8 [h, w, 3] or [n, h, w, 3]; host (pageable or pinned) or CUDA
+            for start, hr in up.push(frame):   # hr: fresh uint8 CUDA [m, H, W, 3], frames start .. start + m - 1, in order
+                encode(hr)
+        for start, hr in up.finish():          # the last windows, reflected about the now-known last frame
+            encode(hr)
+
+    Forwards follow ``sharding.batch_schedule(T, batch)``: batch [i, j) runs as soon as frame j + 2 has arrived (its windows then need
+    no reflection at the end), and the batches whose windows reach past the last frame run in ``finish()``.  `scale` is fixed for the
+    stream; a later ``net.set_scale`` does not change it.
+
+    Ownership: the caller may overwrite or free what it passed to ``push`` as soon as ``push`` returns.  Host frames are staged through
+    the upscaler's own pinned buffers (a staging slot is reused only after the event of its upload); CUDA frames are copied in stream
+    order on the current stream.  Everything runs on the current stream of the net's device, so a ring slot is rewritten only after
+    every forward enqueued before that has read it."""
+
+    def __init__(self, net, lr_size: Tuple[int, int], scale, batch=1, num_frames: int = 7):
+        if net.training:
+            raise RuntimeError("VideoUpscaler is inference only: call net.eval() first")
+        h, w = (int(v) for v in lr_size)
+        if h < 2 or w < 2:
+            raise ValueError(f"LR frames must be at least 2x2, got {h}x{w}")
+        sizes = [int(batch)] if isinstance(batch, int) else [int(b) for b in batch]
+        sharding.batch_schedule(1, batch)                      # refuses empty or non-positive schedules
+        self.net, self.h, self.w, self.batch, self.sizes = net, h, w, batch, sizes
+        self.num_frames, self.pad = num_frames, num_frames // 2
+        self.scale = engine.normalize_scale(scale)
+        self.device = net.gamma.device
+        # Until batch [i, j) has run, the ring holds frames i - pad .. j - 1 + pad, the ones its windows read, and nothing newer.
+        self.capacity = max(sizes) + 2 * self.pad
+        self.ring = torch.empty(self.capacity, h, w, 3, dtype=torch.uint8, device=self.device)
+        self._staging: Optional[torch.Tensor] = None           # pinned twin of the ring for host frames, allocated on first use
+        self._uploaded: List[Optional[torch.cuda.Event]] = [None] * self.capacity
+        self.reset()
+
+    def reset(self) -> None:
+        """Start the next video of the same frame size: the ring, the staging buffers and the module's cached plans are reused."""
+        self.received = 0          # frames pushed
+        self.done = 0              # frames whose HR output has been returned (start of the next batch)
+        self.batches = 0           # forwards run
+        self.finished = False
+
+    def push(self, frames) -> List[Tuple[int, torch.Tensor]]:
+        """Append uint8 BGR frames [h, w, 3] or [n, h, w, 3] (torch or numpy, host or CUDA).  Returns the batches that became ready, as
+        (index of the first frame, uint8 [m, H, W, 3]) in frame order; often none."""
+        if self.finished:
+            raise RuntimeError("push() after finish(): call reset() to start the next video")
+        self._check_net()
+        x = self._frames(frames)
+        out = []
+        with self._on_device():
+            for f in x:
+                self._upload(f)
+                self.received += 1
+                while True:
+                    i, j = self._next_batch()
+                    if j + self.pad > self.received:       # frame j - 1 + pad, the last one its windows read, has not arrived
+                        break
+                    out.append(self._forward(i, j))
+        return out
+
+    def finish(self) -> List[Tuple[int, torch.Tensor]]:
+        """The video has ended: run the remaining windows, reflected about the last frame pushed."""
+        if self.finished:
+            raise RuntimeError("finish() was already called: call reset() to start the next video")
+        self._check_net()
+        sharding.frame_window_indices(0, self.received, self.num_frames)      # too short for reflection padding: ValueError
+        self.finished = True
+        out = []
+        with self._on_device():
+            while self.done < self.received:
+                i, j = self._next_batch()
+                out.append(self._forward(i, min(j, self.received)))
+        return out
+
+    # ------------------------------------------------------------------ internals
+    def _check_net(self) -> None:
+        if self.net.training:
+            raise RuntimeError("VideoUpscaler is inference only: the net was put in train mode")
+
+    def _on_device(self):
+        return torch.cuda.device(self.device) if self.device.type == "cuda" else contextlib.nullcontext()
+
+    def _frames(self, frames) -> torch.Tensor:
+        x = frames if isinstance(frames, torch.Tensor) else torch.as_tensor(frames)
+        if x.dtype != torch.uint8:
+            raise TypeError(f"VideoUpscaler takes uint8 BGR frames, got {x.dtype}")
+        if x.dim() == 3:
+            x = x.unsqueeze(0)
+        if x.dim() != 4 or tuple(x.shape[1:]) != (self.h, self.w, 3):
+            raise ValueError(f"expected uint8 BGR frames [{self.h}, {self.w}, 3] or [n, {self.h}, {self.w}, 3], got {tuple(x.shape)}")
+        if x.device.type != "cpu" and x.device != self.device:
+            raise ValueError(f"frames on {x.device}, the net on {self.device}")
+        return x
+
+    def _upload(self, frame: torch.Tensor) -> None:
+        s = self.received % self.capacity
+        if frame.device.type == "cpu" and self.device.type == "cuda":
+            if self._staging is None:
+                self._staging = torch.empty(self.ring.shape, dtype=torch.uint8, pin_memory=True)
+            ev = self._uploaded[s]
+            if ev is None:
+                ev = self._uploaded[s] = torch.cuda.Event()
+            else:
+                ev.synchronize()                 # the previous upload from this staging slot has been read
+            self._staging[s].copy_(frame)
+            self.ring[s].copy_(self._staging[s], non_blocking=True)
+            ev.record(torch.cuda.current_stream(self.device))
+        else:
+            self.ring[s].copy_(frame, non_blocking=True)
+
+    def _next_batch(self) -> Tuple[int, int]:
+        b = self.sizes[min(self.batches, len(self.sizes) - 1)]
+        return self.done, self.done + b
+
+    def _forward(self, i: int, j: int) -> Tuple[int, torch.Tensor]:
+        R = self.capacity
+        windows = [[f % R for f in sharding.frame_window_indices(c, self.received, self.num_frames)] for c in range(i, j)]
+        hr = self.net._forward_bgr_u8_indexed(self.ring, windows, self.scale)
+        self.done, self.batches = j, self.batches + 1
+        return i, hr
