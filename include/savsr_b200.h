@@ -517,6 +517,30 @@ int savsr_forward_u8(savsr_plan* plan, const uint8_t* x, uint8_t* out, savsr_str
  * savsr_forward / savsr_forward_u8 refuse a frame-table plan. */
 int savsr_forward_u8_frames(savsr_plan* plan, const uint8_t* const* ptrs_host, uint8_t* out, savsr_stream st);
 
+/* ---- YUV 4:2:0 video in and out ------------------------------------------------------------------------------------------------
+ * Decoders hand out and encoders take YUV 4:2:0, the forward reads and writes packed BGR.  These two calls convert on the device,
+ * byte-identically to OpenCV's cv::cvtColor: COLOR_YUV2BGR_I420 / COLOR_YUV2BGR_NV12 (each pixel takes its 2x2 block's chroma sample)
+ * and COLOR_BGR2YUV_I420 (U and V from the top-left pixel of each 2x2 block).  BT.601, limited range; sources tagged otherwise are
+ * converted with the same matrix both ways.  A C host decodes into a ring of BGR frames with savsr_yuv420_to_bgr, runs
+ * savsr_forward_u8_frames on it, and encodes the output with savsr_bgr_to_yuv420.
+ *
+ * A YUV frame of h x w (both even) is described by its planes:
+ *   y, y_pitch        the Y plane, h rows of w bytes, y_pitch >= w bytes apart;
+ *   u, v, c_pitch     the chroma rows (h / 2 of them): chroma sample c of row r is u[r * c_pitch + c * c_step], likewise v;
+ *   c_step            1 for yuv420p (I420: separate U and V planes of w / 2 bytes a row, c_pitch >= w / 2),
+ *                     2 for nv12 (one plane of interleaved U, V bytes, U first: v = u + 1, c_pitch >= w);
+ *   frame_stride      bytes from each plane of frame k to the same plane of frame k + 1.
+ * ffmpeg's rawvideo yuv420p frame of [3h/2][w] bytes at p: y = p, y_pitch = w, u = p + h w, v = u + h w / 4, c_pitch = w / 2,
+ * c_step = 1.  An NVDEC NV12 surface of pitch P at p: y = p, y_pitch = P, u = p + h P, v = u + 1, c_pitch = P, c_step = 2.
+ * The BGR side is contiguous uint8 [n][h][w][3].  Both calls return an error before any launch on odd sizes, a null pointer, a pitch
+ * below the row's width, a c_step other than 1 or 2, or a negative frame_stride; n = 0 launches nothing.
+ * Ownership: every buffer must stay valid, in stream order, until the launch on st has run; the caller may reuse them after that.
+ */
+int savsr_yuv420_to_bgr(savsr_ctx* ctx, const uint8_t* y, int y_pitch, const uint8_t* u, const uint8_t* v, int c_pitch, int c_step,
+                        int64_t frame_stride, int n, int h, int w, uint8_t* bgr, savsr_stream st);
+int savsr_bgr_to_yuv420(savsr_ctx* ctx, const uint8_t* bgr, int n, int h, int w, uint8_t* y, int y_pitch, uint8_t* u, uint8_t* v,
+                        int c_pitch, int c_step, int64_t frame_stride, savsr_stream st);
+
 /* ---- post-processing / metrics on the device (next row 8f3) -------------------------------------------------------
  * tensor2img (lbasicsr/utils/img_util.py:38-94): sr fp32 NCHW [batch][3][H][W] RGB -> uint8 HWC BGR [batch][H][W][3]
  * (clamp, *255, round half to even), and, when gt is given, the per-frame sum of squared Y-channel differences of the two

@@ -187,6 +187,8 @@ SIGNATURES = {
     "savsr_forward_u8": (_I, [_VP, _VP, _VP, _VP]),
     "savsr_forward_u8_frames": (_I, [_VP, _VP, _VP, _VP]),
     "savsr_write_frame_table": (_I, [_VP, _VP, _VP, _I, _VP]),
+    "savsr_yuv420_to_bgr": (_I, [_VP, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _I, _VP, _VP]),
+    "savsr_bgr_to_yuv420": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _VP]),
     "savsr_pack_frames": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),
     "savsr_pack_frames_u8": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),
     "savsr_pack_frames_u8_table": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),

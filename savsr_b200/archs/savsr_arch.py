@@ -23,7 +23,7 @@ from typing import Dict, Optional, Tuple, Union
 import torch
 import torch.nn as nn
 
-from savsr_b200 import engine
+from savsr_b200 import colour, engine
 
 if __name__ == "lbasicsr.archs.savsr_arch":
     # served by savsr_b200.overlay in place of the reference's own file: register in the reference's registry
@@ -264,8 +264,10 @@ class SAVSR(nn.Module):
             self.scale = scale
         return self._forward_bgr_u8_indexed(pool, windows, self.scale)
 
-    def _forward_bgr_u8_indexed(self, pool: torch.Tensor, windows, scale) -> torch.Tensor:
-        """forward_bgr_u8_indexed at `scale`, leaving self.scale as it is (savsr_b200.VideoUpscaler keeps its own scale)."""
+    def _forward_bgr_u8_indexed(self, pool: torch.Tensor, windows, scale, out_format: str = "bgr24") -> torch.Tensor:
+        """forward_bgr_u8_indexed at `scale`, leaving self.scale as it is (savsr_b200.VideoUpscaler keeps its own scale).  With out_format
+        "yuv420p" or "nv12" the HR frames come back as uint8 [b, 3H/2, W] YUV 4:2:0 (savsr_b200.colour), converted from the plan's
+        output staging buffer instead of copied."""
         if self.training:
             raise RuntimeError("forward_bgr_u8_indexed is inference only: call eval() first (training takes fp32 windows through forward)")
         if pool.dtype != torch.uint8:
@@ -285,21 +287,26 @@ class SAVSR(nn.Module):
         b = idx.shape[0]
         self._check_device(pool)
         if b == 0:
-            return pool.new_empty((0, *engine.get_hw(h, w, scale), 3))
+            H, W = engine.get_hw(h, w, scale)
+            return pool.new_empty((0, H, W, 3) if out_format == "bgr24" else (0, *colour.yuv_shape(H, W)))
         idx = idx.to(torch.int64)
         lo, hi = int(idx.min()), int(idx.max())
         if lo < 0 or hi >= n:
             raise IndexError(f"window row index {lo if lo < 0 else hi} out of range for a pool of {n} frames")
         ptrs = (idx.reshape(-1) * (h * w * 3) + pool.data_ptr()).tolist()
-        return self._run_plan(self._plan(b, h, w, pool.device, "bgr_u8_frames", scale), frames=ptrs)
+        return self._run_plan(self._plan(b, h, w, pool.device, "bgr_u8_frames", scale), frames=ptrs, out_format=out_format)
 
-    def _run_plan(self, plan: engine.Plan, x: Optional[torch.Tensor] = None, frames: Optional[list] = None) -> torch.Tensor:
+    def _run_plan(self, plan: engine.Plan, x: Optional[torch.Tensor] = None, frames: Optional[list] = None,
+                  out_format: str = "bgr24") -> torch.Tensor:
         with torch.cuda.device(plan.device):
-            out = torch.empty_like(plan.out)
+            if out_format == "bgr24":
+                out = torch.empty_like(plan.out)
+            else:
+                out = plan.out.new_empty((plan.B, *colour.yuv_shape(plan.H, plan.W)))
             if frames is None:
                 plan.forward_into(x, out, graph=self.use_graph)
             else:
-                plan.forward_frames_into(frames, out, graph=self.use_graph)
+                plan.forward_frames_into(frames, out, graph=self.use_graph, out_format=out_format)
             if self.precision == "fp16" and not plan.__dict__.get("_range_checked"):
                 # fp16 operands meet the <= 1e-3 bound but saturate at 65504: look at every trunk activation of this plan's FIRST forward
                 # (one pass over the arena, once per plan) and refuse to continue silently when the headroom is below 4x

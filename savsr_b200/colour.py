@@ -1,0 +1,151 @@
+"""YUV 4:2:0 <-> packed 8-bit BGR on the device, byte-identical to OpenCV's ``cv2.cvtColor``.
+
+Video decoders hand out YUV 4:2:0 (NVDEC: NV12 surfaces in device memory; ``ffmpeg -f rawvideo -pix_fmt yuv420p``: planar I420) and
+encoders take it back, while ``SAVSR.forward_bgr_u8`` and ``VideoUpscaler`` work on packed BGR [h, w, 3].  The formats carry ffmpeg's
+``pix_fmt`` names:
+
+* ``"bgr24"``: uint8 [h, w, 3], the layout ``cv2.imread`` produces;
+* ``"yuv420p"``: one uint8 [3h/2, w] array per frame: the Y plane, then the U plane (h/2 x w/2), then the V plane, packed;
+* ``"nv12"``: one uint8 [3h/2, w] array per frame: the Y plane, then h/2 rows of interleaved U, V bytes (U first).  It may have a
+  row pitch (``stride(0) >= w``, ``stride(1) == 1``; the UV rows start at row h of the same pitch), as a decoder surface does when it
+  is exposed as a tensor view.  yuv420p frames must have contiguous rows.
+
+Several frames are [n, 3h/2, w].  The conversion is BT.601, limited range, in OpenCV's 20-bit fixed point: decoding gives each pixel
+the chroma sample of its 2x2 block (``COLOR_YUV2BGR_I420`` / ``COLOR_YUV2BGR_NV12``), encoding takes U and V from the top-left
+pixel of each 2x2 block (``COLOR_BGR2YUV_I420``).  Sizes must be even, as cv2 requires.  Each call is one launch on the current
+stream of the tensors' device (savsr_yuv420_to_bgr / savsr_bgr_to_yuv420 of libsavsr_sm100); there is no CPU path.
+"""
+from __future__ import annotations
+
+from typing import Optional, Tuple
+
+import torch
+
+from . import _capi as K, engine
+
+FORMATS = ("bgr24", "yuv420p", "nv12")
+YUV_FORMATS = ("yuv420p", "nv12")
+
+
+def check_format(fmt: str, what: str = "format") -> str:
+    if fmt not in FORMATS:
+        raise ValueError(f"unknown {what} {fmt!r}: expected one of {', '.join(FORMATS)}")
+    return fmt
+
+
+def yuv_shape(h: int, w: int) -> Tuple[int, int]:
+    """The [rows, w] array one YUV 4:2:0 frame of h x w occupies."""
+    return 3 * h // 2, w
+
+
+def yuv_frames(x: torch.Tensor, fmt: str, h: Optional[int] = None, w: Optional[int] = None) -> torch.Tensor:
+    """Check that x holds uint8 `fmt` frames ([3h/2, w] or [n, 3h/2, w]; h x w from the shape when not given) with a layout the
+    kernels read, and return it as [n, 3h/2, w].  Wherever x lives: the device is the caller's concern."""
+    if fmt not in YUV_FORMATS:
+        raise ValueError(f"{fmt!r} is not a YUV 4:2:0 format ({', '.join(YUV_FORMATS)})")
+    if x.dtype != torch.uint8:
+        raise TypeError(f"{fmt} frames are uint8, got {x.dtype}")
+    if h is None:
+        rows, w = (x.shape[-2], x.shape[-1]) if x.dim() in (2, 3) else (0, 0)
+        if rows % 3 or rows == 0:
+            raise ValueError(f"expected uint8 {fmt} frames [3h/2, w] or [n, 3h/2, w], got {tuple(x.shape)}")
+        h = 2 * rows // 3
+    if h % 2 or w % 2:
+        raise ValueError(f"{fmt} needs an even frame size, got {h}x{w}")
+    if x.dim() == 2:
+        x = x.unsqueeze(0)
+    if x.dim() != 3 or tuple(x.shape[1:]) != yuv_shape(h, w):
+        rows = yuv_shape(h, w)[0]
+        raise ValueError(f"expected uint8 {fmt} frames [{rows}, {w}] or [n, {rows}, {w}], got {tuple(x.shape)}")
+    if x.stride(2) != 1:
+        raise ValueError(f"{fmt} frames need a unit column stride, got {x.stride(2)}")
+    if fmt == "yuv420p" and x.stride(1) != w:
+        raise ValueError(f"yuv420p frames must have contiguous rows: row stride {x.stride(1)} != width {w} (only nv12 takes a row pitch)")
+    if x.stride(1) < w:
+        raise ValueError(f"{fmt} row stride {x.stride(1)} is below the width {w}")
+    return x
+
+
+def _planes(x: torch.Tensor, fmt: str, h: int, w: int) -> tuple:
+    """(y, y_pitch, u, v, c_pitch, c_step, frame_stride) of frames x [n, 3h/2, w] (checked by yuv_frames)."""
+    p, pitch = x.data_ptr(), x.stride(1)
+    if fmt == "yuv420p":
+        u = p + h * w
+        return p, w, u, u + (h // 2) * (w // 2), w // 2, 1, x.stride(0)
+    u = p + h * pitch
+    return p, pitch, u, u + 1, pitch, 2, x.stride(0)
+
+
+def _on_cuda(*xs: torch.Tensor) -> torch.device:
+    dev = xs[0].device
+    for x in xs:
+        if not x.is_cuda:
+            raise RuntimeError("savsr_b200.colour runs on CUDA (sm_100a) only; there is no CPU fallback")
+        if x.device != dev:
+            raise ValueError(f"tensors on {dev} and {x.device}")
+    return dev
+
+
+def _bgr(x: torch.Tensor, what: str) -> torch.Tensor:
+    if x.dtype != torch.uint8:
+        raise TypeError(f"{what} takes uint8 BGR frames, got {x.dtype}")
+    if x.dim() == 3:
+        x = x.unsqueeze(0)
+    if x.dim() != 4 or x.shape[3] != 3:
+        raise ValueError(f"{what}: expected uint8 BGR frames [h, w, 3] or [n, h, w, 3], got {tuple(x.shape)}")
+    if not x.is_contiguous():
+        raise ValueError(f"{what}: BGR frames must be contiguous")
+    return x
+
+
+def yuv420_to_bgr(frames: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """uint8 `fmt` frames ("yuv420p" or "nv12", [3h/2, w] or [n, 3h/2, w], CUDA) -> uint8 BGR [h, w, 3] or [n, h, w, 3], as
+    cv2.cvtColor(frame, COLOR_YUV2BGR_I420 or COLOR_YUV2BGR_NV12) of each frame.  Writes `out` (contiguous, that shape) when given,
+    else a fresh tensor.  One launch on the current stream; the frames must stay valid, in stream order, until it has run."""
+    x = yuv_frames(frames, fmt)
+    n, h, w = x.shape[0], 2 * x.shape[1] // 3, x.shape[2]
+    shape = (n, h, w, 3) if frames.dim() == 3 else (h, w, 3)
+    if out is None:
+        _on_cuda(x)
+        out = torch.empty(shape, dtype=torch.uint8, device=x.device)
+    elif tuple(out.shape) != shape or out.dtype != torch.uint8 or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous uint8 tensor of shape {shape}, got {out.dtype} {tuple(out.shape)}")
+    dev = _on_cuda(x, out)
+    if n == 0:
+        return out
+    ctx = engine.context(dev.index)
+    y, yp, u, v, cp, cs, fs = _planes(x, fmt, h, w)
+    with torch.cuda.device(dev):
+        K.check(ctx.lib.savsr_yuv420_to_bgr(ctx.handle, y, yp, u, v, cp, cs, fs, n, h, w, out.data_ptr(),
+                                            torch.cuda.current_stream(dev).cuda_stream))
+    return out
+
+
+def bgr_to_yuv420(bgr: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """uint8 BGR [H, W, 3] or [n, H, W, 3] (contiguous, CUDA, H and W even) -> uint8 `fmt` frames [3H/2, W] or [n, 3H/2, W], as
+    cv2.cvtColor(frame, COLOR_BGR2YUV_I420) of each frame, with U and V interleaved for "nv12".  Writes `out` when given (any layout
+    yuv_frames accepts, e.g. a pitched NV12 surface), else a fresh contiguous tensor.  One launch on the current stream."""
+    if fmt not in YUV_FORMATS:
+        raise ValueError(f"{fmt!r} is not a YUV 4:2:0 format ({', '.join(YUV_FORMATS)})")
+    x = _bgr(bgr, "bgr_to_yuv420")
+    n, H, W = x.shape[:3]
+    shape = (n, *yuv_shape(H, W)) if bgr.dim() == 4 else yuv_shape(H, W)
+    if H % 2 or W % 2:
+        raise ValueError(f"{fmt} needs an even frame size, got {H}x{W}")
+    if out is None:
+        _on_cuda(x)
+        out = torch.empty(shape, dtype=torch.uint8, device=x.device)
+    elif tuple(out.shape) != shape:
+        raise ValueError(f"out must have shape {shape}, got {tuple(out.shape)}")
+    o = yuv_frames(out, fmt, H, W)
+    if n > 1 and o.stride(0) < o.shape[1] * o.stride(1):
+        raise ValueError(f"the frames of out overlap: frame stride {o.stride(0)}")
+    dev = _on_cuda(x, o)
+    if n == 0:
+        return out
+    ctx = engine.context(dev.index)
+    y, yp, u, v, cp, cs, fs = _planes(o, fmt, H, W)
+    with torch.cuda.device(dev):
+        K.check(ctx.lib.savsr_bgr_to_yuv420(ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, cs, fs,
+                                            torch.cuda.current_stream(dev).cuda_stream))
+    return out

@@ -66,6 +66,16 @@ enum IoMode { kIoF32 = 0, kIoU8 = 1, kIoU8Table = 2 };
 // One launch of the frame-table writer carries at most this many pointers in its by-value argument (3.6 KB, under the 4 KB
 // parameter limit of older drivers); 448 = 64 windows of 7 frames.
 constexpr int kFrameTableChunk = 448;
+// BT.601 limited-range YUV <-> 8-bit RGB in OpenCV's 20-bit fixed point (cv::cvtColor YUV 4:2:0 <-> BGR, byte-exact; colour.cu).
+//   decode: y = max(0, Y - 16) * kYuvY, u = U - 128, v = V - 128
+//           R = sat((y + half + kYuvVR v) >> 20), G = sat((y + half + kYuvVG v + kYuvUG u) >> 20), B = sat((y + half + kYuvUB u) >> 20)
+//   encode: Y = (kRgbYR R + kRgbYG G + kRgbYB B + (16 << 20) + half) >> 20, U and V likewise with offset 128 << 20
+// Every intermediate fits in int32; >> is arithmetic.
+constexpr int kYuvShift = 20, kYuvHalf = 1 << (kYuvShift - 1);
+constexpr int kYuvY = 1220542, kYuvVR = 1673527, kYuvVG = -852492, kYuvUG = -409993, kYuvUB = 2116026;
+constexpr int kRgbYR = 269484, kRgbYG = 528482, kRgbYB = 102760;
+constexpr int kRgbUR = -155188, kRgbUG = -305135, kRgbUB = 460324;
+constexpr int kRgbVR = 460324, kRgbVG = -385875, kRgbVB = -74448;
 template <class F>
 inline int ensure_smem_attr(savsr_ctx* ctx, int bit, F func, size_t bytes) {
   if (ctx->attr_mask & (1u << bit)) return 0;

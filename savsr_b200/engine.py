@@ -22,7 +22,7 @@ from typing import Callable, Dict, List, Optional, Sequence, Tuple
 import numpy as np
 import torch
 
-from . import _capi as K
+from . import _capi as K, colour
 
 BN_EPS = 1e-5
 IO_MODES = ("f32", "bgr_u8", "bgr_u8_frames")
@@ -722,18 +722,24 @@ class Plan:
         with torch.cuda.device(self.device):
             K.check(self.lib.savsr_write_frame_table(self.ctx.handle, self.frame_table.data_ptr(), arr, len(ptrs), self._stream().cuda_stream))
 
-    def forward_frames_into(self, ptrs: Sequence[int], out: torch.Tensor, graph: bool = True) -> None:
+    def forward_frames_into(self, ptrs: Sequence[int], out: torch.Tensor, graph: bool = True, out_format: str = "bgr24") -> None:
         """io="bgr_u8_frames": the frames at the B*7 device addresses `ptrs` (see write_frame_table) -> out uint8 [B,H,W,3], all on the
-        device's current stream.  The frames are read in place by the forward: they must stay valid, in stream order, until it has run."""
+        device's current stream.  The frames are read in place by the forward: they must stay valid, in stream order, until it has run.
+        With out_format "yuv420p" or "nv12", out is uint8 [B,3H/2,W] and the colour conversion reads the output staging buffer in place
+        of the copy (colour.bgr_to_yuv420)."""
         if self.io != "bgr_u8_frames":
             raise ValueError(f'forward_frames_into needs a plan with io="bgr_u8_frames", this one has io={self.io!r}')
+        colour.check_format(out_format, "out_format")
         with torch.cuda.device(self.device):
             self.write_frame_table(ptrs)
             if graph:
                 self.run_graph()
             else:
                 self.run()
-            out.copy_(self.out, non_blocking=True)
+            if out_format == "bgr24":
+                out.copy_(self.out, non_blocking=True)
+            else:
+                colour.bgr_to_yuv420(self.out, out_format, out=out)
 
     def activation_absmax(self) -> float:
         """Largest |value| currently held anywhere in the LR arena (every trunk activation of the last forward), read in the plan's

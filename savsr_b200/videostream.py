@@ -3,7 +3,8 @@
 ``VideoUpscaler`` takes frames as a decoder produces them and returns HR frames in order, with the same windows, reflection and
 batch partition as ``sharding.infer_clip(net.forward_bgr_u8, clip, batch=...)`` on the whole clip, so its output is byte-identical to
 that call.  Frames are uploaded once into a device ring and read in place by ``SAVSR.forward_bgr_u8_indexed``; the ring's size depends
-on the largest batch of the schedule, not on the length of the video.
+on the largest batch of the schedule, not on the length of the video.  Frames may come and go as packed BGR or as YUV 4:2:0
+(yuv420p, NV12: savsr_b200.colour), converted on the device on their way into the ring and out of the forward's output buffer.
 """
 from __future__ import annotations
 
@@ -12,11 +13,11 @@ from typing import List, Optional, Tuple
 
 import torch
 
-from . import engine, sharding
+from . import colour, engine, sharding
 
 
 class VideoUpscaler:
-    """Stream uint8 BGR frames through `net` (a SAVSR in eval mode)::
+    """Stream uint8 frames through `net` (a SAVSR in eval mode)::
 
         up = VideoUpscaler(net, lr_size=(h, w), scale=(4, 4), batch=(26, 8))
         for frame in decoder:                  # uint8 [h, w, 3] or [n, h, w, 3]; host (pageable or pinned) or CUDA
@@ -29,12 +30,20 @@ class VideoUpscaler:
     no reflection at the end), and the batches whose windows reach past the last frame run in ``finish()``.  `scale` is fixed for the
     stream; a later ``net.set_scale`` does not change it.
 
+    `in_format` and `out_format` name the frames' layout with ffmpeg's pix_fmt names (savsr_b200.colour): "bgr24" (the default,
+    [h, w, 3]), "yuv420p" or "nv12" (one uint8 [3h/2, w] array per frame, [n, 3h/2, w] for several; an NV12 frame may have a row pitch,
+    like a decoder surface viewed as a tensor).  YUV input is converted to BGR on its way into the ring and YUV output from the forward's
+    output buffer, exactly as cv2.cvtColor converts (COLOR_YUV2BGR_I420 / _NV12, COLOR_BGR2YUV_I420), so the output is
+    enc(infer_clip(net.forward_bgr_u8, dec(frames), batch=...)).  YUV needs even sizes: even h and w for YUV input, an even HR size
+    for YUV output (bgr24 output takes any scale).
+
     Ownership: the caller may overwrite or free what it passed to ``push`` as soon as ``push`` returns.  Host frames are staged through
     the upscaler's own pinned buffers (a staging slot is reused only after the event of its upload); CUDA frames are copied in stream
     order on the current stream.  Everything runs on the current stream of the net's device, so a ring slot is rewritten only after
     every forward enqueued before that has read it."""
 
-    def __init__(self, net, lr_size: Tuple[int, int], scale, batch=1, num_frames: int = 7):
+    def __init__(self, net, lr_size: Tuple[int, int], scale, batch=1, num_frames: int = 7, in_format: str = "bgr24",
+                 out_format: str = "bgr24"):
         if net.training:
             raise RuntimeError("VideoUpscaler is inference only: call net.eval() first")
         h, w = (int(v) for v in lr_size)
@@ -45,11 +54,20 @@ class VideoUpscaler:
         self.net, self.h, self.w, self.batch, self.sizes = net, h, w, batch, sizes
         self.num_frames, self.pad = num_frames, num_frames // 2
         self.scale = engine.normalize_scale(scale)
+        self.in_format = colour.check_format(in_format, "in_format")
+        self.out_format = colour.check_format(out_format, "out_format")
+        if in_format != "bgr24" and (h % 2 or w % 2):
+            raise ValueError(f"{in_format} input needs an even LR size, got {h}x{w}")
+        H, W = engine.get_hw(h, w, self.scale)
+        if out_format != "bgr24" and (H % 2 or W % 2):
+            raise ValueError(f"{out_format} output needs an even HR size: {h}x{w} at scale {self.scale} gives H = {H}, W = {W}; "
+                             "bgr24 output takes any scale")
         self.device = net.gamma.device
         # Until batch [i, j) has run, the ring holds frames i - pad .. j - 1 + pad, the ones its windows read, and nothing newer.
         self.capacity = max(sizes) + 2 * self.pad
         self.ring = torch.empty(self.capacity, h, w, 3, dtype=torch.uint8, device=self.device)
-        self._staging: Optional[torch.Tensor] = None           # pinned twin of the ring for host frames, allocated on first use
+        self._staging: Optional[torch.Tensor] = None           # pinned twin of the ring for host frames (YUV-sized for YUV input), on first use
+        self._yuv_dev: Optional[torch.Tensor] = None           # device staging of one host YUV frame, converted from there into the ring
         self._uploaded: List[Optional[torch.cuda.Event]] = [None] * self.capacity
         self.reset()
 
@@ -61,8 +79,9 @@ class VideoUpscaler:
         self.finished = False
 
     def push(self, frames) -> List[Tuple[int, torch.Tensor]]:
-        """Append uint8 BGR frames [h, w, 3] or [n, h, w, 3] (torch or numpy, host or CUDA).  Returns the batches that became ready, as
-        (index of the first frame, uint8 [m, H, W, 3]) in frame order; often none."""
+        """Append uint8 frames in `in_format`: BGR [h, w, 3] or [n, h, w, 3], YUV [3h/2, w] or [n, 3h/2, w] (torch or numpy, host or
+        CUDA).  Returns the batches that became ready, as (index of the first frame, uint8 [m, H, W, 3], or [m, 3H/2, W] in a YUV
+        out_format) in frame order; often none."""
         if self.finished:
             raise RuntimeError("push() after finish(): call reset() to start the next video")
         self._check_net()
@@ -103,31 +122,40 @@ class VideoUpscaler:
 
     def _frames(self, frames) -> torch.Tensor:
         x = frames if isinstance(frames, torch.Tensor) else torch.as_tensor(frames)
-        if x.dtype != torch.uint8:
-            raise TypeError(f"VideoUpscaler takes uint8 BGR frames, got {x.dtype}")
-        if x.dim() == 3:
-            x = x.unsqueeze(0)
-        if x.dim() != 4 or tuple(x.shape[1:]) != (self.h, self.w, 3):
-            raise ValueError(f"expected uint8 BGR frames [{self.h}, {self.w}, 3] or [n, {self.h}, {self.w}, 3], got {tuple(x.shape)}")
+        if self.in_format != "bgr24":
+            x = colour.yuv_frames(x, self.in_format, self.h, self.w)      # dtype, shape, row pitch and column stride
+        else:
+            if x.dtype != torch.uint8:
+                raise TypeError(f"VideoUpscaler takes uint8 BGR frames, got {x.dtype}")
+            if x.dim() == 3:
+                x = x.unsqueeze(0)
+            if x.dim() != 4 or tuple(x.shape[1:]) != (self.h, self.w, 3):
+                raise ValueError(f"expected uint8 BGR frames [{self.h}, {self.w}, 3] or [n, {self.h}, {self.w}, 3], got {tuple(x.shape)}")
         if x.device.type != "cpu" and x.device != self.device:
             raise ValueError(f"frames on {x.device}, the net on {self.device}")
         return x
 
     def _upload(self, frame: torch.Tensor) -> None:
         s = self.received % self.capacity
+        yuv, ring = self.in_format != "bgr24", self.ring[s]
         if frame.device.type == "cpu" and self.device.type == "cuda":
             if self._staging is None:
-                self._staging = torch.empty(self.ring.shape, dtype=torch.uint8, pin_memory=True)
+                self._staging = torch.empty((self.capacity, *frame.shape), dtype=torch.uint8, pin_memory=True)
+                if yuv:     # one buffer is enough: its next upload follows this frame's conversion in stream order
+                    self._yuv_dev = torch.empty(frame.shape, dtype=torch.uint8, device=self.device)
             ev = self._uploaded[s]
             if ev is None:
                 ev = self._uploaded[s] = torch.cuda.Event()
             else:
                 ev.synchronize()                 # the previous upload from this staging slot has been read
             self._staging[s].copy_(frame)
-            self.ring[s].copy_(self._staging[s], non_blocking=True)
+            frame = self._yuv_dev if yuv else ring
+            frame.copy_(self._staging[s], non_blocking=True)
             ev.record(torch.cuda.current_stream(self.device))
-        else:
-            self.ring[s].copy_(frame, non_blocking=True)
+        if yuv:
+            colour.yuv420_to_bgr(frame, self.in_format, out=ring)      # CUDA frames, pitched NV12 too, are read in place
+        elif frame is not ring:
+            ring.copy_(frame, non_blocking=True)
 
     def _next_batch(self) -> Tuple[int, int]:
         b = self.sizes[min(self.batches, len(self.sizes) - 1)]
@@ -136,6 +164,7 @@ class VideoUpscaler:
     def _forward(self, i: int, j: int) -> Tuple[int, torch.Tensor]:
         R = self.capacity
         windows = [[f % R for f in sharding.frame_window_indices(c, self.received, self.num_frames)] for c in range(i, j)]
-        hr = self.net._forward_bgr_u8_indexed(self.ring, windows, self.scale)
+        yuv_out = {} if self.out_format == "bgr24" else {"out_format": self.out_format}
+        hr = self.net._forward_bgr_u8_indexed(self.ring, windows, self.scale, **yuv_out)
         self.done, self.batches = j, self.batches + 1
         return i, hr
