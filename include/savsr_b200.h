@@ -176,6 +176,13 @@ int savsr_pack_frames_u8(savsr_ctx* ctx, savsr_arena* arena, const uint8_t* x, i
 int savsr_pack_frames_u8_table(savsr_ctx* ctx, savsr_arena* arena, const uint8_t* const* frames, int t, int h, int w, int dst_slot,
                                savsr_stream st);
 /*
+ * The same from a table of 16-bit frames: entry n * t + f points at one contiguous uint16 [h][w][3] BGR frame (bgr48, full scale
+ * 65535), and each value v becomes float(v) / 65535 correctly rounded.  An 8-bit frame widened by 257 gives the slot its 8-bit
+ * original gives.  The table holds frame addresses like the 8-bit one and is written by savsr_write_frame_table; same ownership rule.
+ */
+int savsr_pack_frames_u16_table(savsr_ctx* ctx, savsr_arena* arena, const uint16_t* const* frames, int t, int h, int w, int dst_slot,
+                                savsr_stream st);
+/*
  * Frame table writer: table_dev[i] = ptrs_host[i] for i < n, on stream st.  The pointers travel in the launches' by-value arguments
  * (448 per launch, more launches above that), never through a host-to-device copy, so the call returns at once and can be enqueued
  * in stream order in front of a graph replay that reads the table.  Refuses a null entry before any launch.
@@ -462,6 +469,12 @@ int savsr_satu_hr_u8_table(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_
                            const float* table, const float* base_y, const float* base_x, const void* weights,
                            const float* zbias, const float* tail_bias, const uint8_t* const* frames, int t, int centre, uint8_t* out,
                            savsr_stream st);
+/* The same with 16-bit frames (savsr_pack_frames_u16_table): the skip reads the centre frame through v / 65535, and out is uint16 BGR
+ * [batch][H][W][3], every pixel quantised as tensor2img does with 65535 in place of 255 (clamp to [0, 1], * 65535, round half to even). */
+int savsr_satu_hr_u16_table(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
+                            const float* table, const float* base_y, const float* base_x, const void* weights,
+                            const float* zbias, const float* tail_bias, const uint16_t* const* frames, int t, int centre, uint16_t* out,
+                            savsr_stream st);
 
 /* ---- the forward as one call -----------------------------------------------------------------------------------------------------
  * savsr_plan = an ordered list of recorded launches of the entry points above (argument structures copied at record time), replayed on
@@ -481,9 +494,13 @@ int savsr_plan_set_io_u8(savsr_plan* plan, uint8_t* x_in, size_t x_bytes, uint8_
 /* 8-bit I/O from a frame table: table_dev is the device array of `entries` = batch * 7 frame pointers that the plan's
  * savsr_pack_frames_u8_table and savsr_satu_hr_u8_table launches read, out uint8 BGR [batch][H][W][3].  A third I/O mode. */
 int savsr_plan_set_io_u8_table(savsr_plan* plan, const uint8_t** table_dev, int entries, uint8_t* out, size_t out_bytes, int format);
+/* 16-bit I/O from a frame table of uint16 BGR frames (savsr_pack_frames_u16_table, savsr_satu_hr_u16_table), out uint16 BGR
+ * [batch][H][W][3].  A fourth I/O mode. */
+int savsr_plan_set_io_u16_table(savsr_plan* plan, const uint16_t** table_dev, int entries, uint16_t* out, size_t out_bytes, int format);
 int savsr_plan_add_pack_frames(savsr_plan* plan, savsr_arena* arena, const float* x, int t, int h, int w, int dst_slot);
 int savsr_plan_add_pack_frames_u8(savsr_plan* plan, savsr_arena* arena, const uint8_t* x, int t, int h, int w, int dst_slot);
 int savsr_plan_add_pack_frames_u8_table(savsr_plan* plan, savsr_arena* arena, const uint8_t* const* frames, int t, int h, int w, int dst_slot);
+int savsr_plan_add_pack_frames_u16_table(savsr_plan* plan, savsr_arena* arena, const uint16_t* const* frames, int t, int h, int w, int dst_slot);
 int savsr_plan_add_conv(savsr_plan* plan, savsr_arena* arena, const savsr_conv_group* groups, int ngroups, int ksize, int n_tile,
                         int dst_mode, int impl);
 int savsr_plan_add_osa_prologue(savsr_plan* plan, const savsr_osa_params* convs, int nconvs, int batch, int npart, int npix,
@@ -503,6 +520,9 @@ int savsr_plan_add_satu_hr_u8(savsr_plan* plan, savsr_arena* lr, int x_slot, int
 int savsr_plan_add_satu_hr_u8_table(savsr_plan* plan, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W, const float* table,
                                     const float* base_y, const float* base_x, const void* weights, const float* zbias, const float* tail_bias,
                                     const uint8_t* const* frames, int t, int centre, uint8_t* out);
+int savsr_plan_add_satu_hr_u16_table(savsr_plan* plan, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W, const float* table,
+                                     const float* base_y, const float* base_x, const void* weights, const float* zbias, const float* tail_bias,
+                                     const uint16_t* const* frames, int t, int centre, uint16_t* out);
 int savsr_plan_add_arena_export(savsr_plan* plan, savsr_arena* arena, int slot, float* nchw);   /* debug taps */
 int savsr_plan_run(savsr_plan* plan, savsr_stream st);
 /* x -> the plan's input staging buffer (device-to-device, skipped when x IS that buffer), replay, output staging buffer -> out. */
@@ -516,6 +536,10 @@ int savsr_forward_u8(savsr_plan* plan, const uint8_t* x, uint8_t* out, savsr_str
  * valid, in stream order, until this forward has run.  Returns an error, before any launch, on a plan of another I/O mode, and
  * savsr_forward / savsr_forward_u8 refuse a frame-table plan. */
 int savsr_forward_u8_frames(savsr_plan* plan, const uint8_t* const* ptrs_host, uint8_t* out, savsr_stream st);
+/* The same for a plan with 16-bit frame-table I/O (savsr_plan_set_io_u16_table): each pointer is one contiguous uint16 BGR [h][w][3]
+ * frame, out uint16 BGR [batch][H][W][3].  Same ownership rule; refuses a plan of another I/O mode before any launch, and the other
+ * forward calls refuse this one. */
+int savsr_forward_u16_frames(savsr_plan* plan, const uint16_t* const* ptrs_host, uint16_t* out, savsr_stream st);
 
 /* ---- YUV 4:2:0 video in and out ------------------------------------------------------------------------------------------------
  * Decoders hand out and encoders take YUV 4:2:0, the forward reads and writes packed BGR.  These two calls convert on the device,
@@ -540,6 +564,24 @@ int savsr_yuv420_to_bgr(savsr_ctx* ctx, const uint8_t* y, int y_pitch, const uin
                         int64_t frame_stride, int n, int h, int w, uint8_t* bgr, savsr_stream st);
 int savsr_bgr_to_yuv420(savsr_ctx* ctx, const uint8_t* bgr, int n, int h, int w, uint8_t* y, int y_pitch, uint8_t* u, uint8_t* v,
                         int c_pitch, int c_step, int64_t frame_stride, savsr_stream st);
+/*
+ * 10-bit YUV 4:2:0 <-> 16-bit BGR (bgr48: contiguous uint16 [n][h][w][3], full scale 65535), for HEVC Main10 / 10-bit AV1 decoders and
+ * encoders.  The same matrix and chroma handling as the two 8-bit calls, rescaled: one 10-bit step is a quarter of an 8-bit step, one
+ * 8-bit BGR step is 257 sixteen-bit steps; decoding saturates to [0, 65535].  Each result is within 0.53 of an output step of the
+ * real-valued map (fixed-point forms in savsr_b200/csrc/common.cuh).  The planes are described as above with every pitch and the
+ * frame stride in uint16 elements, and
+ *   msb = 0           yuv420p10le (ffmpeg): the value in bits 0-9; decoding reads s & 0x3ff, encoding writes the value;
+ *   msb = 1           p010 (NVDEC 10-bit surfaces, c_step 2): the value in bits 6-15; decoding reads s >> 6, encoding writes v << 6.
+ * A P010 surface of pitch P bytes at p: y = p, y_pitch = P / 2, u = y + h P / 2, v = u + 1, c_pitch = P / 2, c_step = 2, msb = 1.
+ * Refusals as for the 8-bit calls, and an msb other than 0 or 1.
+ */
+int savsr_yuv420_10_to_bgr48(savsr_ctx* ctx, const uint16_t* y, int y_pitch, const uint16_t* u, const uint16_t* v, int c_pitch, int c_step,
+                             int64_t frame_stride, int msb, int n, int h, int w, uint16_t* bgr, savsr_stream st);
+int savsr_bgr48_to_yuv420_10(savsr_ctx* ctx, const uint16_t* bgr, int n, int h, int w, uint16_t* y, int y_pitch, uint16_t* u, uint16_t* v,
+                             int c_pitch, int c_step, int64_t frame_stride, int msb, savsr_stream st);
+/* uint8 BGR [n][h][w][3] -> uint16 BGR (each value times 257, so v / 65535 of the result is u / 255 of the source): brings 8-bit
+ * frames into a ring of 16-bit frames, for an 8-bit source upscaled to deep output.  Both buffers contiguous; n = 0 launches nothing. */
+int savsr_widen_u8_to_u16(savsr_ctx* ctx, const uint8_t* src, int n, int h, int w, uint16_t* dst, savsr_stream st);
 
 /* ---- post-processing / metrics on the device (next row 8f3) -------------------------------------------------------
  * tensor2img (lbasicsr/utils/img_util.py:38-94): sr fp32 NCHW [batch][3][H][W] RGB -> uint8 HWC BGR [batch][H][W][3]

@@ -170,9 +170,11 @@ SIGNATURES = {
     "savsr_plan_set_io": (_I, [_VP, _VP, _SZ, _VP, _SZ, _I]),
     "savsr_plan_set_io_u8": (_I, [_VP, _VP, _SZ, _VP, _SZ, _I]),
     "savsr_plan_set_io_u8_table": (_I, [_VP, _VP, _I, _VP, _SZ, _I]),
+    "savsr_plan_set_io_u16_table": (_I, [_VP, _VP, _I, _VP, _SZ, _I]),
     "savsr_plan_add_pack_frames": (_I, [_VP, _VP, _VP, _I, _I, _I, _I]),
     "savsr_plan_add_pack_frames_u8": (_I, [_VP, _VP, _VP, _I, _I, _I, _I]),
     "savsr_plan_add_pack_frames_u8_table": (_I, [_VP, _VP, _VP, _I, _I, _I, _I]),
+    "savsr_plan_add_pack_frames_u16_table": (_I, [_VP, _VP, _VP, _I, _I, _I, _I]),
     "savsr_plan_add_conv": (_I, [_VP, _VP, C.POINTER(ConvGroup), _I, _I, _I, _I, _I]),
     "savsr_plan_add_osa_prologue": (_I, [_VP, C.POINTER(OsaParams), _I, _I, _I, _I, _F, _F]),
     "savsr_plan_add_ca_scale_residual": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _VP, _VP, _VP, _VP, _VP]),
@@ -181,17 +183,23 @@ SIGNATURES = {
     "savsr_plan_add_satu_hr": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP]),
     "savsr_plan_add_satu_hr_u8": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP]),
     "savsr_plan_add_satu_hr_u8_table": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP]),
+    "savsr_plan_add_satu_hr_u16_table": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP]),
     "savsr_plan_add_arena_export": (_I, [_VP, _VP, _I, _VP]),
     "savsr_plan_run": (_I, [_VP, _VP]),
     "savsr_forward": (_I, [_VP, _VP, _VP, _VP]),
     "savsr_forward_u8": (_I, [_VP, _VP, _VP, _VP]),
     "savsr_forward_u8_frames": (_I, [_VP, _VP, _VP, _VP]),
+    "savsr_forward_u16_frames": (_I, [_VP, _VP, _VP, _VP]),
     "savsr_write_frame_table": (_I, [_VP, _VP, _VP, _I, _VP]),
     "savsr_yuv420_to_bgr": (_I, [_VP, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _I, _VP, _VP]),
     "savsr_bgr_to_yuv420": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _VP]),
+    "savsr_yuv420_10_to_bgr48": (_I, [_VP, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _I, _I, _VP, _VP]),
+    "savsr_bgr48_to_yuv420_10": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _I, _VP]),
+    "savsr_widen_u8_to_u16": (_I, [_VP, _VP, _I, _I, _I, _VP, _VP]),
     "savsr_pack_frames": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),
     "savsr_pack_frames_u8": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),
     "savsr_pack_frames_u8_table": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),
+    "savsr_pack_frames_u16_table": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),
     "savsr_osa_prologue": (_I, [_VP, C.POINTER(OsaParams), _I, _I, _I, _I, _F, _F, _VP]),
     "savsr_ca_scale_residual": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _VP, _VP, _VP, _VP, _VP, _VP]),
     "savsr_osadapt_mask": (_I, [_VP, _VP, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _VP]),
@@ -200,6 +208,7 @@ SIGNATURES = {
     "savsr_satu_hr": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP, _VP]),
     "savsr_satu_hr_u8": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP, _VP]),
     "savsr_satu_hr_u8_table": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP, _VP]),
+    "savsr_satu_hr_u16_table": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP, _VP, _VP, _I, _I, _VP, _VP]),
     "savsr_img_metrics_blocks": (_I, [_VP, _I, _I]),
     "savsr_img_metrics": (_I, [_VP, _VP, _VP, _I, _I, _I, _VP, _VP, _VP]),
     "savsr_ssim_y_blocks": (_I, [_I, _I]),

@@ -262,18 +262,52 @@ class SAVSR(nn.Module):
         The pool is read on the device's current stream: it must stay valid, in stream order, until the forward has run."""
         if scale is not None:
             self.scale = scale
-        return self._forward_bgr_u8_indexed(pool, windows, self.scale)
+        return self._forward_bgr_u8_indexed(pool, windows, self.scale, dtype=torch.uint8)
 
-    def _forward_bgr_u8_indexed(self, pool: torch.Tensor, windows, scale, out_format: str = "bgr24") -> torch.Tensor:
-        """forward_bgr_u8_indexed at `scale`, leaving self.scale as it is (savsr_b200.VideoUpscaler keeps its own scale).  With out_format
-        "yuv420p" or "nv12" the HR frames come back as uint8 [b, 3H/2, W] YUV 4:2:0 (savsr_b200.colour), converted from the plan's
-        output staging buffer instead of copied."""
+    def forward_bgr48(self, x: torch.Tensor, scale=None) -> torch.Tensor:
+        """Upscale deep video: x uint16 [b, 7, h, w, 3] BGR windows (bgr48, full scale 65535: 16-bit PNG / TIFF frames as
+        cv2.IMREAD_UNCHANGED loads them, or decoded 10-bit video) on CUDA -> a fresh uint16 [b, H, W, 3] BGR tensor.  Bit for bit
+        round(clamp(forward(x') , 0, 1) * 65535) in fp32 with round half to even, where x' = the windows as fp32 RGB planes, v / 65535
+        correctly rounded.  On 257 * x8 it computes what forward_bgr_u8 computes on x8, before the output's quantisation.  The windows
+        are read in place through a frame table (the plan of forward_bgr48_indexed), so x must stay valid, in stream order, until the
+        forward has run.  Inference only; same plan cache, precision and CUDA graphs as forward."""
         if self.training:
-            raise RuntimeError("forward_bgr_u8_indexed is inference only: call eval() first (training takes fp32 windows through forward)")
-        if pool.dtype != torch.uint8:
-            raise TypeError(f"forward_bgr_u8_indexed takes a uint8 frame pool, got {pool.dtype}")
+            raise RuntimeError("forward_bgr48 is inference only: call eval() first (training takes fp32 windows through forward)")
+        if scale is not None:
+            self.scale = scale
+        if x.dtype != torch.uint16:
+            raise TypeError(f"forward_bgr48 takes uint16 windows, got {x.dtype}")
+        if x.dim() != 5 or x.shape[1] != self.num_frame or x.shape[4] != 3:
+            raise ValueError(f"expected uint16 BGR windows [b, {self.num_frame}, h, w, 3], got {tuple(x.shape)}")
+        b, t, h, w, _ = x.shape
+        windows = torch.arange(b * t).reshape(b, t)
+        return self._forward_bgr_u8_indexed(x.reshape(b * t, h, w, 3), windows, self.scale, dtype=torch.uint16)
+
+    def forward_bgr48_indexed(self, pool: torch.Tensor, windows, scale=None) -> torch.Tensor:
+        """forward_bgr48(pool[windows]), bit for bit, without gathering the windows: pool is a contiguous uint16 CUDA tensor [N, h, w, 3]
+        of bgr48 frames, windows as for forward_bgr_u8_indexed.  Returns a fresh uint16 [b, H, W, 3] BGR tensor; the pool is read on
+        the device's current stream and must stay valid, in stream order, until the forward has run."""
+        if scale is not None:
+            self.scale = scale
+        return self._forward_bgr_u8_indexed(pool, windows, self.scale, dtype=torch.uint16)
+
+    def _forward_bgr_u8_indexed(self, pool: torch.Tensor, windows, scale, out_format: Optional[str] = None,
+                                dtype: Optional[torch.dtype] = None) -> torch.Tensor:
+        """forward_bgr_u8_indexed (uint8 pool) or forward_bgr48_indexed (uint16 pool) at `scale`, leaving self.scale as it is
+        (savsr_b200.VideoUpscaler keeps its own scale).  The I/O mode follows the pool's dtype; `dtype`, when given, is the one the
+        public caller takes.  With a YUV out_format of the pool's depth ("yuv420p" / "nv12" for uint8, "yuv420p10le" / "p010" for uint16)
+        the HR frames come back as [b, 3H/2, W] YUV 4:2:0 (savsr_b200.colour), converted from the plan's output staging buffer instead
+        of copied; None is packed BGR."""
+        name = {torch.uint16: "forward_bgr48_indexed"}.get(dtype if dtype is not None else pool.dtype, "forward_bgr_u8_indexed")
+        if self.training:
+            raise RuntimeError(f"{name} is inference only: call eval() first (training takes fp32 windows through forward)")
+        want = (dtype,) if dtype is not None else tuple(engine.FRAME_MODES.values())
+        if pool.dtype not in want:
+            raise TypeError(f"{name} takes a {' or '.join(str(d).replace('torch.', '') for d in want)} frame pool, got {pool.dtype}")
+        io = "bgr48_frames" if pool.dtype == torch.uint16 else "bgr_u8_frames"
+        tn = str(pool.dtype).replace("torch.", "")
         if pool.dim() != 4 or pool.shape[3] != 3:
-            raise ValueError(f"expected a uint8 BGR frame pool [N, h, w, 3], got {tuple(pool.shape)}")
+            raise ValueError(f"expected a {tn} BGR frame pool [N, h, w, 3], got {tuple(pool.shape)}")
         if not pool.is_contiguous():
             raise ValueError("the frame pool must be contiguous (each row one [h, w, 3] frame)")
         idx = torch.as_tensor(windows)
@@ -286,20 +320,24 @@ class SAVSR(nn.Module):
         n, h, w, _ = pool.shape
         b = idx.shape[0]
         self._check_device(pool)
+        bgr = "bgr48le" if io == "bgr48_frames" else "bgr24"
+        out_format = bgr if out_format is None else colour.check_format(out_format, "out_format")
+        if colour.bgr_format(out_format) != bgr:
+            raise ValueError(f"out_format {out_format!r} has another depth than the {tn} frame pool")
         if b == 0:
             H, W = engine.get_hw(h, w, scale)
-            return pool.new_empty((0, H, W, 3) if out_format == "bgr24" else (0, *colour.yuv_shape(H, W)))
+            return pool.new_empty((0, H, W, 3) if out_format == bgr else (0, *colour.yuv_shape(H, W)))
         idx = idx.to(torch.int64)
         lo, hi = int(idx.min()), int(idx.max())
         if lo < 0 or hi >= n:
             raise IndexError(f"window row index {lo if lo < 0 else hi} out of range for a pool of {n} frames")
-        ptrs = (idx.reshape(-1) * (h * w * 3) + pool.data_ptr()).tolist()
-        return self._run_plan(self._plan(b, h, w, pool.device, "bgr_u8_frames", scale), frames=ptrs, out_format=out_format)
+        ptrs = (idx.reshape(-1) * (h * w * 3 * pool.element_size()) + pool.data_ptr()).tolist()
+        return self._run_plan(self._plan(b, h, w, pool.device, io, scale), frames=ptrs, out_format=out_format)
 
     def _run_plan(self, plan: engine.Plan, x: Optional[torch.Tensor] = None, frames: Optional[list] = None,
                   out_format: str = "bgr24") -> torch.Tensor:
         with torch.cuda.device(plan.device):
-            if out_format == "bgr24":
+            if out_format in ("bgr24", "bgr48le"):
                 out = torch.empty_like(plan.out)
             else:
                 out = plan.out.new_empty((plan.B, *colour.yuv_shape(plan.H, plan.W)))
@@ -381,7 +419,8 @@ class SAVSR(nn.Module):
 
     def plan_for(self, x: torch.Tensor, io: str = "f32") -> engine.Plan:
         """The cached plan for windows like `x`: io="f32" takes [b, 7, 3, h, w] (forward), io="bgr_u8" uint8 [b, 7, h, w, 3]
-        (forward_bgr_u8).  Plans of every I/O mode (also "bgr_u8_frames", forward_bgr_u8_indexed) share one WeightStore."""
+        (forward_bgr_u8).  Plans of every I/O mode (also "bgr_u8_frames" and "bgr48_frames", the *_indexed forwards) share one
+        WeightStore."""
         b, h, w = self._window_shape(x, io)
         return self._plan(b, h, w, x.device, io, self.scale)
 

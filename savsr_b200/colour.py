@@ -1,4 +1,4 @@
-"""YUV 4:2:0 <-> packed 8-bit BGR on the device, byte-identical to OpenCV's ``cv2.cvtColor``.
+"""YUV 4:2:0 <-> packed BGR on the device: 8-bit byte-identical to OpenCV's ``cv2.cvtColor``, and 10-bit YUV <-> 16-bit BGR.
 
 Video decoders hand out YUV 4:2:0 (NVDEC: NV12 surfaces in device memory; ``ffmpeg -f rawvideo -pix_fmt yuv420p``: planar I420) and
 encoders take it back, while ``SAVSR.forward_bgr_u8`` and ``VideoUpscaler`` work on packed BGR [h, w, 3].  The formats carry ffmpeg's
@@ -10,10 +10,20 @@ encoders take it back, while ``SAVSR.forward_bgr_u8`` and ``VideoUpscaler`` work
   row pitch (``stride(0) >= w``, ``stride(1) == 1``; the UV rows start at row h of the same pitch), as a decoder surface does when it
   is exposed as a tensor view.  yuv420p frames must have contiguous rows.
 
+Deep video (HEVC Main10, 10-bit AV1, 16-bit PNG / TIFF sequences) has formats of its own, all uint16:
+
+* ``"bgr48le"``: uint16 [h, w, 3] BGR, full scale 65535 (``cv2.imread(path, cv2.IMREAD_UNCHANGED)`` of a 16-bit image);
+* ``"yuv420p10le"``: one uint16 [3h/2, w] array per frame laid out as yuv420p, the 10-bit value in bits 0-9 (ffmpeg's rawvideo);
+* ``"p010"``: one uint16 [3h/2, w] array per frame laid out as nv12, the value in bits 6-15 (NVDEC's 10-bit surfaces); it may have a
+  row pitch like nv12.
+
 Several frames are [n, 3h/2, w].  The conversion is BT.601, limited range, in OpenCV's 20-bit fixed point: decoding gives each pixel
 the chroma sample of its 2x2 block (``COLOR_YUV2BGR_I420`` / ``COLOR_YUV2BGR_NV12``), encoding takes U and V from the top-left
-pixel of each 2x2 block (``COLOR_BGR2YUV_I420``).  Sizes must be even, as cv2 requires.  Each call is one launch on the current
-stream of the tensors' device (savsr_yuv420_to_bgr / savsr_bgr_to_yuv420 of libsavsr_sm100); there is no CPU path.
+pixel of each 2x2 block (``COLOR_BGR2YUV_I420``).  Sizes must be even, as cv2 requires.  The 10-bit formats use the same matrix
+and chroma handling, rescaled (one 10-bit step is a quarter of an 8-bit step, one 8-bit BGR step is 257 sixteen-bit steps), in a
+fixed-point form within 0.53 of an output step of the real-valued map; decoding saturates to [0, 65535].  Each call is one launch on
+the current stream of the tensors' device (savsr_yuv420_to_bgr / savsr_bgr_to_yuv420, savsr_yuv420_10_to_bgr48 /
+savsr_bgr48_to_yuv420_10 of libsavsr_sm100); there is no CPU path.
 """
 from __future__ import annotations
 
@@ -23,8 +33,20 @@ import torch
 
 from . import _capi as K, engine
 
-FORMATS = ("bgr24", "yuv420p", "nv12")
-YUV_FORMATS = ("yuv420p", "nv12")
+FORMATS = ("bgr24", "yuv420p", "nv12", "bgr48le", "yuv420p10le", "p010")
+YUV_FORMATS = ("yuv420p", "nv12", "yuv420p10le", "p010")
+DEEP_FORMATS = ("bgr48le", "yuv420p10le", "p010")
+PITCHED_FORMATS = ("nv12", "p010")          # may have a row pitch; their U, V samples are interleaved
+
+
+def dtype_of(fmt: str) -> torch.dtype:
+    """The sample type of `fmt`: uint16 for the deep formats, uint8 otherwise."""
+    return torch.uint16 if fmt in DEEP_FORMATS else torch.uint8
+
+
+def bgr_format(fmt: str) -> str:
+    """The packed BGR format of the same depth: what the forward reads and writes for `fmt`."""
+    return "bgr48le" if fmt in DEEP_FORMATS else "bgr24"
 
 
 def check_format(fmt: str, what: str = "format") -> str:
@@ -39,16 +61,18 @@ def yuv_shape(h: int, w: int) -> Tuple[int, int]:
 
 
 def yuv_frames(x: torch.Tensor, fmt: str, h: Optional[int] = None, w: Optional[int] = None) -> torch.Tensor:
-    """Check that x holds uint8 `fmt` frames ([3h/2, w] or [n, 3h/2, w]; h x w from the shape when not given) with a layout the
-    kernels read, and return it as [n, 3h/2, w].  Wherever x lives: the device is the caller's concern."""
+    """Check that x holds `fmt` frames (uint8, uint16 for the 10-bit formats; [3h/2, w] or [n, 3h/2, w]; h x w from the shape when not
+    given) with a layout the kernels read, and return it as [n, 3h/2, w].  Wherever x lives: the device is the caller's concern."""
     if fmt not in YUV_FORMATS:
         raise ValueError(f"{fmt!r} is not a YUV 4:2:0 format ({', '.join(YUV_FORMATS)})")
-    if x.dtype != torch.uint8:
-        raise TypeError(f"{fmt} frames are uint8, got {x.dtype}")
+    dt = dtype_of(fmt)
+    tn = str(dt).replace("torch.", "")
+    if x.dtype != dt:
+        raise TypeError(f"{fmt} frames are {tn}, got {x.dtype}")
     if h is None:
         rows, w = (x.shape[-2], x.shape[-1]) if x.dim() in (2, 3) else (0, 0)
         if rows % 3 or rows == 0:
-            raise ValueError(f"expected uint8 {fmt} frames [3h/2, w] or [n, 3h/2, w], got {tuple(x.shape)}")
+            raise ValueError(f"expected {tn} {fmt} frames [3h/2, w] or [n, 3h/2, w], got {tuple(x.shape)}")
         h = 2 * rows // 3
     if h % 2 or w % 2:
         raise ValueError(f"{fmt} needs an even frame size, got {h}x{w}")
@@ -56,24 +80,26 @@ def yuv_frames(x: torch.Tensor, fmt: str, h: Optional[int] = None, w: Optional[i
         x = x.unsqueeze(0)
     if x.dim() != 3 or tuple(x.shape[1:]) != yuv_shape(h, w):
         rows = yuv_shape(h, w)[0]
-        raise ValueError(f"expected uint8 {fmt} frames [{rows}, {w}] or [n, {rows}, {w}], got {tuple(x.shape)}")
+        raise ValueError(f"expected {tn} {fmt} frames [{rows}, {w}] or [n, {rows}, {w}], got {tuple(x.shape)}")
     if x.stride(2) != 1:
         raise ValueError(f"{fmt} frames need a unit column stride, got {x.stride(2)}")
-    if fmt == "yuv420p" and x.stride(1) != w:
-        raise ValueError(f"yuv420p frames must have contiguous rows: row stride {x.stride(1)} != width {w} (only nv12 takes a row pitch)")
+    if fmt not in PITCHED_FORMATS and x.stride(1) != w:
+        raise ValueError(f"{fmt} frames must have contiguous rows: row stride {x.stride(1)} != width {w} "
+                         f"(only {' and '.join(PITCHED_FORMATS)} take a row pitch)")
     if x.stride(1) < w:
         raise ValueError(f"{fmt} row stride {x.stride(1)} is below the width {w}")
     return x
 
 
 def _planes(x: torch.Tensor, fmt: str, h: int, w: int) -> tuple:
-    """(y, y_pitch, u, v, c_pitch, c_step, frame_stride) of frames x [n, 3h/2, w] (checked by yuv_frames)."""
-    p, pitch = x.data_ptr(), x.stride(1)
-    if fmt == "yuv420p":
-        u = p + h * w
-        return p, w, u, u + (h // 2) * (w // 2), w // 2, 1, x.stride(0)
-    u = p + h * pitch
-    return p, pitch, u, u + 1, pitch, 2, x.stride(0)
+    """(y, y_pitch, u, v, c_pitch, c_step, frame_stride) of frames x [n, 3h/2, w] (checked by yuv_frames): addresses in bytes, pitches
+    and the frame stride in elements (bytes for the 8-bit formats, uint16 samples for the 10-bit ones)."""
+    p, pitch, e = x.data_ptr(), x.stride(1), x.element_size()
+    if fmt not in PITCHED_FORMATS:
+        u = p + h * w * e
+        return p, w, u, u + (h // 2) * (w // 2) * e, w // 2, 1, x.stride(0)
+    u = p + h * pitch * e
+    return p, pitch, u, u + e, pitch, 2, x.stride(0)
 
 
 def _on_cuda(*xs: torch.Tensor) -> torch.device:
@@ -86,55 +112,63 @@ def _on_cuda(*xs: torch.Tensor) -> torch.device:
     return dev
 
 
-def _bgr(x: torch.Tensor, what: str) -> torch.Tensor:
-    if x.dtype != torch.uint8:
-        raise TypeError(f"{what} takes uint8 BGR frames, got {x.dtype}")
+def _bgr(x: torch.Tensor, what: str, dt: torch.dtype = torch.uint8) -> torch.Tensor:
+    tn = str(dt).replace("torch.", "")
+    if x.dtype != dt:
+        raise TypeError(f"{what} takes {tn} BGR frames, got {x.dtype}")
     if x.dim() == 3:
         x = x.unsqueeze(0)
     if x.dim() != 4 or x.shape[3] != 3:
-        raise ValueError(f"{what}: expected uint8 BGR frames [h, w, 3] or [n, h, w, 3], got {tuple(x.shape)}")
+        raise ValueError(f"{what}: expected {tn} BGR frames [h, w, 3] or [n, h, w, 3], got {tuple(x.shape)}")
     if not x.is_contiguous():
         raise ValueError(f"{what}: BGR frames must be contiguous")
     return x
 
 
 def yuv420_to_bgr(frames: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """uint8 `fmt` frames ("yuv420p" or "nv12", [3h/2, w] or [n, 3h/2, w], CUDA) -> uint8 BGR [h, w, 3] or [n, h, w, 3], as
-    cv2.cvtColor(frame, COLOR_YUV2BGR_I420 or COLOR_YUV2BGR_NV12) of each frame.  Writes `out` (contiguous, that shape) when given,
-    else a fresh tensor.  One launch on the current stream; the frames must stay valid, in stream order, until it has run."""
+    """`fmt` frames ([3h/2, w] or [n, 3h/2, w], CUDA) -> BGR [h, w, 3] or [n, h, w, 3] of the same depth.  "yuv420p" and "nv12" (uint8)
+    decode to uint8 BGR as cv2.cvtColor(frame, COLOR_YUV2BGR_I420 or COLOR_YUV2BGR_NV12) of each frame; "yuv420p10le" and "p010" (uint16)
+    to uint16 bgr48 with the same matrix.  Writes `out` (contiguous, that shape and dtype) when given, else a fresh tensor.  One launch
+    on the current stream; the frames must stay valid, in stream order, until it has run."""
     x = yuv_frames(frames, fmt)
     n, h, w = x.shape[0], 2 * x.shape[1] // 3, x.shape[2]
     shape = (n, h, w, 3) if frames.dim() == 3 else (h, w, 3)
+    dt = dtype_of(fmt)
     if out is None:
         _on_cuda(x)
-        out = torch.empty(shape, dtype=torch.uint8, device=x.device)
-    elif tuple(out.shape) != shape or out.dtype != torch.uint8 or not out.is_contiguous():
-        raise ValueError(f"out must be a contiguous uint8 tensor of shape {shape}, got {out.dtype} {tuple(out.shape)}")
+        out = torch.empty(shape, dtype=dt, device=x.device)
+    elif tuple(out.shape) != shape or out.dtype != dt or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous {str(dt).replace('torch.', '')} tensor of shape {shape}, got {out.dtype} {tuple(out.shape)}")
     dev = _on_cuda(x, out)
     if n == 0:
         return out
     ctx = engine.context(dev.index)
     y, yp, u, v, cp, cs, fs = _planes(x, fmt, h, w)
+    st = torch.cuda.current_stream(dev).cuda_stream
     with torch.cuda.device(dev):
-        K.check(ctx.lib.savsr_yuv420_to_bgr(ctx.handle, y, yp, u, v, cp, cs, fs, n, h, w, out.data_ptr(),
-                                            torch.cuda.current_stream(dev).cuda_stream))
+        if fmt in DEEP_FORMATS:
+            K.check(ctx.lib.savsr_yuv420_10_to_bgr48(ctx.handle, y, yp, u, v, cp, cs, fs, int(fmt == "p010"), n, h, w, out.data_ptr(), st))
+        else:
+            K.check(ctx.lib.savsr_yuv420_to_bgr(ctx.handle, y, yp, u, v, cp, cs, fs, n, h, w, out.data_ptr(), st))
     return out
 
 
 def bgr_to_yuv420(bgr: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """uint8 BGR [H, W, 3] or [n, H, W, 3] (contiguous, CUDA, H and W even) -> uint8 `fmt` frames [3H/2, W] or [n, 3H/2, W], as
-    cv2.cvtColor(frame, COLOR_BGR2YUV_I420) of each frame, with U and V interleaved for "nv12".  Writes `out` when given (any layout
-    yuv_frames accepts, e.g. a pitched NV12 surface), else a fresh contiguous tensor.  One launch on the current stream."""
+    """BGR [H, W, 3] or [n, H, W, 3] (contiguous, CUDA, H and W even) -> `fmt` frames [3H/2, W] or [n, 3H/2, W].  uint8 BGR to "yuv420p"
+    or "nv12" as cv2.cvtColor(frame, COLOR_BGR2YUV_I420) of each frame, with U and V interleaved for "nv12"; uint16 bgr48 to
+    "yuv420p10le" or "p010" with the same matrix.  Writes `out` when given (any layout yuv_frames accepts, e.g. a pitched NV12 or P010
+    surface), else a fresh contiguous tensor.  One launch on the current stream."""
     if fmt not in YUV_FORMATS:
         raise ValueError(f"{fmt!r} is not a YUV 4:2:0 format ({', '.join(YUV_FORMATS)})")
-    x = _bgr(bgr, "bgr_to_yuv420")
+    dt = dtype_of(fmt)
+    x = _bgr(bgr, f"bgr_to_yuv420 to {fmt}", dt)
     n, H, W = x.shape[:3]
     shape = (n, *yuv_shape(H, W)) if bgr.dim() == 4 else yuv_shape(H, W)
     if H % 2 or W % 2:
         raise ValueError(f"{fmt} needs an even frame size, got {H}x{W}")
     if out is None:
         _on_cuda(x)
-        out = torch.empty(shape, dtype=torch.uint8, device=x.device)
+        out = torch.empty(shape, dtype=dt, device=x.device)
     elif tuple(out.shape) != shape:
         raise ValueError(f"out must have shape {shape}, got {tuple(out.shape)}")
     o = yuv_frames(out, fmt, H, W)
@@ -145,7 +179,26 @@ def bgr_to_yuv420(bgr: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = Non
         return out
     ctx = engine.context(dev.index)
     y, yp, u, v, cp, cs, fs = _planes(o, fmt, H, W)
+    st = torch.cuda.current_stream(dev).cuda_stream
     with torch.cuda.device(dev):
-        K.check(ctx.lib.savsr_bgr_to_yuv420(ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, cs, fs,
-                                            torch.cuda.current_stream(dev).cuda_stream))
+        if fmt in DEEP_FORMATS:
+            K.check(ctx.lib.savsr_bgr48_to_yuv420_10(ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, cs, fs, int(fmt == "p010"), st))
+        else:
+            K.check(ctx.lib.savsr_bgr_to_yuv420(ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, cs, fs, st))
+    return out
+
+
+def widen(bgr: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+    """uint8 BGR [h, w, 3] or [n, h, w, 3] (contiguous, CUDA) -> `out`, uint16 of the same shape (contiguous, CUDA): each value times
+    257, so that out / 65535 is bgr / 255 exactly.  An 8-bit source enters a 16-bit pipeline this way.  One launch on the current stream."""
+    x = _bgr(bgr, "widen")
+    if out.dtype != torch.uint16 or tuple(out.shape) != tuple(bgr.shape) or not out.is_contiguous():
+        raise ValueError(f"out must be a contiguous uint16 tensor of shape {tuple(bgr.shape)}, got {out.dtype} {tuple(out.shape)}")
+    dev = _on_cuda(x, out)
+    n, h, w = x.shape[:3]
+    if n == 0:
+        return out
+    ctx = engine.context(dev.index)
+    with torch.cuda.device(dev):
+        K.check(ctx.lib.savsr_widen_u8_to_u16(ctx.handle, x.data_ptr(), n, h, w, out.data_ptr(), torch.cuda.current_stream(dev).cuda_stream))
     return out

@@ -12,6 +12,10 @@
 // two rows), so every chroma sample is read or written once, and moves each row's bytes with the widest loads and stores the row's
 // alignment allows (all rows of one frame row share it; see load_bytes / store_bytes).  A row's last group may be narrower (w % 8): it
 // takes the byte-wise path.
+//
+// 10-bit YUV 4:2:0 <-> 16-bit BGR (yuv420p10le, p010 <-> bgr48): the same matrix, chroma handling and work split in fixed-point forms
+// rescaled to the deeper samples (common.cuh), with pitches and frame strides in uint16 elements.  A thread's rows are 16 bytes of Y and
+// 48 of BGR, so 16-byte accesses are used where the row's alignment allows.  widen_u8_to_u16 brings 8-bit BGR frames into a 16-bit ring.
 #include "common.cuh"
 
 namespace savsr {
@@ -22,7 +26,13 @@ constexpr int kYuvGroup = 8;   // pixels per thread and row: four 2x2 chroma blo
 template <int N>
 __device__ __forceinline__ void load_bytes(const uint8_t* __restrict__ p, uint32_t (&w)[N / 4]) {
   const unsigned a = static_cast<unsigned>(reinterpret_cast<uintptr_t>(p));
-  if (N % 8 == 0 && (a & 7) == 0) {
+  if (N % 16 == 0 && (a & 15) == 0) {
+#pragma unroll
+    for (int i = 0; i < N / 16; ++i) {
+      const uint4 v = reinterpret_cast<const uint4*>(p)[i];
+      w[4 * i] = v.x; w[4 * i + 1] = v.y; w[4 * i + 2] = v.z; w[4 * i + 3] = v.w;
+    }
+  } else if (N % 8 == 0 && (a & 7) == 0) {
 #pragma unroll
     for (int i = 0; i < N / 8; ++i) {
       const uint2 v = reinterpret_cast<const uint2*>(p)[i];
@@ -46,7 +56,10 @@ __device__ __forceinline__ void load_bytes(const uint8_t* __restrict__ p, uint32
 template <int N>
 __device__ __forceinline__ void store_bytes(uint8_t* __restrict__ p, const uint32_t (&w)[N / 4]) {
   const unsigned a = static_cast<unsigned>(reinterpret_cast<uintptr_t>(p));
-  if (N % 8 == 0 && (a & 7) == 0) {
+  if (N % 16 == 0 && (a & 15) == 0) {
+#pragma unroll
+    for (int i = 0; i < N / 16; ++i) reinterpret_cast<uint4*>(p)[i] = make_uint4(w[4 * i], w[4 * i + 1], w[4 * i + 2], w[4 * i + 3]);
+  } else if (N % 8 == 0 && (a & 7) == 0) {
 #pragma unroll
     for (int i = 0; i < N / 8; ++i) reinterpret_cast<uint2*>(p)[i] = make_uint2(w[2 * i], w[2 * i + 1]);
   } else if ((a & 3) == 0) {
@@ -224,21 +237,209 @@ __global__ void __launch_bounds__(256) bgr_to_yuv420_kernel(const uint8_t* __res
   }
 }
 
-// The checks both entry points make before any launch.
-static int check_yuv420(const char* fn, int n, int h, int w, int y_pitch, int c_pitch, int c_step, long long frame_stride) {
+// ------------------------------------------------------------------------------------------------ 10-bit YUV <-> 16-bit BGR
+template <int N>
+__device__ __forceinline__ int half_at(const uint32_t (&w)[N], int i) { return (w[i >> 1] >> (16 * (i & 1))) & 0xffff; }
+template <int N>
+__device__ __forceinline__ void put_half(uint32_t (&w)[N], int i, int v) { w[i >> 1] |= static_cast<uint32_t>(v) << (16 * (i & 1)); }
+
+__device__ __forceinline__ int sat_u16(int v) { return min(max(v, 0), 65535); }
+// A 10-bit sample from its 16-bit container: p010 keeps it in bits 6-15, yuv420p10le in bits 0-9.
+__device__ __forceinline__ int sample10(int s, int msb) { return msb ? s >> 6 : s & 0x3ff; }
+
+struct Chroma10 {
+  long long r, g, b;
+  Chroma10() = default;
+  __device__ __forceinline__ Chroma10(int U, int V) {
+    const int u = U - 512, v = V - 512;
+    r = kYuv10Half + static_cast<long long>(kYuv10VR) * v;
+    g = kYuv10Half + static_cast<long long>(kYuv10VG) * v + static_cast<long long>(kYuv10UG) * u;
+    b = kYuv10Half + static_cast<long long>(kYuv10UB) * u;
+  }
+  __device__ __forceinline__ void bgr(int Y, int& B, int& G, int& R) const {
+    const long long y = static_cast<long long>(max(Y - 64, 0)) * kYuv10Y;
+    B = sat_u16(static_cast<int>((y + b) >> kYuv10Shift));
+    G = sat_u16(static_cast<int>((y + g) >> kYuv10Shift));
+    R = sat_u16(static_cast<int>((y + r) >> kYuv10Shift));
+  }
+};
+__device__ __forceinline__ int rgb_y10(int R, int G, int B) {
+  return (kRgb10YR * R + kRgb10YG * G + kRgb10YB * B + (64 << kRgb10Shift) + kRgb10Half) >> kRgb10Shift;
+}
+__device__ __forceinline__ int rgb_u10(int R, int G, int B) {
+  return (kRgb10UR * R + kRgb10UG * G + kRgb10UB * B + (512 << kRgb10Shift) + kRgb10Half) >> kRgb10Shift;
+}
+__device__ __forceinline__ int rgb_v10(int R, int G, int B) {
+  return (kRgb10VR * R + kRgb10VG * G + kRgb10VB * B + (512 << kRgb10Shift) + kRgb10Half) >> kRgb10Shift;
+}
+
+// Yuv420Planes in uint16 elements, plus where the 10 bits sit (msb: 1 for p010, 0 for yuv420p10le).
+struct Yuv420Planes16 {
+  uint16_t* y;
+  uint16_t* u;
+  uint16_t* v;
+  int y_pitch, c_pitch, c_step;
+  long long frame_stride;
+  int msb;
+};
+
+template <class T>
+__device__ __forceinline__ const uint8_t* as_bytes(const T* p) { return reinterpret_cast<const uint8_t*>(p); }
+template <class T>
+__device__ __forceinline__ uint8_t* as_bytes(T* p) { return reinterpret_cast<uint8_t*>(p); }
+
+__global__ void __launch_bounds__(256) yuv420_10_to_bgr48_kernel(const Yuv420Planes16 p, int n, int h, int w, uint16_t* __restrict__ bgr) {
+  const int groups = (w + kYuvGroup - 1) / kYuvGroup, half_h = h >> 1;
+  const long long total = static_cast<long long>(n) * half_h * groups;
+  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
+       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
+    int f, rp, x0;
+    yuv_item(idx, groups, half_h, f, rp, x0);
+    const long long fo = f * p.frame_stride;
+    const uint16_t* y0 = p.y + fo + static_cast<long long>(2 * rp) * p.y_pitch + x0;
+    const uint16_t* y1 = y0 + p.y_pitch;
+    const long long co = fo + static_cast<long long>(rp) * p.c_pitch + (x0 >> 1) * p.c_step;
+    const uint16_t* u = p.u + co;
+    const uint16_t* v = p.v + co;
+    uint16_t* o0 = bgr + ((static_cast<long long>(f) * h + 2 * rp) * w + x0) * 3;
+    uint16_t* o1 = o0 + static_cast<long long>(w) * 3;
+    if (x0 + kYuvGroup <= w) {
+      uint32_t ya[4], yb[4], uw[2], vw[2];
+      load_bytes<16>(as_bytes(y0), ya);
+      load_bytes<16>(as_bytes(y1), yb);
+      if (p.c_step == 1) {
+        load_bytes<8>(as_bytes(u), uw);
+        load_bytes<8>(as_bytes(v), vw);
+      } else {                                     // p010: U0 V0 U1 V1 U2 V2 U3 V3, 16 bits each
+        uint32_t uv[4];
+        load_bytes<16>(as_bytes(u), uv);
+        uw[0] = __byte_perm(uv[0], uv[1], 0x5410); uw[1] = __byte_perm(uv[2], uv[3], 0x5410);
+        vw[0] = __byte_perm(uv[0], uv[1], 0x7632); vw[1] = __byte_perm(uv[2], uv[3], 0x7632);
+      }
+      Chroma10 c[kYuvGroup / 2];
+#pragma unroll
+      for (int k = 0; k < kYuvGroup / 2; ++k) c[k] = Chroma10(sample10(half_at(uw, k), p.msb), sample10(half_at(vw, k), p.msb));
+#pragma unroll
+      for (int r = 0; r < 2; ++r) {                // one row at a time: the 48 output bytes of a row stay in 12 registers
+        uint32_t o[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+#pragma unroll
+        for (int j = 0; j < kYuvGroup; ++j) {
+          int B, G, R;
+          c[j >> 1].bgr(sample10(half_at(r ? yb : ya, j), p.msb), B, G, R);
+          put_half(o, 3 * j, B); put_half(o, 3 * j + 1, G); put_half(o, 3 * j + 2, R);
+        }
+        store_bytes<48>(as_bytes(r ? o1 : o0), o);
+      }
+    } else {
+      for (int j = 0; x0 + j < w; j += 2) {
+        const Chroma10 c(sample10(u[(j >> 1) * p.c_step], p.msb), sample10(v[(j >> 1) * p.c_step], p.msb));
+#pragma unroll
+        for (int d = 0; d < 2; ++d) {
+          int B, G, R;
+          c.bgr(sample10(y0[j + d], p.msb), B, G, R);
+          o0[3 * (j + d)] = B; o0[3 * (j + d) + 1] = G; o0[3 * (j + d) + 2] = R;
+          c.bgr(sample10(y1[j + d], p.msb), B, G, R);
+          o1[3 * (j + d)] = B; o1[3 * (j + d) + 1] = G; o1[3 * (j + d) + 2] = R;
+        }
+      }
+    }
+  }
+}
+
+__global__ void __launch_bounds__(256) bgr48_to_yuv420_10_kernel(const uint16_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes16 p) {
+  const int groups = (w + kYuvGroup - 1) / kYuvGroup, half_h = h >> 1;
+  const long long total = static_cast<long long>(n) * half_h * groups;
+  const int sh = p.msb ? 6 : 0;
+  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
+       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
+    int f, rp, x0;
+    yuv_item(idx, groups, half_h, f, rp, x0);
+    const long long fo = f * p.frame_stride;
+    uint16_t* y0 = p.y + fo + static_cast<long long>(2 * rp) * p.y_pitch + x0;
+    uint16_t* y1 = y0 + p.y_pitch;
+    const long long co = fo + static_cast<long long>(rp) * p.c_pitch + (x0 >> 1) * p.c_step;
+    uint16_t* u = p.u + co;
+    uint16_t* v = p.v + co;
+    const uint16_t* i0 = bgr + ((static_cast<long long>(f) * h + 2 * rp) * w + x0) * 3;
+    const uint16_t* i1 = i0 + static_cast<long long>(w) * 3;
+    if (x0 + kYuvGroup <= w) {
+      uint32_t ia[12], ib[12];
+      load_bytes<48>(as_bytes(i0), ia);
+      load_bytes<48>(as_bytes(i1), ib);
+      uint32_t ya[4] = {0, 0, 0, 0}, yb[4] = {0, 0, 0, 0}, uw[2] = {0, 0}, vw[2] = {0, 0};
+#pragma unroll
+      for (int j = 0; j < kYuvGroup; ++j) {
+        const int B = half_at(ia, 3 * j), G = half_at(ia, 3 * j + 1), R = half_at(ia, 3 * j + 2);
+        put_half(ya, j, rgb_y10(R, G, B) << sh);
+        if ((j & 1) == 0) {                        // the top-left pixel of its 2x2 block
+          put_half(uw, j >> 1, rgb_u10(R, G, B) << sh);
+          put_half(vw, j >> 1, rgb_v10(R, G, B) << sh);
+        }
+        put_half(yb, j, rgb_y10(half_at(ib, 3 * j + 2), half_at(ib, 3 * j + 1), half_at(ib, 3 * j)) << sh);
+      }
+      store_bytes<16>(as_bytes(y0), ya);
+      store_bytes<16>(as_bytes(y1), yb);
+      if (p.c_step == 1) {
+        store_bytes<8>(as_bytes(u), uw);
+        store_bytes<8>(as_bytes(v), vw);
+      } else {
+        const uint32_t uv[4] = {__byte_perm(uw[0], vw[0], 0x5410), __byte_perm(uw[0], vw[0], 0x7632),
+                                __byte_perm(uw[1], vw[1], 0x5410), __byte_perm(uw[1], vw[1], 0x7632)};
+        store_bytes<16>(as_bytes(u), uv);
+      }
+    } else {
+      for (int j = 0; x0 + j < w; j += 2) {
+        const uint16_t* a = i0 + 3 * j;
+        u[(j >> 1) * p.c_step] = static_cast<uint16_t>(rgb_u10(a[2], a[1], a[0]) << sh);
+        v[(j >> 1) * p.c_step] = static_cast<uint16_t>(rgb_v10(a[2], a[1], a[0]) << sh);
+#pragma unroll
+        for (int d = 0; d < 2; ++d) {
+          const uint16_t* q0 = i0 + 3 * (j + d);
+          const uint16_t* q1 = i1 + 3 * (j + d);
+          y0[j + d] = static_cast<uint16_t>(rgb_y10(q0[2], q0[1], q0[0]) << sh);
+          y1[j + d] = static_cast<uint16_t>(rgb_y10(q1[2], q1[1], q1[0]) << sh);
+        }
+      }
+    }
+  }
+}
+
+// x 257 (u -> u << 8 | u): 16 bytes in, 32 out per thread where both pointers are 16-byte aligned, one byte at a time otherwise.
+__global__ void __launch_bounds__(256) widen_u8_to_u16_kernel(const uint8_t* __restrict__ src, uint16_t* __restrict__ dst, long long count) {
+  const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
+  const long long first = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;
+  const bool vec = ((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 15) == 0;
+  const long long groups = vec ? count / 16 : 0;
+  for (long long i = first; i < groups; i += stride) {
+    const uint4 s = reinterpret_cast<const uint4*>(src)[i];
+    uint4* d = reinterpret_cast<uint4*>(dst) + 2 * i;
+    d[0] = make_uint4(__byte_perm(s.x, 0, 0x1100), __byte_perm(s.x, 0, 0x3322), __byte_perm(s.y, 0, 0x1100), __byte_perm(s.y, 0, 0x3322));
+    d[1] = make_uint4(__byte_perm(s.z, 0, 0x1100), __byte_perm(s.z, 0, 0x3322), __byte_perm(s.w, 0, 0x1100), __byte_perm(s.w, 0, 0x3322));
+  }
+  for (long long i = groups * 16 + first; i < count; i += stride) dst[i] = static_cast<uint16_t>(src[i] * 257);
+}
+
+// The checks the conversion entry points make before any launch (pitches in bytes for 8-bit planes, in elements for 16-bit ones).
+static int check_yuv420(const char* fn, int n, int h, int w, int y_pitch, int c_pitch, int c_step, long long frame_stride,
+                        bool deep = false) {
   SAVSR_REQUIRE(n >= 0 && h > 0 && w > 0, "%s: bad shape n=%d h=%d w=%d", fn, n, h, w);
   SAVSR_REQUIRE(h % 2 == 0 && w % 2 == 0, "%s: YUV 4:2:0 needs an even frame size, got %dx%d", fn, h, w);
-  SAVSR_REQUIRE(c_step == 1 || c_step == 2, "%s: c_step must be 1 (yuv420p) or 2 (nv12), got %d", fn, c_step);
+  SAVSR_REQUIRE(c_step == 1 || c_step == 2, "%s: c_step must be 1 (%s) or 2 (%s), got %d", fn, deep ? "yuv420p10le" : "yuv420p",
+                deep ? "p010" : "nv12", c_step);
   SAVSR_REQUIRE(y_pitch >= w, "%s: y_pitch %d < width %d", fn, y_pitch, w);
-  SAVSR_REQUIRE(c_pitch >= c_step * (w / 2), "%s: c_pitch %d < chroma row of %d bytes", fn, c_pitch, c_step * (w / 2));
+  SAVSR_REQUIRE(c_pitch >= c_step * (w / 2), "%s: c_pitch %d < chroma row of %d %s", fn, c_pitch, c_step * (w / 2),
+                deep ? "elements" : "bytes");
   SAVSR_REQUIRE(frame_stride >= 0, "%s: negative frame_stride %lld", fn, frame_stride);
   return 0;
 }
 
-static unsigned yuv_blocks(const savsr_ctx* ctx, int n, int h, int w) {
-  const long long items = static_cast<long long>(n) * (h / 2) * ((w + kYuvGroup - 1) / kYuvGroup);
+static unsigned grid_for(const savsr_ctx* ctx, long long items) {
   const long long b = (items + 255) / 256, cap = 16LL * ctx->sm_count;
   return static_cast<unsigned>(b < cap ? b : cap);
+}
+
+static unsigned yuv_blocks(const savsr_ctx* ctx, int n, int h, int w) {
+  return grid_for(ctx, static_cast<long long>(n) * (h / 2) * ((w + kYuvGroup - 1) / kYuvGroup));
 }
 
 }  // namespace savsr
@@ -265,6 +466,44 @@ extern "C" int savsr_bgr_to_yuv420(savsr_ctx* ctx, const uint8_t* bgr, int n, in
   DeviceGuard guard(ctx->device);
   const Yuv420Planes p{y, u, v, y_pitch, c_pitch, c_step, frame_stride};
   bgr_to_yuv420_kernel<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(bgr, n, h, w, p);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int savsr_yuv420_10_to_bgr48(savsr_ctx* ctx, const uint16_t* y, int y_pitch, const uint16_t* u, const uint16_t* v, int c_pitch,
+                                        int c_step, int64_t frame_stride, int msb, int n, int h, int w, uint16_t* bgr, savsr_stream st) {
+  SAVSR_REQUIRE(ctx && y && u && v && bgr, "savsr_yuv420_10_to_bgr48: null pointer");
+  if (check_yuv420("savsr_yuv420_10_to_bgr48", n, h, w, y_pitch, c_pitch, c_step, frame_stride, true)) return 1;
+  SAVSR_REQUIRE(msb == 0 || msb == 1, "savsr_yuv420_10_to_bgr48: msb must be 0 (yuv420p10le) or 1 (p010), got %d", msb);
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const Yuv420Planes16 p{const_cast<uint16_t*>(y), const_cast<uint16_t*>(u), const_cast<uint16_t*>(v), y_pitch, c_pitch, c_step,
+                         frame_stride, msb};
+  yuv420_10_to_bgr48_kernel<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(p, n, h, w, bgr);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int savsr_bgr48_to_yuv420_10(savsr_ctx* ctx, const uint16_t* bgr, int n, int h, int w, uint16_t* y, int y_pitch, uint16_t* u,
+                                        uint16_t* v, int c_pitch, int c_step, int64_t frame_stride, int msb, savsr_stream st) {
+  SAVSR_REQUIRE(ctx && bgr && y && u && v, "savsr_bgr48_to_yuv420_10: null pointer");
+  if (check_yuv420("savsr_bgr48_to_yuv420_10", n, h, w, y_pitch, c_pitch, c_step, frame_stride, true)) return 1;
+  SAVSR_REQUIRE(msb == 0 || msb == 1, "savsr_bgr48_to_yuv420_10: msb must be 0 (yuv420p10le) or 1 (p010), got %d", msb);
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const Yuv420Planes16 p{y, u, v, y_pitch, c_pitch, c_step, frame_stride, msb};
+  bgr48_to_yuv420_10_kernel<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(bgr, n, h, w, p);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int savsr_widen_u8_to_u16(savsr_ctx* ctx, const uint8_t* src, int n, int h, int w, uint16_t* dst, savsr_stream st) {
+  SAVSR_REQUIRE(ctx && src && dst, "savsr_widen_u8_to_u16: null pointer");
+  SAVSR_REQUIRE(n >= 0 && h > 0 && w > 0, "savsr_widen_u8_to_u16: bad shape n=%d h=%d w=%d", n, h, w);
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const long long count = static_cast<long long>(n) * h * w * 3;
+  widen_u8_to_u16_kernel<<<grid_for(ctx, (count + 15) / 16), 256, 0, static_cast<cudaStream_t>(st)>>>(src, dst, count);
   SAVSR_CUDA(cudaGetLastError());
   return 0;
 }

@@ -57,12 +57,14 @@ enum AttrBit { kAttrIgemm = 0 /* + template index, 6 variants */, kAttrBigk = 8,
                kAttrFused = 12, kAttrBigk128 = 13, kAttrSatuHrBf16 = 14, kAttrWgrad = 15, kAttrWgradBatched = 16,
                kAttrOsaAssembleTrain = 17, kAttrOsaUnfoldBwd = 18, kAttrOsaChain = 19, kAttrOsaMatvec = 20 /* + 0, 1, 2: batch 8, 16, 32 */,
                kAttrCaBackward = 23, kAttrSatuHrU8 = 24 /* + format: 8-bit I/O instantiations of satu_hr */,
-               kAttrSatuHrU8Table = 26 /* + format: 8-bit frame-table instantiations of satu_hr */ };
+               kAttrSatuHrU8Table = 26 /* + format: 8-bit frame-table instantiations of satu_hr */,
+               kAttrSatuHrU16Table = 28 /* + format: 16-bit frame-table instantiations of satu_hr */ };
 // Input addressing of the two launches that read a forward's input (pack_frames, satu_hr's bilinear skip):
-//   kIoF32      fp32 NCHW window [batch][t][3][h][w] RGB
-//   kIoU8       uint8 window [batch][t][h][w][3] BGR
-//   kIoU8Table  frame table: device array const uint8_t* [batch][t], entry (n, f) -> one contiguous uint8 [h][w][3] BGR frame
-enum IoMode { kIoF32 = 0, kIoU8 = 1, kIoU8Table = 2 };
+//   kIoF32       fp32 NCHW window [batch][t][3][h][w] RGB
+//   kIoU8        uint8 window [batch][t][h][w][3] BGR
+//   kIoU8Table   frame table: device array const uint8_t* [batch][t], entry (n, f) -> one contiguous uint8 [h][w][3] BGR frame
+//   kIoU16Table  frame table of uint16 frames: const uint16_t* [batch][t] -> one contiguous bgr48 [h][w][3] frame (full scale 65535)
+enum IoMode { kIoF32 = 0, kIoU8 = 1, kIoU8Table = 2, kIoU16Table = 3 };
 // One launch of the frame-table writer carries at most this many pointers in its by-value argument (3.6 KB, under the 4 KB
 // parameter limit of older drivers); 448 = 64 windows of 7 frames.
 constexpr int kFrameTableChunk = 448;
@@ -76,6 +78,22 @@ constexpr int kYuvY = 1220542, kYuvVR = 1673527, kYuvVG = -852492, kYuvUG = -409
 constexpr int kRgbYR = 269484, kRgbYG = 528482, kRgbYB = 102760;
 constexpr int kRgbUR = -155188, kRgbUG = -305135, kRgbUB = 460324;
 constexpr int kRgbVR = 460324, kRgbVG = -385875, kRgbVB = -74448;
+// The same matrix between 10-bit YUV and 16-bit RGB (colour.cu): one 10-bit step is a quarter of an 8-bit step (Y from 64, chroma
+// centred on 512), one 8-bit RGB step is 257 sixteen-bit steps.  Real-valued, R16 = 257 / 4 * (kYuvY (Y10 - 64) + kYuvVR (V10 - 512)) / 2^20
+// and Y10 = 64 + 4 (kRgbYR R16 + kRgbYG G16 + kRgbYB B16) / (257 * 2^20).  Both integer forms are within 0.53 of an output step of that.
+//   decode: int64.  y = max(0, Y - 64) * kYuv10Y, u = U - 512, v = V - 512 (int32),
+//           R = sat16((y + half + kYuv10VR v) >> 22), G, B likewise: the exact map rounded half up (|error| <= 0.5).
+//           The coefficients are 257 times the 8-bit ones (int32); products and sums are int64 (|y + ...| < 2^39).
+//   encode: int32.  Y = (kRgb10YR R + kRgb10YG G + kRgb10YB B + (64 << 21) + half) >> 21, U and V likewise with offset 512 << 21.
+//           The coefficients are round(4 * 2^21 * k / (257 * 2^20)) of the 8-bit ones k; every sum lies in [1.3e8, 2.02e9] for
+//           16-bit inputs, so it fits int32 and never goes negative.  The results lie in [64, 940] (Y) and [64, 960] (U, V).
+constexpr int kYuv10Shift = 22;
+constexpr long long kYuv10Half = 1LL << (kYuv10Shift - 1);
+constexpr int kYuv10Y = 257 * kYuvY, kYuv10VR = 257 * kYuvVR, kYuv10VG = 257 * kYuvVG, kYuv10UG = 257 * kYuvUG, kYuv10UB = 257 * kYuvUB;
+constexpr int kRgb10Shift = 21, kRgb10Half = 1 << (kRgb10Shift - 1);
+constexpr int kRgb10YR = 8389, kRgb10YG = 16451, kRgb10YB = 3199;
+constexpr int kRgb10UR = -4831, kRgb10UG = -9498, kRgb10UB = 14329;
+constexpr int kRgb10VR = 14329, kRgb10VG = -12012, kRgb10VB = -2317;
 template <class F>
 inline int ensure_smem_attr(savsr_ctx* ctx, int bit, F func, size_t bytes) {
   if (ctx->attr_mask & (1u << bit)) return 0;
@@ -153,9 +171,22 @@ __device__ __forceinline__ float u8_to_unit(uint8_t u) {
   return __fmaf_rn(__fmaf_rn(-q, 255.0f, a), r, q);
 }
 __device__ __forceinline__ int unit_to_u8(float v) { return __float2int_rn(fminf(fmaxf(v, 0.f), 1.f) * 255.0f); }
-// Entry i of a frame table (kIoU8Table), through the read-only cache: every thread of a launch reads the same few entries.
-__device__ __forceinline__ const uint8_t* frame_at(const uint8_t* const* table, long i) {
-  return reinterpret_cast<const uint8_t*>(__ldg(reinterpret_cast<const unsigned long long*>(table) + i));
+// 16-bit sample <-> [0, 1] float, the same two conversions with full scale 65535.  In: v / 65535 correctly rounded, by the same
+// reciprocal-and-one-fma form (exact for all 65536 values, checked exhaustively in tests/test_video_deep.py).  Since 257 u / 65535 =
+// u / 255, u16_to_unit(257 u) == u8_to_unit(u): an 8-bit frame widened by 257 enters the network exactly as the 8-bit frame does.
+// Out: tensor2img's quantiser with 65535 in place of 255.
+__device__ __forceinline__ float u16_to_unit(uint16_t u) {
+  const float a = static_cast<float>(u), r = 1.0f / 65535.0f;
+  const float q = __fmul_rn(a, r);
+  return __fmaf_rn(__fmaf_rn(-q, 65535.0f, a), r, q);
+}
+__device__ __forceinline__ int unit_to_u16(float v) { return __float2int_rn(fminf(fmaxf(v, 0.f), 1.f) * 65535.0f); }
+__device__ __forceinline__ float to_unit(uint8_t u) { return u8_to_unit(u); }
+__device__ __forceinline__ float to_unit(uint16_t u) { return u16_to_unit(u); }
+// Entry i of a frame table (kIoU8Table, kIoU16Table), through the read-only cache: every thread of a launch reads the same few entries.
+template <class T>
+__device__ __forceinline__ const T* frame_at(const T* const* table, long i) {
+  return reinterpret_cast<const T*>(__ldg(reinterpret_cast<const unsigned long long*>(table) + i));
 }
 __device__ __forceinline__ float h_to_float(uint16_t raw, int fmt) { return h_lo(raw, fmt); }
 __device__ __forceinline__ uint16_t float_to_h(float x, int fmt) { return static_cast<uint16_t>(pack_h2(x, 0.f, fmt) & 0xffffu); }

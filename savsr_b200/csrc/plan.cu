@@ -12,11 +12,12 @@
 struct savsr_plan {
   savsr_ctx* ctx;
   std::vector<std::function<int(savsr_stream)>> ops;
-  void* x_in = nullptr;            // input staging buffer, or the frame table (kIoU8Table)
+  void* x_in = nullptr;            // input staging buffer, or the frame table (kIoU8Table, kIoU16Table)
   void* out = nullptr;
   size_t x_bytes = 0, out_bytes = 0;
   int format = SAVSR_FMT_BF16;
-  int io = savsr::kIoF32;          // I/O mode: fp32 (savsr_forward), uint8 BGR (savsr_forward_u8), frame table (savsr_forward_u8_frames)
+  int io = savsr::kIoF32;          // I/O mode: fp32 (savsr_forward), uint8 BGR (savsr_forward_u8), frame table (savsr_forward_u8_frames),
+                                   // uint16 frame table (savsr_forward_u16_frames)
 };
 
 using namespace savsr;
@@ -54,6 +55,13 @@ extern "C" int savsr_plan_set_io_u8_table(savsr_plan* plan, const uint8_t** tabl
                 kIoU8Table);
 }
 
+extern "C" int savsr_plan_set_io_u16_table(savsr_plan* plan, const uint16_t** table_dev, int entries, uint16_t* out, size_t out_bytes,
+                                          int format) {
+  SAVSR_REQUIRE(entries >= 0, "savsr_plan_set_io_u16_table: negative entry count %d", entries);
+  return set_io("savsr_plan_set_io_u16_table", plan, const_cast<uint16_t**>(table_dev), entries * sizeof(*table_dev), out, out_bytes, format,
+                kIoU16Table);
+}
+
 extern "C" int savsr_plan_add_pack_frames(savsr_plan* plan, savsr_arena* arena, const float* x, int t, int h, int w, int dst_slot) {
   SAVSR_REQUIRE(plan && arena && x, "savsr_plan_add_pack_frames: null pointer");
   savsr_ctx* ctx = plan->ctx;
@@ -73,6 +81,14 @@ extern "C" int savsr_plan_add_pack_frames_u8_table(savsr_plan* plan, savsr_arena
   SAVSR_REQUIRE(plan && arena && frames, "savsr_plan_add_pack_frames_u8_table: null pointer");
   savsr_ctx* ctx = plan->ctx;
   plan->ops.push_back([=](savsr_stream st) { return savsr_pack_frames_u8_table(ctx, arena, frames, t, h, w, dst_slot, st); });
+  return 0;
+}
+
+extern "C" int savsr_plan_add_pack_frames_u16_table(savsr_plan* plan, savsr_arena* arena, const uint16_t* const* frames, int t, int h, int w,
+                                                    int dst_slot) {
+  SAVSR_REQUIRE(plan && arena && frames, "savsr_plan_add_pack_frames_u16_table: null pointer");
+  savsr_ctx* ctx = plan->ctx;
+  plan->ops.push_back([=](savsr_stream st) { return savsr_pack_frames_u16_table(ctx, arena, frames, t, h, w, dst_slot, st); });
   return 0;
 }
 
@@ -154,6 +170,19 @@ extern "C" int savsr_plan_add_satu_hr_u8_table(savsr_plan* plan, savsr_arena* lr
   return 0;
 }
 
+extern "C" int savsr_plan_add_satu_hr_u16_table(savsr_plan* plan, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
+                                                const float* table, const float* base_y, const float* base_x, const void* weights,
+                                                const float* zbias, const float* tail_bias, const uint16_t* const* frames, int t, int centre,
+                                                uint16_t* out) {
+  SAVSR_REQUIRE(plan && lr, "savsr_plan_add_satu_hr_u16_table: null pointer");
+  savsr_ctx* ctx = plan->ctx;
+  plan->ops.push_back([=](savsr_stream st) {
+    return savsr_satu_hr_u16_table(ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias, frames, t, centre,
+                                   out, st);
+  });
+  return 0;
+}
+
 extern "C" int savsr_plan_add_arena_export(savsr_plan* plan, savsr_arena* arena, int slot, float* nchw) {
   SAVSR_REQUIRE(plan && arena && nchw, "savsr_plan_add_arena_export: null pointer");
   plan->ops.push_back([=](savsr_stream st) { return savsr_arena_export(arena, slot, nchw, st); });
@@ -172,10 +201,11 @@ extern "C" int savsr_plan_run(savsr_plan* plan, savsr_stream st) {
 
 // Refuses a call of the wrong I/O mode before any copy or launch.
 static int check_io(const char* name, const savsr_plan* plan, int io) {
-  static const char* const kModeName[] = {"fp32", "uint8 BGR", "uint8 BGR frame-table"};
-  static const char* const kForward[] = {"savsr_forward", "savsr_forward_u8", "savsr_forward_u8_frames"};
+  static const char* const kModeName[] = {"fp32", "uint8 BGR", "uint8 BGR frame-table", "uint16 BGR frame-table"};
+  static const char* const kForward[] = {"savsr_forward", "savsr_forward_u8", "savsr_forward_u8_frames", "savsr_forward_u16_frames"};
   SAVSR_REQUIRE(plan->x_in && plan->out,
-                "%s: the plan has no I/O staging buffers (savsr_plan_set_io / savsr_plan_set_io_u8 / savsr_plan_set_io_u8_table)", name);
+                "%s: the plan has no I/O staging buffers (savsr_plan_set_io / savsr_plan_set_io_u8 / savsr_plan_set_io_u8_table / "
+                "savsr_plan_set_io_u16_table)", name);
   SAVSR_REQUIRE(plan->io == io, "%s: the plan was set up for %s I/O; call %s", name, kModeName[plan->io], kForward[plan->io]);
   return 0;
 }
@@ -199,13 +229,24 @@ extern "C" int savsr_forward_u8(savsr_plan* plan, const uint8_t* x, uint8_t* out
   return forward("savsr_forward_u8", plan, x, out, kIoU8, st);
 }
 
-extern "C" int savsr_forward_u8_frames(savsr_plan* plan, const uint8_t* const* ptrs_host, uint8_t* out, savsr_stream st) {
-  SAVSR_REQUIRE(plan && ptrs_host && out, "savsr_forward_u8_frames: null pointer");
-  if (int rc = check_io("savsr_forward_u8_frames", plan, kIoU8Table)) return rc;
+// Both frame-table modes: the table holds frame addresses whatever the sample type, written by the same kernel.
+static int forward_frames(const char* name, savsr_plan* plan, const void* const* ptrs_host, void* out, int io, savsr_stream st) {
+  SAVSR_REQUIRE(plan && ptrs_host && out, "%s: null pointer", name);
+  if (int rc = check_io(name, plan, io)) return rc;
   DeviceGuard guard(plan->ctx->device);
-  const int entries = static_cast<int>(plan->x_bytes / sizeof(const uint8_t*));
-  if (int rc = savsr_write_frame_table(plan->ctx, static_cast<const uint8_t**>(plan->x_in), ptrs_host, entries, st)) return rc;
+  const int entries = static_cast<int>(plan->x_bytes / sizeof(const void*));
+  if (int rc = savsr_write_frame_table(plan->ctx, static_cast<const uint8_t**>(plan->x_in), reinterpret_cast<const uint8_t* const*>(ptrs_host),
+                                       entries, st))
+    return rc;
   if (int rc = savsr_plan_run(plan, st)) return rc;
   if (out != plan->out) SAVSR_CUDA(cudaMemcpyAsync(out, plan->out, plan->out_bytes, cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(st)));
   return 0;
+}
+
+extern "C" int savsr_forward_u8_frames(savsr_plan* plan, const uint8_t* const* ptrs_host, uint8_t* out, savsr_stream st) {
+  return forward_frames("savsr_forward_u8_frames", plan, reinterpret_cast<const void* const*>(ptrs_host), out, kIoU8Table, st);
+}
+
+extern "C" int savsr_forward_u16_frames(savsr_plan* plan, const uint16_t* const* ptrs_host, uint16_t* out, savsr_stream st) {
+  return forward_frames("savsr_forward_u16_frames", plan, reinterpret_cast<const void* const*>(ptrs_host), out, kIoU16Table, st);
 }

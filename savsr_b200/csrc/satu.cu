@@ -346,7 +346,8 @@ __device__ __forceinline__ int swz(int r, int c) { return r * 128 + ((c ^ (r & 7
 // I/O modes (template IO, enum IoMode): fp32 (the module's forward contract) reads the skip from the fp32 window and stores fp32 NCHW;
 // 8-bit reads it from the uint8 BGR window [batch][t][h][w][3], or from the centre frame's entry of a frame table, through the same
 // u / 255 as the first layer, so the skip is the same fp32 number, and stores tensor2img's uint8 HWC BGR [batch][H][W][3] of the same
-// fp32 value the fp32 mode would have written.
+// fp32 value the fp32 mode would have written.  16-bit (frame table only) reads the centre frame's bgr48 samples through v / 65535 and
+// stores uint16 BGR [batch][H][W][3], the same quantiser with 65535 in place of 255.
 struct HrParams {
   const __nv_bfloat16* lr;
   const float* table;        // [H*W][8]: offset x,y | st_offset x,y | r0..r3
@@ -356,8 +357,8 @@ struct HrParams {
   const float* zbias;        // [32]: zb[tap*3+c], 27 used
   const float* tail_bias;    // [3]
   const void* x_in;          // bilinear skip of the centre frame: fp32 [batch][t][3][h][w], uint8 BGR [batch][t][h][w][3], or the
-                             // frame table const uint8_t* [batch][t]
-  void* out;                 // fp32 [batch][3][H][W], or uint8 BGR [batch][H][W][3]
+                             // frame table const uint8_t* [batch][t] or const uint16_t* [batch][t]
+  void* out;                 // fp32 [batch][3][H][W], or uint8 / uint16 BGR [batch][H][W][3]
   int batch, hp, wp, h, w, H, W;
   int x_slot, sta_slot;
   int t, centre;
@@ -503,7 +504,11 @@ __global__ void __launch_bounds__(kHrThreads, 1) satu_hr_kernel(const __grid_con
 #pragma unroll
           for (int ch = 0; ch < 3; ++ch) {
             float a, bb, cc, d;
-            if constexpr (IO != kIoF32) {
+            if constexpr (IO == kIoU16Table) {
+              const uint16_t* pl = frame_at(static_cast<const uint16_t* const*>(p.x_in), n * p.t + p.centre) + 2 - ch;
+              a = u16_to_unit(__ldg(pl + 3 * o00)); bb = u16_to_unit(__ldg(pl + 3 * o01));
+              cc = u16_to_unit(__ldg(pl + 3 * o10)); d = u16_to_unit(__ldg(pl + 3 * o11));
+            } else if constexpr (IO != kIoF32) {
               const uint8_t* pl = (IO == kIoU8Table ? fc : static_cast<const uint8_t*>(p.x_in) + xc) + 2 - ch;
               a = u8_to_unit(__ldg(pl + 3 * o00)); bb = u8_to_unit(__ldg(pl + 3 * o01));
               cc = u8_to_unit(__ldg(pl + 3 * o10)); d = u8_to_unit(__ldg(pl + 3 * o11));
@@ -526,7 +531,12 @@ __global__ void __launch_bounds__(kHrThreads, 1) satu_hr_kernel(const __grid_con
               acc2 += v ? __half2float(z[2 * kHrPix]) : 0.f;
             }
           }
-          if constexpr (IO != kIoF32) {
+          if constexpr (IO == kIoU16Table) {
+            // 6 bytes per pixel, 2-byte aligned: three 16-bit stores (a warp row is 192 contiguous bytes)
+            uint16_t* o = static_cast<uint16_t*>(p.out) + (static_cast<long>(n) * NPIX + static_cast<long>(Y) * p.W + X) * 3;
+            o[0] = static_cast<uint16_t>(unit_to_u16(acc2 + sk[2])); o[1] = static_cast<uint16_t>(unit_to_u16(acc1 + sk[1]));
+            o[2] = static_cast<uint16_t>(unit_to_u16(acc0 + sk[0]));
+          } else if constexpr (IO != kIoF32) {
             // 3 bytes per pixel: W * 3 has any alignment, so plain byte stores (a warp row is 96 contiguous bytes)
             uint8_t* o = static_cast<uint8_t*>(p.out) + (static_cast<long>(n) * NPIX + static_cast<long>(Y) * p.W + X) * 3;
             o[0] = static_cast<uint8_t>(unit_to_u8(acc2 + sk[2])); o[1] = static_cast<uint8_t>(unit_to_u8(acc1 + sk[1]));
@@ -791,7 +801,8 @@ static int satu_hr(const char* name, savsr_ctx* ctx, savsr_arena* lr, int x_slot
   if (lr->batch == 0) return 0;
   const bool fp16 = ctx->fmt == SAVSR_FMT_FP16;
   auto kernel = fp16 ? satu_hr_kernel<SAVSR_FMT_FP16, IO> : satu_hr_kernel<SAVSR_FMT_BF16, IO>;
-  const int bit = IO == kIoU8Table ? kAttrSatuHrU8Table + (fp16 ? 1 : 0)
+  const int bit = IO == kIoU16Table ? kAttrSatuHrU16Table + (fp16 ? 1 : 0)
+                : IO == kIoU8Table ? kAttrSatuHrU8Table + (fp16 ? 1 : 0)
                 : IO == kIoU8      ? kAttrSatuHrU8 + (fp16 ? 1 : 0)
                                    : (fp16 ? kAttrSatuHr : kAttrSatuHrBf16);
   if (int rc = ensure_smem_attr(ctx, bit, kernel, kHrSmem)) return rc;
@@ -830,4 +841,12 @@ extern "C" int savsr_satu_hr_u8_table(savsr_ctx* ctx, savsr_arena* lr, int x_slo
                                       uint8_t* out, savsr_stream st) {
   return satu_hr<kIoU8Table>("savsr_satu_hr_u8_table", ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias, tail_bias,
                              frames, t, centre, out, st);
+}
+
+extern "C" int savsr_satu_hr_u16_table(savsr_ctx* ctx, savsr_arena* lr, int x_slot, int sta_slot, int h, int w, int H, int W,
+                                       const float* table, const float* base_y, const float* base_x, const void* weights,
+                                       const float* zbias, const float* tail_bias, const uint16_t* const* frames, int t, int centre,
+                                       uint16_t* out, savsr_stream st) {
+  return satu_hr<kIoU16Table>("savsr_satu_hr_u16_table", ctx, lr, x_slot, sta_slot, h, w, H, W, table, base_y, base_x, weights, zbias,
+                              tail_bias, frames, t, centre, out, st);
 }

@@ -13,7 +13,8 @@ namespace savsr {
 // reflect-padded to the even arena size (savsr_arch.py:670-690).  With this slot the first-layer convs (conv_c / conv_sup,
 // savsr_arch.py:456-457) run on the tensor-core kernel with zero-expanded weights.  T = float: fp32 NCHW window [B][t][3][h][w] RGB;
 // T = uint8_t: the decoded 8-bit window [B][t][h][w][3] BGR, converted exactly as the reference's img.astype(np.float32) / 255.;
-// T = const uint8_t*: a frame table (x[n * t + f] -> frame f of sample n, [h][w][3] BGR), read through the same conversion.
+// T = const uint8_t*: a frame table (x[n * t + f] -> frame f of sample n, [h][w][3] BGR), read through the same conversion;
+// T = const uint16_t*: a frame table of bgr48 frames, read through u16_to_unit (v / 65535, correctly rounded).
 template <class T>
 __global__ void __launch_bounds__(256) pack_frames_kernel(const T* __restrict__ x, __nv_bfloat16* __restrict__ dst, int batch,
                                                           int t, int h, int w, int hp, int wp, int fmt) {
@@ -32,7 +33,7 @@ __global__ void __launch_bounds__(256) pack_frames_kernel(const T* __restrict__ 
       const int ch = chunk * 8 + e;
       if constexpr (std::is_pointer<T>::value) {
         const int f = ch / 3, c = ch - 3 * f;
-        v[e] = ch < 3 * t ? u8_to_unit(__ldg(frame_at(x, static_cast<long>(n) * t + f) + (static_cast<long>(ry) * w + rx) * 3 + 2 - c)) : 0.f;
+        v[e] = ch < 3 * t ? to_unit(__ldg(frame_at(x, static_cast<long>(n) * t + f) + (static_cast<long>(ry) * w + rx) * 3 + 2 - c)) : 0.f;
       } else if constexpr (sizeof(T) == 1) {
         const int f = ch / 3, c = ch - 3 * f;
         v[e] = ch < 3 * t ? u8_to_unit(__ldg(x + ((static_cast<long>(n) * t + f) * h + ry) * w * 3 + rx * 3 + 2 - c)) : 0.f;
@@ -580,6 +581,11 @@ extern "C" int savsr_pack_frames_u8(savsr_ctx* ctx, savsr_arena* arena, const ui
 extern "C" int savsr_pack_frames_u8_table(savsr_ctx* ctx, savsr_arena* arena, const uint8_t* const* frames, int t, int h, int w, int dst_slot,
                                           savsr_stream st) {
   return pack_frames("savsr_pack_frames_u8_table", ctx, arena, frames, t, h, w, dst_slot, st);
+}
+
+extern "C" int savsr_pack_frames_u16_table(savsr_ctx* ctx, savsr_arena* arena, const uint16_t* const* frames, int t, int h, int w, int dst_slot,
+                                           savsr_stream st) {
+  return pack_frames("savsr_pack_frames_u16_table", ctx, arena, frames, t, h, w, dst_slot, st);
 }
 
 namespace savsr {

@@ -25,7 +25,8 @@ import torch
 from . import _capi as K, colour
 
 BN_EPS = 1e-5
-IO_MODES = ("f32", "bgr_u8", "bgr_u8_frames")
+IO_MODES = ("f32", "bgr_u8", "bgr_u8_frames", "bgr48_frames")
+FRAME_MODES = {"bgr_u8_frames": torch.uint8, "bgr48_frames": torch.uint16}     # I/O modes that read frames in place, and their sample type
 
 
 def normalize_scale(scale) -> Tuple[float, float]:
@@ -163,8 +164,10 @@ class Plan:
     """I/O modes (`io`): "f32" stages the module's forward contract, x fp32 [B,7,3,h,w] RGB in [0, 1] -> out fp32 [B,3,H,W];
     "bgr_u8" stages decoded 8-bit video, x uint8 [B,7,h,w,3] BGR -> out uint8 [B,H,W,3] BGR, the image tensor2img makes of the
     fp32 output of x / 255; "bgr_u8_frames" has no input staging: it reads B*7 uint8 BGR [h,w,3] frames in place through a device
-    table of frame pointers (`frame_table`, written per forward by forward_frames_into) -> out uint8 [B,H,W,3] as "bgr_u8".
-    The modes differ only in their first and last launch (savsr_pack_frames[_u8[_table]], savsr_satu_hr[_u8[_table]])."""
+    table of frame pointers (`frame_table`, written per forward by forward_frames_into) -> out uint8 [B,H,W,3] as "bgr_u8";
+    "bgr48_frames" is the same for deep video: B*7 uint16 bgr48 [h,w,3] frames, each value v entering as v / 65535 -> out uint16
+    [B,H,W,3], the fp32 output clamped, * 65535 and rounded half to even.
+    The modes differ only in their first and last launch (savsr_pack_frames[_u8[_table] | _u16_table], savsr_satu_hr[...])."""
     io = "f32"
 
     def __init__(self, params: Dict[str, torch.Tensor], batch: int, h: int, w: int, scale, device: torch.device,
@@ -211,9 +214,10 @@ class Plan:
             if self.cplan is not None:
                 if self._recorded == len(self.ops):
                     out_bytes = self.out.numel() * self.out.element_size()
-                    if self.io == "bgr_u8_frames":
-                        K.check(self.lib.savsr_plan_set_io_u8_table(self.cplan.handle, self.frame_table.data_ptr(), self.frame_table.numel(),
-                                                                    self.out.data_ptr(), out_bytes, self.fmt))
+                    if self.io in FRAME_MODES:
+                        set_io = self.lib.savsr_plan_set_io_u8_table if self.io == "bgr_u8_frames" else self.lib.savsr_plan_set_io_u16_table
+                        K.check(set_io(self.cplan.handle, self.frame_table.data_ptr(), self.frame_table.numel(), self.out.data_ptr(), out_bytes,
+                                       self.fmt))
                     else:
                         set_io = self.lib.savsr_plan_set_io_u8 if self.io == "bgr_u8" else self.lib.savsr_plan_set_io
                         K.check(set_io(self.cplan.handle, self.x_in.data_ptr(), self.x_in.numel() * self.x_in.element_size(), self.out.data_ptr(),
@@ -418,10 +422,10 @@ class Plan:
         self.arena_lr_t.zero_()                  # the zero slot must be zero; the rest so that activation_absmax never reads stale memory
         self.lr = K.Arena(self.ctx, self.arena_lr_t.data_ptr(), self.n_lr_slots, B, self.hp, self.wp)
         lr = self.lr
-        if self.io == "bgr_u8_frames":
+        if self.io in FRAME_MODES:
             self.x_in = None
-            self.frame_table = self._buf(B * t, dtype=torch.int64)         # const uint8_t* [B][t], rewritten before every forward
-            self.out = self._buf(B, self.H, self.W, 3, dtype=torch.uint8)
+            self.frame_table = self._buf(B * t, dtype=torch.int64)         # const uint8_t* / uint16_t* [B][t], rewritten before every forward
+            self.out = self._buf(B, self.H, self.W, 3, dtype=FRAME_MODES[self.io])
             xin = self.frame_table.data_ptr()
         else:
             if self.io == "bgr_u8":
@@ -431,7 +435,7 @@ class Plan:
                 self.x_in = self._buf(B, t, 3, self.h, self.w)
                 self.out = self._buf(B, 3, self.H, self.W)
             xin = self.x_in.data_ptr()
-        sfx = {"f32": "", "bgr_u8": "_u8", "bgr_u8_frames": "_u8_table"}[self.io]   # the first and the last launch; everything between is shared
+        sfx = {"f32": "", "bgr_u8": "_u8", "bgr_u8_frames": "_u8_table", "bgr48_frames": "_u16_table"}[self.io]   # the first and the last launch; everything between is shared
         pack_frames, add_pack_frames = getattr(lib, "savsr_pack_frames" + sfx), getattr(lib, "savsr_plan_add_pack_frames" + sfx)
         satu_hr, add_satu_hr = getattr(lib, "savsr_satu_hr" + sfx), getattr(lib, "savsr_plan_add_satu_hr" + sfx)
 
@@ -702,8 +706,8 @@ class Plan:
     def forward_into(self, x: torch.Tensor, out: torch.Tensor, graph: bool = True) -> None:
         """x -> out through the plan's staging buffers (graph replay reads / writes fixed addresses), all on the device's current
         stream: fp32 [B,7,3,h,w] -> [B,3,H,W], or with io="bgr_u8" uint8 [B,7,h,w,3] -> [B,H,W,3]."""
-        if self.io == "bgr_u8_frames":
-            raise ValueError('a plan with io="bgr_u8_frames" reads frames in place: call forward_frames_into')
+        if self.io in FRAME_MODES:
+            raise ValueError(f'a plan with io="{self.io}" reads frames in place: call forward_frames_into')
         with torch.cuda.device(self.device):
             self.x_in.copy_(x, non_blocking=True)
             if graph:
@@ -713,30 +717,34 @@ class Plan:
             out.copy_(self.out, non_blocking=True)
 
     def write_frame_table(self, ptrs: Sequence[int]) -> None:
-        """Enqueue the writer of the frame table (io="bgr_u8_frames") on the device's current stream: B*7 device addresses of uint8 BGR
-        [h,w,3] frames, window n = ptrs[7n : 7n + 7].  The addresses travel in the launch arguments (savsr_write_frame_table), so nothing
-        waits for the stream; the writer runs in stream order before the forward that reads the table, outside any captured graph."""
+        """Enqueue the writer of the frame table (io="bgr_u8_frames" or "bgr48_frames") on the device's current stream: B*7 device
+        addresses of BGR [h,w,3] frames of the mode's sample type, window n = ptrs[7n : 7n + 7].  The addresses travel in the launch
+        arguments (savsr_write_frame_table), so nothing waits for the stream; the writer runs in stream order before the forward that reads the table, outside any captured graph."""
         if len(ptrs) != self.frame_table.numel():
             raise ValueError(f"plan built for {self.frame_table.numel()} frame pointers, got {len(ptrs)}")
         arr = (C.c_void_p * len(ptrs))(*ptrs)
         with torch.cuda.device(self.device):
             K.check(self.lib.savsr_write_frame_table(self.ctx.handle, self.frame_table.data_ptr(), arr, len(ptrs), self._stream().cuda_stream))
 
-    def forward_frames_into(self, ptrs: Sequence[int], out: torch.Tensor, graph: bool = True, out_format: str = "bgr24") -> None:
-        """io="bgr_u8_frames": the frames at the B*7 device addresses `ptrs` (see write_frame_table) -> out uint8 [B,H,W,3], all on the
-        device's current stream.  The frames are read in place by the forward: they must stay valid, in stream order, until it has run.
-        With out_format "yuv420p" or "nv12", out is uint8 [B,3H/2,W] and the colour conversion reads the output staging buffer in place
-        of the copy (colour.bgr_to_yuv420)."""
-        if self.io != "bgr_u8_frames":
-            raise ValueError(f'forward_frames_into needs a plan with io="bgr_u8_frames", this one has io={self.io!r}')
-        colour.check_format(out_format, "out_format")
+    def forward_frames_into(self, ptrs: Sequence[int], out: torch.Tensor, graph: bool = True, out_format: Optional[str] = None) -> None:
+        """io="bgr_u8_frames" or "bgr48_frames": the frames at the B*7 device addresses `ptrs` (see write_frame_table) -> out BGR
+        [B,H,W,3] of the mode's sample type, all on the device's current stream.  The frames are read in place by the forward: they must
+        stay valid, in stream order, until it has run.  With a YUV out_format of the same depth ("yuv420p" or "nv12" for uint8,
+        "yuv420p10le" or "p010" for uint16), out is [B,3H/2,W] and the colour conversion reads the output staging buffer in place of the
+        copy (colour.bgr_to_yuv420).  out_format None is the mode's packed BGR ("bgr24", "bgr48le")."""
+        if self.io not in FRAME_MODES:
+            raise ValueError(f'forward_frames_into needs a plan with io="bgr_u8_frames" or "bgr48_frames", this one has io={self.io!r}')
+        bgr = "bgr48le" if self.io == "bgr48_frames" else "bgr24"
+        out_format = bgr if out_format is None else colour.check_format(out_format, "out_format")
+        if colour.bgr_format(out_format) != bgr:
+            raise ValueError(f'out_format {out_format!r} has another depth than the frames of io="{self.io}" ({bgr})')
         with torch.cuda.device(self.device):
             self.write_frame_table(ptrs)
             if graph:
                 self.run_graph()
             else:
                 self.run()
-            if out_format == "bgr24":
+            if out_format == bgr:
                 out.copy_(self.out, non_blocking=True)
             else:
                 colour.bgr_to_yuv420(self.out, out_format, out=out)
@@ -754,8 +762,8 @@ class Plan:
         eagerly on the device's current stream -- what a non-Python host would call.  Shapes and dtypes as in forward_into."""
         if self.cplan is None:
             raise K.SavsrError("this plan has no C-side launch list")
-        if self.io == "bgr_u8_frames":
-            raise ValueError('a plan with io="bgr_u8_frames" reads frames in place: call forward_frames_c')
+        if self.io in FRAME_MODES:
+            raise ValueError(f'a plan with io="{self.io}" reads frames in place: call forward_frames_c')
         u8 = self.io == "bgr_u8"
         dt = torch.uint8 if u8 else torch.float32
         if not (x.is_cuda and out.is_cuda and x.is_contiguous() and out.is_contiguous() and x.dtype == out.dtype == dt):
@@ -767,17 +775,22 @@ class Plan:
             K.check(fwd(self.cplan.handle, x.data_ptr(), out.data_ptr(), self._stream().cuda_stream))
 
     def forward_frames_c(self, ptrs: Sequence[int], out: torch.Tensor) -> None:
-        """io="bgr_u8_frames": as forward_frames_into through ONE C call (savsr_forward_u8_frames: table writer + the recorded launch list
-        + the output copy), eagerly on the device's current stream -- what a non-Python host would call."""
+        """io="bgr_u8_frames" or "bgr48_frames": as forward_frames_into through ONE C call (savsr_forward_u8_frames /
+        savsr_forward_u16_frames: table writer + the recorded launch list + the output copy), eagerly on the device's current stream --
+        what a non-Python host would call."""
         if self.cplan is None:
             raise K.SavsrError("this plan has no C-side launch list")
+        if self.io not in FRAME_MODES:
+            raise ValueError(f'forward_frames_c needs a plan with io="bgr_u8_frames" or "bgr48_frames", this one has io={self.io!r}')
         if len(ptrs) != self.frame_table.numel():
             raise ValueError(f"plan built for {self.frame_table.numel()} frame pointers, got {len(ptrs)}")
-        if not (out.is_cuda and out.is_contiguous() and out.dtype == torch.uint8 and tuple(out.shape) == tuple(self.out.shape)):
-            raise ValueError(f"savsr_forward_u8_frames writes a contiguous uint8 CUDA tensor of shape {tuple(self.out.shape)}")
+        dt = FRAME_MODES[self.io]
+        name = "savsr_forward_u8_frames" if dt == torch.uint8 else "savsr_forward_u16_frames"
+        if not (out.is_cuda and out.is_contiguous() and out.dtype == dt and tuple(out.shape) == tuple(self.out.shape)):
+            raise ValueError(f"{name} writes a contiguous {str(dt).replace('torch.', '')} CUDA tensor of shape {tuple(self.out.shape)}")
         arr = (C.c_void_p * len(ptrs))(*ptrs)
         with torch.cuda.device(self.device):
-            K.check(self.lib.savsr_forward_u8_frames(self.cplan.handle, arr, out.data_ptr(), self._stream().cuda_stream))
+            K.check(getattr(self.lib, name)(self.cplan.handle, arr, out.data_ptr(), self._stream().cuda_stream))
 
     def release(self) -> None:
         """Drop the CUDA graph and every device buffer now (plan-cache eviction), instead of waiting for the collector."""

@@ -1,10 +1,11 @@
-"""Frame-in / frame-out upscaling of decoded 8-bit video of any length.
+"""Frame-in / frame-out upscaling of decoded 8-bit or deep (10- and 16-bit) video of any length.
 
 ``VideoUpscaler`` takes frames as a decoder produces them and returns HR frames in order, with the same windows, reflection and
 batch partition as ``sharding.infer_clip(net.forward_bgr_u8, clip, batch=...)`` on the whole clip, so its output is byte-identical to
 that call.  Frames are uploaded once into a device ring and read in place by ``SAVSR.forward_bgr_u8_indexed``; the ring's size depends
 on the largest batch of the schedule, not on the length of the video.  Frames may come and go as packed BGR or as YUV 4:2:0
-(yuv420p, NV12: savsr_b200.colour), converted on the device on their way into the ring and out of the forward's output buffer.
+(yuv420p, NV12: savsr_b200.colour), converted on the device on their way into the ring and out of the forward's output buffer.  Deep
+video (bgr48le, yuv420p10le, P010) streams through a ring of uint16 frames and ``SAVSR.forward_bgr48_indexed``.
 """
 from __future__ import annotations
 
@@ -37,6 +38,12 @@ class VideoUpscaler:
     enc(infer_clip(net.forward_bgr_u8, dec(frames), batch=...)).  YUV needs even sizes: even h and w for YUV input, an even HR size
     for YUV output (bgr24 output takes any scale).
 
+    Deep formats: "bgr48le" (uint16 [h, w, 3]), "yuv420p10le" and "p010" (one uint16 [3h/2, w] array per frame; a P010 frame may have
+    a row pitch).  When either side is deep the ring holds uint16 BGR frames and the forward is net.forward_bgr48: 8-bit input is
+    decoded as above and widened by 257 on its way into the ring, so it enters the network exactly as the 8-bit path feeds it, and the
+    output is enc(infer_clip(net.forward_bgr48, dec(frames), batch=...)) with dec of an 8-bit source widened.  An 8-bit source gets
+    deep output this way, without 8-bit banding; deep input with 8-bit output is refused.
+
     Ownership: the caller may overwrite or free what it passed to ``push`` as soon as ``push`` returns.  Host frames are staged through
     the upscaler's own pinned buffers (a staging slot is reused only after the event of its upload); CUDA frames are copied in stream
     order on the current stream.  Everything runs on the current stream of the net's device, so a ring slot is rewritten only after
@@ -56,18 +63,24 @@ class VideoUpscaler:
         self.scale = engine.normalize_scale(scale)
         self.in_format = colour.check_format(in_format, "in_format")
         self.out_format = colour.check_format(out_format, "out_format")
-        if in_format != "bgr24" and (h % 2 or w % 2):
+        deep_in, deep_out = in_format in colour.DEEP_FORMATS, out_format in colour.DEEP_FORMATS
+        if deep_in and not deep_out:
+            raise ValueError(f"deep input {in_format} with 8-bit output {out_format} is not supported: choose an output of "
+                             f"{', '.join(colour.DEEP_FORMATS)}")
+        if in_format in colour.YUV_FORMATS and (h % 2 or w % 2):
             raise ValueError(f"{in_format} input needs an even LR size, got {h}x{w}")
         H, W = engine.get_hw(h, w, self.scale)
-        if out_format != "bgr24" and (H % 2 or W % 2):
+        if out_format in colour.YUV_FORMATS and (H % 2 or W % 2):
             raise ValueError(f"{out_format} output needs an even HR size: {h}x{w} at scale {self.scale} gives H = {H}, W = {W}; "
-                             "bgr24 output takes any scale")
+                             f"{colour.bgr_format(out_format)} output takes any scale")
         self.device = net.gamma.device
         # Until batch [i, j) has run, the ring holds frames i - pad .. j - 1 + pad, the ones its windows read, and nothing newer.
         self.capacity = max(sizes) + 2 * self.pad
-        self.ring = torch.empty(self.capacity, h, w, 3, dtype=torch.uint8, device=self.device)
+        self.ring = torch.empty(self.capacity, h, w, 3, dtype=torch.uint16 if deep_out else torch.uint8, device=self.device)
+        self._widen = deep_out and not deep_in                  # 8-bit frames into a 16-bit ring: decoded to uint8 BGR, then x 257
         self._staging: Optional[torch.Tensor] = None           # pinned twin of the ring for host frames (YUV-sized for YUV input), on first use
         self._yuv_dev: Optional[torch.Tensor] = None           # device staging of one host YUV frame, converted from there into the ring
+        self._bgr8_dev: Optional[torch.Tensor] = None          # one uint8 BGR frame on its way into a 16-bit ring, widened from there
         self._uploaded: List[Optional[torch.cuda.Event]] = [None] * self.capacity
         self.reset()
 
@@ -79,9 +92,9 @@ class VideoUpscaler:
         self.finished = False
 
     def push(self, frames) -> List[Tuple[int, torch.Tensor]]:
-        """Append uint8 frames in `in_format`: BGR [h, w, 3] or [n, h, w, 3], YUV [3h/2, w] or [n, 3h/2, w] (torch or numpy, host or
-        CUDA).  Returns the batches that became ready, as (index of the first frame, uint8 [m, H, W, 3], or [m, 3H/2, W] in a YUV
-        out_format) in frame order; often none."""
+        """Append frames in `in_format` (uint8, uint16 for the deep formats): BGR [h, w, 3] or [n, h, w, 3], YUV [3h/2, w] or
+        [n, 3h/2, w] (torch or numpy, host or CUDA).  Returns the batches that became ready, as (index of the first frame, [m, H, W, 3],
+        or [m, 3H/2, W] in a YUV out_format, of out_format's sample type) in frame order; often none."""
         if self.finished:
             raise RuntimeError("push() after finish(): call reset() to start the next video")
         self._check_net()
@@ -122,40 +135,52 @@ class VideoUpscaler:
 
     def _frames(self, frames) -> torch.Tensor:
         x = frames if isinstance(frames, torch.Tensor) else torch.as_tensor(frames)
-        if self.in_format != "bgr24":
+        if self.in_format in colour.YUV_FORMATS:
             x = colour.yuv_frames(x, self.in_format, self.h, self.w)      # dtype, shape, row pitch and column stride
         else:
-            if x.dtype != torch.uint8:
-                raise TypeError(f"VideoUpscaler takes uint8 BGR frames, got {x.dtype}")
+            dt = colour.dtype_of(self.in_format)
+            tn = str(dt).replace("torch.", "")
+            if x.dtype != dt:
+                raise TypeError(f"VideoUpscaler takes {tn} BGR frames for {self.in_format}, got {x.dtype}")
             if x.dim() == 3:
                 x = x.unsqueeze(0)
             if x.dim() != 4 or tuple(x.shape[1:]) != (self.h, self.w, 3):
-                raise ValueError(f"expected uint8 BGR frames [{self.h}, {self.w}, 3] or [n, {self.h}, {self.w}, 3], got {tuple(x.shape)}")
+                raise ValueError(f"expected {tn} BGR frames [{self.h}, {self.w}, 3] or [n, {self.h}, {self.w}, 3], got {tuple(x.shape)}")
         if x.device.type != "cpu" and x.device != self.device:
             raise ValueError(f"frames on {x.device}, the net on {self.device}")
         return x
 
     def _upload(self, frame: torch.Tensor) -> None:
         s = self.received % self.capacity
-        yuv, ring = self.in_format != "bgr24", self.ring[s]
+        yuv, ring = self.in_format in colour.YUV_FORMATS, self.ring[s]
+        # where the frame's BGR goes: the ring slot, or for an 8-bit frame into a 16-bit ring one uint8 scratch frame widened from there
+        # (one buffer is enough: its next use follows this frame's widening in stream order)
+        if self._widen and self._bgr8_dev is None:
+            self._bgr8_dev = torch.empty(self.h, self.w, 3, dtype=torch.uint8, device=self.device)
+        bgr = self._bgr8_dev if self._widen else ring
         if frame.device.type == "cpu" and self.device.type == "cuda":
             if self._staging is None:
-                self._staging = torch.empty((self.capacity, *frame.shape), dtype=torch.uint8, pin_memory=True)
+                self._staging = torch.empty((self.capacity, *frame.shape), dtype=frame.dtype, pin_memory=True)
                 if yuv:     # one buffer is enough: its next upload follows this frame's conversion in stream order
-                    self._yuv_dev = torch.empty(frame.shape, dtype=torch.uint8, device=self.device)
+                    self._yuv_dev = torch.empty(frame.shape, dtype=frame.dtype, device=self.device)
             ev = self._uploaded[s]
             if ev is None:
                 ev = self._uploaded[s] = torch.cuda.Event()
             else:
                 ev.synchronize()                 # the previous upload from this staging slot has been read
             self._staging[s].copy_(frame)
-            frame = self._yuv_dev if yuv else ring
+            frame = self._yuv_dev if yuv else bgr
             frame.copy_(self._staging[s], non_blocking=True)
             ev.record(torch.cuda.current_stream(self.device))
         if yuv:
-            colour.yuv420_to_bgr(frame, self.in_format, out=ring)      # CUDA frames, pitched NV12 too, are read in place
-        elif frame is not ring:
-            ring.copy_(frame, non_blocking=True)
+            colour.yuv420_to_bgr(frame, self.in_format, out=bgr)       # CUDA frames, pitched NV12 / P010 too, are read in place
+        elif frame is not bgr:
+            if self._widen and frame.is_contiguous():
+                bgr = frame                      # a CUDA frame is widened where it is
+            else:
+                bgr.copy_(frame, non_blocking=True)
+        if self._widen:
+            colour.widen(bgr, out=ring)
 
     def _next_batch(self) -> Tuple[int, int]:
         b = self.sizes[min(self.batches, len(self.sizes) - 1)]
@@ -164,7 +189,7 @@ class VideoUpscaler:
     def _forward(self, i: int, j: int) -> Tuple[int, torch.Tensor]:
         R = self.capacity
         windows = [[f % R for f in sharding.frame_window_indices(c, self.received, self.num_frames)] for c in range(i, j)]
-        yuv_out = {} if self.out_format == "bgr24" else {"out_format": self.out_format}
+        yuv_out = {} if self.out_format == colour.bgr_format(self.out_format) else {"out_format": self.out_format}
         hr = self.net._forward_bgr_u8_indexed(self.ring, windows, self.scale, **yuv_out)
         self.done, self.batches = j, self.batches + 1
         return i, hr
