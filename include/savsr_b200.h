@@ -544,8 +544,8 @@ int savsr_forward_u16_frames(savsr_plan* plan, const uint16_t* const* ptrs_host,
 /* ---- YUV 4:2:0 video in and out ------------------------------------------------------------------------------------------------
  * Decoders hand out and encoders take YUV 4:2:0, the forward reads and writes packed BGR.  These two calls convert on the device,
  * byte-identically to OpenCV's cv::cvtColor: COLOR_YUV2BGR_I420 / COLOR_YUV2BGR_NV12 (each pixel takes its 2x2 block's chroma sample)
- * and COLOR_BGR2YUV_I420 (U and V from the top-left pixel of each 2x2 block).  BT.601, limited range; sources tagged otherwise are
- * converted with the same matrix both ways.  A C host decodes into a ring of BGR frames with savsr_yuv420_to_bgr, runs
+ * and COLOR_BGR2YUV_I420 (U and V from the top-left pixel of each 2x2 block), with OpenCV's BT.601 limited-range matrix.  Video in another
+ * matrix or range goes through the _cs calls below.  A C host decodes into a ring of BGR frames with savsr_yuv420_to_bgr, runs
  * savsr_forward_u8_frames on it, and encodes the output with savsr_bgr_to_yuv420.
  *
  * A YUV frame of h x w (both even) is described by its planes:
@@ -579,6 +579,29 @@ int savsr_yuv420_10_to_bgr48(savsr_ctx* ctx, const uint16_t* y, int y_pitch, con
                              int64_t frame_stride, int msb, int n, int h, int w, uint16_t* bgr, savsr_stream st);
 int savsr_bgr48_to_yuv420_10(savsr_ctx* ctx, const uint16_t* bgr, int n, int h, int w, uint16_t* y, int y_pitch, uint16_t* u, uint16_t* v,
                              int c_pitch, int c_step, int64_t frame_stride, int msb, savsr_stream st);
+/* ---- colour matrix and range (names as ffmpeg's -colorspace and -color_range) -------------------------------------------------------
+ * The four conversions above for video in another matrix or range: each _cs call takes its plain call's arguments plus colorspace and
+ * range.  (BT601, TV) launches exactly what the plain call launches (OpenCV's constants).  Every other pair converts with the
+ * Y'CbCr <-> R'G'B' map of ITU-T H.273 (Kr, Kb: BT.601 0.299, 0.114; BT.709 0.2126, 0.0722; BT.2020 0.2627, 0.0593): tv range has
+ * its black level at 16 and spans of 219 (Y) and 224 (U, V) 8-bit steps, pc range uses every code value (0 .. 2^n - 1, chroma
+ * centred on 2^(n-1)).  Decoding rounds and saturates to [0, 255] or [0, 65535] without clamping Y at the black level; encoding rounds
+ * and saturates to [0, 2^n - 1].  Integer forms within 0.55 of an output step of the real-valued map (savsr_b200/csrc/common.cuh).
+ * Chroma handling, layouts, pitches and refusals are those of the plain calls; an unknown colorspace or range is refused, before any
+ * launch, with a savsr_last_error() naming the value.  Only R'G'B' code values are produced: no transfer function (PQ, HLG) is applied,
+ * and BT.2020 is the non-constant-luminance matrix.
+ */
+enum savsr_colorspace { SAVSR_COLORSPACE_BT601 = 0, SAVSR_COLORSPACE_BT709 = 1, SAVSR_COLORSPACE_BT2020NC = 2 };
+enum savsr_color_range { SAVSR_RANGE_TV = 0, SAVSR_RANGE_PC = 1 };
+int savsr_yuv420_to_bgr_cs(savsr_ctx* ctx, const uint8_t* y, int y_pitch, const uint8_t* u, const uint8_t* v, int c_pitch, int c_step,
+                           int64_t frame_stride, int n, int h, int w, uint8_t* bgr, int colorspace, int range, savsr_stream st);
+int savsr_bgr_to_yuv420_cs(savsr_ctx* ctx, const uint8_t* bgr, int n, int h, int w, uint8_t* y, int y_pitch, uint8_t* u, uint8_t* v,
+                           int c_pitch, int c_step, int64_t frame_stride, int colorspace, int range, savsr_stream st);
+int savsr_yuv420_10_to_bgr48_cs(savsr_ctx* ctx, const uint16_t* y, int y_pitch, const uint16_t* u, const uint16_t* v, int c_pitch,
+                                int c_step, int64_t frame_stride, int msb, int n, int h, int w, uint16_t* bgr, int colorspace, int range,
+                                savsr_stream st);
+int savsr_bgr48_to_yuv420_10_cs(savsr_ctx* ctx, const uint16_t* bgr, int n, int h, int w, uint16_t* y, int y_pitch, uint16_t* u,
+                                uint16_t* v, int c_pitch, int c_step, int64_t frame_stride, int msb, int colorspace, int range,
+                                savsr_stream st);
 /* uint8 BGR [n][h][w][3] -> uint16 BGR (each value times 257, so v / 65535 of the result is u / 255 of the source): brings 8-bit
  * frames into a ring of 16-bit frames, for an 8-bit source upscaled to deep output.  Both buffers contiguous; n = 0 launches nothing. */
 int savsr_widen_u8_to_u16(savsr_ctx* ctx, const uint8_t* src, int n, int h, int w, uint16_t* dst, savsr_stream st);

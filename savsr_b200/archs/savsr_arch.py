@@ -292,12 +292,13 @@ class SAVSR(nn.Module):
         return self._forward_bgr_u8_indexed(pool, windows, self.scale, dtype=torch.uint16)
 
     def _forward_bgr_u8_indexed(self, pool: torch.Tensor, windows, scale, out_format: Optional[str] = None,
-                                dtype: Optional[torch.dtype] = None) -> torch.Tensor:
+                                dtype: Optional[torch.dtype] = None, out_colorspace: str = "bt601",
+                                out_color_range: str = "tv") -> torch.Tensor:
         """forward_bgr_u8_indexed (uint8 pool) or forward_bgr48_indexed (uint16 pool) at `scale`, leaving self.scale as it is
         (savsr_b200.VideoUpscaler keeps its own scale).  The I/O mode follows the pool's dtype; `dtype`, when given, is the one the
         public caller takes.  With a YUV out_format of the pool's depth ("yuv420p" / "nv12" for uint8, "yuv420p10le" / "p010" for uint16)
         the HR frames come back as [b, 3H/2, W] YUV 4:2:0 (savsr_b200.colour), converted from the plan's output staging buffer instead
-        of copied; None is packed BGR."""
+        of copied, with the matrix out_colorspace and the range out_color_range; None is packed BGR."""
         name = {torch.uint16: "forward_bgr48_indexed"}.get(dtype if dtype is not None else pool.dtype, "forward_bgr_u8_indexed")
         if self.training:
             raise RuntimeError(f"{name} is inference only: call eval() first (training takes fp32 windows through forward)")
@@ -324,6 +325,11 @@ class SAVSR(nn.Module):
         out_format = bgr if out_format is None else colour.check_format(out_format, "out_format")
         if colour.bgr_format(out_format) != bgr:
             raise ValueError(f"out_format {out_format!r} has another depth than the {tn} frame pool")
+        out_colorspace = colour.check_colorspace(out_colorspace, "out_colorspace")
+        out_color_range = colour.check_color_range(out_color_range, "out_color_range")
+        if out_format == bgr and (out_colorspace, out_color_range) != ("bt601", "tv"):
+            raise ValueError(f"out_colorspace / out_color_range ({out_colorspace!r}, {out_color_range!r}) need a YUV out_format: "
+                             f"{out_format} output is not converted")
         if b == 0:
             H, W = engine.get_hw(h, w, scale)
             return pool.new_empty((0, H, W, 3) if out_format == bgr else (0, *colour.yuv_shape(H, W)))
@@ -332,10 +338,11 @@ class SAVSR(nn.Module):
         if lo < 0 or hi >= n:
             raise IndexError(f"window row index {lo if lo < 0 else hi} out of range for a pool of {n} frames")
         ptrs = (idx.reshape(-1) * (h * w * 3 * pool.element_size()) + pool.data_ptr()).tolist()
-        return self._run_plan(self._plan(b, h, w, pool.device, io, scale), frames=ptrs, out_format=out_format)
+        return self._run_plan(self._plan(b, h, w, pool.device, io, scale), frames=ptrs, out_format=out_format,
+                              out_colorspace=out_colorspace, out_color_range=out_color_range)
 
     def _run_plan(self, plan: engine.Plan, x: Optional[torch.Tensor] = None, frames: Optional[list] = None,
-                  out_format: str = "bgr24") -> torch.Tensor:
+                  out_format: str = "bgr24", out_colorspace: str = "bt601", out_color_range: str = "tv") -> torch.Tensor:
         with torch.cuda.device(plan.device):
             if out_format in ("bgr24", "bgr48le"):
                 out = torch.empty_like(plan.out)
@@ -344,7 +351,9 @@ class SAVSR(nn.Module):
             if frames is None:
                 plan.forward_into(x, out, graph=self.use_graph)
             else:
-                plan.forward_frames_into(frames, out, graph=self.use_graph, out_format=out_format)
+                cs = {} if (out_colorspace, out_color_range) == ("bt601", "tv") else \
+                    {"out_colorspace": out_colorspace, "out_color_range": out_color_range}
+                plan.forward_frames_into(frames, out, graph=self.use_graph, out_format=out_format, **cs)
             if self.precision == "fp16" and not plan.__dict__.get("_range_checked"):
                 # fp16 operands meet the <= 1e-3 bound but saturate at 65504: look at every trunk activation of this plan's FIRST forward
                 # (one pass over the arena, once per plan) and refuse to continue silently when the headroom is below 4x

@@ -17,13 +17,22 @@ Deep video (HEVC Main10, 10-bit AV1, 16-bit PNG / TIFF sequences) has formats of
 * ``"p010"``: one uint16 [3h/2, w] array per frame laid out as nv12, the value in bits 6-15 (NVDEC's 10-bit surfaces); it may have a
   row pitch like nv12.
 
-Several frames are [n, 3h/2, w].  The conversion is BT.601, limited range, in OpenCV's 20-bit fixed point: decoding gives each pixel
-the chroma sample of its 2x2 block (``COLOR_YUV2BGR_I420`` / ``COLOR_YUV2BGR_NV12``), encoding takes U and V from the top-left
-pixel of each 2x2 block (``COLOR_BGR2YUV_I420``).  Sizes must be even, as cv2 requires.  The 10-bit formats use the same matrix
-and chroma handling, rescaled (one 10-bit step is a quarter of an 8-bit step, one 8-bit BGR step is 257 sixteen-bit steps), in a
-fixed-point form within 0.53 of an output step of the real-valued map; decoding saturates to [0, 65535].  Each call is one launch on
-the current stream of the tensors' device (savsr_yuv420_to_bgr / savsr_bgr_to_yuv420, savsr_yuv420_10_to_bgr48 /
-savsr_bgr48_to_yuv420_10 of libsavsr_sm100); there is no CPU path.
+Several frames are [n, 3h/2, w].  By default the conversion is BT.601, limited range, in OpenCV's 20-bit fixed point: decoding gives
+each pixel the chroma sample of its 2x2 block (``COLOR_YUV2BGR_I420`` / ``COLOR_YUV2BGR_NV12``), encoding takes U and V from the
+top-left pixel of each 2x2 block (``COLOR_BGR2YUV_I420``).  Sizes must be even, as cv2 requires.  The 10-bit formats use the same
+matrix and chroma handling, rescaled (one 10-bit step is a quarter of an 8-bit step, one 8-bit BGR step is 257 sixteen-bit steps), in
+a fixed-point form within 0.53 of an output step of the real-valued map; decoding saturates to [0, 65535].
+
+Other colour matrices and ranges, named as ffmpeg's ``-colorspace`` and ``-color_range`` options (``COLORSPACES``, ``COLOR_RANGES``):
+``colorspace`` "bt601" (aliases "bt470bg", "smpte170m"), "bt709" or "bt2020nc" ("bt2020"), ``color_range`` "tv" ("limited", "mpeg")
+or "pc" ("full", "jpeg").  Every pair but the default ("bt601", "tv") converts with the Y'CbCr <-> R'G'B' map of ITU-T H.273 (the
+same chroma handling), in integer forms within 0.55 of an output step of the real-valued map at both depths: tv has its black level
+at 16 (64 in 10 bits) and spans of 219 and 224 steps, pc uses every code value.  Decoding saturates to the BGR range and does not clamp
+Y at the black level; encoding saturates to [0, 2^n - 1].  Only code values are converted: no transfer function (PQ / HLG, tone
+mapping) is applied, and BT.2020 is the non-constant-luminance matrix.  The default pair keeps OpenCV's constants exactly.
+
+Each call is one launch on the current stream of the tensors' device (savsr_yuv420_to_bgr / savsr_bgr_to_yuv420,
+savsr_yuv420_10_to_bgr48 / savsr_bgr48_to_yuv420_10 of libsavsr_sm100, and their _cs forms for the other pairs); there is no CPU path.
 """
 from __future__ import annotations
 
@@ -37,6 +46,10 @@ FORMATS = ("bgr24", "yuv420p", "nv12", "bgr48le", "yuv420p10le", "p010")
 YUV_FORMATS = ("yuv420p", "nv12", "yuv420p10le", "p010")
 DEEP_FORMATS = ("bgr48le", "yuv420p10le", "p010")
 PITCHED_FORMATS = ("nv12", "p010")          # may have a row pitch; their U, V samples are interleaved
+COLORSPACES = {"bt601": 0, "bt709": 1, "bt2020nc": 2}      # enum savsr_colorspace
+COLOR_RANGES = {"tv": 0, "pc": 1}                          # enum savsr_color_range
+_COLORSPACE_ALIASES = {"bt470bg": "bt601", "smpte170m": "bt601", "bt2020": "bt2020nc"}
+_COLOR_RANGE_ALIASES = {"limited": "tv", "mpeg": "tv", "full": "pc", "jpeg": "pc"}
 
 
 def dtype_of(fmt: str) -> torch.dtype:
@@ -53,6 +66,30 @@ def check_format(fmt: str, what: str = "format") -> str:
     if fmt not in FORMATS:
         raise ValueError(f"unknown {what} {fmt!r}: expected one of {', '.join(FORMATS)}")
     return fmt
+
+
+def check_colorspace(name: str, what: str = "colorspace") -> str:
+    """The canonical name of colour matrix `name` (ffmpeg's -colorspace names and aliases)."""
+    cs = _COLORSPACE_ALIASES.get(name, name)
+    if cs not in COLORSPACES:
+        names = [*COLORSPACES, *_COLORSPACE_ALIASES]
+        raise ValueError(f"unknown {what} {name!r}: expected one of {', '.join(names)}")
+    return cs
+
+
+def check_color_range(name: str, what: str = "color_range") -> str:
+    """The canonical name of colour range `name`: "tv" (limited) or "pc" (full), ffmpeg's -color_range names and aliases."""
+    r = _COLOR_RANGE_ALIASES.get(name, name)
+    if r not in COLOR_RANGES:
+        names = [*COLOR_RANGES, *_COLOR_RANGE_ALIASES]
+        raise ValueError(f"unknown {what} {name!r}: expected one of {', '.join(names)}")
+    return r
+
+
+def _cs_args(colorspace: str, color_range: str) -> tuple:
+    """() for the default pair ("bt601", "tv"), which the plain entry points convert; else the enumerator values for the _cs ones."""
+    cs, r = check_colorspace(colorspace), check_color_range(color_range)
+    return () if (cs, r) == ("bt601", "tv") else (COLORSPACES[cs], COLOR_RANGES[r])
 
 
 def yuv_shape(h: int, w: int) -> Tuple[int, int]:
@@ -125,11 +162,14 @@ def _bgr(x: torch.Tensor, what: str, dt: torch.dtype = torch.uint8) -> torch.Ten
     return x
 
 
-def yuv420_to_bgr(frames: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+def yuv420_to_bgr(frames: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None, colorspace: str = "bt601",
+                  color_range: str = "tv") -> torch.Tensor:
     """`fmt` frames ([3h/2, w] or [n, 3h/2, w], CUDA) -> BGR [h, w, 3] or [n, h, w, 3] of the same depth.  "yuv420p" and "nv12" (uint8)
     decode to uint8 BGR as cv2.cvtColor(frame, COLOR_YUV2BGR_I420 or COLOR_YUV2BGR_NV12) of each frame; "yuv420p10le" and "p010" (uint16)
-    to uint16 bgr48 with the same matrix.  Writes `out` (contiguous, that shape and dtype) when given, else a fresh tensor.  One launch
-    on the current stream; the frames must stay valid, in stream order, until it has run."""
+    to uint16 bgr48 with the same matrix.  Another `colorspace` / `color_range` than ("bt601", "tv") decodes with that pair's H.273
+    map.  Writes `out` (contiguous, that shape and dtype) when given, else a fresh tensor.  One launch on the current stream; the
+    frames must stay valid, in stream order, until it has run."""
+    cs = _cs_args(colorspace, color_range)
     x = yuv_frames(frames, fmt)
     n, h, w = x.shape[0], 2 * x.shape[1] // 3, x.shape[2]
     shape = (n, h, w, 3) if frames.dim() == 3 else (h, w, 3)
@@ -143,21 +183,26 @@ def yuv420_to_bgr(frames: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = 
     if n == 0:
         return out
     ctx = engine.context(dev.index)
-    y, yp, u, v, cp, cs, fs = _planes(x, fmt, h, w)
+    y, yp, u, v, cp, c_step, fs = _planes(x, fmt, h, w)
     st = torch.cuda.current_stream(dev).cuda_stream
     with torch.cuda.device(dev):
         if fmt in DEEP_FORMATS:
-            K.check(ctx.lib.savsr_yuv420_10_to_bgr48(ctx.handle, y, yp, u, v, cp, cs, fs, int(fmt == "p010"), n, h, w, out.data_ptr(), st))
+            args = (ctx.handle, y, yp, u, v, cp, c_step, fs, int(fmt == "p010"), n, h, w, out.data_ptr(), *cs, st)
+            K.check((ctx.lib.savsr_yuv420_10_to_bgr48_cs if cs else ctx.lib.savsr_yuv420_10_to_bgr48)(*args))
         else:
-            K.check(ctx.lib.savsr_yuv420_to_bgr(ctx.handle, y, yp, u, v, cp, cs, fs, n, h, w, out.data_ptr(), st))
+            args = (ctx.handle, y, yp, u, v, cp, c_step, fs, n, h, w, out.data_ptr(), *cs, st)
+            K.check((ctx.lib.savsr_yuv420_to_bgr_cs if cs else ctx.lib.savsr_yuv420_to_bgr)(*args))
     return out
 
 
-def bgr_to_yuv420(bgr: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+def bgr_to_yuv420(bgr: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None, colorspace: str = "bt601",
+                  color_range: str = "tv") -> torch.Tensor:
     """BGR [H, W, 3] or [n, H, W, 3] (contiguous, CUDA, H and W even) -> `fmt` frames [3H/2, W] or [n, 3H/2, W].  uint8 BGR to "yuv420p"
     or "nv12" as cv2.cvtColor(frame, COLOR_BGR2YUV_I420) of each frame, with U and V interleaved for "nv12"; uint16 bgr48 to
-    "yuv420p10le" or "p010" with the same matrix.  Writes `out` when given (any layout yuv_frames accepts, e.g. a pitched NV12 or P010
-    surface), else a fresh contiguous tensor.  One launch on the current stream."""
+    "yuv420p10le" or "p010" with the same matrix.  Another `colorspace` / `color_range` than ("bt601", "tv") encodes with that pair's
+    H.273 map.  Writes `out` when given (any layout yuv_frames accepts, e.g. a pitched NV12 or P010 surface), else a fresh contiguous
+    tensor.  One launch on the current stream."""
+    cs = _cs_args(colorspace, color_range)
     if fmt not in YUV_FORMATS:
         raise ValueError(f"{fmt!r} is not a YUV 4:2:0 format ({', '.join(YUV_FORMATS)})")
     dt = dtype_of(fmt)
@@ -178,13 +223,15 @@ def bgr_to_yuv420(bgr: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = Non
     if n == 0:
         return out
     ctx = engine.context(dev.index)
-    y, yp, u, v, cp, cs, fs = _planes(o, fmt, H, W)
+    y, yp, u, v, cp, c_step, fs = _planes(o, fmt, H, W)
     st = torch.cuda.current_stream(dev).cuda_stream
     with torch.cuda.device(dev):
         if fmt in DEEP_FORMATS:
-            K.check(ctx.lib.savsr_bgr48_to_yuv420_10(ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, cs, fs, int(fmt == "p010"), st))
+            args = (ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, c_step, fs, int(fmt == "p010"), *cs, st)
+            K.check((ctx.lib.savsr_bgr48_to_yuv420_10_cs if cs else ctx.lib.savsr_bgr48_to_yuv420_10)(*args))
         else:
-            K.check(ctx.lib.savsr_bgr_to_yuv420(ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, cs, fs, st))
+            args = (ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, c_step, fs, *cs, st)
+            K.check((ctx.lib.savsr_bgr_to_yuv420_cs if cs else ctx.lib.savsr_bgr_to_yuv420)(*args))
     return out
 
 

@@ -16,6 +16,9 @@
 // 10-bit YUV 4:2:0 <-> 16-bit BGR (yuv420p10le, p010 <-> bgr48): the same matrix, chroma handling and work split in fixed-point forms
 // rescaled to the deeper samples (common.cuh), with pitches and frame strides in uint16 elements.  A thread's rows are 16 bytes of Y and
 // 48 of BGR, so 16-byte accesses are used where the row's alignment allows.  widen_u8_to_u16 brings 8-bit BGR frames into a 16-bit ring.
+//
+// Other colour matrices and ranges (the _cs entry points): the same four kernel bodies over the H.273 map of one (colorspace, range)
+// pair, one instantiation per pair with the coefficients of common.cuh's kYuvCoeffs8 / kYuvCoeffs10 as compile-time constants.
 #include "common.cuh"
 
 namespace savsr {
@@ -107,6 +110,39 @@ __device__ __forceinline__ int rgb_y(int R, int G, int B) { return (kRgbYR * R +
 __device__ __forceinline__ int rgb_u(int R, int G, int B) { return (kRgbUR * R + kRgbUG * G + kRgbUB * B + (128 << kYuvShift) + kYuvHalf) >> kYuvShift; }
 __device__ __forceinline__ int rgb_v(int R, int G, int B) { return (kRgbVR * R + kRgbVG * G + kRgbVB * B + (128 << kYuvShift) + kYuvHalf) >> kYuvShift; }
 
+// The kernel bodies are written over a pixel map: chroma(U, V) once per 2x2 block and pixel(c, Y, B, G, R) per pixel (decode), and
+// y, u, v of (R, G, B) (encode).  Cv2Map8: the cv2-exact BT.601 limited-range functions above.  CsMap8<CS, RNG>: the H.273 map of
+// one (matrix, range) pair, its coefficients compile-time constants from kYuvCoeffs8 (one instantiation per pair: with the
+// coefficients passed by value instead, the 8-bit encode needed 62 registers instead of 40 and ran 17 % slower at 1080p x 26).
+struct Cv2Map8 {
+  using Chroma = savsr::Chroma;
+  __device__ __forceinline__ Chroma chroma(int U, int V) const { return Chroma(U, V); }
+  __device__ __forceinline__ void pixel(const Chroma& c, int Y, int& B, int& G, int& R) const { c.bgr(Y, B, G, R); }
+  __device__ __forceinline__ int y(int R, int G, int B) const { return rgb_y(R, G, B); }
+  __device__ __forceinline__ int u(int R, int G, int B) const { return rgb_u(R, G, B); }
+  __device__ __forceinline__ int v(int R, int G, int B) const { return rgb_v(R, G, B); }
+};
+
+template <int CS, int RNG>
+struct CsMap8 {
+  struct Chroma { int r, g, b; };
+  static constexpr YuvCoeffs k = kYuvCoeffs8[CS][RNG];
+  static constexpr int kHalf = 1 << (kCs8Shift - 1);
+  __device__ __forceinline__ Chroma chroma(int U, int V) const {
+    const int u = U - 128, v = V - 128;
+    return {kHalf + k.dvr * v, kHalf + k.dvg * v + k.dug * u, kHalf + k.dub * u};
+  }
+  __device__ __forceinline__ void pixel(const Chroma& c, int Y, int& B, int& G, int& R) const {
+    const int y = (Y - k.y0) * k.dy;
+    B = sat_u8((y + c.b) >> kCs8Shift);
+    G = sat_u8((y + c.g) >> kCs8Shift);
+    R = sat_u8((y + c.r) >> kCs8Shift);
+  }
+  __device__ __forceinline__ int y(int R, int G, int B) const { return sat_u8(k.y0 + ((k.eyr * R + k.eyg * G + k.eyb * B + kHalf) >> kCs8Shift)); }
+  __device__ __forceinline__ int u(int R, int G, int B) const { return sat_u8(128 + ((k.eur * R + k.eug * G + k.eub * B + kHalf) >> kCs8Shift)); }
+  __device__ __forceinline__ int v(int R, int G, int B) const { return sat_u8(128 + ((k.evr * R + k.evg * G + k.evb * B + kHalf) >> kCs8Shift)); }
+};
+
 struct Yuv420Planes {
   uint8_t* y;
   uint8_t* u;
@@ -123,7 +159,8 @@ __device__ __forceinline__ void yuv_item(long long idx, int groups, int half_h, 
   f = static_cast<int>(rest / half_h);
 }
 
-__global__ void __launch_bounds__(256) yuv420_to_bgr_kernel(const Yuv420Planes p, int n, int h, int w, uint8_t* __restrict__ bgr) {
+template <class Map>
+__device__ __forceinline__ void yuv420_to_bgr_body(const Yuv420Planes& p, int n, int h, int w, uint8_t* __restrict__ bgr, const Map& m) {
   const int groups = (w + kYuvGroup - 1) / kYuvGroup, half_h = h >> 1;
   const long long total = static_cast<long long>(n) * half_h * groups;
   for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
@@ -151,29 +188,29 @@ __global__ void __launch_bounds__(256) yuv420_to_bgr_kernel(const Yuv420Planes p
         uw[0] = __byte_perm(uv[0], uv[1], 0x6420);
         vw[0] = __byte_perm(uv[0], uv[1], 0x7531);
       }
-      Chroma c[kYuvGroup / 2];
+      typename Map::Chroma c[kYuvGroup / 2];
 #pragma unroll
-      for (int k = 0; k < kYuvGroup / 2; ++k) c[k] = Chroma(byte_at(uw, k), byte_at(vw, k));
+      for (int k = 0; k < kYuvGroup / 2; ++k) c[k] = m.chroma(byte_at(uw, k), byte_at(vw, k));
 #pragma unroll
       for (int r = 0; r < 2; ++r) {                // one row at a time: the 24 output bytes of a row stay in 6 registers
         uint32_t o[6] = {0, 0, 0, 0, 0, 0};
 #pragma unroll
         for (int j = 0; j < kYuvGroup; ++j) {
           int B, G, R;
-          c[j >> 1].bgr(byte_at(r ? yb : ya, j), B, G, R);
+          m.pixel(c[j >> 1], byte_at(r ? yb : ya, j), B, G, R);
           put_byte(o, 3 * j, B); put_byte(o, 3 * j + 1, G); put_byte(o, 3 * j + 2, R);
         }
         store_bytes<24>(r ? o1 : o0, o);
       }
     } else {
       for (int j = 0; x0 + j < w; j += 2) {
-        const Chroma c(u[(j >> 1) * p.c_step], v[(j >> 1) * p.c_step]);
+        const typename Map::Chroma c = m.chroma(u[(j >> 1) * p.c_step], v[(j >> 1) * p.c_step]);
 #pragma unroll
         for (int d = 0; d < 2; ++d) {
           int B, G, R;
-          c.bgr(y0[j + d], B, G, R);
+          m.pixel(c, y0[j + d], B, G, R);
           o0[3 * (j + d)] = B; o0[3 * (j + d) + 1] = G; o0[3 * (j + d) + 2] = R;
-          c.bgr(y1[j + d], B, G, R);
+          m.pixel(c, y1[j + d], B, G, R);
           o1[3 * (j + d)] = B; o1[3 * (j + d) + 1] = G; o1[3 * (j + d) + 2] = R;
         }
       }
@@ -181,7 +218,16 @@ __global__ void __launch_bounds__(256) yuv420_to_bgr_kernel(const Yuv420Planes p
   }
 }
 
-__global__ void __launch_bounds__(256) bgr_to_yuv420_kernel(const uint8_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes p) {
+__global__ void __launch_bounds__(256) yuv420_to_bgr_kernel(const Yuv420Planes p, int n, int h, int w, uint8_t* __restrict__ bgr) {
+  yuv420_to_bgr_body(p, n, h, w, bgr, Cv2Map8{});
+}
+template <int CS, int RNG>
+__global__ void __launch_bounds__(256) yuv420_to_bgr_cs_kernel(const Yuv420Planes p, int n, int h, int w, uint8_t* __restrict__ bgr) {
+  yuv420_to_bgr_body(p, n, h, w, bgr, CsMap8<CS, RNG>{});
+}
+
+template <class Map>
+__device__ __forceinline__ void bgr_to_yuv420_body(const uint8_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes& p, const Map& m) {
   const int groups = (w + kYuvGroup - 1) / kYuvGroup, half_h = h >> 1;
   const long long total = static_cast<long long>(n) * half_h * groups;
   for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
@@ -204,12 +250,12 @@ __global__ void __launch_bounds__(256) bgr_to_yuv420_kernel(const uint8_t* __res
 #pragma unroll
       for (int j = 0; j < kYuvGroup; ++j) {
         const int B = byte_at(ia, 3 * j), G = byte_at(ia, 3 * j + 1), R = byte_at(ia, 3 * j + 2);
-        put_byte(ya, j, rgb_y(R, G, B));
+        put_byte(ya, j, m.y(R, G, B));
         if ((j & 1) == 0) {                        // the top-left pixel of its 2x2 block
-          put_byte(uw, j >> 1, rgb_u(R, G, B));
-          put_byte(vw, j >> 1, rgb_v(R, G, B));
+          put_byte(uw, j >> 1, m.u(R, G, B));
+          put_byte(vw, j >> 1, m.v(R, G, B));
         }
-        put_byte(yb, j, rgb_y(byte_at(ib, 3 * j + 2), byte_at(ib, 3 * j + 1), byte_at(ib, 3 * j)));
+        put_byte(yb, j, m.y(byte_at(ib, 3 * j + 2), byte_at(ib, 3 * j + 1), byte_at(ib, 3 * j)));
       }
       store_bytes<8>(y0, ya);
       store_bytes<8>(y1, yb);
@@ -223,18 +269,26 @@ __global__ void __launch_bounds__(256) bgr_to_yuv420_kernel(const uint8_t* __res
     } else {
       for (int j = 0; x0 + j < w; j += 2) {
         const uint8_t* a = i0 + 3 * j;
-        u[(j >> 1) * p.c_step] = static_cast<uint8_t>(rgb_u(a[2], a[1], a[0]));
-        v[(j >> 1) * p.c_step] = static_cast<uint8_t>(rgb_v(a[2], a[1], a[0]));
+        u[(j >> 1) * p.c_step] = static_cast<uint8_t>(m.u(a[2], a[1], a[0]));
+        v[(j >> 1) * p.c_step] = static_cast<uint8_t>(m.v(a[2], a[1], a[0]));
 #pragma unroll
         for (int d = 0; d < 2; ++d) {
           const uint8_t* q0 = i0 + 3 * (j + d);
           const uint8_t* q1 = i1 + 3 * (j + d);
-          y0[j + d] = static_cast<uint8_t>(rgb_y(q0[2], q0[1], q0[0]));
-          y1[j + d] = static_cast<uint8_t>(rgb_y(q1[2], q1[1], q1[0]));
+          y0[j + d] = static_cast<uint8_t>(m.y(q0[2], q0[1], q0[0]));
+          y1[j + d] = static_cast<uint8_t>(m.y(q1[2], q1[1], q1[0]));
         }
       }
     }
   }
+}
+
+__global__ void __launch_bounds__(256) bgr_to_yuv420_kernel(const uint8_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes p) {
+  bgr_to_yuv420_body(bgr, n, h, w, p, Cv2Map8{});
+}
+template <int CS, int RNG>
+__global__ void __launch_bounds__(256) bgr_to_yuv420_cs_kernel(const uint8_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes p) {
+  bgr_to_yuv420_body(bgr, n, h, w, p, CsMap8<CS, RNG>{});
 }
 
 // ------------------------------------------------------------------------------------------------ 10-bit YUV <-> 16-bit BGR
@@ -272,6 +326,45 @@ __device__ __forceinline__ int rgb_u10(int R, int G, int B) {
 __device__ __forceinline__ int rgb_v10(int R, int G, int B) {
   return (kRgb10VR * R + kRgb10VG * G + kRgb10VB * B + (512 << kRgb10Shift) + kRgb10Half) >> kRgb10Shift;
 }
+__device__ __forceinline__ int sat_u10(int v) { return min(max(v, 0), 1023); }
+
+// The 10-bit pixel maps, as Cv2Map8 / CsMap8 (10-bit YUV samples, 16-bit BGR; coefficients from kYuvCoeffs10).
+struct Cv2Map10 {
+  using Chroma = Chroma10;
+  __device__ __forceinline__ Chroma chroma(int U, int V) const { return Chroma(U, V); }
+  __device__ __forceinline__ void pixel(const Chroma& c, int Y, int& B, int& G, int& R) const { c.bgr(Y, B, G, R); }
+  __device__ __forceinline__ int y(int R, int G, int B) const { return rgb_y10(R, G, B); }
+  __device__ __forceinline__ int u(int R, int G, int B) const { return rgb_u10(R, G, B); }
+  __device__ __forceinline__ int v(int R, int G, int B) const { return rgb_v10(R, G, B); }
+};
+
+template <int CS, int RNG>
+struct CsMap10 {
+  struct Chroma { long long r, g, b; };
+  static constexpr YuvCoeffs k = kYuvCoeffs10[CS][RNG];
+  static constexpr long long kDecHalf = 1LL << (kCs10DecShift - 1);
+  static constexpr int kEncHalf = 1 << (kCs10EncShift - 1);
+  __device__ __forceinline__ Chroma chroma(int U, int V) const {
+    const int u = U - 512, v = V - 512;
+    return {kDecHalf + static_cast<long long>(k.dvr) * v, kDecHalf + static_cast<long long>(k.dvg) * v + static_cast<long long>(k.dug) * u,
+            kDecHalf + static_cast<long long>(k.dub) * u};
+  }
+  __device__ __forceinline__ void pixel(const Chroma& c, int Y, int& B, int& G, int& R) const {
+    const long long y = static_cast<long long>(Y - k.y0) * k.dy;
+    B = sat_u16(static_cast<int>((y + c.b) >> kCs10DecShift));
+    G = sat_u16(static_cast<int>((y + c.g) >> kCs10DecShift));
+    R = sat_u16(static_cast<int>((y + c.r) >> kCs10DecShift));
+  }
+  __device__ __forceinline__ int y(int R, int G, int B) const {
+    return sat_u10(k.y0 + ((k.eyr * R + k.eyg * G + k.eyb * B + kEncHalf) >> kCs10EncShift));
+  }
+  __device__ __forceinline__ int u(int R, int G, int B) const {
+    return sat_u10(512 + ((k.eur * R + k.eug * G + k.eub * B + kEncHalf) >> kCs10EncShift));
+  }
+  __device__ __forceinline__ int v(int R, int G, int B) const {
+    return sat_u10(512 + ((k.evr * R + k.evg * G + k.evb * B + kEncHalf) >> kCs10EncShift));
+  }
+};
 
 // Yuv420Planes in uint16 elements, plus where the 10 bits sit (msb: 1 for p010, 0 for yuv420p10le).
 struct Yuv420Planes16 {
@@ -288,7 +381,8 @@ __device__ __forceinline__ const uint8_t* as_bytes(const T* p) { return reinterp
 template <class T>
 __device__ __forceinline__ uint8_t* as_bytes(T* p) { return reinterpret_cast<uint8_t*>(p); }
 
-__global__ void __launch_bounds__(256) yuv420_10_to_bgr48_kernel(const Yuv420Planes16 p, int n, int h, int w, uint16_t* __restrict__ bgr) {
+template <class Map>
+__device__ __forceinline__ void yuv420_10_to_bgr48_body(const Yuv420Planes16& p, int n, int h, int w, uint16_t* __restrict__ bgr, const Map& m) {
   const int groups = (w + kYuvGroup - 1) / kYuvGroup, half_h = h >> 1;
   const long long total = static_cast<long long>(n) * half_h * groups;
   for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
@@ -316,29 +410,29 @@ __global__ void __launch_bounds__(256) yuv420_10_to_bgr48_kernel(const Yuv420Pla
         uw[0] = __byte_perm(uv[0], uv[1], 0x5410); uw[1] = __byte_perm(uv[2], uv[3], 0x5410);
         vw[0] = __byte_perm(uv[0], uv[1], 0x7632); vw[1] = __byte_perm(uv[2], uv[3], 0x7632);
       }
-      Chroma10 c[kYuvGroup / 2];
+      typename Map::Chroma c[kYuvGroup / 2];
 #pragma unroll
-      for (int k = 0; k < kYuvGroup / 2; ++k) c[k] = Chroma10(sample10(half_at(uw, k), p.msb), sample10(half_at(vw, k), p.msb));
+      for (int k = 0; k < kYuvGroup / 2; ++k) c[k] = m.chroma(sample10(half_at(uw, k), p.msb), sample10(half_at(vw, k), p.msb));
 #pragma unroll
       for (int r = 0; r < 2; ++r) {                // one row at a time: the 48 output bytes of a row stay in 12 registers
         uint32_t o[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
 #pragma unroll
         for (int j = 0; j < kYuvGroup; ++j) {
           int B, G, R;
-          c[j >> 1].bgr(sample10(half_at(r ? yb : ya, j), p.msb), B, G, R);
+          m.pixel(c[j >> 1], sample10(half_at(r ? yb : ya, j), p.msb), B, G, R);
           put_half(o, 3 * j, B); put_half(o, 3 * j + 1, G); put_half(o, 3 * j + 2, R);
         }
         store_bytes<48>(as_bytes(r ? o1 : o0), o);
       }
     } else {
       for (int j = 0; x0 + j < w; j += 2) {
-        const Chroma10 c(sample10(u[(j >> 1) * p.c_step], p.msb), sample10(v[(j >> 1) * p.c_step], p.msb));
+        const typename Map::Chroma c = m.chroma(sample10(u[(j >> 1) * p.c_step], p.msb), sample10(v[(j >> 1) * p.c_step], p.msb));
 #pragma unroll
         for (int d = 0; d < 2; ++d) {
           int B, G, R;
-          c.bgr(sample10(y0[j + d], p.msb), B, G, R);
+          m.pixel(c, sample10(y0[j + d], p.msb), B, G, R);
           o0[3 * (j + d)] = B; o0[3 * (j + d) + 1] = G; o0[3 * (j + d) + 2] = R;
-          c.bgr(sample10(y1[j + d], p.msb), B, G, R);
+          m.pixel(c, sample10(y1[j + d], p.msb), B, G, R);
           o1[3 * (j + d)] = B; o1[3 * (j + d) + 1] = G; o1[3 * (j + d) + 2] = R;
         }
       }
@@ -346,7 +440,17 @@ __global__ void __launch_bounds__(256) yuv420_10_to_bgr48_kernel(const Yuv420Pla
   }
 }
 
-__global__ void __launch_bounds__(256) bgr48_to_yuv420_10_kernel(const uint16_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes16 p) {
+__global__ void __launch_bounds__(256) yuv420_10_to_bgr48_kernel(const Yuv420Planes16 p, int n, int h, int w, uint16_t* __restrict__ bgr) {
+  yuv420_10_to_bgr48_body(p, n, h, w, bgr, Cv2Map10{});
+}
+template <int CS, int RNG>
+__global__ void __launch_bounds__(256) yuv420_10_to_bgr48_cs_kernel(const Yuv420Planes16 p, int n, int h, int w, uint16_t* __restrict__ bgr) {
+  yuv420_10_to_bgr48_body(p, n, h, w, bgr, CsMap10<CS, RNG>{});
+}
+
+template <class Map>
+__device__ __forceinline__ void bgr48_to_yuv420_10_body(const uint16_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes16& p,
+                                                        const Map& m) {
   const int groups = (w + kYuvGroup - 1) / kYuvGroup, half_h = h >> 1;
   const long long total = static_cast<long long>(n) * half_h * groups;
   const int sh = p.msb ? 6 : 0;
@@ -370,12 +474,12 @@ __global__ void __launch_bounds__(256) bgr48_to_yuv420_10_kernel(const uint16_t*
 #pragma unroll
       for (int j = 0; j < kYuvGroup; ++j) {
         const int B = half_at(ia, 3 * j), G = half_at(ia, 3 * j + 1), R = half_at(ia, 3 * j + 2);
-        put_half(ya, j, rgb_y10(R, G, B) << sh);
+        put_half(ya, j, m.y(R, G, B) << sh);
         if ((j & 1) == 0) {                        // the top-left pixel of its 2x2 block
-          put_half(uw, j >> 1, rgb_u10(R, G, B) << sh);
-          put_half(vw, j >> 1, rgb_v10(R, G, B) << sh);
+          put_half(uw, j >> 1, m.u(R, G, B) << sh);
+          put_half(vw, j >> 1, m.v(R, G, B) << sh);
         }
-        put_half(yb, j, rgb_y10(half_at(ib, 3 * j + 2), half_at(ib, 3 * j + 1), half_at(ib, 3 * j)) << sh);
+        put_half(yb, j, m.y(half_at(ib, 3 * j + 2), half_at(ib, 3 * j + 1), half_at(ib, 3 * j)) << sh);
       }
       store_bytes<16>(as_bytes(y0), ya);
       store_bytes<16>(as_bytes(y1), yb);
@@ -390,18 +494,26 @@ __global__ void __launch_bounds__(256) bgr48_to_yuv420_10_kernel(const uint16_t*
     } else {
       for (int j = 0; x0 + j < w; j += 2) {
         const uint16_t* a = i0 + 3 * j;
-        u[(j >> 1) * p.c_step] = static_cast<uint16_t>(rgb_u10(a[2], a[1], a[0]) << sh);
-        v[(j >> 1) * p.c_step] = static_cast<uint16_t>(rgb_v10(a[2], a[1], a[0]) << sh);
+        u[(j >> 1) * p.c_step] = static_cast<uint16_t>(m.u(a[2], a[1], a[0]) << sh);
+        v[(j >> 1) * p.c_step] = static_cast<uint16_t>(m.v(a[2], a[1], a[0]) << sh);
 #pragma unroll
         for (int d = 0; d < 2; ++d) {
           const uint16_t* q0 = i0 + 3 * (j + d);
           const uint16_t* q1 = i1 + 3 * (j + d);
-          y0[j + d] = static_cast<uint16_t>(rgb_y10(q0[2], q0[1], q0[0]) << sh);
-          y1[j + d] = static_cast<uint16_t>(rgb_y10(q1[2], q1[1], q1[0]) << sh);
+          y0[j + d] = static_cast<uint16_t>(m.y(q0[2], q0[1], q0[0]) << sh);
+          y1[j + d] = static_cast<uint16_t>(m.y(q1[2], q1[1], q1[0]) << sh);
         }
       }
     }
   }
+}
+
+__global__ void __launch_bounds__(256) bgr48_to_yuv420_10_kernel(const uint16_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes16 p) {
+  bgr48_to_yuv420_10_body(bgr, n, h, w, p, Cv2Map10{});
+}
+template <int CS, int RNG>
+__global__ void __launch_bounds__(256) bgr48_to_yuv420_10_cs_kernel(const uint16_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes16 p) {
+  bgr48_to_yuv420_10_body(bgr, n, h, w, p, CsMap10<CS, RNG>{});
 }
 
 // x 257 (u -> u << 8 | u): 16 bytes in, 32 out per thread where both pointers are 16-byte aligned, one byte at a time otherwise.
@@ -442,59 +554,140 @@ static unsigned yuv_blocks(const savsr_ctx* ctx, int n, int h, int w) {
   return grid_for(ctx, static_cast<long long>(n) * (h / 2) * ((w + kYuvGroup - 1) / kYuvGroup));
 }
 
+// The kernel of (colorspace, range) for the _cs entry points: the cv2-exact kernel of the plain entry point for (BT601, TV), else the
+// pair's H.273 instantiation; an error naming the value for anything not in enum savsr_colorspace / savsr_color_range.
+template <class F>
+static int cs_kernel(const char* fn, int colorspace, int range, F plain, const F (&table)[3][2], F* k) {
+  SAVSR_REQUIRE(colorspace >= SAVSR_COLORSPACE_BT601 && colorspace <= SAVSR_COLORSPACE_BT2020NC,
+                "%s: unknown colorspace %d (0 BT601, 1 BT709, 2 BT2020NC)", fn, colorspace);
+  SAVSR_REQUIRE(range == SAVSR_RANGE_TV || range == SAVSR_RANGE_PC, "%s: unknown color range %d (0 TV, 1 PC)", fn, range);
+  *k = colorspace == SAVSR_COLORSPACE_BT601 && range == SAVSR_RANGE_TV ? plain : table[colorspace][range];
+  return 0;
+}
+#define SAVSR_CS_TABLE(kernel) {{nullptr, kernel<0, 1>}, {kernel<1, 0>, kernel<1, 1>}, {kernel<2, 0>, kernel<2, 1>}}
+using Dec8Kernel = void (*)(const Yuv420Planes, int, int, int, uint8_t*);
+using Enc8Kernel = void (*)(const uint8_t*, int, int, int, const Yuv420Planes);
+using Dec10Kernel = void (*)(const Yuv420Planes16, int, int, int, uint16_t*);
+using Enc10Kernel = void (*)(const uint16_t*, int, int, int, const Yuv420Planes16);
+static const Dec8Kernel kDec8Cs[3][2] = SAVSR_CS_TABLE(yuv420_to_bgr_cs_kernel);
+static const Enc8Kernel kEnc8Cs[3][2] = SAVSR_CS_TABLE(bgr_to_yuv420_cs_kernel);
+static const Dec10Kernel kDec10Cs[3][2] = SAVSR_CS_TABLE(yuv420_10_to_bgr48_cs_kernel);
+static const Enc10Kernel kEnc10Cs[3][2] = SAVSR_CS_TABLE(bgr48_to_yuv420_10_cs_kernel);
+#undef SAVSR_CS_TABLE
+
+// The four conversions, with the kernel to launch.
+static int yuv420_to_bgr(const char* fn, savsr_ctx* ctx, const uint8_t* y, int y_pitch, const uint8_t* u, const uint8_t* v, int c_pitch,
+                         int c_step, int64_t frame_stride, int n, int h, int w, uint8_t* bgr, Dec8Kernel k, savsr_stream st) {
+  SAVSR_REQUIRE(ctx && y && u && v && bgr, "%s: null pointer", fn);
+  if (check_yuv420(fn, n, h, w, y_pitch, c_pitch, c_step, frame_stride)) return 1;
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const Yuv420Planes p{const_cast<uint8_t*>(y), const_cast<uint8_t*>(u), const_cast<uint8_t*>(v), y_pitch, c_pitch, c_step, frame_stride};
+  k<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(p, n, h, w, bgr);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
+}
+
+static int bgr_to_yuv420(const char* fn, savsr_ctx* ctx, const uint8_t* bgr, int n, int h, int w, uint8_t* y, int y_pitch, uint8_t* u,
+                         uint8_t* v, int c_pitch, int c_step, int64_t frame_stride, Enc8Kernel k, savsr_stream st) {
+  SAVSR_REQUIRE(ctx && bgr && y && u && v, "%s: null pointer", fn);
+  if (check_yuv420(fn, n, h, w, y_pitch, c_pitch, c_step, frame_stride)) return 1;
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const Yuv420Planes p{y, u, v, y_pitch, c_pitch, c_step, frame_stride};
+  k<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(bgr, n, h, w, p);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
+}
+
+static int yuv420_10_to_bgr48(const char* fn, savsr_ctx* ctx, const uint16_t* y, int y_pitch, const uint16_t* u, const uint16_t* v,
+                              int c_pitch, int c_step, int64_t frame_stride, int msb, int n, int h, int w, uint16_t* bgr, Dec10Kernel k,
+                              savsr_stream st) {
+  SAVSR_REQUIRE(ctx && y && u && v && bgr, "%s: null pointer", fn);
+  if (check_yuv420(fn, n, h, w, y_pitch, c_pitch, c_step, frame_stride, true)) return 1;
+  SAVSR_REQUIRE(msb == 0 || msb == 1, "%s: msb must be 0 (yuv420p10le) or 1 (p010), got %d", fn, msb);
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const Yuv420Planes16 p{const_cast<uint16_t*>(y), const_cast<uint16_t*>(u), const_cast<uint16_t*>(v), y_pitch, c_pitch, c_step,
+                         frame_stride, msb};
+  k<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(p, n, h, w, bgr);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
+}
+
+static int bgr48_to_yuv420_10(const char* fn, savsr_ctx* ctx, const uint16_t* bgr, int n, int h, int w, uint16_t* y, int y_pitch,
+                              uint16_t* u, uint16_t* v, int c_pitch, int c_step, int64_t frame_stride, int msb, Enc10Kernel k,
+                              savsr_stream st) {
+  SAVSR_REQUIRE(ctx && bgr && y && u && v, "%s: null pointer", fn);
+  if (check_yuv420(fn, n, h, w, y_pitch, c_pitch, c_step, frame_stride, true)) return 1;
+  SAVSR_REQUIRE(msb == 0 || msb == 1, "%s: msb must be 0 (yuv420p10le) or 1 (p010), got %d", fn, msb);
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const Yuv420Planes16 p{y, u, v, y_pitch, c_pitch, c_step, frame_stride, msb};
+  k<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(bgr, n, h, w, p);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
+}
+
 }  // namespace savsr
 
 using namespace savsr;
 
 extern "C" int savsr_yuv420_to_bgr(savsr_ctx* ctx, const uint8_t* y, int y_pitch, const uint8_t* u, const uint8_t* v, int c_pitch,
                                    int c_step, int64_t frame_stride, int n, int h, int w, uint8_t* bgr, savsr_stream st) {
-  SAVSR_REQUIRE(ctx && y && u && v && bgr, "savsr_yuv420_to_bgr: null pointer");
-  if (check_yuv420("savsr_yuv420_to_bgr", n, h, w, y_pitch, c_pitch, c_step, frame_stride)) return 1;
-  if (n == 0) return 0;
-  DeviceGuard guard(ctx->device);
-  const Yuv420Planes p{const_cast<uint8_t*>(y), const_cast<uint8_t*>(u), const_cast<uint8_t*>(v), y_pitch, c_pitch, c_step, frame_stride};
-  yuv420_to_bgr_kernel<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(p, n, h, w, bgr);
-  SAVSR_CUDA(cudaGetLastError());
-  return 0;
+  return savsr::yuv420_to_bgr("savsr_yuv420_to_bgr", ctx, y, y_pitch, u, v, c_pitch, c_step, frame_stride, n, h, w, bgr, yuv420_to_bgr_kernel, st);
+}
+
+extern "C" int savsr_yuv420_to_bgr_cs(savsr_ctx* ctx, const uint8_t* y, int y_pitch, const uint8_t* u, const uint8_t* v, int c_pitch,
+                                      int c_step, int64_t frame_stride, int n, int h, int w, uint8_t* bgr, int colorspace, int range,
+                                      savsr_stream st) {
+  const char* fn = "savsr_yuv420_to_bgr_cs";
+  Dec8Kernel k;
+  if (cs_kernel(fn, colorspace, range, static_cast<Dec8Kernel>(yuv420_to_bgr_kernel), kDec8Cs, &k)) return 1;
+  return savsr::yuv420_to_bgr(fn, ctx, y, y_pitch, u, v, c_pitch, c_step, frame_stride, n, h, w, bgr, k, st);
 }
 
 extern "C" int savsr_bgr_to_yuv420(savsr_ctx* ctx, const uint8_t* bgr, int n, int h, int w, uint8_t* y, int y_pitch, uint8_t* u, uint8_t* v,
                                    int c_pitch, int c_step, int64_t frame_stride, savsr_stream st) {
-  SAVSR_REQUIRE(ctx && bgr && y && u && v, "savsr_bgr_to_yuv420: null pointer");
-  if (check_yuv420("savsr_bgr_to_yuv420", n, h, w, y_pitch, c_pitch, c_step, frame_stride)) return 1;
-  if (n == 0) return 0;
-  DeviceGuard guard(ctx->device);
-  const Yuv420Planes p{y, u, v, y_pitch, c_pitch, c_step, frame_stride};
-  bgr_to_yuv420_kernel<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(bgr, n, h, w, p);
-  SAVSR_CUDA(cudaGetLastError());
-  return 0;
+  return savsr::bgr_to_yuv420("savsr_bgr_to_yuv420", ctx, bgr, n, h, w, y, y_pitch, u, v, c_pitch, c_step, frame_stride, bgr_to_yuv420_kernel, st);
+}
+
+extern "C" int savsr_bgr_to_yuv420_cs(savsr_ctx* ctx, const uint8_t* bgr, int n, int h, int w, uint8_t* y, int y_pitch, uint8_t* u,
+                                      uint8_t* v, int c_pitch, int c_step, int64_t frame_stride, int colorspace, int range, savsr_stream st) {
+  const char* fn = "savsr_bgr_to_yuv420_cs";
+  Enc8Kernel k;
+  if (cs_kernel(fn, colorspace, range, static_cast<Enc8Kernel>(bgr_to_yuv420_kernel), kEnc8Cs, &k)) return 1;
+  return savsr::bgr_to_yuv420(fn, ctx, bgr, n, h, w, y, y_pitch, u, v, c_pitch, c_step, frame_stride, k, st);
 }
 
 extern "C" int savsr_yuv420_10_to_bgr48(savsr_ctx* ctx, const uint16_t* y, int y_pitch, const uint16_t* u, const uint16_t* v, int c_pitch,
                                         int c_step, int64_t frame_stride, int msb, int n, int h, int w, uint16_t* bgr, savsr_stream st) {
-  SAVSR_REQUIRE(ctx && y && u && v && bgr, "savsr_yuv420_10_to_bgr48: null pointer");
-  if (check_yuv420("savsr_yuv420_10_to_bgr48", n, h, w, y_pitch, c_pitch, c_step, frame_stride, true)) return 1;
-  SAVSR_REQUIRE(msb == 0 || msb == 1, "savsr_yuv420_10_to_bgr48: msb must be 0 (yuv420p10le) or 1 (p010), got %d", msb);
-  if (n == 0) return 0;
-  DeviceGuard guard(ctx->device);
-  const Yuv420Planes16 p{const_cast<uint16_t*>(y), const_cast<uint16_t*>(u), const_cast<uint16_t*>(v), y_pitch, c_pitch, c_step,
-                         frame_stride, msb};
-  yuv420_10_to_bgr48_kernel<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(p, n, h, w, bgr);
-  SAVSR_CUDA(cudaGetLastError());
-  return 0;
+  return savsr::yuv420_10_to_bgr48("savsr_yuv420_10_to_bgr48", ctx, y, y_pitch, u, v, c_pitch, c_step, frame_stride, msb, n, h, w, bgr,
+                                   yuv420_10_to_bgr48_kernel, st);
+}
+
+extern "C" int savsr_yuv420_10_to_bgr48_cs(savsr_ctx* ctx, const uint16_t* y, int y_pitch, const uint16_t* u, const uint16_t* v,
+                                           int c_pitch, int c_step, int64_t frame_stride, int msb, int n, int h, int w, uint16_t* bgr,
+                                           int colorspace, int range, savsr_stream st) {
+  const char* fn = "savsr_yuv420_10_to_bgr48_cs";
+  Dec10Kernel k;
+  if (cs_kernel(fn, colorspace, range, static_cast<Dec10Kernel>(yuv420_10_to_bgr48_kernel), kDec10Cs, &k)) return 1;
+  return savsr::yuv420_10_to_bgr48(fn, ctx, y, y_pitch, u, v, c_pitch, c_step, frame_stride, msb, n, h, w, bgr, k, st);
 }
 
 extern "C" int savsr_bgr48_to_yuv420_10(savsr_ctx* ctx, const uint16_t* bgr, int n, int h, int w, uint16_t* y, int y_pitch, uint16_t* u,
                                         uint16_t* v, int c_pitch, int c_step, int64_t frame_stride, int msb, savsr_stream st) {
-  SAVSR_REQUIRE(ctx && bgr && y && u && v, "savsr_bgr48_to_yuv420_10: null pointer");
-  if (check_yuv420("savsr_bgr48_to_yuv420_10", n, h, w, y_pitch, c_pitch, c_step, frame_stride, true)) return 1;
-  SAVSR_REQUIRE(msb == 0 || msb == 1, "savsr_bgr48_to_yuv420_10: msb must be 0 (yuv420p10le) or 1 (p010), got %d", msb);
-  if (n == 0) return 0;
-  DeviceGuard guard(ctx->device);
-  const Yuv420Planes16 p{y, u, v, y_pitch, c_pitch, c_step, frame_stride, msb};
-  bgr48_to_yuv420_10_kernel<<<yuv_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(bgr, n, h, w, p);
-  SAVSR_CUDA(cudaGetLastError());
-  return 0;
+  return savsr::bgr48_to_yuv420_10("savsr_bgr48_to_yuv420_10", ctx, bgr, n, h, w, y, y_pitch, u, v, c_pitch, c_step, frame_stride, msb,
+                                   bgr48_to_yuv420_10_kernel, st);
+}
+
+extern "C" int savsr_bgr48_to_yuv420_10_cs(savsr_ctx* ctx, const uint16_t* bgr, int n, int h, int w, uint16_t* y, int y_pitch, uint16_t* u,
+                                           uint16_t* v, int c_pitch, int c_step, int64_t frame_stride, int msb, int colorspace, int range,
+                                           savsr_stream st) {
+  const char* fn = "savsr_bgr48_to_yuv420_10_cs";
+  Enc10Kernel k;
+  if (cs_kernel(fn, colorspace, range, static_cast<Enc10Kernel>(bgr48_to_yuv420_10_kernel), kEnc10Cs, &k)) return 1;
+  return savsr::bgr48_to_yuv420_10(fn, ctx, bgr, n, h, w, y, y_pitch, u, v, c_pitch, c_step, frame_stride, msb, k, st);
 }
 
 extern "C" int savsr_widen_u8_to_u16(savsr_ctx* ctx, const uint8_t* src, int n, int h, int w, uint16_t* dst, savsr_stream st) {

@@ -94,6 +94,44 @@ constexpr int kRgb10Shift = 21, kRgb10Half = 1 << (kRgb10Shift - 1);
 constexpr int kRgb10YR = 8389, kRgb10YG = 16451, kRgb10YB = 3199;
 constexpr int kRgb10UR = -4831, kRgb10UG = -9498, kRgb10UB = 14329;
 constexpr int kRgb10VR = 14329, kRgb10VG = -12012, kRgb10VB = -2317;
+// Y'CbCr <-> R'G'B' of ITU-T H.273 for the other (matrix, range) pairs (the _cs entry points; colour.cu).  Kr, Kb: BT.601 0.299,
+// 0.114; BT.709 0.2126, 0.0722; BT.2020 non-constant luminance 0.2627, 0.0593; Kg = 1 - Kr - Kb.  n = YUV bit depth (8, 10), M = BGR
+// full scale (255, 65535), s = 2^(n-8).  Range tv: black level y0 = 16 s, luma span ys = 219 s, chroma span cs = 224 s; pc: y0 = 0,
+// ys = cs = 2^n - 1.  Real-valued, with u = U - 2^(n-1), v = V - 2^(n-1):
+//   decode  R = M ((Y - y0) / ys + 2 (1 - Kr) v / cs), B = M ((Y - y0) / ys + 2 (1 - Kb) u / cs),
+//           G = M ((Y - y0) / ys - 2 Kr (1 - Kr) v / (Kg cs) - 2 Kb (1 - Kb) u / (Kg cs)), each rounded and saturated to [0, M];
+//           Y is not clamped at the black level
+//   encode  Y = y0 + ys (Kr R + Kg G + Kb B) / M, U = 2^(n-1) + cs (B - Y') / (2 (1 - Kb) M), V likewise with R and Kr
+//           (Y' = Kr R + Kg G + Kb B), each rounded and saturated to [0, 2^n - 1]
+// Rule: every coefficient is the exact rational above times 2^shift, rounded to the nearest integer (ties away from zero).
+//   decode  (dy (Y - y0) + dvr v + half) >> shift for R, (dy (Y - y0) + dvg v + dug u + half) >> shift for G, (... + dub u ...) for B
+//   encode  y0 + ((eyr R + eyg G + eyb B + half) >> shift), 2^(n-1) + ((eur R + eug G + eub B + half) >> shift), V likewise; the
+//           offset is added after the shift (exact, the offsets being integers), so the sums stay within int32
+// Shifts: 8-bit 20 both ways (int32); 10-bit decode 22 (int32 coefficients, int64 products and sums), 16-bit -> 10-bit encode 21
+// (int32: |sum| <= 32736 * 65535 + 2^20 < 2^31).  Each result is within 0.5 + (sum of |x_i| / 2) / 2^shift <= 0.547 of an output
+// step of the real-valued map, for 8-bit and 10-bit, both ways.  (BT601, TV) is listed for completeness: the library converts that
+// pair with the cv2-exact constants above.
+struct YuvCoeffs {
+  int y0;                           // black level
+  int dy, dvr, dvg, dug, dub;       // decode
+  int eyr, eyg, eyb, eur, eug, eub, evr, evg, evb;   // encode
+};
+constexpr int kCs8Shift = 20, kCs10DecShift = 22, kCs10EncShift = 21;
+// [colorspace][range]: enum savsr_colorspace x enum savsr_color_range
+constexpr YuvCoeffs kYuvCoeffs8[3][2] = {
+    {{16, 1220945, 1673555, -852458, -410793, 2115221, 269262, 528618, 102662, -155423, -305128, 460551, 460551, -385654, -74897},
+     {0, 1048576, 1470104, -748826, -360853, 1858077, 313524, 615514, 119538, -176932, -347356, 524288, 524288, -439026, -85262}},
+    {{16, 1220945, 1879825, -558796, -223607, 2215014, 191455, 644067, 65019, -105533, -355018, 460551, 460551, -418321, -42230},
+     {0, 1048576, 1651297, -490864, -196424, 1945738, 222927, 749942, 75707, -120138, -404150, 524288, 524288, -476214, -48074}},
+    {{16, 1220945, 1760217, -682019, -196426, 2245811, 236572, 610567, 53402, -128614, -331937, 460551, 460551, -423510, -37041},
+     {0, 1048576, 1546230, -599107, -172546, 1972791, 275461, 710935, 62181, -146413, -377875, 524288, 524288, -482120, -42168}}};
+constexpr YuvCoeffs kYuvCoeffs10[3][2] = {
+    {{64, 313782777, 430103733, -219081799, -105573682, 543611851, 8382, 16455, 3196, -4838, -9498, 14336, 14336, -12005, -2331},
+     {0, 268693756, 376708646, -191883961, -92467271, 476125336, 9788, 19216, 3732, -5524, -10844, 16368, 16368, -13706, -2662}},
+    {{64, 313782777, 483115092, -143610555, -57467096, 569258550, 5960, 20049, 2024, -3285, -11051, 14336, 14336, -13022, -1315},
+     {0, 268693756, 423138927, -125782069, -50332863, 498588134, 6960, 23413, 2364, -3751, -12618, 16368, 16368, -14867, -1501}},
+    {{64, 313782777, 452375867, -175278968, -50481394, 577173441, 7364, 19006, 1662, -4004, -10333, 14336, 14336, -13183, -1153},
+     {0, 268693756, 396215813, -153519018, -44214398, 505520433, 8600, 22195, 1941, -4571, -11797, 16368, 16368, -15052, -1316}}};
 template <class F>
 inline int ensure_smem_attr(savsr_ctx* ctx, int bit, F func, size_t bytes) {
   if (ctx->attr_mask & (1u << bit)) return 0;

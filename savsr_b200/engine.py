@@ -726,18 +726,23 @@ class Plan:
         with torch.cuda.device(self.device):
             K.check(self.lib.savsr_write_frame_table(self.ctx.handle, self.frame_table.data_ptr(), arr, len(ptrs), self._stream().cuda_stream))
 
-    def forward_frames_into(self, ptrs: Sequence[int], out: torch.Tensor, graph: bool = True, out_format: Optional[str] = None) -> None:
+    def forward_frames_into(self, ptrs: Sequence[int], out: torch.Tensor, graph: bool = True, out_format: Optional[str] = None,
+                            out_colorspace: str = "bt601", out_color_range: str = "tv") -> None:
         """io="bgr_u8_frames" or "bgr48_frames": the frames at the B*7 device addresses `ptrs` (see write_frame_table) -> out BGR
         [B,H,W,3] of the mode's sample type, all on the device's current stream.  The frames are read in place by the forward: they must
         stay valid, in stream order, until it has run.  With a YUV out_format of the same depth ("yuv420p" or "nv12" for uint8,
         "yuv420p10le" or "p010" for uint16), out is [B,3H/2,W] and the colour conversion reads the output staging buffer in place of the
-        copy (colour.bgr_to_yuv420).  out_format None is the mode's packed BGR ("bgr24", "bgr48le")."""
+        copy (colour.bgr_to_yuv420, with the matrix out_colorspace and the range out_color_range).  out_format None is the mode's packed
+        BGR ("bgr24", "bgr48le"), which takes only the default colour pair: there is nothing to convert."""
         if self.io not in FRAME_MODES:
             raise ValueError(f'forward_frames_into needs a plan with io="bgr_u8_frames" or "bgr48_frames", this one has io={self.io!r}')
         bgr = "bgr48le" if self.io == "bgr48_frames" else "bgr24"
         out_format = bgr if out_format is None else colour.check_format(out_format, "out_format")
         if colour.bgr_format(out_format) != bgr:
             raise ValueError(f'out_format {out_format!r} has another depth than the frames of io="{self.io}" ({bgr})')
+        cs = (colour.check_colorspace(out_colorspace, "out_colorspace"), colour.check_color_range(out_color_range, "out_color_range"))
+        if out_format == bgr and cs != ("bt601", "tv"):
+            raise ValueError(f"out_colorspace / out_color_range {cs} need a YUV out_format: {out_format} output is not converted")
         with torch.cuda.device(self.device):
             self.write_frame_table(ptrs)
             if graph:
@@ -747,7 +752,7 @@ class Plan:
             if out_format == bgr:
                 out.copy_(self.out, non_blocking=True)
             else:
-                colour.bgr_to_yuv420(self.out, out_format, out=out)
+                colour.bgr_to_yuv420(self.out, out_format, out=out, colorspace=cs[0], color_range=cs[1])
 
     def activation_absmax(self) -> float:
         """Largest |value| currently held anywhere in the LR arena (every trunk activation of the last forward), read in the plan's

@@ -4,8 +4,9 @@
 batch partition as ``sharding.infer_clip(net.forward_bgr_u8, clip, batch=...)`` on the whole clip, so its output is byte-identical to
 that call.  Frames are uploaded once into a device ring and read in place by ``SAVSR.forward_bgr_u8_indexed``; the ring's size depends
 on the largest batch of the schedule, not on the length of the video.  Frames may come and go as packed BGR or as YUV 4:2:0
-(yuv420p, NV12: savsr_b200.colour), converted on the device on their way into the ring and out of the forward's output buffer.  Deep
-video (bgr48le, yuv420p10le, P010) streams through a ring of uint16 frames and ``SAVSR.forward_bgr48_indexed``.
+(yuv420p, NV12: savsr_b200.colour), converted on the device on their way into the ring and out of the forward's output buffer, each
+side with its own colour matrix and range (BT.601, BT.709, BT.2020; tv or pc).  Deep video (bgr48le, yuv420p10le, P010) streams through
+a ring of uint16 frames and ``SAVSR.forward_bgr48_indexed``.
 """
 from __future__ import annotations
 
@@ -44,13 +45,22 @@ class VideoUpscaler:
     output is enc(infer_clip(net.forward_bgr48, dec(frames), batch=...)) with dec of an 8-bit source widened.  An 8-bit source gets
     deep output this way, without 8-bit banding; deep input with 8-bit output is refused.
 
+    Colour: YUV input is decoded with the matrix `in_colorspace` and the range `in_color_range`, YUV output encoded with
+    `out_colorspace` and `out_color_range` (ffmpeg's -colorspace / -color_range names: "bt601", "bt709", "bt2020nc"; "tv", "pc";
+    savsr_b200.colour).  The default ("bt601", "tv") is the cv2-exact conversion above; the other pairs use the H.273 map.  An SD
+    source upscaled to HD is ``in_colorspace="bt601", out_colorspace="bt709"``, so the output carries HD's usual tag.  dec and enc of
+    the compositions above are then the conversions of these pairs (an 8-bit source for a 16-bit ring is decoded with the input pair,
+    then widened).  A packed BGR side has nothing to convert and takes only the defaults.  No transfer function is applied: BT.2020
+    frames are converted as code values.
+
     Ownership: the caller may overwrite or free what it passed to ``push`` as soon as ``push`` returns.  Host frames are staged through
     the upscaler's own pinned buffers (a staging slot is reused only after the event of its upload); CUDA frames are copied in stream
     order on the current stream.  Everything runs on the current stream of the net's device, so a ring slot is rewritten only after
     every forward enqueued before that has read it."""
 
     def __init__(self, net, lr_size: Tuple[int, int], scale, batch=1, num_frames: int = 7, in_format: str = "bgr24",
-                 out_format: str = "bgr24"):
+                 out_format: str = "bgr24", in_colorspace: str = "bt601", in_color_range: str = "tv", out_colorspace: str = "bt601",
+                 out_color_range: str = "tv"):
         if net.training:
             raise RuntimeError("VideoUpscaler is inference only: call net.eval() first")
         h, w = (int(v) for v in lr_size)
@@ -67,6 +77,13 @@ class VideoUpscaler:
         if deep_in and not deep_out:
             raise ValueError(f"deep input {in_format} with 8-bit output {out_format} is not supported: choose an output of "
                              f"{', '.join(colour.DEEP_FORMATS)}")
+        self.in_colour = (colour.check_colorspace(in_colorspace, "in_colorspace"), colour.check_color_range(in_color_range, "in_color_range"))
+        self.out_colour = (colour.check_colorspace(out_colorspace, "out_colorspace"),
+                           colour.check_color_range(out_color_range, "out_color_range"))
+        for side, fmt, pair in (("in", in_format, self.in_colour), ("out", out_format, self.out_colour)):
+            if fmt not in colour.YUV_FORMATS and pair != ("bt601", "tv"):
+                raise ValueError(f"{side}_colorspace / {side}_color_range {pair} need a YUV {side}_format: {side}_format {fmt} is packed "
+                                 f"BGR and is not converted")
         if in_format in colour.YUV_FORMATS and (h % 2 or w % 2):
             raise ValueError(f"{in_format} input needs an even LR size, got {h}x{w}")
         H, W = engine.get_hw(h, w, self.scale)
@@ -172,8 +189,8 @@ class VideoUpscaler:
             frame = self._yuv_dev if yuv else bgr
             frame.copy_(self._staging[s], non_blocking=True)
             ev.record(torch.cuda.current_stream(self.device))
-        if yuv:
-            colour.yuv420_to_bgr(frame, self.in_format, out=bgr)       # CUDA frames, pitched NV12 / P010 too, are read in place
+        if yuv:                                  # CUDA frames, pitched NV12 / P010 too, are read in place
+            colour.yuv420_to_bgr(frame, self.in_format, out=bgr, **self._colour_kw(self.in_colour, "colorspace", "color_range"))
         elif frame is not bgr:
             if self._widen and frame.is_contiguous():
                 bgr = frame                      # a CUDA frame is widened where it is
@@ -182,6 +199,11 @@ class VideoUpscaler:
         if self._widen:
             colour.widen(bgr, out=ring)
 
+    @staticmethod
+    def _colour_kw(pair: Tuple[str, str], cs_key: str, range_key: str) -> dict:
+        """Keyword arguments of a conversion with colour `pair`: none for the default pair, whose calls stay exactly as they were."""
+        return {} if pair == ("bt601", "tv") else {cs_key: pair[0], range_key: pair[1]}
+
     def _next_batch(self) -> Tuple[int, int]:
         b = self.sizes[min(self.batches, len(self.sizes) - 1)]
         return self.done, self.done + b
@@ -189,7 +211,8 @@ class VideoUpscaler:
     def _forward(self, i: int, j: int) -> Tuple[int, torch.Tensor]:
         R = self.capacity
         windows = [[f % R for f in sharding.frame_window_indices(c, self.received, self.num_frames)] for c in range(i, j)]
-        yuv_out = {} if self.out_format == colour.bgr_format(self.out_format) else {"out_format": self.out_format}
+        yuv_out = {} if self.out_format == colour.bgr_format(self.out_format) else \
+            {"out_format": self.out_format, **self._colour_kw(self.out_colour, "out_colorspace", "out_color_range")}
         hr = self.net._forward_bgr_u8_indexed(self.ring, windows, self.scale, **yuv_out)
         self.done, self.batches = j, self.batches + 1
         return i, hr
