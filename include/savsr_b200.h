@@ -606,6 +606,49 @@ int savsr_bgr48_to_yuv420_10_cs(savsr_ctx* ctx, const uint16_t* bgr, int n, int 
  * frames into a ring of 16-bit frames, for an 8-bit source upscaled to deep output.  Both buffers contiguous; n = 0 launches nothing. */
 int savsr_widen_u8_to_u16(savsr_ctx* ctx, const uint8_t* src, int n, int h, int w, uint16_t* dst, savsr_stream st);
 
+/* ---- scene cuts in a streamed video ---------------------------------------------------------------------------------------------
+ * A window that straddles a cut would mix two unrelated shots; instead each window is folded into its own shot, the reflection padding
+ * the reference applies at the ends of a clip.  For the shot [start, stop) of frame c, L = stop - start, index i = c + o (o in -3 .. 3)
+ * becomes start when L = 1, else start + r with r = (i - start) mod 2(L - 1) (non-negative), r replaced by 2(L - 1) - r when r >= L.
+ * For L >= 4 this is the single reflection of a clip's ends.
+ *
+ * The caller keeps a ring of R >= 7 contiguous BGR [h][w][3] frames (frame t in slot t % R, as for savsr_forward_u8_frames) and three
+ * small device arrays, sized by R alone: cut uint8 [R] and sad uint64 [R] (slot t % R belongs to frame t) and scratch uint64
+ * [SAVSR_SCENE_SCRATCH_WORDS], zeroed once before the first call (each call leaves it ready for the next).  One detector state per ring.
+ *
+ * savsr_scene_score_u8 / _u16: after frame t has been written into its slot, scores it against frame t - 1:
+ *   SAD_t = sum of |ring[t] - ring[t - 1]| over all 3hw samples (SAD_0 = 0),   m_t = min(SAD_t, |SAD_t - SAD_{t-1}|)
+ * (ffmpeg scdet's min(mafd, |mafd - prev_mafd|), scaled), and writes sad[t % R] = SAD_t and cut[t % R] = 1 when t >= 1 and
+ * m_t >= bound, or when `marked` (a cut the caller knows of, e.g. from an edit list), else 0.  For a threshold tau in percent, the
+ * score 100 m_t / (3hw maxval) reaches tau exactly when m_t >= bound = ceil(tau * 3hw * maxval / 100), maxval 255 or 65535, which the
+ * host computes from the exact value of tau.
+ * Because maxval is the full scale, an 8-bit source widened by 257 gets the decisions of the 8-bit frames.  A cut that ends a 1-frame
+ * shot is not detected: its SAD and the one before it cancel in |SAD_t - SAD_{t-1}|, as scdet suppresses a flash; mark such cuts.
+ * Call once per frame, t = 0, 1, 2, ... in order on one stream (frame t reads sad[(t - 1) % R] written by the call of t - 1); t = 0
+ * starts a new video.  One launch, integer arithmetic: the result does not depend on the launch configuration.
+ *
+ * savsr_write_scene_frame_table: writes the 7 * count table entries of the windows of frames first .. first + count - 1, each folded into
+ * its shot, where a shot starts at frame 0 and at every frame whose cut flag is set: entry 7n + k = ring + ((window entry k of frame
+ * first + n) % R) * frame_bytes.  `received` frames have been scored so far; `finished` = 1 once the stream has ended (the last shot
+ * ends at `received`), else every window must lie inside the received frames (first + count + 2 < received).  It reads only the flags
+ * of frames c - 2 .. c + 3 of each window, never a frame not yet received, so the host needs no read-back of the flags.
+ *
+ * Composition on one stream (what savsr_b200.VideoUpscaler does with a plan of savsr_plan_set_io_u8_table / _u16_table): per frame t,
+ * write it into slot t % R and call savsr_scene_score; when frame j + 2 has arrived (or at the end), call savsr_write_scene_frame_table
+ * with the plan's table and count = the plan's batch, then savsr_plan_run (or a graph replay of it), then read the plan's output.  The
+ * table writer replaces savsr_write_frame_table and runs, like it, in stream order outside any captured graph.
+ * Ownership: the ring, the arrays and the table must stay valid, in stream order, until the launches that read them have run; a ring slot
+ * may be rewritten only after every launch that reads it was enqueued.  Both calls return an error before any launch on a null pointer,
+ * R < 7, a non-positive bound or frame size, and (the writer) a batch that reaches past the received frames or beyond the ring.
+ */
+#define SAVSR_SCENE_SCRATCH_WORDS 1024
+int savsr_scene_score_u8(savsr_ctx* ctx, const uint8_t* ring, int R, int h, int w, long long t, int marked, long long bound, uint8_t* cut,
+                         unsigned long long* sad, unsigned long long* scratch, savsr_stream st);
+int savsr_scene_score_u16(savsr_ctx* ctx, const uint16_t* ring, int R, int h, int w, long long t, int marked, long long bound, uint8_t* cut,
+                          unsigned long long* sad, unsigned long long* scratch, savsr_stream st);
+int savsr_write_scene_frame_table(savsr_ctx* ctx, const uint8_t** table_dev, const void* ring, long long frame_bytes, int R, const uint8_t* cut,
+                                  long long first, int count, long long received, int finished, savsr_stream st);
+
 /* ---- post-processing / metrics on the device (next row 8f3) -------------------------------------------------------
  * tensor2img (lbasicsr/utils/img_util.py:38-94): sr fp32 NCHW [batch][3][H][W] RGB -> uint8 HWC BGR [batch][H][W][3]
  * (clamp, *255, round half to even), and, when gt is given, the per-frame sum of squared Y-channel differences of the two

@@ -25,6 +25,7 @@ FMT_NAMES = {"bf16": FMT_BF16, "fp16": FMT_FP16}
 OPT_BIGK_ALL, OPT_BIGK_ISSUERS, OPT_PDL = 0, 1, 2   # enum savsr_option
 WGRAD_OIHW, WGRAD_TIO = 0, 1     # enum savsr_wgrad_layout
 ROWS_LINEAR, ROWS_QUAD = 0, 1     # enum savsr_row_order: QUAD for everything savsr_conv / savsr_satu_kconv_sta consume with n_tile 64
+SCENE_SCRATCH_WORDS = 1024        # SAVSR_SCENE_SCRATCH_WORDS: uint64 scratch of one scene detector
 
 # SAVSR_LIB_PATH: alternative build of the same ABI (A/B timing of kernel variants); default = the in-tree library
 LIB_PATH = os.environ.get("SAVSR_LIB_PATH") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "lib", "libsavsr_sm100.so")
@@ -126,7 +127,7 @@ MAX_TRAIN_ENTRIES = 32
 
 
 # name -> (restype, argtypes); every symbol declared in include/savsr_b200.h
-_VP, _I, _F, _SZ = C.c_void_p, C.c_int, C.c_float, C.c_size_t
+_VP, _I, _F, _SZ, _LL = C.c_void_p, C.c_int, C.c_float, C.c_size_t, C.c_longlong
 SIGNATURES = {
     "savsr_abi_version": (_I, []),
     "savsr_last_error": (C.c_char_p, []),
@@ -200,6 +201,9 @@ SIGNATURES = {
     "savsr_yuv420_10_to_bgr48_cs": (_I, [_VP, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _I, _I, _VP, _I, _I, _VP]),
     "savsr_bgr48_to_yuv420_10_cs": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _I, _VP]),
     "savsr_widen_u8_to_u16": (_I, [_VP, _VP, _I, _I, _I, _VP, _VP]),
+    "savsr_scene_score_u8": (_I, [_VP, _VP, _I, _I, _I, _LL, _I, _LL, _VP, _VP, _VP, _VP]),
+    "savsr_scene_score_u16": (_I, [_VP, _VP, _I, _I, _I, _LL, _I, _LL, _VP, _VP, _VP, _VP]),
+    "savsr_write_scene_frame_table": (_I, [_VP, _VP, _VP, _LL, _I, _VP, _LL, _I, _LL, _I, _VP]),
     "savsr_pack_frames": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),
     "savsr_pack_frames_u8": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),
     "savsr_pack_frames_u8_table": (_I, [_VP, _VP, _VP, _I, _I, _I, _I, _VP]),

@@ -341,18 +341,40 @@ class SAVSR(nn.Module):
         return self._run_plan(self._plan(b, h, w, pool.device, io, scale), frames=ptrs, out_format=out_format,
                               out_colorspace=out_colorspace, out_color_range=out_color_range)
 
+    def _forward_ring_scenes(self, ring: torch.Tensor, cut: torch.Tensor, first: int, count: int, received: int, finished: bool, scale,
+                             out_format: Optional[str] = None, out_colorspace: str = "bt601", out_color_range: str = "tv") -> torch.Tensor:
+        """The forward of savsr_b200.VideoUpscaler with scene detection: the windows of frames first .. first + count - 1 of a stream
+        whose frame t sits in slot t % R of `ring` (uint8 or uint16 [R, h, w, 3]), each folded into its shot as the device cut flags
+        `cut` (uint8 [R], savsr_b200.scenes.Detector) mark it.  The frame table is written on the device (Plan.forward_scene_frames_into),
+        so no flag is read back.  Output, formats and colour as _forward_bgr_u8_indexed at `scale`."""
+        if self.training:
+            raise RuntimeError("_forward_ring_scenes is inference only: call eval() first")
+        if ring.dtype not in engine.FRAME_MODES.values() or ring.dim() != 4 or ring.shape[3] != 3 or not ring.is_contiguous():
+            raise ValueError(f"expected a contiguous uint8 or uint16 BGR ring [R, h, w, 3], got {ring.dtype} {tuple(ring.shape)}")
+        self._check_device(ring)
+        io = "bgr48_frames" if ring.dtype == torch.uint16 else "bgr_u8_frames"
+        out_format = ("bgr48le" if io == "bgr48_frames" else "bgr24") if out_format is None else colour.check_format(out_format, "out_format")
+        out_colorspace = colour.check_colorspace(out_colorspace, "out_colorspace")
+        out_color_range = colour.check_color_range(out_color_range, "out_color_range")
+        return self._run_plan(self._plan(int(count), ring.shape[1], ring.shape[2], ring.device, io, scale), out_format=out_format,
+                              out_colorspace=out_colorspace, out_color_range=out_color_range,
+                              scene=(ring, cut, int(first), int(received), bool(finished)))
+
     def _run_plan(self, plan: engine.Plan, x: Optional[torch.Tensor] = None, frames: Optional[list] = None,
-                  out_format: str = "bgr24", out_colorspace: str = "bt601", out_color_range: str = "tv") -> torch.Tensor:
+                  out_format: str = "bgr24", out_colorspace: str = "bt601", out_color_range: str = "tv",
+                  scene: Optional[tuple] = None) -> torch.Tensor:
         with torch.cuda.device(plan.device):
             if out_format in ("bgr24", "bgr48le"):
                 out = torch.empty_like(plan.out)
             else:
                 out = plan.out.new_empty((plan.B, *colour.yuv_shape(plan.H, plan.W)))
-            if frames is None:
+            cs = {} if (out_colorspace, out_color_range) == ("bt601", "tv") else \
+                {"out_colorspace": out_colorspace, "out_color_range": out_color_range}
+            if scene is not None:
+                plan.forward_scene_frames_into(*scene, out, graph=self.use_graph, out_format=out_format, **cs)
+            elif frames is None:
                 plan.forward_into(x, out, graph=self.use_graph)
             else:
-                cs = {} if (out_colorspace, out_color_range) == ("bt601", "tv") else \
-                    {"out_colorspace": out_colorspace, "out_color_range": out_color_range}
                 plan.forward_frames_into(frames, out, graph=self.use_graph, out_format=out_format, **cs)
             if self.precision == "fp16" and not plan.__dict__.get("_range_checked"):
                 # fp16 operands meet the <= 1e-3 bound but saturate at 65504: look at every trunk activation of this plan's FIRST forward

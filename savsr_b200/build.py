@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libsavsr_sm100.so")
-SOURCES = ["capi.cu", "conv_igemm.cu", "conv_wgrad.cu", "train_ops.cu", "train_attn.cu", "train_mask.cu", "plan.cu", "small_ops.cu", "satu.cu", "datapath.cu", "colour.cu"]
+SOURCES = ["capi.cu", "conv_igemm.cu", "conv_wgrad.cu", "train_ops.cu", "train_attn.cu", "train_mask.cu", "plan.cu", "small_ops.cu", "satu.cu", "datapath.cu", "colour.cu", "scenes.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "--expt-relaxed-constexpr"]
 

@@ -734,6 +734,37 @@ class Plan:
         "yuv420p10le" or "p010" for uint16), out is [B,3H/2,W] and the colour conversion reads the output staging buffer in place of the
         copy (colour.bgr_to_yuv420, with the matrix out_colorspace and the range out_color_range).  out_format None is the mode's packed
         BGR ("bgr24", "bgr48le"), which takes only the default colour pair: there is nothing to convert."""
+        self._forward_table_into(lambda: self.write_frame_table(ptrs), out, graph, out_format, out_colorspace, out_color_range)
+
+    def write_scene_frame_table(self, ring: torch.Tensor, cut: torch.Tensor, first: int, received: int, finished: bool) -> None:
+        """Enqueue savsr_write_scene_frame_table on the device's current stream: the table of the B windows of frames first .. first + B - 1
+        of a stream whose frame t sits in slot t % R of `ring` (contiguous [R, h, w, 3] of the mode's sample type), each window folded into
+        its shot as the device cut flags `cut` (uint8 [R], written by scenes.Detector) mark it.  `received`: frames scored so far;
+        `finished`: the stream has ended at `received`.  Nothing is read back: the host does not need to know the cuts."""
+        if self.io not in FRAME_MODES:
+            raise ValueError(f'write_scene_frame_table needs a plan with io="bgr_u8_frames" or "bgr48_frames", this one has io={self.io!r}')
+        if ring.dtype != FRAME_MODES[self.io] or ring.dim() != 4 or tuple(ring.shape[1:]) != (self.h, self.w, 3) or not ring.is_contiguous():
+            raise ValueError(f"the ring must be a contiguous {str(FRAME_MODES[self.io]).replace('torch.', '')} tensor [R, {self.h}, {self.w}, 3], "
+                             f"got {ring.dtype} {tuple(ring.shape)}")
+        if cut.dtype != torch.uint8 or tuple(cut.shape) != (ring.shape[0],):
+            raise ValueError(f"cut must be a uint8 tensor [{ring.shape[0]}], got {cut.dtype} {tuple(cut.shape)}")
+        fb = self.h * self.w * 3 * ring.element_size()
+        with torch.cuda.device(self.device):
+            K.check(self.lib.savsr_write_scene_frame_table(self.ctx.handle, self.frame_table.data_ptr(), ring.data_ptr(), fb, ring.shape[0],
+                                                            cut.data_ptr(), int(first), self.B, int(received), int(bool(finished)),
+                                                            self._stream().cuda_stream))
+
+    def forward_scene_frames_into(self, ring: torch.Tensor, cut: torch.Tensor, first: int, received: int, finished: bool, out: torch.Tensor,
+                                  graph: bool = True, out_format: Optional[str] = None, out_colorspace: str = "bt601",
+                                  out_color_range: str = "tv") -> None:
+        """forward_frames_into with the table written on the device by write_scene_frame_table instead of from host pointers: the windows
+        of frames first .. first + B - 1 of the ring, folded at the cuts the device flags mark.  The launch list, the graph and the
+        output conversion are those of forward_frames_into."""
+        self._forward_table_into(lambda: self.write_scene_frame_table(ring, cut, first, received, finished), out, graph, out_format,
+                                 out_colorspace, out_color_range)
+
+    def _forward_table_into(self, write_table: Callable[[], None], out: torch.Tensor, graph: bool, out_format: Optional[str],
+                            out_colorspace: str, out_color_range: str) -> None:
         if self.io not in FRAME_MODES:
             raise ValueError(f'forward_frames_into needs a plan with io="bgr_u8_frames" or "bgr48_frames", this one has io={self.io!r}')
         bgr = "bgr48le" if self.io == "bgr48_frames" else "bgr24"
@@ -744,7 +775,7 @@ class Plan:
         if out_format == bgr and cs != ("bt601", "tv"):
             raise ValueError(f"out_colorspace / out_color_range {cs} need a YUV out_format: {out_format} output is not converted")
         with torch.cuda.device(self.device):
-            self.write_frame_table(ptrs)
+            write_table()
             if graph:
                 self.run_graph()
             else:

@@ -7,6 +7,7 @@ path; only the optional gather of results uses ``torch.distributed`` (NCCL on GP
 """
 from __future__ import annotations
 
+import bisect
 from typing import Callable, List, Optional, Sequence
 
 import torch
@@ -30,6 +31,48 @@ def frame_window_indices(crt_idx: int, n_frames: int, num_frames: int = 7) -> Li
     return out
 
 
+def scene_window_indices(c: int, start: int, stop: int, num_frames: int = 7) -> List[int]:
+    """Window of frame `c` inside the shot [start, stop): each index c + o, |o| <= num_frames // 2, folded into the shot.  A shot of one
+    frame repeats it; otherwise the index is reflected at the shot's ends, as often as it takes (period 2 (L - 1)).  For a shot of
+    num_frames // 2 + 1 frames or more this is exactly frame_window_indices(c - start, L) + start, the reference's padding at a clip's
+    ends, applied at every cut; shorter shots, which a clip cannot be, get the repeated fold."""
+    if num_frames % 2 != 1:
+        raise ValueError("num_frames should be an odd number.")
+    L = stop - start
+    if L < 1 or not (start <= c < stop):
+        raise ValueError(f"frame {c} is not inside the shot [{start}, {stop})")
+    pad = num_frames // 2
+    if L == 1:
+        return [start] * num_frames
+    period = 2 * (L - 1)
+    out = []
+    for i in range(c - pad, c + pad + 1):
+        r = (i - start) % period
+        if r >= L:
+            r = period - r
+        out.append(start + r)
+    return out
+
+
+def check_cuts(cuts: Sequence[int], n_frames: int) -> tuple:
+    """`cuts` as a tuple of ints: sorted, distinct frame indices in [0, n_frames), each the first frame of a shot."""
+    out = tuple(int(f) for f in cuts)
+    if any(b <= a for a, b in zip(out, out[1:])) or (out and (out[0] < 0 or out[-1] >= n_frames)):
+        raise ValueError(f"cuts must be sorted, distinct frame indices in [0, {n_frames}), got {list(out)}")
+    return out
+
+
+def clip_window_indices(c: int, n_frames: int, cuts: Optional[Sequence[int]] = None, num_frames: int = 7) -> List[int]:
+    """Window of frame `c` of a clip of `n_frames` frames: frame_window_indices with `cuts` None, else the window folded into the shot of
+    `c` (scene_window_indices), where a shot starts at frame 0 and at every frame of the sorted `cuts`."""
+    if cuts is None:
+        return frame_window_indices(c, n_frames, num_frames)
+    k = bisect.bisect_right(cuts, c)
+    start = cuts[k - 1] if k > 0 else 0
+    stop = cuts[k] if k < len(cuts) else n_frames
+    return scene_window_indices(c, start, stop, num_frames)
+
+
 def shard_frames(n_frames: int, rank: int, world_size: int, contiguous: bool = False) -> List[int]:
     """Frames of a clip owned by `rank`.  Default = the reference's rank-strided loop
     (video_base_model.py:50); `contiguous` gives equal contiguous chunks instead."""
@@ -44,23 +87,28 @@ def shard_frames(n_frames: int, rank: int, world_size: int, contiguous: bool = F
 _WINDOW_INDEX_CACHE: "dict[tuple, torch.Tensor]" = {}
 
 
-def _window_index(T: int, frames: Sequence[int], num_frames: int, device: torch.device) -> torch.Tensor:
+def _window_index(T: int, frames: Sequence[int], num_frames: int, device: torch.device, cuts: Optional[tuple] = None) -> torch.Tensor:
     """Flat gather index of the windows of `frames`, resident on `device`.  Cached: building it per call costs a host-to-device copy from
-    pageable memory, which blocks the host until the stream has drained -- between two batches of a clip that is an idle GPU."""
-    key = (T, tuple(int(f) for f in frames), num_frames, device.type, device.index)
+    pageable memory, which blocks the host until the stream has drained -- between two batches of a clip that is an idle GPU.
+    `cuts` (checked, a tuple) is part of the key, so clips of one length with different cuts get their own index."""
+    key = (T, tuple(int(f) for f in frames), num_frames, device.type, device.index) + (() if cuts is None else (cuts,))
     idx = _WINDOW_INDEX_CACHE.get(key)
     if idx is None:
         if len(_WINDOW_INDEX_CACHE) >= 256:
             _WINDOW_INDEX_CACHE.clear()
-        idx = torch.tensor([frame_window_indices(f, T, num_frames) for f in key[1]], dtype=torch.long).reshape(-1).to(device)
+        if cuts is not None and T <= num_frames // 2:      # the refusal of a whole clip this short stays, with or without cuts
+            frame_window_indices(0, T, num_frames)
+        idx = torch.tensor([clip_window_indices(f, T, cuts, num_frames) for f in key[1]], dtype=torch.long).reshape(-1).to(device)
         _WINDOW_INDEX_CACHE[key] = idx
     return idx
 
 
-def gather_windows(clip: torch.Tensor, frames: Sequence[int], num_frames: int = 7) -> torch.Tensor:
+def gather_windows(clip: torch.Tensor, frames: Sequence[int], num_frames: int = 7, cuts: Optional[Sequence[int]] = None) -> torch.Tensor:
     """clip [T, ...] -> windows [len(frames), num_frames, ...] (temporal halo = duplicated input): fp32 [T, 3, h, w] planes for
-    SAVSR.forward, or uint8 [T, h, w, 3] BGR frames for SAVSR.forward_bgr_u8."""
-    idx = _window_index(clip.shape[0], frames, num_frames, clip.device)
+    SAVSR.forward, or uint8 [T, h, w, 3] BGR frames for SAVSR.forward_bgr_u8.  `cuts`: sorted frame indices that each start a new
+    shot; every window is then folded into its own shot (scene_window_indices) instead of mixing frames of two shots."""
+    c = None if cuts is None else check_cuts(cuts, clip.shape[0])
+    idx = _window_index(clip.shape[0], frames, num_frames, clip.device, c)
     return clip.index_select(0, idx).reshape(len(frames), num_frames, *clip.shape[1:])
 
 
@@ -82,12 +130,14 @@ def batch_schedule(n: int, batch) -> list:
 
 def infer_clip(net: Callable[[torch.Tensor], torch.Tensor], clip: torch.Tensor, frames: Optional[Sequence[int]] = None,
                batch=1, num_frames: int = 7, out: Optional[torch.Tensor] = None, copy_stream: Optional["torch.cuda.Stream"] = None,
-               join: bool = True) -> torch.Tensor:
+               join: bool = True, cuts: Optional[Sequence[int]] = None) -> torch.Tensor:
     """Run `net` on the windows of `frames` (default: all), `batch` windows per forward (int or a schedule, see batch_schedule).
     Returns [len(frames), ...] of whatever `net` returns per window: [n, 3, H, W] fp32 for SAVSR (clip [T, 3, h, w] fp32), or
     [n, H, W, 3] uint8 BGR for SAVSR.forward_bgr_u8 (clip [T, h, w, 3] uint8).  The last, ragged batch is run at its own size.
     If `out` (e.g. a pinned host tensor) is given, each batch is copied into it on a side stream while the next
     batch computes, and `out` is returned once all copies are enqueued behind the current stream.
+    `cuts`: sorted frame indices of the clip that each start a new shot (a scene cut); each window is folded into its own shot
+    (scene_window_indices), so no output frame is made of two shots.  None (the default) is one shot, reflected at the clip's ends.
     `copy_stream` / `join=False`: for a stream of clips -- the caller owns ONE copy stream, the compute stream does not wait for the copies
     (the next clip's forwards overlap this clip's last copy), and the caller synchronises the copy stream before reading `out`."""
     frames = list(range(clip.shape[0])) if frames is None else list(frames)
@@ -96,7 +146,7 @@ def infer_clip(net: Callable[[torch.Tensor], torch.Tensor], clip: torch.Tensor, 
     outs = []
     for i, j in batch_schedule(len(frames), batch):
         chunk = frames[i:j]
-        y = net(gather_windows(clip, chunk, num_frames))
+        y = net(gather_windows(clip, chunk, num_frames) if cuts is None else gather_windows(clip, chunk, num_frames, cuts))
         if out is None:
             outs.append(y)
         elif copy_stream is None:

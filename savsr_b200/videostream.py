@@ -6,7 +6,8 @@ that call.  Frames are uploaded once into a device ring and read in place by ``S
 on the largest batch of the schedule, not on the length of the video.  Frames may come and go as packed BGR or as YUV 4:2:0
 (yuv420p, NV12: savsr_b200.colour), converted on the device on their way into the ring and out of the forward's output buffer, each
 side with its own colour matrix and range (BT.601, BT.709, BT.2020; tv or pc).  Deep video (bgr48le, yuv420p10le, P010) streams through
-a ring of uint16 frames and ``SAVSR.forward_bgr48_indexed``.
+a ring of uint16 frames and ``SAVSR.forward_bgr48_indexed``.  Scene cuts, marked by the caller or detected on the device
+(savsr_b200.scenes), fold each window into its own shot, so that no output frame is made of two shots.
 """
 from __future__ import annotations
 
@@ -15,7 +16,7 @@ from typing import List, Optional, Tuple
 
 import torch
 
-from . import colour, engine, sharding
+from . import colour, engine, scenes, sharding
 
 
 class VideoUpscaler:
@@ -56,11 +57,22 @@ class VideoUpscaler:
     Ownership: the caller may overwrite or free what it passed to ``push`` as soon as ``push`` returns.  Host frames are staged through
     the upscaler's own pinned buffers (a staging slot is reused only after the event of its upload); CUDA frames are copied in stream
     order on the current stream.  Everything runs on the current stream of the net's device, so a ring slot is rewritten only after
-    every forward enqueued before that has read it."""
+    every forward enqueued before that has read it.
+
+    Scene cuts: ``push(frames, new_scene=True)`` marks the first of those frames as the start of a shot (from an edit list, or the
+    encoder's own detector), and with `scene_threshold` set (percent, in (0, 100]) every pushed frame is also scored on the device
+    against the one before it, after any YUV decode or widening (savsr_b200.scenes: ffmpeg scdet's rule in exact integers), and starts a
+    shot when its score reaches the threshold.  Each window is then folded into its own shot (sharding.scene_window_indices, the
+    reference's reflection at a clip's ends applied at every cut), and the output is enc(infer_clip(net..., dec(frames), batch=...,
+    cuts=up.scene_cuts())) with the same batches as without cuts.  About 10, scdet's default, is a starting point for the threshold; it
+    has not been tuned on real footage.  A cut that ends a 1-frame shot (a flash) is not detected by design: mark it.  Detected cuts are
+    resolved on the device when the frame table is written, so push and finish never wait for a score; without a threshold, marked
+    cuts are resolved on the host into the usual frame pointers, and with no cut marked the launches are exactly those of a stream
+    without cuts.  Fades and dissolves are not detected."""
 
     def __init__(self, net, lr_size: Tuple[int, int], scale, batch=1, num_frames: int = 7, in_format: str = "bgr24",
                  out_format: str = "bgr24", in_colorspace: str = "bt601", in_color_range: str = "tv", out_colorspace: str = "bt601",
-                 out_color_range: str = "tv"):
+                 out_color_range: str = "tv", scene_threshold=None):
         if net.training:
             raise RuntimeError("VideoUpscaler is inference only: call net.eval() first")
         h, w = (int(v) for v in lr_size)
@@ -90,6 +102,8 @@ class VideoUpscaler:
         if out_format in colour.YUV_FORMATS and (H % 2 or W % 2):
             raise ValueError(f"{out_format} output needs an even HR size: {h}x{w} at scale {self.scale} gives H = {H}, W = {W}; "
                              f"{colour.bgr_format(out_format)} output takes any scale")
+        if scene_threshold is not None:
+            scenes.check_threshold(scene_threshold)
         self.device = net.gamma.device
         # Until batch [i, j) has run, the ring holds frames i - pad .. j - 1 + pad, the ones its windows read, and nothing newer.
         self.capacity = max(sizes) + 2 * self.pad
@@ -99,6 +113,10 @@ class VideoUpscaler:
         self._yuv_dev: Optional[torch.Tensor] = None           # device staging of one host YUV frame, converted from there into the ring
         self._bgr8_dev: Optional[torch.Tensor] = None          # one uint8 BGR frame on its way into a 16-bit ring, widened from there
         self._uploaded: List[Optional[torch.cuda.Event]] = [None] * self.capacity
+        # scene detection: per-slot cut flags and SADs beside the ring (sized by it), and a host log of each frame's flag, copied
+        # back asynchronously for scene_cuts() in chunks of pinned memory that are reused by the next video
+        self.detector = None if scene_threshold is None else scenes.Detector(self.ring, scene_threshold)
+        self._cut_log: List[torch.Tensor] = []
         self.reset()
 
     def reset(self) -> None:
@@ -107,19 +125,27 @@ class VideoUpscaler:
         self.done = 0              # frames whose HR output has been returned (start of the next batch)
         self.batches = 0           # forwards run
         self.finished = False
+        self._marked: List[int] = []   # frames > 0 marked with push(..., new_scene=True)
 
-    def push(self, frames) -> List[Tuple[int, torch.Tensor]]:
+    def push(self, frames, new_scene: bool = False) -> List[Tuple[int, torch.Tensor]]:
         """Append frames in `in_format` (uint8, uint16 for the deep formats): BGR [h, w, 3] or [n, h, w, 3], YUV [3h/2, w] or
         [n, 3h/2, w] (torch or numpy, host or CUDA).  Returns the batches that became ready, as (index of the first frame, [m, H, W, 3],
-        or [m, 3H/2, W] in a YUV out_format, of out_format's sample type) in frame order; often none."""
+        or [m, 3H/2, W] in a YUV out_format, of out_format's sample type) in frame order; often none.  `new_scene`: the first of these
+        frames starts a new shot (the first frame of a video always does)."""
         if self.finished:
             raise RuntimeError("push() after finish(): call reset() to start the next video")
         self._check_net()
         x = self._frames(frames)
+        if new_scene and x.shape[0] == 0:
+            raise ValueError("push(new_scene=True) needs at least one frame: new_scene marks the first frame of the push")
+        if new_scene and self.received > 0:
+            self._marked.append(self.received)
         out = []
         with self._on_device():
-            for f in x:
+            for k, f in enumerate(x):
                 self._upload(f)
+                if self.detector is not None:
+                    self._score(self.received, bool(new_scene) and k == 0)
                 self.received += 1
                 while True:
                     i, j = self._next_batch()
@@ -142,7 +168,29 @@ class VideoUpscaler:
                 out.append(self._forward(i, min(j, self.received)))
         return out
 
+    def scene_cuts(self) -> List[int]:
+        """The sorted frames that started a new shot so far, marked or detected (frame 0 is not listed).  With detection on this waits
+        for the scores of the pushed frames: it synchronises with the device's current stream."""
+        if self.detector is None:
+            return list(self._marked)
+        with self._on_device():
+            if self.device.type == "cuda":
+                torch.cuda.current_stream(self.device).synchronize()
+        n = self.received
+        flags = torch.cat(self._cut_log)[:n] if n else torch.zeros(0, dtype=torch.uint8)
+        return [int(f) for f in torch.nonzero(flags[1:]).flatten().add(1)]
+
     # ------------------------------------------------------------------ internals
+    _LOG_CHUNK = 4096
+
+    def _score(self, t: int, marked: bool) -> None:
+        """Score frame t on the device (after its upload, in stream order) and queue the copy of its flag into the host log."""
+        self.detector.score(t, marked)
+        k, r = divmod(t, self._LOG_CHUNK)
+        if k == len(self._cut_log):
+            self._cut_log.append(torch.zeros(self._LOG_CHUNK, dtype=torch.uint8, pin_memory=self.device.type == "cuda"))
+        self._cut_log[k][r:r + 1].copy_(self.detector.cut[t % self.capacity:t % self.capacity + 1], non_blocking=True)
+
     def _check_net(self) -> None:
         if self.net.training:
             raise RuntimeError("VideoUpscaler is inference only: the net was put in train mode")
@@ -210,9 +258,15 @@ class VideoUpscaler:
 
     def _forward(self, i: int, j: int) -> Tuple[int, torch.Tensor]:
         R = self.capacity
-        windows = [[f % R for f in sharding.frame_window_indices(c, self.received, self.num_frames)] for c in range(i, j)]
         yuv_out = {} if self.out_format == colour.bgr_format(self.out_format) else \
             {"out_format": self.out_format, **self._colour_kw(self.out_colour, "out_colorspace", "out_color_range")}
-        hr = self.net._forward_bgr_u8_indexed(self.ring, windows, self.scale, **yuv_out)
+        if self.detector is not None:          # the cuts are on the device: the table is written there
+            hr = self.net._forward_ring_scenes(self.ring, self.detector.cut, i, j - i, self.received, self.finished, self.scale, **yuv_out)
+        else:
+            # marked cuts only: folded on the host into the pointers (before the end, the windows lie inside the received frames, so
+            # `received` stands in for the end of the last shot)
+            cuts = self._marked if self._marked else None
+            windows = [[f % R for f in sharding.clip_window_indices(c, self.received, cuts, self.num_frames)] for c in range(i, j)]
+            hr = self.net._forward_bgr_u8_indexed(self.ring, windows, self.scale, **yuv_out)
         self.done, self.batches = j, self.batches + 1
         return i, hr
