@@ -602,6 +602,37 @@ int savsr_yuv420_10_to_bgr48_cs(savsr_ctx* ctx, const uint16_t* y, int y_pitch, 
 int savsr_bgr48_to_yuv420_10_cs(savsr_ctx* ctx, const uint16_t* bgr, int n, int h, int w, uint16_t* y, int y_pitch, uint16_t* u,
                                 uint16_t* v, int c_pitch, int c_step, int64_t frame_stride, int msb, int colorspace, int range,
                                 savsr_stream st);
+/* ---- YUV 4:2:2 video in and out (mezzanine formats, capture devices) -----------------------------------------------------------
+ * 4:2:2 halves the chroma horizontally only: frame row r has chroma row r, and each horizontal pixel pair shares one (U, V).  The
+ * frame width must be even; any height is accepted.  Decoding gives both pixels of a pair its chroma (nearest neighbour: byte for byte
+ * cv::cvtColor COLOR_YUV2BGR_YUYV / _UYVY at (BT601, TV)).  Encoding computes Y exactly as the 4:2:0 calls do and takes U and V from
+ * the LEFT pixel of each pair: the co-sited chroma position of H.264, HEVC and ProRes 4:2:2 and the 4:2:0 calls' top-left rule, so a
+ * 4:2:0 encode equals the 4:2:2 encode with its odd chroma rows dropped.  This is not COLOR_BGR2YUV_YUYV, which averages the pair's
+ * chroma and rounds Y differently.  Every (colorspace, range) converts with the pixel map of the 4:2:0 calls: OpenCV's constants at
+ * (BT601, TV), the H.273 map otherwise.  The planes are described as for 4:2:0, with chroma row r for frame row r, plus
+ *   y_step            the distance between the Y samples of a row: 1 for the planar and semi-planar layouts, 2 for the packed ones;
+ * and the layouts are
+ *   yuv422p           y_step 1, c_step 1: Y plane, then U and V planes of h rows of w / 2 bytes (c_pitch >= w / 2); ffmpeg's [2h][w]
+ *                     frame at p: y = p, y_pitch = w, u = p + h w, v = u + h w / 2, c_pitch = w / 2;
+ *   nv16              y_step 1, c_step 2: Y plane, then h rows of interleaved U, V bytes, U first (v = u + 1, c_pitch >= w);
+ *   yuyv422           y_step 2, c_step 4: rows of Y0 U0 Y1 V0 ...: u = y + 1, v = y + 3, c_pitch = y_pitch >= 2w;
+ *   uyvy422           y_step 2, c_step 4: rows of U0 Y0 V0 Y1 ...: u = y - 1, v = y + 1, c_pitch = y_pitch >= 2w.
+ * The 10-bit calls take yuv422p10le (c_step 1, msb 0) and p210 (c_step 2, msb 1: the value in bits 6-15, read as s >> 6, which also
+ * reads 10-bit content in a P216 surface) with every pitch and the frame stride in uint16 elements, and bgr48 on the BGR side.
+ * Refused before any launch, with a savsr_last_error() naming the value: an odd width, a (y_step, c_step) other than the layouts
+ * above, a pitch below the row, a packed layout whose u and v are not those above, v != u + 1 for c_step 2, a null pointer, a negative
+ * frame_stride, an msb other than 0 or 1, an unknown colorspace or range.  n = 0 launches nothing.  Ownership as for 4:2:0.
+ */
+int savsr_yuv422_to_bgr_cs(savsr_ctx* ctx, const uint8_t* y, int y_pitch, int y_step, const uint8_t* u, const uint8_t* v, int c_pitch,
+                           int c_step, int64_t frame_stride, int n, int h, int w, uint8_t* bgr, int colorspace, int range, savsr_stream st);
+int savsr_bgr_to_yuv422_cs(savsr_ctx* ctx, const uint8_t* bgr, int n, int h, int w, uint8_t* y, int y_pitch, int y_step, uint8_t* u,
+                           uint8_t* v, int c_pitch, int c_step, int64_t frame_stride, int colorspace, int range, savsr_stream st);
+int savsr_yuv422_10_to_bgr48_cs(savsr_ctx* ctx, const uint16_t* y, int y_pitch, int y_step, const uint16_t* u, const uint16_t* v,
+                                int c_pitch, int c_step, int64_t frame_stride, int msb, int n, int h, int w, uint16_t* bgr, int colorspace,
+                                int range, savsr_stream st);
+int savsr_bgr48_to_yuv422_10_cs(savsr_ctx* ctx, const uint16_t* bgr, int n, int h, int w, uint16_t* y, int y_pitch, int y_step,
+                                uint16_t* u, uint16_t* v, int c_pitch, int c_step, int64_t frame_stride, int msb, int colorspace, int range,
+                                savsr_stream st);
 /* uint8 BGR [n][h][w][3] -> uint16 BGR (each value times 257, so v / 65535 of the result is u / 255 of the source): brings 8-bit
  * frames into a ring of 16-bit frames, for an 8-bit source upscaled to deep output.  Both buffers contiguous; n = 0 launches nothing. */
 int savsr_widen_u8_to_u16(savsr_ctx* ctx, const uint8_t* src, int n, int h, int w, uint16_t* dst, savsr_stream st);

@@ -200,6 +200,10 @@ SIGNATURES = {
     "savsr_bgr_to_yuv420_cs": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _VP]),
     "savsr_yuv420_10_to_bgr48_cs": (_I, [_VP, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _I, _I, _VP, _I, _I, _VP]),
     "savsr_bgr48_to_yuv420_10_cs": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _I, _VP]),
+    "savsr_yuv422_to_bgr_cs": (_I, [_VP, _VP, _I, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _I, _VP, _I, _I, _VP]),
+    "savsr_bgr_to_yuv422_cs": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _VP]),
+    "savsr_yuv422_10_to_bgr48_cs": (_I, [_VP, _VP, _I, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _I, _I, _VP, _I, _I, _VP]),
+    "savsr_bgr48_to_yuv422_10_cs": (_I, [_VP, _VP, _I, _I, _I, _VP, _I, _I, _VP, _VP, _I, _I, C.c_int64, _I, _I, _I, _VP]),
     "savsr_widen_u8_to_u16": (_I, [_VP, _VP, _I, _I, _I, _VP, _VP]),
     "savsr_scene_score_u8": (_I, [_VP, _VP, _I, _I, _I, _LL, _I, _LL, _VP, _VP, _VP, _VP]),
     "savsr_scene_score_u16": (_I, [_VP, _VP, _I, _I, _I, _LL, _I, _LL, _VP, _VP, _VP, _VP]),

@@ -296,8 +296,8 @@ class SAVSR(nn.Module):
                                 out_color_range: str = "tv") -> torch.Tensor:
         """forward_bgr_u8_indexed (uint8 pool) or forward_bgr48_indexed (uint16 pool) at `scale`, leaving self.scale as it is
         (savsr_b200.VideoUpscaler keeps its own scale).  The I/O mode follows the pool's dtype; `dtype`, when given, is the one the
-        public caller takes.  With a YUV out_format of the pool's depth ("yuv420p" / "nv12" for uint8, "yuv420p10le" / "p010" for uint16)
-        the HR frames come back as [b, 3H/2, W] YUV 4:2:0 (savsr_b200.colour), converted from the plan's output staging buffer instead
+        public caller takes.  With a YUV out_format of the pool's depth (4:2:0 or 4:2:2, savsr_b200.colour) the HR frames come back as
+        [b, *colour.yuv_shape(H, W, out_format)], converted from the plan's output staging buffer instead
         of copied, with the matrix out_colorspace and the range out_color_range; None is packed BGR."""
         name = {torch.uint16: "forward_bgr48_indexed"}.get(dtype if dtype is not None else pool.dtype, "forward_bgr_u8_indexed")
         if self.training:
@@ -332,7 +332,7 @@ class SAVSR(nn.Module):
                              f"{out_format} output is not converted")
         if b == 0:
             H, W = engine.get_hw(h, w, scale)
-            return pool.new_empty((0, H, W, 3) if out_format == bgr else (0, *colour.yuv_shape(H, W)))
+            return pool.new_empty((0, H, W, 3) if out_format == bgr else (0, *colour.yuv_shape(H, W, out_format)))
         idx = idx.to(torch.int64)
         lo, hi = int(idx.min()), int(idx.max())
         if lo < 0 or hi >= n:
@@ -367,7 +367,7 @@ class SAVSR(nn.Module):
             if out_format in ("bgr24", "bgr48le"):
                 out = torch.empty_like(plan.out)
             else:
-                out = plan.out.new_empty((plan.B, *colour.yuv_shape(plan.H, plan.W)))
+                out = plan.out.new_empty((plan.B, *colour.yuv_shape(plan.H, plan.W, out_format)))
             cs = {} if (out_colorspace, out_color_range) == ("bt601", "tv") else \
                 {"out_colorspace": out_colorspace, "out_color_range": out_color_range}
             if scene is not None:

@@ -31,8 +31,25 @@ at 16 (64 in 10 bits) and spans of 219 and 224 steps, pc uses every code value. 
 Y at the black level; encoding saturates to [0, 2^n - 1].  Only code values are converted: no transfer function (PQ / HLG, tone
 mapping) is applied, and BT.2020 is the non-constant-luminance matrix.  The default pair keeps OpenCV's constants exactly.
 
+YUV 4:2:2 (mezzanine and mastering formats such as ProRes 422, broadcast SDI, capture cards) halves the chroma horizontally only.  Its
+width must be even; any height works:
+
+* ``"yuv422p"``: one uint8 [2h, w] array per frame: the Y plane, then the U plane (h x w/2), then the V plane, packed, contiguous rows;
+* ``"nv16"``: one uint8 [2h, w] array per frame: the Y plane, then h rows of interleaved U, V bytes (U first); may have a row pitch;
+* ``"yuyv422"`` / ``"uyvy422"``: one uint8 [h, 2w] array per frame, rows of Y0 U0 Y1 V0 ... / U0 Y0 V0 Y1 ...; may have a row pitch;
+* ``"yuv422p10le"``: uint16 [2h, w] laid out as yuv422p, the value in bits 0-9;
+* ``"p210"``: uint16 [2h, w] laid out as nv16, the value in bits 6-15 (read as v >> 6); may have a row pitch.
+
+Decoding gives both pixels of each horizontal pair the pair's (U, V): the 4:2:0 decode's rule, byte for byte
+``COLOR_YUV2BGR_YUYV`` / ``_UYVY`` at the default pair.  Encoding computes Y as the 4:2:0 encode does and takes U and V from the left
+pixel of each pair, the co-sited chroma position of H.264, HEVC and ProRes 4:2:2, so a 4:2:0 encode is the 4:2:2 encode with its odd
+chroma rows dropped.  That is deliberately not cv2's ``COLOR_BGR2YUV_YUYV``, which averages the pair's chroma and rounds Y otherwise.
+Every colour pair uses the same per-pixel map as for 4:2:0.
+
 Each call is one launch on the current stream of the tensors' device (savsr_yuv420_to_bgr / savsr_bgr_to_yuv420,
-savsr_yuv420_10_to_bgr48 / savsr_bgr48_to_yuv420_10 of libsavsr_sm100, and their _cs forms for the other pairs); there is no CPU path.
+savsr_yuv420_10_to_bgr48 / savsr_bgr48_to_yuv420_10 of libsavsr_sm100, and their _cs forms for the other pairs; the four
+savsr_yuv422_* / savsr_bgr*_to_yuv422* _cs calls for 4:2:2); there is no CPU path.  yuv_to_bgr and bgr_to_yuv pick the conversion of
+a format's subsampling.
 """
 from __future__ import annotations
 
@@ -42,10 +59,13 @@ import torch
 
 from . import _capi as K, engine
 
-FORMATS = ("bgr24", "yuv420p", "nv12", "bgr48le", "yuv420p10le", "p010")
-YUV_FORMATS = ("yuv420p", "nv12", "yuv420p10le", "p010")
-DEEP_FORMATS = ("bgr48le", "yuv420p10le", "p010")
-PITCHED_FORMATS = ("nv12", "p010")          # may have a row pitch; their U, V samples are interleaved
+FORMATS = ("bgr24", "yuv420p", "nv12", "bgr48le", "yuv420p10le", "p010", "yuv422p", "nv16", "yuyv422", "uyvy422", "yuv422p10le", "p210")
+YUV420_FORMATS = ("yuv420p", "nv12", "yuv420p10le", "p010")
+YUV422_FORMATS = ("yuv422p", "nv16", "yuyv422", "uyvy422", "yuv422p10le", "p210")
+YUV_FORMATS = YUV420_FORMATS + YUV422_FORMATS
+DEEP_FORMATS = ("bgr48le", "yuv420p10le", "p010", "yuv422p10le", "p210")
+PITCHED_FORMATS = ("nv12", "p010", "nv16", "p210", "yuyv422", "uyvy422")   # may have a row pitch; their U, V samples are interleaved
+PACKED_FORMATS = ("yuyv422", "uyvy422")     # [h, 2w]: Y, U and V in one plane of 4-byte macropixels
 COLORSPACES = {"bt601": 0, "bt709": 1, "bt2020nc": 2}      # enum savsr_colorspace
 COLOR_RANGES = {"tv": 0, "pc": 1}                          # enum savsr_color_range
 _COLORSPACE_ALIASES = {"bt470bg": "bt601", "smpte170m": "bt601", "bt2020": "bt2020nc"}
@@ -86,57 +106,93 @@ def check_color_range(name: str, what: str = "color_range") -> str:
     return r
 
 
-def _cs_args(colorspace: str, color_range: str) -> tuple:
-    """() for the default pair ("bt601", "tv"), which the plain entry points convert; else the enumerator values for the _cs ones."""
-    cs, r = check_colorspace(colorspace), check_color_range(color_range)
-    return () if (cs, r) == ("bt601", "tv") else (COLORSPACES[cs], COLOR_RANGES[r])
+def _cs_values(colorspace: str, color_range: str) -> tuple:
+    """The enumerator values (enum savsr_colorspace, enum savsr_color_range) of a colour pair."""
+    return COLORSPACES[check_colorspace(colorspace)], COLOR_RANGES[check_color_range(color_range)]
 
 
-def yuv_shape(h: int, w: int) -> Tuple[int, int]:
-    """The [rows, w] array one YUV 4:2:0 frame of h x w occupies."""
+def yuv_shape(h: int, w: int, fmt: str = "yuv420p") -> Tuple[int, int]:
+    """The [rows, cols] array one `fmt` frame of h x w occupies: [3h/2, w] for 4:2:0, [2h, w] for planar and semi-planar 4:2:2,
+    [h, 2w] for packed 4:2:2."""
+    if fmt in PACKED_FORMATS:
+        return h, 2 * w
+    if fmt in YUV422_FORMATS:
+        return 2 * h, w
     return 3 * h // 2, w
 
 
+def frame_size(x: torch.Tensor, fmt: str) -> Tuple[int, int]:
+    """(h, w) of the `fmt` frames x [n, rows, cols] (checked by yuv_frames)."""
+    rows, cols = x.shape[-2], x.shape[-1]
+    if fmt in PACKED_FORMATS:
+        return rows, cols // 2
+    return (rows // 2 if fmt in YUV422_FORMATS else 2 * rows // 3), cols
+
+
 def yuv_frames(x: torch.Tensor, fmt: str, h: Optional[int] = None, w: Optional[int] = None) -> torch.Tensor:
-    """Check that x holds `fmt` frames (uint8, uint16 for the 10-bit formats; [3h/2, w] or [n, 3h/2, w]; h x w from the shape when not
-    given) with a layout the kernels read, and return it as [n, 3h/2, w].  Wherever x lives: the device is the caller's concern."""
+    """Check that x holds `fmt` frames (uint8, uint16 for the 10-bit formats; one [rows, cols] array per frame as yuv_shape gives it,
+    [n, rows, cols] for several; h x w from the shape when not given) with a layout the kernels read, and return it as [n, rows, cols].
+    4:2:0 needs an even frame size, 4:2:2 an even width.  Wherever x lives: the device is the caller's concern."""
     if fmt not in YUV_FORMATS:
-        raise ValueError(f"{fmt!r} is not a YUV 4:2:0 format ({', '.join(YUV_FORMATS)})")
+        raise ValueError(f"{fmt!r} is not a YUV format ({', '.join(YUV_FORMATS)})")
     dt = dtype_of(fmt)
     tn = str(dt).replace("torch.", "")
     if x.dtype != dt:
         raise TypeError(f"{fmt} frames are {tn}, got {x.dtype}")
+    four22 = fmt in YUV422_FORMATS
     if h is None:
-        rows, w = (x.shape[-2], x.shape[-1]) if x.dim() in (2, 3) else (0, 0)
-        if rows % 3 or rows == 0:
-            raise ValueError(f"expected {tn} {fmt} frames [3h/2, w] or [n, 3h/2, w], got {tuple(x.shape)}")
-        h = 2 * rows // 3
-    if h % 2 or w % 2:
+        rows, cols = (x.shape[-2], x.shape[-1]) if x.dim() in (2, 3) else (0, 0)
+        if fmt in PACKED_FORMATS:
+            bad, form = cols % 2 or cols == 0 or rows == 0, "[h, 2w] or [n, h, 2w]"
+        elif four22:
+            bad, form = rows % 2 or rows == 0, "[2h, w] or [n, 2h, w]"
+        else:
+            bad, form = rows % 3 or rows == 0, "[3h/2, w] or [n, 3h/2, w]"
+        if bad:
+            raise ValueError(f"expected {tn} {fmt} frames {form}, got {tuple(x.shape)}")
+        h, w = frame_size(x, fmt)
+    if four22 and w % 2:
+        raise ValueError(f"{fmt} needs an even width, got {h}x{w}")
+    if not four22 and (h % 2 or w % 2):
         raise ValueError(f"{fmt} needs an even frame size, got {h}x{w}")
     if x.dim() == 2:
         x = x.unsqueeze(0)
-    if x.dim() != 3 or tuple(x.shape[1:]) != yuv_shape(h, w):
-        rows = yuv_shape(h, w)[0]
-        raise ValueError(f"expected {tn} {fmt} frames [{rows}, {w}] or [n, {rows}, {w}], got {tuple(x.shape)}")
+    rows, cols = yuv_shape(h, w, fmt)
+    if x.dim() != 3 or tuple(x.shape[1:]) != (rows, cols):
+        raise ValueError(f"expected {tn} {fmt} frames [{rows}, {cols}] or [n, {rows}, {cols}], got {tuple(x.shape)}")
     if x.stride(2) != 1:
         raise ValueError(f"{fmt} frames need a unit column stride, got {x.stride(2)}")
-    if fmt not in PITCHED_FORMATS and x.stride(1) != w:
+    if fmt not in PITCHED_FORMATS and x.stride(1) != cols:
         raise ValueError(f"{fmt} frames must have contiguous rows: row stride {x.stride(1)} != width {w} "
-                         f"(only {' and '.join(PITCHED_FORMATS)} take a row pitch)")
-    if x.stride(1) < w:
-        raise ValueError(f"{fmt} row stride {x.stride(1)} is below the width {w}")
+                         f"(only {', '.join(PITCHED_FORMATS)} take a row pitch)")
+    if x.stride(1) < cols:
+        raise ValueError(f"{fmt} row stride {x.stride(1)} is below the " + (f"width {w}" if cols == w else f"row of {cols} samples"))
     return x
 
 
 def _planes(x: torch.Tensor, fmt: str, h: int, w: int) -> tuple:
-    """(y, y_pitch, u, v, c_pitch, c_step, frame_stride) of frames x [n, 3h/2, w] (checked by yuv_frames): addresses in bytes, pitches
-    and the frame stride in elements (bytes for the 8-bit formats, uint16 samples for the 10-bit ones)."""
+    """(y, y_pitch, u, v, c_pitch, c_step, frame_stride) of 4:2:0 frames x [n, 3h/2, w] (checked by yuv_frames): addresses in bytes,
+    pitches and the frame stride in elements (bytes for the 8-bit formats, uint16 samples for the 10-bit ones)."""
     p, pitch, e = x.data_ptr(), x.stride(1), x.element_size()
     if fmt not in PITCHED_FORMATS:
         u = p + h * w * e
         return p, w, u, u + (h // 2) * (w // 2) * e, w // 2, 1, x.stride(0)
     u = p + h * pitch * e
     return p, pitch, u, u + e, pitch, 2, x.stride(0)
+
+
+def _planes422(x: torch.Tensor, fmt: str, h: int, w: int) -> tuple:
+    """(y, y_pitch, y_step, u, v, c_pitch, c_step, frame_stride) of 4:2:2 frames x (checked by yuv_frames), units as _planes."""
+    p, pitch, e = x.data_ptr(), x.stride(1), x.element_size()
+    if fmt == "yuyv422":
+        return p, pitch, 2, p + 1, p + 3, pitch, 4, x.stride(0)
+    if fmt == "uyvy422":
+        return p + 1, pitch, 2, p, p + 2, pitch, 4, x.stride(0)
+    if fmt in PITCHED_FORMATS:                 # nv16, p210
+        u = p + h * pitch * e
+        return p, pitch, 1, u, u + e, pitch, 2, x.stride(0)
+    u = p + h * w * e
+    return p, w, 1, u, u + h * (w // 2) * e, w // 2, 1, x.stride(0)
 
 
 def _on_cuda(*xs: torch.Tensor) -> torch.device:
@@ -169,9 +225,55 @@ def yuv420_to_bgr(frames: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = 
     to uint16 bgr48 with the same matrix.  Another `colorspace` / `color_range` than ("bt601", "tv") decodes with that pair's H.273
     map.  Writes `out` (contiguous, that shape and dtype) when given, else a fresh tensor.  One launch on the current stream; the
     frames must stay valid, in stream order, until it has run."""
-    cs = _cs_args(colorspace, color_range)
+    return _decode(frames, fmt, out, colorspace, color_range, YUV420_FORMATS)
+
+
+def yuv422_to_bgr(frames: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None, colorspace: str = "bt601",
+                  color_range: str = "tv") -> torch.Tensor:
+    """yuv420_to_bgr for the 4:2:2 formats: both pixels of each horizontal pair take the pair's (U, V).  For "yuyv422" / "uyvy422" at the
+    default pair this is cv2.cvtColor(frame, COLOR_YUV2BGR_YUYV / _UYVY) of each frame."""
+    return _decode(frames, fmt, out, colorspace, color_range, YUV422_FORMATS)
+
+
+def bgr_to_yuv420(bgr: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None, colorspace: str = "bt601",
+                  color_range: str = "tv") -> torch.Tensor:
+    """BGR [H, W, 3] or [n, H, W, 3] (contiguous, CUDA, H and W even) -> `fmt` frames [3H/2, W] or [n, 3H/2, W].  uint8 BGR to "yuv420p"
+    or "nv12" as cv2.cvtColor(frame, COLOR_BGR2YUV_I420) of each frame, with U and V interleaved for "nv12"; uint16 bgr48 to
+    "yuv420p10le" or "p010" with the same matrix.  Another `colorspace` / `color_range` than ("bt601", "tv") encodes with that pair's
+    H.273 map.  Writes `out` when given (any layout yuv_frames accepts, e.g. a pitched NV12 or P010 surface), else a fresh contiguous
+    tensor.  One launch on the current stream."""
+    return _encode(bgr, fmt, out, colorspace, color_range, YUV420_FORMATS)
+
+
+def bgr_to_yuv422(bgr: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None, colorspace: str = "bt601",
+                  color_range: str = "tv") -> torch.Tensor:
+    """bgr_to_yuv420 for the 4:2:2 formats (W even, any H): Y as the 4:2:0 encode computes it, U and V from the left pixel of each
+    horizontal pair (co-sited, as H.264, HEVC and ProRes 4:2:2 site them), so the 4:2:0 encode is this one with its odd chroma rows
+    dropped.  Not cv2's COLOR_BGR2YUV_YUYV, which averages the pair's chroma and rounds Y otherwise."""
+    return _encode(bgr, fmt, out, colorspace, color_range, YUV422_FORMATS)
+
+
+def yuv_to_bgr(frames: torch.Tensor, fmt: str, **kw) -> torch.Tensor:
+    """yuv420_to_bgr or yuv422_to_bgr, as `fmt` subsamples; the keyword arguments are passed on as given."""
+    return (yuv422_to_bgr if fmt in YUV422_FORMATS else yuv420_to_bgr)(frames, fmt, **kw)
+
+
+def bgr_to_yuv(bgr: torch.Tensor, fmt: str, **kw) -> torch.Tensor:
+    """bgr_to_yuv420 or bgr_to_yuv422, as `fmt` subsamples; the keyword arguments are passed on as given."""
+    return (bgr_to_yuv422 if fmt in YUV422_FORMATS else bgr_to_yuv420)(bgr, fmt, **kw)
+
+
+def _family(fmt: str, family: tuple) -> None:
+    if fmt not in family:
+        raise ValueError(f"{fmt!r} is not a YUV {'4:2:2' if family is YUV422_FORMATS else '4:2:0'} format ({', '.join(family)})")
+
+
+def _decode(frames, fmt, out, colorspace, color_range, family) -> torch.Tensor:
+    pair = _cs_values(colorspace, color_range)
+    cs = () if pair == (0, 0) else pair         # the plain 4:2:0 entry points convert the default pair
+    _family(fmt, family)
     x = yuv_frames(frames, fmt)
-    n, h, w = x.shape[0], 2 * x.shape[1] // 3, x.shape[2]
+    n, (h, w) = x.shape[0], frame_size(x, fmt)
     shape = (n, h, w, 3) if frames.dim() == 3 else (h, w, 3)
     dt = dtype_of(fmt)
     if out is None:
@@ -183,9 +285,16 @@ def yuv420_to_bgr(frames: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = 
     if n == 0:
         return out
     ctx = engine.context(dev.index)
-    y, yp, u, v, cp, c_step, fs = _planes(x, fmt, h, w)
     st = torch.cuda.current_stream(dev).cuda_stream
     with torch.cuda.device(dev):
+        if family is YUV422_FORMATS:            # one _cs entry point per depth; the default pair is (0, 0)
+            planes = _planes422(x, fmt, h, w)
+            if fmt in DEEP_FORMATS:
+                K.check(ctx.lib.savsr_yuv422_10_to_bgr48_cs(ctx.handle, *planes, int(fmt == "p210"), n, h, w, out.data_ptr(), *pair, st))
+            else:
+                K.check(ctx.lib.savsr_yuv422_to_bgr_cs(ctx.handle, *planes, n, h, w, out.data_ptr(), *pair, st))
+            return out
+        y, yp, u, v, cp, c_step, fs = _planes(x, fmt, h, w)
         if fmt in DEEP_FORMATS:
             args = (ctx.handle, y, yp, u, v, cp, c_step, fs, int(fmt == "p010"), n, h, w, out.data_ptr(), *cs, st)
             K.check((ctx.lib.savsr_yuv420_10_to_bgr48_cs if cs else ctx.lib.savsr_yuv420_10_to_bgr48)(*args))
@@ -195,21 +304,18 @@ def yuv420_to_bgr(frames: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = 
     return out
 
 
-def bgr_to_yuv420(bgr: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = None, colorspace: str = "bt601",
-                  color_range: str = "tv") -> torch.Tensor:
-    """BGR [H, W, 3] or [n, H, W, 3] (contiguous, CUDA, H and W even) -> `fmt` frames [3H/2, W] or [n, 3H/2, W].  uint8 BGR to "yuv420p"
-    or "nv12" as cv2.cvtColor(frame, COLOR_BGR2YUV_I420) of each frame, with U and V interleaved for "nv12"; uint16 bgr48 to
-    "yuv420p10le" or "p010" with the same matrix.  Another `colorspace` / `color_range` than ("bt601", "tv") encodes with that pair's
-    H.273 map.  Writes `out` when given (any layout yuv_frames accepts, e.g. a pitched NV12 or P010 surface), else a fresh contiguous
-    tensor.  One launch on the current stream."""
-    cs = _cs_args(colorspace, color_range)
-    if fmt not in YUV_FORMATS:
-        raise ValueError(f"{fmt!r} is not a YUV 4:2:0 format ({', '.join(YUV_FORMATS)})")
+def _encode(bgr, fmt, out, colorspace, color_range, family) -> torch.Tensor:
+    pair = _cs_values(colorspace, color_range)
+    cs = () if pair == (0, 0) else pair         # the plain 4:2:0 entry points convert the default pair
+    _family(fmt, family)
+    four22 = family is YUV422_FORMATS
     dt = dtype_of(fmt)
-    x = _bgr(bgr, f"bgr_to_yuv420 to {fmt}", dt)
+    x = _bgr(bgr, f"bgr_to_yuv{'422' if four22 else '420'} to {fmt}", dt)
     n, H, W = x.shape[:3]
-    shape = (n, *yuv_shape(H, W)) if bgr.dim() == 4 else yuv_shape(H, W)
-    if H % 2 or W % 2:
+    shape = (n, *yuv_shape(H, W, fmt)) if bgr.dim() == 4 else yuv_shape(H, W, fmt)
+    if four22 and W % 2:
+        raise ValueError(f"{fmt} needs an even width, got {H}x{W}")
+    if not four22 and (H % 2 or W % 2):
         raise ValueError(f"{fmt} needs an even frame size, got {H}x{W}")
     if out is None:
         _on_cuda(x)
@@ -223,9 +329,16 @@ def bgr_to_yuv420(bgr: torch.Tensor, fmt: str, out: Optional[torch.Tensor] = Non
     if n == 0:
         return out
     ctx = engine.context(dev.index)
-    y, yp, u, v, cp, c_step, fs = _planes(o, fmt, H, W)
     st = torch.cuda.current_stream(dev).cuda_stream
     with torch.cuda.device(dev):
+        if four22:
+            planes = _planes422(o, fmt, H, W)
+            if fmt in DEEP_FORMATS:
+                K.check(ctx.lib.savsr_bgr48_to_yuv422_10_cs(ctx.handle, x.data_ptr(), n, H, W, *planes, int(fmt == "p210"), *pair, st))
+            else:
+                K.check(ctx.lib.savsr_bgr_to_yuv422_cs(ctx.handle, x.data_ptr(), n, H, W, *planes, *pair, st))
+            return out
+        y, yp, u, v, cp, c_step, fs = _planes(o, fmt, H, W)
         if fmt in DEEP_FORMATS:
             args = (ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, c_step, fs, int(fmt == "p010"), *cs, st)
             K.check((ctx.lib.savsr_bgr48_to_yuv420_10_cs if cs else ctx.lib.savsr_bgr48_to_yuv420_10)(*args))

@@ -531,6 +531,274 @@ __global__ void __launch_bounds__(256) widen_u8_to_u16_kernel(const uint8_t* __r
   for (long long i = groups * 16 + first; i < count; i += stride) dst[i] = static_cast<uint16_t>(src[i] * 257);
 }
 
+// ------------------------------------------------------------------------------------------------ YUV 4:2:2 <-> BGR
+// 4:2:2 halves the chroma horizontally only: frame row r has chroma row r, and each horizontal pixel pair shares one (U, V).  Decoding
+// gives both pixels of a pair its chroma (cv2's COLOR_YUV2BGR_YUYV / _UYVY); encoding takes U and V from the pair's left pixel, the
+// co-sited position of H.264, HEVC and ProRes 4:2:2 and the 4:2:0 encode's point-sampling rule, so a 4:2:0 encode is the 4:2:2 encode
+// with its odd chroma rows dropped.  (cv2's COLOR_BGR2YUV_YUYV averages the pair's chroma and rounds Y otherwise: it is not this.)
+// The pixel maps are those of 4:2:0.  A thread owns kYuvGroup pixels of one row (four pairs), so odd heights need nothing special;
+// every sample is read or written once, with the widest accesses the row's alignment allows, and a row's last w % 8 pixels take the
+// sample-wise path.
+//
+// Plane description: Yuv420Planes plus y_step, the distance between Y samples of a row: 1 for the planar layout (yuv422p: c_step 1) and
+// the semi-planar one (nv16: one interleaved U, V plane, v = u + 1, c_step 2), 2 for the packed ones, whose y, u and v point into the
+// same rows of 4-byte macropixels (c_step 4): yuyv422 Y0 U0 Y1 V0 (u = y + 1, v = y + 3), uyvy422 U0 Y0 V0 Y1 (u = y - 1, v = y + 1).
+struct Yuv422Planes {
+  uint8_t* y;
+  uint8_t* u;
+  uint8_t* v;
+  int y_pitch, y_step, c_pitch, c_step;
+  long long frame_stride;
+};
+
+template <class Map>
+__device__ __forceinline__ void yuv422_to_bgr_body(const Yuv422Planes& p, int n, int h, int w, uint8_t* __restrict__ bgr, const Map& m) {
+  const int groups = (w + kYuvGroup - 1) / kYuvGroup;
+  const long long total = static_cast<long long>(n) * h * groups;
+  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
+       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
+    int f, r, x0;
+    yuv_item(idx, groups, h, f, r, x0);
+    const long long fo = f * p.frame_stride;
+    const uint8_t* y = p.y + fo + static_cast<long long>(r) * p.y_pitch + x0 * p.y_step;
+    const long long co = fo + static_cast<long long>(r) * p.c_pitch + (x0 >> 1) * p.c_step;
+    const uint8_t* u = p.u + co;
+    const uint8_t* v = p.v + co;
+    uint8_t* o = bgr + ((static_cast<long long>(f) * h + r) * w + x0) * 3;
+    if (x0 + kYuvGroup <= w) {
+      uint32_t yw[2], uw[1], vw[1];
+      if (p.y_step == 2) {                         // four macropixels, from whichever of y and u comes first
+        const bool uyvy = u < y;
+        uint32_t q[4];
+        load_bytes<16>(uyvy ? u : y, q);
+        const unsigned sy = uyvy ? 0x7531 : 0x6420, sc = uyvy ? 0x6420 : 0x7531;
+        yw[0] = __byte_perm(q[0], q[1], sy);
+        yw[1] = __byte_perm(q[2], q[3], sy);
+        const uint32_t c01 = __byte_perm(q[0], q[1], sc), c23 = __byte_perm(q[2], q[3], sc);     // U0 V0 U1 V1, U2 V2 U3 V3
+        uw[0] = __byte_perm(c01, c23, 0x6420);
+        vw[0] = __byte_perm(c01, c23, 0x7531);
+      } else {
+        load_bytes<8>(y, yw);
+        if (p.c_step == 1) {
+          load_bytes<4>(u, uw);
+          load_bytes<4>(v, vw);
+        } else {                                   // nv16: U0 V0 U1 V1 U2 V2 U3 V3
+          uint32_t uv[2];
+          load_bytes<8>(u, uv);
+          uw[0] = __byte_perm(uv[0], uv[1], 0x6420);
+          vw[0] = __byte_perm(uv[0], uv[1], 0x7531);
+        }
+      }
+      typename Map::Chroma c[kYuvGroup / 2];
+#pragma unroll
+      for (int k = 0; k < kYuvGroup / 2; ++k) c[k] = m.chroma(byte_at(uw, k), byte_at(vw, k));
+      uint32_t out[6] = {0, 0, 0, 0, 0, 0};
+#pragma unroll
+      for (int j = 0; j < kYuvGroup; ++j) {
+        int B, G, R;
+        m.pixel(c[j >> 1], byte_at(yw, j), B, G, R);
+        put_byte(out, 3 * j, B); put_byte(out, 3 * j + 1, G); put_byte(out, 3 * j + 2, R);
+      }
+      store_bytes<24>(o, out);
+    } else {
+      for (int j = 0; x0 + j < w; j += 2) {
+        const typename Map::Chroma c = m.chroma(u[(j >> 1) * p.c_step], v[(j >> 1) * p.c_step]);
+#pragma unroll
+        for (int d = 0; d < 2; ++d) {
+          int B, G, R;
+          m.pixel(c, y[(j + d) * p.y_step], B, G, R);
+          o[3 * (j + d)] = B; o[3 * (j + d) + 1] = G; o[3 * (j + d) + 2] = R;
+        }
+      }
+    }
+  }
+}
+
+template <class Map>
+__global__ void __launch_bounds__(256) yuv422_to_bgr_kernel(const Yuv422Planes p, int n, int h, int w, uint8_t* __restrict__ bgr) {
+  yuv422_to_bgr_body(p, n, h, w, bgr, Map{});
+}
+
+template <class Map>
+__device__ __forceinline__ void bgr_to_yuv422_body(const uint8_t* __restrict__ bgr, int n, int h, int w, const Yuv422Planes& p, const Map& m) {
+  const int groups = (w + kYuvGroup - 1) / kYuvGroup;
+  const long long total = static_cast<long long>(n) * h * groups;
+  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
+       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
+    int f, r, x0;
+    yuv_item(idx, groups, h, f, r, x0);
+    const long long fo = f * p.frame_stride;
+    uint8_t* y = p.y + fo + static_cast<long long>(r) * p.y_pitch + x0 * p.y_step;
+    const long long co = fo + static_cast<long long>(r) * p.c_pitch + (x0 >> 1) * p.c_step;
+    uint8_t* u = p.u + co;
+    uint8_t* v = p.v + co;
+    const uint8_t* in = bgr + ((static_cast<long long>(f) * h + r) * w + x0) * 3;
+    if (x0 + kYuvGroup <= w) {
+      uint32_t ia[6];
+      load_bytes<24>(in, ia);
+      uint32_t yw[2] = {0, 0}, uw[1] = {0}, vw[1] = {0};
+#pragma unroll
+      for (int j = 0; j < kYuvGroup; ++j) {
+        const int B = byte_at(ia, 3 * j), G = byte_at(ia, 3 * j + 1), R = byte_at(ia, 3 * j + 2);
+        put_byte(yw, j, m.y(R, G, B));
+        if ((j & 1) == 0) {                        // the left pixel of its pair
+          put_byte(uw, j >> 1, m.u(R, G, B));
+          put_byte(vw, j >> 1, m.v(R, G, B));
+        }
+      }
+      if (p.y_step == 2) {
+        const bool uyvy = u < y;
+        const uint32_t c01 = __byte_perm(uw[0], vw[0], 0x5140), c23 = __byte_perm(uw[0], vw[0], 0x7362);   // U0 V0 U1 V1, U2 V2 U3 V3
+        const unsigned s0 = uyvy ? 0x1504 : 0x5140, s1 = uyvy ? 0x3726 : 0x7362;
+        const uint32_t q[4] = {__byte_perm(yw[0], c01, s0), __byte_perm(yw[0], c01, s1), __byte_perm(yw[1], c23, s0),
+                               __byte_perm(yw[1], c23, s1)};
+        store_bytes<16>(uyvy ? u : y, q);
+      } else {
+        store_bytes<8>(y, yw);
+        if (p.c_step == 1) {
+          store_bytes<4>(u, uw);
+          store_bytes<4>(v, vw);
+        } else {
+          const uint32_t uv[2] = {__byte_perm(uw[0], vw[0], 0x5140), __byte_perm(uw[0], vw[0], 0x7362)};
+          store_bytes<8>(u, uv);
+        }
+      }
+    } else {
+      for (int j = 0; x0 + j < w; j += 2) {
+        const uint8_t* a = in + 3 * j;
+        u[(j >> 1) * p.c_step] = static_cast<uint8_t>(m.u(a[2], a[1], a[0]));
+        v[(j >> 1) * p.c_step] = static_cast<uint8_t>(m.v(a[2], a[1], a[0]));
+#pragma unroll
+        for (int d = 0; d < 2; ++d) {
+          const uint8_t* q = in + 3 * (j + d);
+          y[(j + d) * p.y_step] = static_cast<uint8_t>(m.y(q[2], q[1], q[0]));
+        }
+      }
+    }
+  }
+}
+
+template <class Map>
+__global__ void __launch_bounds__(256) bgr_to_yuv422_kernel(const uint8_t* __restrict__ bgr, int n, int h, int w, const Yuv422Planes p) {
+  bgr_to_yuv422_body(bgr, n, h, w, p, Map{});
+}
+
+// 10-bit 4:2:2 (yuv422p10le, p210): Yuv420Planes16 describes the planes, y_step is 1.  A thread's row is 16 bytes of Y, 8 of U and of V
+// (or 16 of interleaved U, V) and 48 of BGR.
+template <class Map>
+__device__ __forceinline__ void yuv422_10_to_bgr48_body(const Yuv420Planes16& p, int n, int h, int w, uint16_t* __restrict__ bgr, const Map& m) {
+  const int groups = (w + kYuvGroup - 1) / kYuvGroup;
+  const long long total = static_cast<long long>(n) * h * groups;
+  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
+       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
+    int f, r, x0;
+    yuv_item(idx, groups, h, f, r, x0);
+    const long long fo = f * p.frame_stride;
+    const uint16_t* y = p.y + fo + static_cast<long long>(r) * p.y_pitch + x0;
+    const long long co = fo + static_cast<long long>(r) * p.c_pitch + (x0 >> 1) * p.c_step;
+    const uint16_t* u = p.u + co;
+    const uint16_t* v = p.v + co;
+    uint16_t* o = bgr + ((static_cast<long long>(f) * h + r) * w + x0) * 3;
+    if (x0 + kYuvGroup <= w) {
+      uint32_t yw[4], uw[2], vw[2];
+      load_bytes<16>(as_bytes(y), yw);
+      if (p.c_step == 1) {
+        load_bytes<8>(as_bytes(u), uw);
+        load_bytes<8>(as_bytes(v), vw);
+      } else {                                     // p210: U0 V0 U1 V1 U2 V2 U3 V3, 16 bits each
+        uint32_t uv[4];
+        load_bytes<16>(as_bytes(u), uv);
+        uw[0] = __byte_perm(uv[0], uv[1], 0x5410); uw[1] = __byte_perm(uv[2], uv[3], 0x5410);
+        vw[0] = __byte_perm(uv[0], uv[1], 0x7632); vw[1] = __byte_perm(uv[2], uv[3], 0x7632);
+      }
+      typename Map::Chroma c[kYuvGroup / 2];
+#pragma unroll
+      for (int k = 0; k < kYuvGroup / 2; ++k) c[k] = m.chroma(sample10(half_at(uw, k), p.msb), sample10(half_at(vw, k), p.msb));
+      uint32_t out[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};
+#pragma unroll
+      for (int j = 0; j < kYuvGroup; ++j) {
+        int B, G, R;
+        m.pixel(c[j >> 1], sample10(half_at(yw, j), p.msb), B, G, R);
+        put_half(out, 3 * j, B); put_half(out, 3 * j + 1, G); put_half(out, 3 * j + 2, R);
+      }
+      store_bytes<48>(as_bytes(o), out);
+    } else {
+      for (int j = 0; x0 + j < w; j += 2) {
+        const typename Map::Chroma c = m.chroma(sample10(u[(j >> 1) * p.c_step], p.msb), sample10(v[(j >> 1) * p.c_step], p.msb));
+#pragma unroll
+        for (int d = 0; d < 2; ++d) {
+          int B, G, R;
+          m.pixel(c, sample10(y[j + d], p.msb), B, G, R);
+          o[3 * (j + d)] = B; o[3 * (j + d) + 1] = G; o[3 * (j + d) + 2] = R;
+        }
+      }
+    }
+  }
+}
+
+template <class Map>
+__global__ void __launch_bounds__(256) yuv422_10_to_bgr48_kernel(const Yuv420Planes16 p, int n, int h, int w, uint16_t* __restrict__ bgr) {
+  yuv422_10_to_bgr48_body(p, n, h, w, bgr, Map{});
+}
+
+template <class Map>
+__device__ __forceinline__ void bgr48_to_yuv422_10_body(const uint16_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes16& p,
+                                                        const Map& m) {
+  const int groups = (w + kYuvGroup - 1) / kYuvGroup;
+  const long long total = static_cast<long long>(n) * h * groups;
+  const int sh = p.msb ? 6 : 0;
+  for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total;
+       idx += static_cast<long long>(gridDim.x) * blockDim.x) {
+    int f, r, x0;
+    yuv_item(idx, groups, h, f, r, x0);
+    const long long fo = f * p.frame_stride;
+    uint16_t* y = p.y + fo + static_cast<long long>(r) * p.y_pitch + x0;
+    const long long co = fo + static_cast<long long>(r) * p.c_pitch + (x0 >> 1) * p.c_step;
+    uint16_t* u = p.u + co;
+    uint16_t* v = p.v + co;
+    const uint16_t* in = bgr + ((static_cast<long long>(f) * h + r) * w + x0) * 3;
+    if (x0 + kYuvGroup <= w) {
+      uint32_t ia[12];
+      load_bytes<48>(as_bytes(in), ia);
+      uint32_t yw[4] = {0, 0, 0, 0}, uw[2] = {0, 0}, vw[2] = {0, 0};
+#pragma unroll
+      for (int j = 0; j < kYuvGroup; ++j) {
+        const int B = half_at(ia, 3 * j), G = half_at(ia, 3 * j + 1), R = half_at(ia, 3 * j + 2);
+        put_half(yw, j, m.y(R, G, B) << sh);
+        if ((j & 1) == 0) {                        // the left pixel of its pair
+          put_half(uw, j >> 1, m.u(R, G, B) << sh);
+          put_half(vw, j >> 1, m.v(R, G, B) << sh);
+        }
+      }
+      store_bytes<16>(as_bytes(y), yw);
+      if (p.c_step == 1) {
+        store_bytes<8>(as_bytes(u), uw);
+        store_bytes<8>(as_bytes(v), vw);
+      } else {
+        const uint32_t uv[4] = {__byte_perm(uw[0], vw[0], 0x5410), __byte_perm(uw[0], vw[0], 0x7632),
+                                __byte_perm(uw[1], vw[1], 0x5410), __byte_perm(uw[1], vw[1], 0x7632)};
+        store_bytes<16>(as_bytes(u), uv);
+      }
+    } else {
+      for (int j = 0; x0 + j < w; j += 2) {
+        const uint16_t* a = in + 3 * j;
+        u[(j >> 1) * p.c_step] = static_cast<uint16_t>(m.u(a[2], a[1], a[0]) << sh);
+        v[(j >> 1) * p.c_step] = static_cast<uint16_t>(m.v(a[2], a[1], a[0]) << sh);
+#pragma unroll
+        for (int d = 0; d < 2; ++d) {
+          const uint16_t* q = in + 3 * (j + d);
+          y[j + d] = static_cast<uint16_t>(m.y(q[2], q[1], q[0]) << sh);
+        }
+      }
+    }
+  }
+}
+
+template <class Map>
+__global__ void __launch_bounds__(256) bgr48_to_yuv422_10_kernel(const uint16_t* __restrict__ bgr, int n, int h, int w, const Yuv420Planes16 p) {
+  bgr48_to_yuv422_10_body(bgr, n, h, w, p, Map{});
+}
+
 // The checks the conversion entry points make before any launch (pitches in bytes for 8-bit planes, in elements for 16-bit ones).
 static int check_yuv420(const char* fn, int n, int h, int w, int y_pitch, int c_pitch, int c_step, long long frame_stride,
                         bool deep = false) {
@@ -629,6 +897,47 @@ static int bgr48_to_yuv420_10(const char* fn, savsr_ctx* ctx, const uint16_t* bg
   return 0;
 }
 
+// The 4:2:2 kernels of each (colorspace, range): [BT601][TV] is the cv2-exact map, the others their H.273 maps.
+#define SAVSR_422_TABLE(kernel, M)                                                                        \
+  {{kernel<Cv2Map##M>, kernel<CsMap##M<0, 1>>}, {kernel<CsMap##M<1, 0>>, kernel<CsMap##M<1, 1>>}, \
+   {kernel<CsMap##M<2, 0>>, kernel<CsMap##M<2, 1>>}}
+using Dec422Kernel = void (*)(const Yuv422Planes, int, int, int, uint8_t*);
+using Enc422Kernel = void (*)(const uint8_t*, int, int, int, const Yuv422Planes);
+static const Dec422Kernel kDec422[3][2] = SAVSR_422_TABLE(yuv422_to_bgr_kernel, 8);
+static const Enc422Kernel kEnc422[3][2] = SAVSR_422_TABLE(bgr_to_yuv422_kernel, 8);
+static const Dec10Kernel kDec422_10[3][2] = SAVSR_422_TABLE(yuv422_10_to_bgr48_kernel, 10);
+static const Enc10Kernel kEnc422_10[3][2] = SAVSR_422_TABLE(bgr48_to_yuv422_10_kernel, 10);
+#undef SAVSR_422_TABLE
+
+// The checks of the 4:2:2 entry points before any launch; T is the sample type (pitches and strides in its elements).
+template <class T>
+static int check_yuv422(const char* fn, int n, int h, int w, const T* y, int y_pitch, int y_step, const T* u, const T* v, int c_pitch,
+                        int c_step, long long frame_stride) {
+  constexpr bool deep = sizeof(T) == 2;
+  SAVSR_REQUIRE(n >= 0 && h > 0 && w > 0, "%s: bad shape n=%d h=%d w=%d", fn, n, h, w);
+  SAVSR_REQUIRE(w % 2 == 0, "%s: YUV 4:2:2 needs an even width, got %dx%d", fn, h, w);
+  if (deep) {
+    SAVSR_REQUIRE(y_step == 1 && (c_step == 1 || c_step == 2),
+                  "%s: (y_step, c_step) must be (1, 1) (yuv422p10le) or (1, 2) (p210), got (%d, %d)", fn, y_step, c_step);
+  } else {
+    SAVSR_REQUIRE((y_step == 1 && (c_step == 1 || c_step == 2)) || (y_step == 2 && c_step == 4),
+                  "%s: (y_step, c_step) must be (1, 1) (yuv422p), (1, 2) (nv16) or (2, 4) (yuyv422, uyvy422), got (%d, %d)", fn, y_step,
+                  c_step);
+  }
+  SAVSR_REQUIRE(y_pitch >= y_step * w, "%s: y_pitch %d < row of %d %s", fn, y_pitch, y_step * w, deep ? "elements" : "bytes");
+  SAVSR_REQUIRE(c_pitch >= c_step * (w / 2), "%s: c_pitch %d < chroma row of %d %s", fn, c_pitch, c_step * (w / 2),
+                deep ? "elements" : "bytes");
+  SAVSR_REQUIRE(c_step != 2 || v == u + 1, "%s: interleaved chroma (c_step 2) needs v = u + 1", fn);
+  SAVSR_REQUIRE(y_step != 2 || (c_pitch == y_pitch && ((u == y + 1 && v == y + 3) || (u == y - 1 && v == y + 1))),
+                "%s: packed 4:2:2 needs c_pitch = y_pitch and yuyv422 (u = y + 1, v = y + 3) or uyvy422 (u = y - 1, v = y + 1)", fn);
+  SAVSR_REQUIRE(frame_stride >= 0, "%s: negative frame_stride %lld", fn, frame_stride);
+  return 0;
+}
+
+static unsigned yuv422_blocks(const savsr_ctx* ctx, int n, int h, int w) {
+  return grid_for(ctx, static_cast<long long>(n) * h * ((w + kYuvGroup - 1) / kYuvGroup));
+}
+
 }  // namespace savsr
 
 using namespace savsr;
@@ -688,6 +997,74 @@ extern "C" int savsr_bgr48_to_yuv420_10_cs(savsr_ctx* ctx, const uint16_t* bgr, 
   Enc10Kernel k;
   if (cs_kernel(fn, colorspace, range, static_cast<Enc10Kernel>(bgr48_to_yuv420_10_kernel), kEnc10Cs, &k)) return 1;
   return savsr::bgr48_to_yuv420_10(fn, ctx, bgr, n, h, w, y, y_pitch, u, v, c_pitch, c_step, frame_stride, msb, k, st);
+}
+
+extern "C" int savsr_yuv422_to_bgr_cs(savsr_ctx* ctx, const uint8_t* y, int y_pitch, int y_step, const uint8_t* u, const uint8_t* v,
+                                      int c_pitch, int c_step, int64_t frame_stride, int n, int h, int w, uint8_t* bgr, int colorspace,
+                                      int range, savsr_stream st) {
+  const char* fn = "savsr_yuv422_to_bgr_cs";
+  Dec422Kernel k;
+  if (cs_kernel(fn, colorspace, range, kDec422[0][0], kDec422, &k)) return 1;
+  SAVSR_REQUIRE(ctx && y && u && v && bgr, "%s: null pointer", fn);
+  if (check_yuv422(fn, n, h, w, y, y_pitch, y_step, u, v, c_pitch, c_step, frame_stride)) return 1;
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const Yuv422Planes p{const_cast<uint8_t*>(y), const_cast<uint8_t*>(u), const_cast<uint8_t*>(v), y_pitch, y_step, c_pitch, c_step,
+                       frame_stride};
+  k<<<yuv422_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(p, n, h, w, bgr);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int savsr_bgr_to_yuv422_cs(savsr_ctx* ctx, const uint8_t* bgr, int n, int h, int w, uint8_t* y, int y_pitch, int y_step,
+                                      uint8_t* u, uint8_t* v, int c_pitch, int c_step, int64_t frame_stride, int colorspace, int range,
+                                      savsr_stream st) {
+  const char* fn = "savsr_bgr_to_yuv422_cs";
+  Enc422Kernel k;
+  if (cs_kernel(fn, colorspace, range, kEnc422[0][0], kEnc422, &k)) return 1;
+  SAVSR_REQUIRE(ctx && bgr && y && u && v, "%s: null pointer", fn);
+  if (check_yuv422<uint8_t>(fn, n, h, w, y, y_pitch, y_step, u, v, c_pitch, c_step, frame_stride)) return 1;
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const Yuv422Planes p{y, u, v, y_pitch, y_step, c_pitch, c_step, frame_stride};
+  k<<<yuv422_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(bgr, n, h, w, p);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int savsr_yuv422_10_to_bgr48_cs(savsr_ctx* ctx, const uint16_t* y, int y_pitch, int y_step, const uint16_t* u, const uint16_t* v,
+                                           int c_pitch, int c_step, int64_t frame_stride, int msb, int n, int h, int w, uint16_t* bgr,
+                                           int colorspace, int range, savsr_stream st) {
+  const char* fn = "savsr_yuv422_10_to_bgr48_cs";
+  Dec10Kernel k;
+  if (cs_kernel(fn, colorspace, range, kDec422_10[0][0], kDec422_10, &k)) return 1;
+  SAVSR_REQUIRE(ctx && y && u && v && bgr, "%s: null pointer", fn);
+  if (check_yuv422(fn, n, h, w, y, y_pitch, y_step, u, v, c_pitch, c_step, frame_stride)) return 1;
+  SAVSR_REQUIRE(msb == 0 || msb == 1, "%s: msb must be 0 (yuv422p10le) or 1 (p210), got %d", fn, msb);
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const Yuv420Planes16 p{const_cast<uint16_t*>(y), const_cast<uint16_t*>(u), const_cast<uint16_t*>(v), y_pitch, c_pitch, c_step,
+                         frame_stride, msb};
+  k<<<yuv422_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(p, n, h, w, bgr);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
+}
+
+extern "C" int savsr_bgr48_to_yuv422_10_cs(savsr_ctx* ctx, const uint16_t* bgr, int n, int h, int w, uint16_t* y, int y_pitch, int y_step,
+                                           uint16_t* u, uint16_t* v, int c_pitch, int c_step, int64_t frame_stride, int msb,
+                                           int colorspace, int range, savsr_stream st) {
+  const char* fn = "savsr_bgr48_to_yuv422_10_cs";
+  Enc10Kernel k;
+  if (cs_kernel(fn, colorspace, range, kEnc422_10[0][0], kEnc422_10, &k)) return 1;
+  SAVSR_REQUIRE(ctx && bgr && y && u && v, "%s: null pointer", fn);
+  if (check_yuv422<uint16_t>(fn, n, h, w, y, y_pitch, y_step, u, v, c_pitch, c_step, frame_stride)) return 1;
+  SAVSR_REQUIRE(msb == 0 || msb == 1, "%s: msb must be 0 (yuv422p10le) or 1 (p210), got %d", fn, msb);
+  if (n == 0) return 0;
+  DeviceGuard guard(ctx->device);
+  const Yuv420Planes16 p{y, u, v, y_pitch, c_pitch, c_step, frame_stride, msb};
+  k<<<yuv422_blocks(ctx, n, h, w), 256, 0, static_cast<cudaStream_t>(st)>>>(bgr, n, h, w, p);
+  SAVSR_CUDA(cudaGetLastError());
+  return 0;
 }
 
 extern "C" int savsr_widen_u8_to_u16(savsr_ctx* ctx, const uint8_t* src, int n, int h, int w, uint16_t* dst, savsr_stream st) {

@@ -730,9 +730,9 @@ class Plan:
                             out_colorspace: str = "bt601", out_color_range: str = "tv") -> None:
         """io="bgr_u8_frames" or "bgr48_frames": the frames at the B*7 device addresses `ptrs` (see write_frame_table) -> out BGR
         [B,H,W,3] of the mode's sample type, all on the device's current stream.  The frames are read in place by the forward: they must
-        stay valid, in stream order, until it has run.  With a YUV out_format of the same depth ("yuv420p" or "nv12" for uint8,
-        "yuv420p10le" or "p010" for uint16), out is [B,3H/2,W] and the colour conversion reads the output staging buffer in place of the
-        copy (colour.bgr_to_yuv420, with the matrix out_colorspace and the range out_color_range).  out_format None is the mode's packed
+        stay valid, in stream order, until it has run.  With a YUV out_format of the same depth (4:2:0 or 4:2:2; uint8 or uint16), out is
+        [B, *colour.yuv_shape(H, W, out_format)] and the colour conversion reads the output staging buffer in place of the copy
+        (colour.bgr_to_yuv, with the matrix out_colorspace and the range out_color_range).  out_format None is the mode's packed
         BGR ("bgr24", "bgr48le"), which takes only the default colour pair: there is nothing to convert."""
         self._forward_table_into(lambda: self.write_frame_table(ptrs), out, graph, out_format, out_colorspace, out_color_range)
 
@@ -783,7 +783,7 @@ class Plan:
             if out_format == bgr:
                 out.copy_(self.out, non_blocking=True)
             else:
-                colour.bgr_to_yuv420(self.out, out_format, out=out, colorspace=cs[0], color_range=cs[1])
+                colour.bgr_to_yuv(self.out, out_format, out=out, colorspace=cs[0], color_range=cs[1])
 
     def activation_absmax(self) -> float:
         """Largest |value| currently held anywhere in the LR arena (every trunk activation of the last forward), read in the plan's

@@ -3,10 +3,10 @@
 ``VideoUpscaler`` takes frames as a decoder produces them and returns HR frames in order, with the same windows, reflection and
 batch partition as ``sharding.infer_clip(net.forward_bgr_u8, clip, batch=...)`` on the whole clip, so its output is byte-identical to
 that call.  Frames are uploaded once into a device ring and read in place by ``SAVSR.forward_bgr_u8_indexed``; the ring's size depends
-on the largest batch of the schedule, not on the length of the video.  Frames may come and go as packed BGR or as YUV 4:2:0
-(yuv420p, NV12: savsr_b200.colour), converted on the device on their way into the ring and out of the forward's output buffer, each
-side with its own colour matrix and range (BT.601, BT.709, BT.2020; tv or pc).  Deep video (bgr48le, yuv420p10le, P010) streams through
-a ring of uint16 frames and ``SAVSR.forward_bgr48_indexed``.  Scene cuts, marked by the caller or detected on the device
+on the largest batch of the schedule, not on the length of the video.  Frames may come and go as packed BGR, as YUV 4:2:0 (yuv420p,
+NV12) or as YUV 4:2:2 (yuv422p, NV16, YUYV, UYVY: savsr_b200.colour), converted on the device on their way into the ring and out of
+the forward's output buffer, each side with its own colour matrix and range (BT.601, BT.709, BT.2020; tv or pc).  Deep video (bgr48le,
+yuv420p10le, P010, yuv422p10le, P210) streams through a ring of uint16 frames and ``SAVSR.forward_bgr48_indexed``.  Scene cuts, marked by the caller or detected on the device
 (savsr_b200.scenes), fold each window into its own shot, so that no output frame is made of two shots.
 """
 from __future__ import annotations
@@ -45,6 +45,11 @@ class VideoUpscaler:
     decoded as above and widened by 257 on its way into the ring, so it enters the network exactly as the 8-bit path feeds it, and the
     output is enc(infer_clip(net.forward_bgr48, dec(frames), batch=...)) with dec of an 8-bit source widened.  An 8-bit source gets
     deep output this way, without 8-bit banding; deep input with 8-bit output is refused.
+
+    4:2:2 formats (savsr_b200.colour): "yuv422p", "nv16" (uint8 [2h, w]), "yuyv422", "uyvy422" (uint8 [h, 2w]), "yuv422p10le" and
+    "p210" (uint16 [2h, w]); all but yuv422p and yuv422p10le may have a row pitch.  They need an even width only: an even LR width for
+    4:2:2 input, an even HR width (any HR height) for 4:2:2 output.  Decoding gives both pixels of a horizontal pair the pair's chroma,
+    encoding takes it from the pair's left pixel; either side may be 4:2:0 or 4:2:2 independently of the other.
 
     Colour: YUV input is decoded with the matrix `in_colorspace` and the range `in_color_range`, YUV output encoded with
     `out_colorspace` and `out_color_range` (ffmpeg's -colorspace / -color_range names: "bt601", "bt709", "bt2020nc"; "tv", "pc";
@@ -96,11 +101,16 @@ class VideoUpscaler:
             if fmt not in colour.YUV_FORMATS and pair != ("bt601", "tv"):
                 raise ValueError(f"{side}_colorspace / {side}_color_range {pair} need a YUV {side}_format: {side}_format {fmt} is packed "
                                  f"BGR and is not converted")
-        if in_format in colour.YUV_FORMATS and (h % 2 or w % 2):
+        if in_format in colour.YUV420_FORMATS and (h % 2 or w % 2):
             raise ValueError(f"{in_format} input needs an even LR size, got {h}x{w}")
+        if in_format in colour.YUV422_FORMATS and w % 2:
+            raise ValueError(f"{in_format} input needs an even LR width, got {h}x{w}")
         H, W = engine.get_hw(h, w, self.scale)
-        if out_format in colour.YUV_FORMATS and (H % 2 or W % 2):
+        if out_format in colour.YUV420_FORMATS and (H % 2 or W % 2):
             raise ValueError(f"{out_format} output needs an even HR size: {h}x{w} at scale {self.scale} gives H = {H}, W = {W}; "
+                             f"{colour.bgr_format(out_format)} output takes any scale")
+        if out_format in colour.YUV422_FORMATS and W % 2:
+            raise ValueError(f"{out_format} output needs an even HR width: {h}x{w} at scale {self.scale} gives W = {W}; "
                              f"{colour.bgr_format(out_format)} output takes any scale")
         if scene_threshold is not None:
             scenes.check_threshold(scene_threshold)
@@ -128,9 +138,10 @@ class VideoUpscaler:
         self._marked: List[int] = []   # frames > 0 marked with push(..., new_scene=True)
 
     def push(self, frames, new_scene: bool = False) -> List[Tuple[int, torch.Tensor]]:
-        """Append frames in `in_format` (uint8, uint16 for the deep formats): BGR [h, w, 3] or [n, h, w, 3], YUV [3h/2, w] or
-        [n, 3h/2, w] (torch or numpy, host or CUDA).  Returns the batches that became ready, as (index of the first frame, [m, H, W, 3],
-        or [m, 3H/2, W] in a YUV out_format, of out_format's sample type) in frame order; often none.  `new_scene`: the first of these
+        """Append frames in `in_format` (uint8, uint16 for the deep formats): BGR [h, w, 3] or [n, h, w, 3], YUV one
+        colour.yuv_shape(h, w, in_format) array per frame or [n, ...] (torch or numpy, host or CUDA).  Returns the batches that became
+        ready, as (index of the first frame, [m, H, W, 3], or [m, *colour.yuv_shape(H, W, out_format)] in a YUV out_format, of
+        out_format's sample type) in frame order; often none.  `new_scene`: the first of these
         frames starts a new shot (the first frame of a video always does)."""
         if self.finished:
             raise RuntimeError("push() after finish(): call reset() to start the next video")
@@ -237,8 +248,8 @@ class VideoUpscaler:
             frame = self._yuv_dev if yuv else bgr
             frame.copy_(self._staging[s], non_blocking=True)
             ev.record(torch.cuda.current_stream(self.device))
-        if yuv:                                  # CUDA frames, pitched NV12 / P010 too, are read in place
-            colour.yuv420_to_bgr(frame, self.in_format, out=bgr, **self._colour_kw(self.in_colour, "colorspace", "color_range"))
+        if yuv:                                  # CUDA frames, pitched ones too, are read in place
+            colour.yuv_to_bgr(frame, self.in_format, out=bgr, **self._colour_kw(self.in_colour, "colorspace", "color_range"))
         elif frame is not bgr:
             if self._widen and frame.is_contiguous():
                 bgr = frame                      # a CUDA frame is widened where it is
