@@ -129,6 +129,22 @@ def frame_size(x: torch.Tensor, fmt: str) -> Tuple[int, int]:
     return (rows // 2 if fmt in YUV422_FORMATS else 2 * rows // 3), cols
 
 
+def _uneven(fmt: str, h: int, w: int) -> str:
+    """What of an h x w frame must be even for `fmt` and is not: "size" (4:2:0: height and width), "width" (4:2:2), or "" when
+    the size suits `fmt` (and for packed BGR, which takes any size)."""
+    if fmt in YUV420_FORMATS and (h % 2 or w % 2):
+        return "size"
+    if fmt in YUV422_FORMATS and w % 2:
+        return "width"
+    return ""
+
+
+def _check_even(fmt: str, h: int, w: int) -> None:
+    need = _uneven(fmt, h, w)
+    if need:
+        raise ValueError(f"{fmt} needs an even {'frame size' if need == 'size' else 'width'}, got {h}x{w}")
+
+
 def yuv_frames(x: torch.Tensor, fmt: str, h: Optional[int] = None, w: Optional[int] = None) -> torch.Tensor:
     """Check that x holds `fmt` frames (uint8, uint16 for the 10-bit formats; one [rows, cols] array per frame as yuv_shape gives it,
     [n, rows, cols] for several; h x w from the shape when not given) with a layout the kernels read, and return it as [n, rows, cols].
@@ -151,10 +167,7 @@ def yuv_frames(x: torch.Tensor, fmt: str, h: Optional[int] = None, w: Optional[i
         if bad:
             raise ValueError(f"expected {tn} {fmt} frames {form}, got {tuple(x.shape)}")
         h, w = frame_size(x, fmt)
-    if four22 and w % 2:
-        raise ValueError(f"{fmt} needs an even width, got {h}x{w}")
-    if not four22 and (h % 2 or w % 2):
-        raise ValueError(f"{fmt} needs an even frame size, got {h}x{w}")
+    _check_even(fmt, h, w)
     if x.dim() == 2:
         x = x.unsqueeze(0)
     rows, cols = yuv_shape(h, w, fmt)
@@ -171,28 +184,19 @@ def yuv_frames(x: torch.Tensor, fmt: str, h: Optional[int] = None, w: Optional[i
 
 
 def _planes(x: torch.Tensor, fmt: str, h: int, w: int) -> tuple:
-    """(y, y_pitch, u, v, c_pitch, c_step, frame_stride) of 4:2:0 frames x [n, 3h/2, w] (checked by yuv_frames): addresses in bytes,
-    pitches and the frame stride in elements (bytes for the 8-bit formats, uint16 samples for the 10-bit ones)."""
-    p, pitch, e = x.data_ptr(), x.stride(1), x.element_size()
-    if fmt not in PITCHED_FORMATS:
-        u = p + h * w * e
-        return p, w, u, u + (h // 2) * (w // 2) * e, w // 2, 1, x.stride(0)
-    u = p + h * pitch * e
-    return p, pitch, u, u + e, pitch, 2, x.stride(0)
-
-
-def _planes422(x: torch.Tensor, fmt: str, h: int, w: int) -> tuple:
-    """(y, y_pitch, y_step, u, v, c_pitch, c_step, frame_stride) of 4:2:2 frames x (checked by yuv_frames), units as _planes."""
+    """(y, y_pitch, y_step, u, v, c_pitch, c_step, frame_stride) of `fmt` frames x (checked by yuv_frames), as the kernels take them:
+    addresses in bytes, pitches and the frame stride in elements (bytes for the 8-bit formats, uint16 samples for the 10-bit ones)."""
     p, pitch, e = x.data_ptr(), x.stride(1), x.element_size()
     if fmt == "yuyv422":
         return p, pitch, 2, p + 1, p + 3, pitch, 4, x.stride(0)
     if fmt == "uyvy422":
         return p + 1, pitch, 2, p, p + 2, pitch, 4, x.stride(0)
-    if fmt in PITCHED_FORMATS:                 # nv16, p210
+    if fmt in PITCHED_FORMATS:                 # nv12, p010, nv16, p210: the U, V rows follow the h Y rows at the same pitch
         u = p + h * pitch * e
         return p, pitch, 1, u, u + e, pitch, 2, x.stride(0)
+    c_rows = h if fmt in YUV422_FORMATS else h // 2
     u = p + h * w * e
-    return p, w, 1, u, u + h * (w // 2) * e, w // 2, 1, x.stride(0)
+    return p, w, 1, u, u + c_rows * (w // 2) * e, w // 2, 1, x.stride(0)
 
 
 def _on_cuda(*xs: torch.Tensor) -> torch.device:
@@ -270,7 +274,6 @@ def _family(fmt: str, family: tuple) -> None:
 
 def _decode(frames, fmt, out, colorspace, color_range, family) -> torch.Tensor:
     pair = _cs_values(colorspace, color_range)
-    cs = () if pair == (0, 0) else pair         # the plain 4:2:0 entry points convert the default pair
     _family(fmt, family)
     x = yuv_frames(frames, fmt)
     n, (h, w) = x.shape[0], frame_size(x, fmt)
@@ -284,39 +287,19 @@ def _decode(frames, fmt, out, colorspace, color_range, family) -> torch.Tensor:
     dev = _on_cuda(x, out)
     if n == 0:
         return out
-    ctx = engine.context(dev.index)
-    st = torch.cuda.current_stream(dev).cuda_stream
-    with torch.cuda.device(dev):
-        if family is YUV422_FORMATS:            # one _cs entry point per depth; the default pair is (0, 0)
-            planes = _planes422(x, fmt, h, w)
-            if fmt in DEEP_FORMATS:
-                K.check(ctx.lib.savsr_yuv422_10_to_bgr48_cs(ctx.handle, *planes, int(fmt == "p210"), n, h, w, out.data_ptr(), *pair, st))
-            else:
-                K.check(ctx.lib.savsr_yuv422_to_bgr_cs(ctx.handle, *planes, n, h, w, out.data_ptr(), *pair, st))
-            return out
-        y, yp, u, v, cp, c_step, fs = _planes(x, fmt, h, w)
-        if fmt in DEEP_FORMATS:
-            args = (ctx.handle, y, yp, u, v, cp, c_step, fs, int(fmt == "p010"), n, h, w, out.data_ptr(), *cs, st)
-            K.check((ctx.lib.savsr_yuv420_10_to_bgr48_cs if cs else ctx.lib.savsr_yuv420_10_to_bgr48)(*args))
-        else:
-            args = (ctx.handle, y, yp, u, v, cp, c_step, fs, n, h, w, out.data_ptr(), *cs, st)
-            K.check((ctx.lib.savsr_yuv420_to_bgr_cs if cs else ctx.lib.savsr_yuv420_to_bgr)(*args))
+    _convert(dev, True, fmt, pair, _planes(x, fmt, h, w), out.data_ptr(), n, h, w)
     return out
 
 
 def _encode(bgr, fmt, out, colorspace, color_range, family) -> torch.Tensor:
     pair = _cs_values(colorspace, color_range)
-    cs = () if pair == (0, 0) else pair         # the plain 4:2:0 entry points convert the default pair
     _family(fmt, family)
     four22 = family is YUV422_FORMATS
     dt = dtype_of(fmt)
     x = _bgr(bgr, f"bgr_to_yuv{'422' if four22 else '420'} to {fmt}", dt)
     n, H, W = x.shape[:3]
     shape = (n, *yuv_shape(H, W, fmt)) if bgr.dim() == 4 else yuv_shape(H, W, fmt)
-    if four22 and W % 2:
-        raise ValueError(f"{fmt} needs an even width, got {H}x{W}")
-    if not four22 and (H % 2 or W % 2):
-        raise ValueError(f"{fmt} needs an even frame size, got {H}x{W}")
+    _check_even(fmt, H, W)
     if out is None:
         _on_cuda(x)
         out = torch.empty(shape, dtype=dt, device=x.device)
@@ -328,24 +311,35 @@ def _encode(bgr, fmt, out, colorspace, color_range, family) -> torch.Tensor:
     dev = _on_cuda(x, o)
     if n == 0:
         return out
-    ctx = engine.context(dev.index)
-    st = torch.cuda.current_stream(dev).cuda_stream
-    with torch.cuda.device(dev):
-        if four22:
-            planes = _planes422(o, fmt, H, W)
-            if fmt in DEEP_FORMATS:
-                K.check(ctx.lib.savsr_bgr48_to_yuv422_10_cs(ctx.handle, x.data_ptr(), n, H, W, *planes, int(fmt == "p210"), *pair, st))
-            else:
-                K.check(ctx.lib.savsr_bgr_to_yuv422_cs(ctx.handle, x.data_ptr(), n, H, W, *planes, *pair, st))
-            return out
-        y, yp, u, v, cp, c_step, fs = _planes(o, fmt, H, W)
-        if fmt in DEEP_FORMATS:
-            args = (ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, c_step, fs, int(fmt == "p010"), *cs, st)
-            K.check((ctx.lib.savsr_bgr48_to_yuv420_10_cs if cs else ctx.lib.savsr_bgr48_to_yuv420_10)(*args))
-        else:
-            args = (ctx.handle, x.data_ptr(), n, H, W, y, yp, u, v, cp, c_step, fs, *cs, st)
-            K.check((ctx.lib.savsr_bgr_to_yuv420_cs if cs else ctx.lib.savsr_bgr_to_yuv420)(*args))
+    _convert(dev, False, fmt, pair, _planes(o, fmt, H, W), x.data_ptr(), n, H, W)
     return out
+
+
+# The C entry point of each (decode, 4:2:2, deep).  4:2:0 has a plain form for the default colour pair and a _cs form for any pair;
+# 4:2:2 has only the _cs form.
+_C_CALLS = {
+    (True, False, False): "savsr_yuv420_to_bgr", (True, False, True): "savsr_yuv420_10_to_bgr48",
+    (True, True, False): "savsr_yuv422_to_bgr_cs", (True, True, True): "savsr_yuv422_10_to_bgr48_cs",
+    (False, False, False): "savsr_bgr_to_yuv420", (False, False, True): "savsr_bgr48_to_yuv420_10",
+    (False, True, False): "savsr_bgr_to_yuv422_cs", (False, True, True): "savsr_bgr48_to_yuv422_10_cs",
+}
+
+
+def _convert(dev: torch.device, decode: bool, fmt: str, pair: tuple, planes: tuple, bgr: int, n: int, h: int, w: int) -> None:
+    """One conversion between `fmt` frames with `planes` (as _planes gives them) and BGR at address `bgr`, on the current stream."""
+    four22, deep = fmt in YUV422_FORMATS, fmt in DEEP_FORMATS
+    name, cs = _C_CALLS[decode, four22, deep], pair
+    if not four22:
+        planes = planes[:2] + planes[3:]        # the 4:2:0 entry points take no y_step
+        if pair == (0, 0):
+            cs = ()                             # the plain form converts the default pair
+        else:
+            name += "_cs"
+    msb = (int(fmt in ("p010", "p210")),) if deep else ()
+    args = (*planes, *msb, n, h, w, bgr) if decode else (bgr, n, h, w, *planes, *msb)
+    ctx = engine.context(dev.index)
+    with torch.cuda.device(dev):
+        K.check(getattr(ctx.lib, name)(ctx.handle, *args, *cs, torch.cuda.current_stream(dev).cuda_stream))
 
 
 def widen(bgr: torch.Tensor, out: torch.Tensor) -> torch.Tensor:

@@ -101,16 +101,14 @@ class VideoUpscaler:
             if fmt not in colour.YUV_FORMATS and pair != ("bt601", "tv"):
                 raise ValueError(f"{side}_colorspace / {side}_color_range {pair} need a YUV {side}_format: {side}_format {fmt} is packed "
                                  f"BGR and is not converted")
-        if in_format in colour.YUV420_FORMATS and (h % 2 or w % 2):
-            raise ValueError(f"{in_format} input needs an even LR size, got {h}x{w}")
-        if in_format in colour.YUV422_FORMATS and w % 2:
-            raise ValueError(f"{in_format} input needs an even LR width, got {h}x{w}")
+        need = colour._uneven(in_format, h, w)
+        if need:
+            raise ValueError(f"{in_format} input needs an even LR {need}, got {h}x{w}")
         H, W = engine.get_hw(h, w, self.scale)
-        if out_format in colour.YUV420_FORMATS and (H % 2 or W % 2):
-            raise ValueError(f"{out_format} output needs an even HR size: {h}x{w} at scale {self.scale} gives H = {H}, W = {W}; "
-                             f"{colour.bgr_format(out_format)} output takes any scale")
-        if out_format in colour.YUV422_FORMATS and W % 2:
-            raise ValueError(f"{out_format} output needs an even HR width: {h}x{w} at scale {self.scale} gives W = {W}; "
+        need = colour._uneven(out_format, H, W)
+        if need:
+            gives = f"H = {H}, W = {W}" if need == "size" else f"W = {W}"
+            raise ValueError(f"{out_format} output needs an even HR {need}: {h}x{w} at scale {self.scale} gives {gives}; "
                              f"{colour.bgr_format(out_format)} output takes any scale")
         if scene_threshold is not None:
             scenes.check_threshold(scene_threshold)
